@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # our arm (N>1: launched by torchrun, one rank per GPU)
   python bench.py --impl reference --gpus N --steps K ...  # the reference's ffmpeg-mjpeg CPU path on the host cores
+  python bench.py --steps K --dump-outputs DIR             # also writes what the last timed step computed, DIR/<name>.npy
 
 A step is one pass of the hot path over one batch of `--frames` distinct frames (default 2048 x 1080p = 6.4 GB
 of input, larger than the 126 MB L2, so nothing is served from cache between steps).
@@ -62,7 +63,16 @@ def parse_args():
     ap.add_argument("--no-other-configs", action="store_true", help="skip the 4K and 1918x1078 records (BASELINE.json configs[3])")
     ap.add_argument("--parity-frames", type=int, default=16, help="frames of the last timed launch compared with the oracle")
     ap.add_argument("--sustain-seconds", type=float, default=3.0, help="length of the sustained device-resident pass (0 = skip)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed step of the device-resident "
+                                                          "pass computed as DIR/<name>.npy (rank 0's frames; see dump_outputs).  The "
+                                                          "frames are read after the timed region, except with more sub-batches than "
+                                                          "slots: then a reused slot's are read inside it, which the timing includes")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs dumps the GPU path's outputs; the reference arm has none to write")
+    return a
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -407,40 +417,59 @@ def sample_indices(n, count, seed):
     return sorted(pick)
 
 
-def device_pass(cx, enc, streams, d_frames, stride, fb, F, SB, NS, w, h, steps, warmup, profile_every, sample=0, min_seconds=0.0, chroma_format=0):
+def device_pass(cx, enc, streams, d_frames, stride, fb, F, SB, NS, w, h, steps, warmup, profile_every, sample=0, min_seconds=0.0, chroma_format=0,
+                keep_frames=()):
     """The device-resident pass: `steps` steps of F frames in sub-batches of SB on NS slots, CUDA-event timed.  After
     the timed region `sample` frames of the LAST timed launch are fetched from the device and compared with the oracle.
-    min_seconds > 0: keep stepping until the timed region has lasted that long (sustained figure)."""
+    min_seconds > 0: keep stepping until the timed region has lasted that long (sustained figure).
+    keep_frames: frames (indices within a step) whose JPEG bytes the last timed step keeps; out["last_step"] then holds
+    them and the sizes and status of every frame of that step.  They are read after the timed region, except from a slot
+    that the step reuses (more sub-batches than slots): that slot's are read before its next submit, inside the region."""
     torch = cx.torch
     nsub = F // SB
     main = torch.cuda.current_stream(cx.dev)
     kernel_ms, kernel_calls = {}, {}
     sizes_total = [0]
     last = {}
+    kept = {"sizes": np.zeros(F, np.int64), "status": np.zeros(F, np.int64), "jpeg": {}, "launches": []}
 
     def harvest(slot):
         for name, ms in enc.kernel_ms(slot):
             kernel_ms[name] = kernel_ms.get(name, 0.0) + ms
             kernel_calls[name] = kernel_calls.get(name, 0) + 1
 
-    def collect(slot, first_frame, record):
+    def collect(slot, first_frame, record, keep):
         d_out, cap, sizes, st = enc.collect_device(slot)
         if record:
             harvest(slot)
             sizes_total[0] += int(sizes.sum())
             last.update(slot=slot, first_frame=first_frame, d_out=d_out, cap=cap, sizes=sizes, status=st)
+        if keep:
+            kept["sizes"][first_frame: first_frame + len(sizes)] = sizes
+            kept["status"][first_frame: first_frame + len(st)] = st
+            kept["launches"].append((first_frame, d_out, cap, sizes))
 
-    def step(record=False):
+    def read_kept():
+        for first_frame, d_out, cap, sizes in kept["launches"]:
+            for i in keep_frames:
+                j = i - first_frame
+                if 0 <= j < len(sizes):
+                    kept["jpeg"][i] = np.frombuffer(enc.read_device(d_out + j * cap, int(sizes[j])), np.uint8)
+        kept["launches"].clear()
+
+    def step(record=False, keep=False):
         inflight = []
         for i in range(nsub):
             slot = i % NS
             if len(inflight) == NS:
                 s0, f0 = inflight.pop(0)
-                collect(s0, f0, record)
+                collect(s0, f0, record, keep)
+                if keep:
+                    read_kept()
             enc.submit_device(slot, d_frames.data_ptr() + i * SB * stride, stride, SB, w, h)
             inflight.append((slot, i * SB))
         for s0, f0 in inflight:
-            collect(s0, f0, record)
+            collect(s0, f0, record, keep)
 
     for _ in range(warmup):
         step()
@@ -458,7 +487,7 @@ def device_pass(cx, enc, streams, d_frames, stride, fb, F, SB, NS, w, h, steps, 
         # per-kernel event brackets on a sample of the timed steps: a bracket leaves the GPU idle for a few microseconds at
         # every kernel boundary (eight per step), which is instrumentation, not the encoder
         enc.set_profile(profile_every > 0 and done % max(1, profile_every) == 0)
-        step(record=True)
+        step(record=True, keep=bool(keep_frames) and done == steps - 1 and min_seconds <= 0)
         done += 1
     for st in streams:
         main.wait_stream(st)
@@ -472,6 +501,9 @@ def device_pass(cx, enc, streams, d_frames, stride, fb, F, SB, NS, w, h, steps, 
            "launches": enc.kernel_launches - launches0, "kernel_ms": kernel_ms, "kernel_calls": kernel_calls,
            "avg_jpeg": sizes_total[0] / max(1, F * done), "parity": None}
     out["value"] = cx.world * F * done / (out["dev_ms_max"] / 1000.0)
+    if keep_frames:
+        read_kept()
+        out["last_step"] = {"sizes": kept["sizes"], "status": kept["status"], "jpeg": kept["jpeg"]}
     if sample > 0 and last:
         # frames of the launch that was just timed (the slot's output stays valid until the next submit)
         try:
@@ -600,6 +632,35 @@ def algorithmic_bytes(w, h, fb, nblk, avg_jpeg, avg_image_bytes=None):
         "stuff_kernel": 2 * avg_jpeg,
         "huffman_kernel": nblk * 2,
     }
+
+
+DUMP_BYTES = 64_000_000  # --dump-outputs writes at most this much
+
+
+def dump_sample(F):
+    """Frames of a step whose JPEG bytes --dump-outputs keeps: the first, the last and seeded random ones, 16 in all."""
+    return sample_indices(F, 16, seed=F)
+
+
+def dump_outputs(path, last):
+    """What the last timed step handed its caller, as path/<name>.npy:
+      jpeg_sizes         float64 [F]  bytes of every frame's JPEG
+      status             float64 [F]  every frame's status (0 = ok)
+      sample_frames      float64 [S]  the kept frames (dump_sample), in order, as many as fit DUMP_BYTES in all
+      sample_jpeg_bytes  float32      the JPEG bytes of those frames, concatenated in frame order"""
+    os.makedirs(path, exist_ok=True)
+    room = (DUMP_BYTES - 16 * len(last["sizes"]) - 4 * 4096) // 4  # float32 bytes left after the per-frame arrays and npy headers
+    frames = []
+    for i in sorted(last["jpeg"]):
+        room -= len(last["jpeg"][i]) + 2  # + 2: the frame's entry in sample_frames
+        if room < 0:
+            break
+        frames.append(i)
+    arrays = {"jpeg_sizes": last["sizes"].astype(np.float64), "status": last["status"].astype(np.float64),
+              "sample_frames": np.array(frames, np.float64),
+              "sample_jpeg_bytes": np.concatenate([np.zeros(0, np.uint8)] + [last["jpeg"][i] for i in frames]).astype(np.float32)}
+    for name, arr in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), arr)
 
 
 def hbm_peak():
@@ -886,7 +947,11 @@ def run_ours(a):
         enc.set_stream(s_i, st.cuda_stream)
 
     # ---- value: device-resident, with a parity sample out of the timed launches ----------------------
-    dp = device_pass(cx, enc, streams, d_frames, stride, fb, F, SB, NS, w, h, a.steps, a.warmup, a.profile_every, sample=a.parity_frames)
+    keep = dump_sample(F) if a.dump_outputs and rank == 0 else ()
+    dp = device_pass(cx, enc, streams, d_frames, stride, fb, F, SB, NS, w, h, a.steps, a.warmup, a.profile_every, sample=a.parity_frames,
+                     keep_frames=keep)
+    if keep:
+        dump_outputs(a.dump_outputs, dp["last_step"])
     value, dev_ms_max, clocks = dp["value"], dp["dev_ms_max"], dp["clocks"]
     if world > 1:  # every rank's own time and clock, so that a slow GPU (power cap, clocks) shows in the line
         flags = cx.gather(1.0 if clocks.get("reasons") and clocks["reasons"] != ["no samples"] else 0.0)

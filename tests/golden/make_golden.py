@@ -15,6 +15,14 @@
   golden_frames_fmt.json   the same encoder at 4:2:2 and 4:4:4 (DESIGN.md row f3): sha256 / size of what the libavcodec the
                        reference vendors makes of integer-generated yuvj422p / yuvj444p frames, opened the way the reference
                        opens it (oracle/ref_harness.cpp ref_mjpeg_encode_fmt).  `python make_golden.py formats` writes only this.
+  reference_cases.json digests of what the reference makes of the inputs of tests/test_oracle_vs_reference.py (4:2:0 frames,
+                       pts / pix_fmt variants, FDCT blocks, libswscale range conversion, 4:2:2 / 4:4:4 frames), so
+                       that those tests compare with the reference where it is absent.  `python make_golden.py cases`
+                       writes only this.  `python make_golden.py cases-from-oracle` writes it from the oracle instead and
+                       says so in "made_with": valid only at a commit whose tests/test_oracle_vs_reference.py passed live
+                       against the reference with the same oracle and the same inputs (that run pinned oracle == reference
+                       on every encode, FDCT and range case; for the pts / pix_fmt and 4:2:0-entry frames it pinned that the
+                       reference's outputs agree with each other, and the digests are the oracle's output of those frames).
 """
 import hashlib
 import json
@@ -193,9 +201,69 @@ def main():
     print("done")
 
 
+def main_cases(from_oracle=False):
+    from tests import test_oracle_vs_reference as T
+
+    L = orc.oracle()
+    if from_oracle:
+        made_with = ("the CPU oracle (oracle/mjpeg_oracle.c) at a commit whose tests/test_oracle_vs_reference.py passed live against "
+                     "the compiled reference (Lavc58.117.101) on these inputs")
+        enc = lambda y, u, v, pts=orc.NOPTS, pix_fmt=0: orc.oracle_encode(y, u, v, pts=pts)[0]  # noqa: E731 (the oracle has no pix_fmt)
+        enc_fmt = lambda y, u, v, fmt: orc.oracle_encode(y, u, v, chroma_format=fmt)[0]  # noqa: E731
+
+        def fdct(b):
+            for i in range(len(b)):
+                L.orc_fdct_sse2(b[i].ctypes.data)
+
+        def rng_conv(w, h, y, u, v, flags):
+            return T.oracle_range(orc, w, h, y, u, v)
+    else:
+        R = orc.reference()
+        made_with = "the compiled reference, " + R.ref_version().decode()
+        enc, enc_fmt = orc.reference_encode, orc.reference_encode_fmt
+
+        def fdct(b):
+            assert R.ref_fdct(b.ctypes.data, len(b)) == 1
+
+        def rng_conv(w, h, y, u, v, flags):
+            oy = np.zeros_like(y); ou = np.zeros_like(u); ov = np.zeros_like(v)
+            assert R.ref_sws_limited_to_full(y.ctypes.data, u.ctypes.data, v.ctypes.data, w, h, flags, oy.ctypes.data, ou.ctypes.data, ov.ctypes.data) == 1
+            return oy, ou, ov
+
+    out = {"generator": "tests/golden/make_golden.py " + ("cases-from-oracle" if from_oracle else "cases"), "made_with": made_with,
+           "encode_420": {}, "encode_fmt": {}, "range": {}}
+    for (w, h, kind, amp) in T.CASES:
+        y, u, v = orc.synth_planes(w, h, kind, seed=w * 7 + h, amp=amp)
+        j = enc(y, u, v)
+        out["encode_420"][f"{w}x{h}_{kind}_{amp}"] = {"planes_sha256": T.sha(y, u, v), "size": len(j), "sha256": T.sha(j)}
+    w, h, kind, seed, amp = T.PTS_FRAME
+    y, u, v = orc.synth_planes(w, h, kind, seed=seed, amp=amp)
+    variants = {"base": T.sha(enc(y, u, v)), "pix_fmt=12": T.sha(enc(y, u, v, pix_fmt=12))}
+    variants.update({f"pts={p}": T.sha(enc(y, u, v, pts=p)) for p in T.PTS})
+    out["pts_pix_fmt"] = {"planes_sha256": T.sha(y, u, v), "sha256": variants}
+    blocks = T.fdct_blocks()
+    coefs = blocks.copy()
+    fdct(coefs)
+    out["fdct"] = {"blocks_sha256": T.sha(blocks), "fdct_sha256": T.sha(coefs)}
+    for (w, h, y, u, v) in T.range_planes():
+        out["range"][f"{w}x{h}"] = {"planes_sha256": T.sha(y, u, v)}
+        out["range"][f"{w}x{h}"].update({f"flags={f}": T.sha(*rng_conv(w, h, y, u, v, f)) for f in T.RANGE_FLAGS})
+    for fmt in (orc.CHROMA_422, orc.CHROMA_444):
+        for i, (w, h, kind, amp) in enumerate(T.FMT_CASES):
+            y, u, v = orc.synth_planes_fmt(w, h, fmt, kind, seed=50 + i, amp=amp)
+            j = enc_fmt(y, u, v, fmt)
+            out["encode_fmt"][f"{fmt}_{w}x{h}_{kind}_{amp}"] = {"planes_sha256": T.sha(y, u, v), "size": len(j), "sha256": T.sha(j)}
+    w, h, kind, seed = T.FMT0_FRAME
+    y, u, v = orc.synth_planes(w, h, kind, seed=seed)
+    out["fmt0_entry"] = {"planes_sha256": T.sha(y, u, v), "sha256_fmt_entry": T.sha(enc_fmt(y, u, v, 0)), "sha256_default_entry": T.sha(enc(y, u, v))}
+    json.dump(out, open(os.path.join(HERE, "reference_cases.json"), "w"), indent=1)
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "formats":
         main_formats()
+    elif len(sys.argv) > 1 and sys.argv[1] in ("cases", "cases-from-oracle"):
+        main_cases(from_oracle=sys.argv[1] == "cases-from-oracle")
     else:
         main()
         main_formats()

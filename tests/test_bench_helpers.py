@@ -66,6 +66,33 @@ def test_sample_indices_hold_first_last_and_stay_in_range():
         assert all(0 <= i < n for i in pick)
 
 
+def test_dump_outputs_stay_within_budget_as_float_arrays(tmp_path):
+    """The dump's frame sample is fixed by the arguments; the frames written are the sample's first ones that fit DUMP_BYTES,
+    all of them when the JPEGs are small, none when not even one fits."""
+    import numpy as np
+
+    import bench
+
+    F = 2048
+    pick = bench.dump_sample(F)
+    assert pick == bench.dump_sample(F) and pick[0] == 0 and pick[-1] == F - 1 and len(pick) == 16
+    rng = np.random.default_rng(3)
+    for size, n_written in ((300_000, 16), (2 * 1024 * 1024, 7), (17_000_000, 0)):
+        last = {"sizes": np.full(F, size, np.int64), "status": np.zeros(F, np.int64),
+                "jpeg": {i: rng.integers(0, 256, size, dtype=np.uint8) for i in pick}}
+        out = tmp_path / str(size)
+        bench.dump_outputs(str(out), last)
+        files = sorted(os.listdir(out))
+        assert files == ["jpeg_sizes.npy", "sample_frames.npy", "sample_jpeg_bytes.npy", "status.npy"]
+        assert sum(os.path.getsize(out / f) for f in files) <= bench.DUMP_BYTES
+        got = {f[:-4]: np.load(out / f) for f in files}
+        assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+        assert got["sample_frames"].tolist() == pick[:n_written]
+        assert (got["jpeg_sizes"] == size).all() and (got["status"] == 0).all()
+        want = np.concatenate([np.zeros(0, np.uint8)] + [last["jpeg"][i] for i in pick[:n_written]])
+        assert got["sample_jpeg_bytes"].shape == want.shape and (got["sample_jpeg_bytes"].astype(np.uint8) == want).all()
+
+
 def test_device_plans(monkeypatch, tmp_path):
     import bench
 
