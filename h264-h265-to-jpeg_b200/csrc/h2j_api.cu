@@ -75,7 +75,8 @@ struct h2j_encoder {
     std::string comment;
     std::string err;
     int sm_count = 0;
-    size_t out_cap = 0;           // per-frame JPEG capacity (multiple of 16)
+    size_t out_cap = 0;           // per-frame output stride: jpeg_cap rounded up to 16 bytes
+    size_t jpeg_cap = 0;          // max_jpeg_bytes exactly: the largest JPEG a frame may have
     long long scan_cap_words = 0;
     long long images_cap = 0;     // K2 tile images per frame at max geometry, rounded up to whole K4 tiles
     long long blocks_cap = 0;     // images_cap * 96
@@ -332,7 +333,7 @@ int launch_pipeline(h2j_encoder *e, Slot &sl, const uint8_t *d_frames, int n, in
     }
     {
         ScopedTiming t(e, sl, "huffman_kernel");
-        huffman_kernel<<<4 * n, kHuffGroup, 0, st>>>(L, sl.d_tabs, sl.d_state, n, sl.d_out, (long long)e->out_cap,
+        huffman_kernel<<<4 * n, kHuffGroup, 0, st>>>(L, sl.d_tabs, sl.d_state, n, sl.d_out, (long long)e->out_cap, (long long)e->jpeg_cap,
                                                                        e->d_comment, (int)e->comment.size());
         e->launches++;
     }
@@ -369,7 +370,7 @@ int launch_pipeline(h2j_encoder *e, Slot &sl, const uint8_t *d_frames, int n, in
         ScopedTiming t(e, sl, "stuff_kernel");
         static const int stuff_ctas_env = getenv("H2J_STUFF_CTAS") ? atoi(getenv("H2J_STUFF_CTAS")) : 0;  // tuning knob
         stuff_kernel<<<dim3(stuff_ctas_env > 0 ? stuff_ctas_env : e->stuff_ctas, n), kStuffThreads, 0, st>>>(sl.d_tabs, sl.d_state, sl.d_scan, e->scan_cap_words, sl.d_chunk_ff,
-                                                                      e->chunks_cap, sl.d_out, (long long)e->out_cap);
+                                                                      e->chunks_cap, sl.d_out, (long long)e->out_cap, (long long)e->jpeg_cap);
         e->launches++;
     }
     CU(e, cudaGetLastError());
@@ -400,7 +401,7 @@ int enqueue_pack_and_sizes(h2j_encoder *e, Slot &sl, bool pack)
     cudaStream_t st = sl.stream;
     {
         ScopedTiming t(e, sl, "pack_offsets_kernel");
-        pack_offsets_kernel<<<1, kPackOffsetsThreads, 0, st>>>(sl.d_tabs, sl.n, (long long)e->out_cap, sl.d_offsets, sl.d_status);
+        pack_offsets_kernel<<<1, kPackOffsetsThreads, 0, st>>>(sl.d_tabs, sl.n, (long long)e->jpeg_cap, sl.d_offsets, sl.d_status);
         e->launches++;
     }
     sl.packed = pack;
@@ -588,7 +589,8 @@ int h2j_create(const h2j_settings *s, h2j_encoder **out)
     CUB(cudaGetDeviceProperties(&prop, s->device));
     e->sm_count = prop.multiProcessorCount;
 
-    e->out_cap = align_up(s->max_jpeg_bytes ? s->max_jpeg_bytes : (size_t)2 * 1024 * 1024, 16);
+    e->jpeg_cap = s->max_jpeg_bytes ? s->max_jpeg_bytes : (size_t)2 * 1024 * 1024;
+    e->out_cap = align_up(e->jpeg_cap, 16);
     e->scan_cap_words = (long long)(e->out_cap / 4);
     const int fmt = s->chroma_format;
     const int mcu_w = (s->max_width + fmt_mcu_px_w(fmt) - 1) / fmt_mcu_px_w(fmt), mcu_h = (s->max_height + 15) >> 4;
@@ -945,7 +947,7 @@ int h2j_encode_frame(h2j_encoder *e, const uint8_t *const planes[3], const int s
     memcpy(&st, sl.h_tail + (offsetof(FrameTab, status) - kTabTailOff), sizeof st);
     memcpy(&jpeg_bytes, sl.h_tail + (offsetof(FrameTab, jpeg_bytes) - kTabTailOff), sizeof jpeg_bytes);
     if (st != 0) return fail(e, st, "the frame failed: %s", h2j_status_string(st));
-    if (jpeg_bytes < 0 || (size_t)jpeg_bytes > e->out_cap) return fail(e, H2J_ERR_OUTPUT_TOO_SMALL, "JPEG of %lld bytes exceeds max_jpeg_bytes", jpeg_bytes);
+    if (jpeg_bytes < 0 || (size_t)jpeg_bytes > e->jpeg_cap) return fail(e, H2J_ERR_OUTPUT_TOO_SMALL, "JPEG of %lld bytes exceeds max_jpeg_bytes", jpeg_bytes);
     const size_t n_out = (size_t)jpeg_bytes;
     *out_size = n_out;
     if (n_out > out_capacity) return fail(e, H2J_ERR_OUTPUT_TOO_SMALL, "JPEG is %zu bytes, caller gave %zu", n_out, out_capacity);

@@ -394,8 +394,10 @@ __device__ uint8_t header_byte(int i, const HeaderPlan &h, const FrameTab *T, co
 // grid 4 * frames CTAs of one group each: one table per CTA.  blockIdx.x / frames picks the table, AC tables first (they
 // take ~10x longer than the DC ones and decide the kernel's duration: with one CTA per FRAME the four scratch areas
 // allowed two CTAs per SM, and 512 frames needed two waves of them).  The frame's CTA that finishes last writes the header.
+// Frame f's output starts at out + f * out_cap; jpeg_cap (<= out_cap) is the largest JPEG allowed, and no byte at or past
+// it is written.
 __global__ void __launch_bounds__(kHuffGroup) huffman_kernel(FrameLayout L, FrameTab *__restrict__ tabs, FrameState *__restrict__ state,
-                                                             int n_frames, uint8_t *__restrict__ out, long long out_cap,
+                                                             int n_frames, uint8_t *__restrict__ out, long long out_cap, long long jpeg_cap,
                                                              const char *__restrict__ comment, int comment_len)
 {
     __shared__ HuffScratch scratch;
@@ -423,10 +425,10 @@ __global__ void __launch_bounds__(kHuffGroup) huffman_kernel(FrameLayout L, Fram
     const HeaderPlan h = header_plan(nvals, comment_len);
     uint8_t *o = out + (long long)f * out_cap;
     for (int i = tid; i < h.total; i += kHuffGroup)
-        if (i < out_cap) o[i] = header_byte(i, h, T, L, comment, comment_len);
+        if (i < jpeg_cap) o[i] = header_byte(i, h, T, L, comment, comment_len);
     if (tid == 0) {
         T->header_bytes = h.total;
-        if (h.total > out_cap) T->status = -4;
+        if (h.total > jpeg_cap) T->status = -4;
     }
 }
 

@@ -9,7 +9,7 @@ namespace h2j {
 // offsets[n+1] is computed by block 0 of pack_offsets_kernel.
 // ------------------------------------------------------------------------------------------------
 constexpr int kPackOffsetsThreads = 256;
-__global__ void __launch_bounds__(kPackOffsetsThreads) pack_offsets_kernel(const FrameTab *__restrict__ tabs, int n, long long out_cap,
+__global__ void __launch_bounds__(kPackOffsetsThreads) pack_offsets_kernel(const FrameTab *__restrict__ tabs, int n, long long jpeg_cap,
                                                                            unsigned long long *__restrict__ offsets, int *__restrict__ status)
 {
     // one CTA: exclusive scan of the JPEG sizes, a chunk of kPackOffsetsThreads frames at a time
@@ -25,7 +25,7 @@ __global__ void __launch_bounds__(kPackOffsetsThreads) pack_offsets_kernel(const
             const int st = tabs[i].status;
             status[i] = st;
             const long long b = tabs[i].jpeg_bytes;
-            sz = (st != 0 || b > out_cap) ? 0ull : (unsigned long long)b;
+            sz = (st != 0 || b > jpeg_cap) ? 0ull : (unsigned long long)b;
         }
         unsigned long long incl = sz;
 #pragma unroll

@@ -8,7 +8,8 @@
 //     bytes, ORed into the pre-zeroed image at its byte offset (two or three shared-memory atomics, no byte loop);
 //   * the image starts at the byte offset the chunk's output has inside its 16-byte line in global memory, so image
 //     quads and output quads coincide: one LDS.128 + one STG.128 per 16 bytes, bytewise only for the two ragged ends.
-// The CTA that owns the last chunk appends EOI and publishes the frame's size.
+// The CTA that owns the last chunk appends EOI and publishes the frame's size.  Frame f's output starts at out + f * out_cap;
+// jpeg_cap (<= out_cap) is the largest JPEG allowed, and no byte at or past it is written.
 // (The first form of this kernel expanded byte by byte whenever ANY lane of the warp had a 0xFF -- 86 % of the warps --
 // and realigned the image with funnel shifts on the way out: 39 thread instructions per byte; this one needs about 8.)
 #pragma once
@@ -36,7 +37,7 @@ __device__ __forceinline__ void stuff_put(unsigned int *img, unsigned q, unsigne
 __global__ void __launch_bounds__(kStuffThreads, 8) stuff_kernel(FrameTab *__restrict__ tabs, const FrameState *__restrict__ state,
                                                               const uint32_t *__restrict__ scan, long long scan_cap_words,
                                                               const unsigned int *__restrict__ chunk_ff, int chunks_cap,
-                                                              uint8_t *__restrict__ out, long long out_cap)
+                                                              uint8_t *__restrict__ out, long long out_cap, long long jpeg_cap)
 {
     __shared__ __align__(16) unsigned int s_img[kStuffImageWords];
     __shared__ unsigned s_warp[kStuffThreads / 32];
@@ -51,7 +52,7 @@ __global__ void __launch_bounds__(kStuffThreads, 8) stuff_kernel(FrameTab *__res
     // a frame that outgrew its capacity (reported by K4b, status -4) is cut at the capacity: nothing behind it exists
     const int nchunks = min((int)((nwords + kChunkWords - 1) >> kChunkShift), chunks_cap);
     const unsigned hdr = (unsigned)T->header_bytes;
-    const unsigned cap = (unsigned)min(out_cap, (long long)0xffffffffu);
+    const unsigned cap = (unsigned)min(jpeg_cap, (long long)0xffffffffu);
     const unsigned scan_cap = (unsigned)min(scan_cap_words, (long long)0xffffffffu);
     const uint32_t *gs = scan + (long long)f * scan_cap_words;
     const unsigned int *cff = chunk_ff + (long long)f * chunks_cap;
@@ -145,7 +146,7 @@ __global__ void __launch_bounds__(kStuffThreads, 8) stuff_kernel(FrameTab *__res
         if (c == nchunks - 1 && tid == 0) {
             const long long ff = (long long)before + chunk_total;
             const long long end = (long long)hdr + nbytes + ff;
-            if (end + 2 <= out_cap) { o[end] = 0xff; o[end + 1] = 0xd9; }
+            if (end + 2 <= jpeg_cap) { o[end] = 0xff; o[end + 1] = 0xd9; }
             else T->status = -4;
             T->scan_bits = bits;
             T->stuffed_ff = ff;

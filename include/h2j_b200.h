@@ -75,7 +75,8 @@ typedef struct h2j_settings {
     int range_mode;        /* h2j_range_mode */
     int fixed_qscale;      /* 0: the reference's first-frame rate control decides (default);
                               1..31: force it (AV_CODEC_FLAG_QSCALE equivalent; not used by the reference) */
-    size_t max_jpeg_bytes; /* per-frame output capacity; 0 = 2 MiB, the reference's HEAP_SIZE; at most 256 MiB */
+    size_t max_jpeg_bytes; /* largest JPEG a frame may have, exactly (a larger one fails with H2J_ERR_OUTPUT_TOO_SMALL);
+                              0 = 2 MiB, the reference's HEAP_SIZE; at most 256 MiB */
     const char *comment;   /* COM segment payload; NULL = "Lavc58.117.101", the LIBAVCODEC_IDENT of the
                               ffmpeg build the reference links on x86-64 (lib/ffmpeg/x86_64_shared) */
     int profile;           /* non-zero: bracket every kernel with CUDA events (see h2j_slot_kernel_ms) */
@@ -120,7 +121,8 @@ int h2j_encode_frame(h2j_encoder *e, const uint8_t *const planes[3], const int s
  *                    call returns the failed frames' status.  If `out` itself is too short for the batch the call returns
  *                    H2J_ERR_BUFFER_TOO_SMALL with offsets[] filled in and the slot still collectable.
  * h2j_collect_device:waits for the slot and only reports where the JPEGs are on the device: frame i is
- *                    at (*d_out) + i * (*d_frame_capacity), sizes[i] bytes long (sizes is a host array).
+ *                    at (*d_out) + i * (*d_frame_capacity), sizes[i] bytes long (sizes is a host array);
+ *                    *d_frame_capacity is max_jpeg_bytes rounded up to a multiple of 16.
  *                    The memory stays valid until the slot is submitted to again.
  * status[i] (optional, may be NULL) receives a per-frame h2j_status.
  *

@@ -43,7 +43,7 @@ int main(int argc, char **argv)
     for (int rep = 0; rep < 5; rep++) {
         cudaMemcpy(st, &h, sizeof h, cudaMemcpyHostToDevice);
         cudaEventRecord(e0);
-        huffman_kernel<<<4, kHuffGroup>>>(L, tab, st, 1, out, 1 << 20, comment, 14);
+        huffman_kernel<<<4, kHuffGroup>>>(L, tab, st, 1, out, 1 << 20, 1 << 20, comment, 14);
         cudaEventRecord(e1);
         cudaDeviceSynchronize();
         float ms;
