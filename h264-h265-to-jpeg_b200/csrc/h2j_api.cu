@@ -88,6 +88,7 @@ struct h2j_encoder {
     int stuff_ctas = 32;          // K5 CTAs per frame
     int fdct_tiles_per_cta = 16;  // upper bound of consecutive K2 tiles one CTA walks
     int force_fdct_tiles = 0;     // h2j_debug_set_knob("fdct_tiles_per_cta"): exactly this many, whatever the batch size
+    int force_sp_prepass = 0;     // h2j_debug_set_knob("semiplanar_prepass"): split semi-planar frames first even when aligned
     size_t frame_bytes_cap = 0;
     uint8_t *d_qscale_lut = nullptr;
     char *d_comment = nullptr;
@@ -171,6 +172,17 @@ int chroma_w(int w, int fmt) { return (w + (1 << fmt_hshift(fmt)) - 1) >> fmt_hs
 int chroma_h(int h, int fmt) { return (h + (1 << fmt_vshift(fmt)) - 1) >> fmt_vshift(fmt); }
 size_t tight_frame_bytes(int w, int h, int fmt) { return (size_t)w * h + 2 * (size_t)chroma_w(w, fmt) * chroma_h(h, fmt); }
 
+// the vector-load flags of a planar layout whose frames start at `base`
+void set_alignment(FrameLayout *L, const uint8_t *base)
+{
+    auto al = [&](int a) {
+        return ((uintptr_t)base % a) == 0 && (L->frame_stride % a) == 0 && (L->u_off % a) == 0 && (L->v_off % a) == 0 &&
+               (L->y_pitch % a) == 0 && (L->c_pitch % a) == 0;
+    };
+    L->aligned8 = al(8) ? 1 : 0;
+    L->aligned16 = ((uintptr_t)base % 16) == 0 && (L->frame_stride % 16) == 0 && (L->y_pitch % 16) == 0 ? 1 : 0;
+}
+
 int make_layout(h2j_encoder *e, const uint8_t *base, size_t frame_stride, int w, int h, FrameLayout *L)
 {
     if (w < 2 || h < 2 || w > 65500 || h > 65500) return fail(e, H2J_ERR_UNSUPPORTED, "unsupported frame size %dx%d", w, h);
@@ -190,12 +202,7 @@ int make_layout(h2j_encoder *e, const uint8_t *base, size_t frame_stride, int w,
     L->mcu_w = (w + fmt_mcu_px_w(fmt) - 1) / fmt_mcu_px_w(fmt); L->mcu_h = (h + 15) >> 4;
     L->n_mcu = L->mcu_w * L->mcu_h;
     L->n_blocks = L->n_mcu * fmt_mcu_blocks(fmt);
-    auto al = [&](int a) {
-        return ((uintptr_t)base % a) == 0 && (frame_stride % a) == 0 && (L->u_off % a) == 0 && (L->v_off % a) == 0 &&
-               (L->y_pitch % a) == 0 && (L->c_pitch % a) == 0;
-    };
-    L->aligned8 = al(8) ? 1 : 0;
-    L->aligned16 = ((uintptr_t)base % 16) == 0 && (frame_stride % 16) == 0 && (L->y_pitch % 16) == 0 ? 1 : 0;
+    set_alignment(L, base);
     L->range_mode = e->s.range_mode;
     L->fixed_qscale = e->s.fixed_qscale;
     L->nv12 = 0;
@@ -226,10 +233,10 @@ FrameLayout pitched_layout(const FrameLayout &T)
     return P;
 }
 
-int prepare_input(h2j_encoder *e, Slot &sl, const uint8_t *d_src, size_t src_stride, int n, int w, int h, const uint8_t **pipe_src)
+// sl.L describes the n frames at d_src (any planar layout); src_end is the end of the last one's last plane
+int repitch_if_unaligned(h2j_encoder *e, Slot &sl, const uint8_t *d_src, const uint8_t *src_end, int n, const uint8_t **pipe_src)
 {
-    int rc = make_layout(e, d_src, src_stride, w, h, &sl.L);
-    if (rc) return rc;
+    const int w = sl.L.w, h = sl.L.h;
     *pipe_src = d_src;
     static const bool no_repitch = getenv("H2J_NO_REPITCH") != nullptr;  // measurement knob
     if (sl.L.aligned8 || no_repitch) return H2J_OK;
@@ -244,13 +251,20 @@ int prepare_input(h2j_encoder *e, Slot &sl, const uint8_t *d_src, size_t src_str
     const FrameLayout T = sl.L;
     const FrameLayout P = pitched_layout(T);
     const int fch = chroma_h(h, T.fmt);
-    const uint8_t *src_end = d_src + (size_t)(n - 1) * src_stride + tight_frame_bytes(w, h, T.fmt);
     repitch_kernel<<<dim3((w + 128 * 16 - 1) / (128 * 16), (h + 2 * fch + kPlaneRowsPerCta - 1) / kPlaneRowsPerCta, n), 128, 0, sl.stream>>>(d_src, T, fch, sl.d_pitched, P, d_src, src_end);
     e->launches++;
     CU(e, cudaGetLastError());
     sl.L = P;
     *pipe_src = sl.d_pitched;
     return H2J_OK;
+}
+
+int prepare_input(h2j_encoder *e, Slot &sl, const uint8_t *d_src, size_t src_stride, int n, int w, int h, const uint8_t **pipe_src)
+{
+    int rc = make_layout(e, d_src, src_stride, w, h, &sl.L);
+    if (rc) return rc;
+    const uint8_t *src_end = d_src + (size_t)(n - 1) * src_stride + tight_frame_bytes(w, h, sl.L.fmt);
+    return repitch_if_unaligned(e, sl, d_src, src_end, n, pipe_src);
 }
 
 struct ScopedTiming {
@@ -325,8 +339,10 @@ int launch_pipeline(h2j_encoder *e, Slot &sl, const uint8_t *d_frames, int n, in
         // occupancy experiment knob (DESIGN.md section 4): extra dynamic shared memory limits the CTAs resident per SM
         static const int extra_smem = getenv("H2J_K2_EXTRA_SMEM") ? atoi(getenv("H2J_K2_EXTRA_SMEM")) : 0;
         const dim3 grid(fmt_roles(L.fmt) * ((n_tiles + tiles_per_cta - 1) / tiles_per_cta), n);
-        if (L.fmt == kFmt422) fdct_quant_fmt_kernel<kFmt422><<<grid, kFdctThreads, 0, st>>>(d_frames, L, sl.d_state, sl.d_tabs, sl.d_images, e->images_cap, tiles_per_cta);
-        else if (L.fmt == kFmt444) fdct_quant_fmt_kernel<kFmt444><<<grid, kFdctThreads, 0, st>>>(d_frames, L, sl.d_state, sl.d_tabs, sl.d_images, e->images_cap, tiles_per_cta);
+        if (L.fmt == kFmt422 && L.nv12) fdct_quant_fmt_kernel<kFmt422, true><<<grid, kFdctThreads, 0, st>>>(d_frames, L, sl.d_state, sl.d_tabs, sl.d_images, e->images_cap, tiles_per_cta);
+        else if (L.fmt == kFmt422) fdct_quant_fmt_kernel<kFmt422, false><<<grid, kFdctThreads, 0, st>>>(d_frames, L, sl.d_state, sl.d_tabs, sl.d_images, e->images_cap, tiles_per_cta);
+        else if (L.fmt == kFmt444 && L.nv12) fdct_quant_fmt_kernel<kFmt444, true><<<grid, kFdctThreads, 0, st>>>(d_frames, L, sl.d_state, sl.d_tabs, sl.d_images, e->images_cap, tiles_per_cta);
+        else if (L.fmt == kFmt444) fdct_quant_fmt_kernel<kFmt444, false><<<grid, kFdctThreads, 0, st>>>(d_frames, L, sl.d_state, sl.d_tabs, sl.d_images, e->images_cap, tiles_per_cta);
         else if (L.nv12) fdct_quant_kernel<true><<<grid, kFdctThreads, extra_smem, st>>>(d_frames, L, sl.d_state, sl.d_tabs, sl.d_images, e->images_cap, tiles_per_cta);
         else fdct_quant_kernel<false><<<grid, kFdctThreads, extra_smem, st>>>(d_frames, L, sl.d_state, sl.d_tabs, sl.d_images, e->images_cap, tiles_per_cta);
         e->launches++;
@@ -688,8 +704,8 @@ int h2j_submit_device(h2j_encoder *e, int slot, const uint8_t *d_frames, size_t 
     return H2J_OK;
 }
 
-int h2j_submit_device_nv12(h2j_encoder *e, int slot, const uint8_t *d_frames, size_t frame_stride, int pitch, size_t uv_offset, int n,
-                           int width, int height)
+int h2j_submit_device_semiplanar(h2j_encoder *e, int slot, const uint8_t *d_frames, size_t frame_stride, int pitch, size_t uv_offset,
+                                 int n, int width, int height)
 {
     int rc = check_slot(e, slot);
     if (rc) return rc;
@@ -697,12 +713,12 @@ int h2j_submit_device_nv12(h2j_encoder *e, int slot, const uint8_t *d_frames, si
     if (sl.busy) return fail(e, H2J_ERR_BUSY, "slot %d has a batch in flight", slot);
     if (!d_frames || n < 1 || n > e->s.max_batch) return fail(e, H2J_ERR_INVALID_ARG, "bad frames pointer or batch size %d (max %d)", n, e->s.max_batch);
     if (width < 2 || height < 2) return fail(e, H2J_ERR_UNSUPPORTED, "unsupported frame size %dx%d", width, height);
-    if (e->s.chroma_format != H2J_CHROMA_420) return fail(e, H2J_ERR_UNSUPPORTED, "NV12 is a 4:2:0 layout; this encoder was created for another chroma format");
-    const int fcw = (width + 1) >> 1, fch = (height + 1) >> 1;
+    const int fmt = e->s.chroma_format;
+    const int fcw = chroma_w(width, fmt), fch = chroma_h(height, fmt);  // pairs per row, rows of the pair plane
     if (pitch < width || pitch < 2 * fcw) return fail(e, H2J_ERR_INVALID_ARG, "pitch %d smaller than a row of %d samples", pitch, width);
     if (uv_offset < (size_t)pitch * height || frame_stride < uv_offset + (size_t)pitch * (fch - 1) + 2 * (size_t)fcw)
-        return fail(e, H2J_ERR_INVALID_ARG, "uv_offset / frame_stride do not hold an NV12 frame of %dx%d at pitch %d", width, height, pitch);
-    const size_t fb = tight_frame_bytes(width, height, e->s.chroma_format);
+        return fail(e, H2J_ERR_INVALID_ARG, "uv_offset / frame_stride do not hold a semi-planar frame of %dx%d at pitch %d", width, height, pitch);
+    const size_t fb = tight_frame_bytes(width, height, fmt);
     const size_t dstride = align_up(fb, 256);
     if (dstride > e->frame_bytes_cap) return fail(e, H2J_ERR_UNSUPPORTED, "frame %dx%d exceeds the configured maximum", width, height);
     ON_DEVICE(e);
@@ -710,11 +726,11 @@ int h2j_submit_device_nv12(h2j_encoder *e, int slot, const uint8_t *d_frames, si
     if (rc) return rc;
     sl.n = n;
     CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
-    // Rows on 8-byte boundaries (what decoders produce): the pipeline reads the NV12 frames where they are -- K1 only looks
-    // at luma, K2's chroma warps fetch the pairs and split them in registers.  Otherwise the pairs are split into the
-    // slot's I420 buffer first (one more pass over the frame).
+    // Rows on 8-byte boundaries (what decoders produce): the pipeline reads the frames where they are -- K1 only looks at
+    // luma, K2's chroma roles fetch the pairs and keep their component in registers.  Otherwise the pairs are split into
+    // the slot's planar frame buffer first (one more pass over the frame).
     static const bool force_prepass = getenv("H2J_NV12_PREPASS") != nullptr;  // measurement knob
-    if (!force_prepass && (uintptr_t)d_frames % 8 == 0 && frame_stride % 8 == 0 && pitch % 8 == 0 && uv_offset % 8 == 0) {
+    if (!force_prepass && !e->force_sp_prepass && (uintptr_t)d_frames % 8 == 0 && frame_stride % 8 == 0 && pitch % 8 == 0 && uv_offset % 8 == 0) {
         FrameLayout &L = sl.L;
         L.y_pitch = pitch;
         L.c_pitch = pitch;
@@ -737,6 +753,56 @@ int h2j_submit_device_nv12(h2j_encoder *e, int slot, const uint8_t *d_frames, si
     CU(e, cudaGetLastError());
     const uint8_t *pipe_src = nullptr;
     rc = prepare_input(e, sl, sl.d_frames, dstride, n, width, height, &pipe_src);  // (odd widths: once more, to a 16-byte pitch)
+    if (rc) return rc;
+    rc = launch_pipeline(e, sl, pipe_src, n, TAIL_SIZES);
+    if (rc) return rc;
+    sl.busy = true;
+    return H2J_OK;
+}
+
+int h2j_submit_device_nv12(h2j_encoder *e, int slot, const uint8_t *d_frames, size_t frame_stride, int pitch, size_t uv_offset, int n,
+                           int width, int height)
+{
+    int rc = check_slot(e, slot);
+    if (rc) return rc;
+    if (e->slots[slot].busy) return fail(e, H2J_ERR_BUSY, "slot %d has a batch in flight", slot);
+    if (!d_frames || n < 1 || n > e->s.max_batch) return fail(e, H2J_ERR_INVALID_ARG, "bad frames pointer or batch size %d (max %d)", n, e->s.max_batch);
+    if (width < 2 || height < 2) return fail(e, H2J_ERR_UNSUPPORTED, "unsupported frame size %dx%d", width, height);
+    if (e->s.chroma_format != H2J_CHROMA_420) return fail(e, H2J_ERR_UNSUPPORTED, "NV12 is a 4:2:0 layout; this encoder was created for another chroma format");
+    return h2j_submit_device_semiplanar(e, slot, d_frames, frame_stride, pitch, uv_offset, n, width, height);
+}
+
+int h2j_submit_device_pitched(h2j_encoder *e, int slot, const uint8_t *d_frames, size_t frame_stride, int y_pitch, int c_pitch,
+                              size_t u_offset, size_t v_offset, int n, int width, int height)
+{
+    int rc = check_slot(e, slot);
+    if (rc) return rc;
+    Slot &sl = e->slots[slot];
+    if (sl.busy) return fail(e, H2J_ERR_BUSY, "slot %d has a batch in flight", slot);
+    if (!d_frames || n < 1 || n > e->s.max_batch) return fail(e, H2J_ERR_INVALID_ARG, "bad frames pointer or batch size %d (max %d)", n, e->s.max_batch);
+    if (width < 2 || height < 2) return fail(e, H2J_ERR_UNSUPPORTED, "unsupported frame size %dx%d", width, height);
+    const int fmt = e->s.chroma_format;
+    const int fcw = chroma_w(width, fmt), fch = chroma_h(height, fmt);
+    if (y_pitch < width || c_pitch < fcw) return fail(e, H2J_ERR_INVALID_ARG, "pitches %d / %d smaller than rows of %d / %d samples", y_pitch, c_pitch, width, fcw);
+    const size_t y_end = (size_t)y_pitch * (height - 1) + width;
+    const size_t u_end = u_offset + (size_t)c_pitch * (fch - 1) + fcw, v_end = v_offset + (size_t)c_pitch * (fch - 1) + fcw;
+    if (y_end > frame_stride || u_end > frame_stride || v_end > frame_stride)
+        return fail(e, H2J_ERR_INVALID_ARG, "a plane of the %dx%d frame reaches past frame_stride %zu", width, height, frame_stride);
+    ON_DEVICE(e);
+    rc = make_layout(e, d_frames, frame_stride, width, height, &sl.L);
+    if (rc) return rc;
+    FrameLayout &L = sl.L;
+    L.y_pitch = y_pitch;
+    L.c_pitch = c_pitch;
+    L.u_off = (long long)u_offset;
+    L.v_off = (long long)v_offset;
+    set_alignment(&L, d_frames);
+    sl.n = n;
+    CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
+    // rows on 8-byte boundaries: the pipeline reads the frames where they are; otherwise one copy to a 16-byte pitch
+    const uint8_t *pipe_src = nullptr;
+    const uint8_t *src_end = d_frames + (size_t)(n - 1) * frame_stride + std::max(y_end, std::max(u_end, v_end));
+    rc = repitch_if_unaligned(e, sl, d_frames, src_end, n, &pipe_src);
     if (rc) return rc;
     rc = launch_pipeline(e, sl, pipe_src, n, TAIL_SIZES);
     if (rc) return rc;
@@ -1075,6 +1141,11 @@ int h2j_debug_set_knob(h2j_encoder *e, const char *name, int value)
     if (!strcmp(name, "fdct_tiles_per_cta")) {
         if (value < 0 || value > 4096) return fail(e, H2J_ERR_INVALID_ARG, "fdct_tiles_per_cta %d out of range", value);
         e->force_fdct_tiles = value;
+        return H2J_OK;
+    }
+    if (!strcmp(name, "semiplanar_prepass")) {
+        if (value < 0 || value > 1) return fail(e, H2J_ERR_INVALID_ARG, "semiplanar_prepass %d is not 0 or 1", value);
+        e->force_sp_prepass = value;
         return H2J_OK;
     }
     return fail(e, H2J_ERR_INVALID_ARG, "unknown knob %s", name);

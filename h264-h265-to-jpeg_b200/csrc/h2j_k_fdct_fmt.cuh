@@ -9,19 +9,25 @@
 // is the component's last block of the MCU in front of the role's range, rebuilt from its pixel sum by eight helper lanes
 // (the DC output of ff_fdct_sse2 is the sum of the 64 samples) -- for every tile, there is no chroma carry to keep.
 // blockIdx.x = tile group * roles + role, single-warp CTAs, tiles_per_cta consecutive tiles per CTA.
+// SP (semi-planar, L.nv12): chroma is ONE plane of interleaved Cb/Cr pairs (NV16 at 4:2:2, NV24 at 4:4:4), read in place.
+// A chroma block's eight samples of a row are the 16 bytes of its eight pairs; every role holds one component, so each
+// chroma lane fetches the whole 16 bytes and keeps its half (no lane trade as in fdct_quant_kernel's NV12 path).
 #pragma once
 #include "h2j_k_fdct.cuh"
 
 namespace h2j {
 
 // component c (0 Y, 1 Cb, 2 Cr), k-th block of that component inside the MCU (coding order)
-template <int FMT> __device__ __forceinline__ PlaneRef plane_ref_fmt(const uint8_t *base, const FrameLayout &L, int c, int k)
+template <int FMT, bool SP> __device__ __forceinline__ PlaneRef plane_ref_fmt(const uint8_t *base, const FrameLayout &L, int c, int k)
 {
     PlaneRef r;
     if (c == 0) {
         r.P = base; r.pitch = L.y_pitch; r.pw = L.w; r.ph = L.h; r.step = 16;
         if (FMT == kFmt444) { r.xstep = 8; r.xoff = 0; r.yoff = k * 8; }          // Y top, Y bottom of an 8x16 MCU
         else { r.xstep = 16; r.xoff = (k & 1) * 8; r.yoff = (k >> 1) * 8; }       // Y0 Y1 / Y2 Y3
+    } else if (SP) {  // the pair plane, positions in bytes: a block is 16 bytes wide, pw = the pairs the encoder reads
+        r.P = base + L.u_off; r.pitch = L.c_pitch; r.pw = 2 * L.cw; r.ph = L.ch;
+        r.step = 16; r.xstep = 16; r.xoff = 0; r.yoff = k * 8;
     } else {
         r.P = base + (c == 1 ? L.u_off : L.v_off); r.pitch = L.c_pitch; r.pw = L.cw; r.ph = L.ch;
         r.step = 16; r.xstep = 8; r.xoff = 0; r.yoff = k * 8;                      // top, bottom; chroma MCU step 8 x 16 in both formats
@@ -30,7 +36,101 @@ template <int FMT> __device__ __forceinline__ PlaneRef plane_ref_fmt(const uint8
     return r;
 }
 
-template <int FMT>
+// ---- SP chroma lanes: `odd` = 0 for Cb (even bytes of the pair plane), 1 for Cr ----
+// The second 8 bytes of each row of the block and of the predecessor row (the first 8 ride in BlockFetch).  Both halves
+// are requested a tile ahead, as in the planar path: requesting the second halves at the top of the tile instead (16 fewer
+// registers in flight across the statistics walk) left their latency exposed -- NV16 in place at 1.005x the prepass instead
+// of 1.09x (DESIGN.md row (f)(4)).
+struct PairHalves {
+    uint2 hi[8];
+    uint2 prow_hi;
+};
+__device__ __forceinline__ bool sp_is_fast(const PlaneRef &R, int bx) { return R.can_fast && bx + 16 <= R.pw; }
+// sample c of the block at byte bx of a row, the right edge replicated: never a byte past the row's 2 * cw
+__device__ __forceinline__ int sp_sample_at(const uint8_t *row, const PlaneRef &R, int bx, int c, int odd)
+{
+    return row[2 * min((bx >> 1) + c, (R.pw >> 1) - 1) + odd];
+}
+
+// as fetch_issue<false, false>, with the 16 bytes of each row as two 8-byte loads (the rows are 8-byte aligned), and the
+// predecessor rows of the helper lanes likewise
+__device__ __forceinline__ void sp_fetch_issue(BlockFetch &F, PairHalves &H, const uint8_t *safe, const PlaneRef &R, const BlockPos &bp,
+                                               bool valid, const PlaneRef &Q, const BlockPos &pp, bool phelp, int prow_idx)
+{
+    const bool pf = phelp && sp_is_fast(Q, pp.bx);
+    const uint8_t *pq = pf ? Q.P + (long long)min(pp.by + prow_idx, Q.ph - 1) * Q.pitch + pp.bx : safe;
+    F.prow = ldg64(pq);
+    H.prow_hi = ldg64(pq + 8);
+    const bool rf = valid && sp_is_fast(R, bp.bx);
+    if (!rf || bp.by + 8 <= R.ph) {
+        const uint8_t *p = rf ? R.P + (long long)bp.by * R.pitch + bp.bx : safe;
+        const int pitch = rf ? R.pitch : 0;
+#pragma unroll
+        for (int r = 0; r < 8; r++) {
+            F.rows[r] = ldg64(p);
+            H.hi[r] = ldg64(p + 8);
+            p += pitch;
+        }
+    } else {
+#pragma unroll
+        for (int r = 0; r < 8; r++) {
+            const uint8_t *p = R.P + (long long)min(bp.by + r, R.ph - 1) * R.pitch + bp.bx;
+            F.rows[r] = ldg64(p);
+            H.hi[r] = ldg64(p + 8);
+        }
+    }
+}
+
+__device__ __forceinline__ void sp_fetch_consume(const BlockFetch &F, const PairHalves &H, const PlaneRef &R, const BlockPos &bp, int odd,
+                                                 const uint8_t *lut, int (&v)[64])
+{
+    const unsigned sel = odd ? 0x7531u : 0x6420u;  // the Cr / Cb byte of four pairs
+#pragma unroll
+    for (int r = 0; r < 8; r++) {
+        const unsigned lo4 = __byte_perm(F.rows[r].x, F.rows[r].y, sel), hi4 = __byte_perm(H.hi[r].x, H.hi[r].y, sel);
+        v[r * 8 + 0] = (int)__byte_perm(lo4, 0u, 0x4440);
+        v[r * 8 + 1] = (int)__byte_perm(lo4, 0u, 0x4441);
+        v[r * 8 + 2] = (int)__byte_perm(lo4, 0u, 0x4442);
+        v[r * 8 + 3] = (int)__byte_perm(lo4, 0u, 0x4443);
+        v[r * 8 + 4] = (int)__byte_perm(hi4, 0u, 0x4440);
+        v[r * 8 + 5] = (int)__byte_perm(hi4, 0u, 0x4441);
+        v[r * 8 + 6] = (int)__byte_perm(hi4, 0u, 0x4442);
+        v[r * 8 + 7] = (int)__byte_perm(hi4, 0u, 0x4443);
+    }
+    if (!sp_is_fast(R, bp.bx)) {
+#pragma unroll
+        for (int r = 0; r < 8; r++) {
+            const uint8_t *row = R.P + (long long)min(bp.by + r, R.ph - 1) * R.pitch;
+#pragma unroll
+            for (int c = 0; c < 8; c++) v[r * 8 + c] = sp_sample_at(row, R, bp.bx, c, odd);
+        }
+    }
+    if (lut) {
+#pragma unroll
+        for (int i = 0; i < 64; i++) v[i] = lut[v[i]];
+    }
+}
+
+// this lane's share (one pixel row) of the predecessor block's sample sum
+__device__ __forceinline__ int sp_pred_rowsum(const BlockFetch &F, const PairHalves &H, const PlaneRef &Q, const BlockPos &pp, bool phelp,
+                                              int prow_idx, int odd, const uint8_t *lut)
+{
+    const unsigned sel = odd ? 0x7531u : 0x6420u;
+    int s = (int)__dp4a(__byte_perm(H.prow_hi.x, H.prow_hi.y, sel), 0x01010101u, __dp4a(__byte_perm(F.prow.x, F.prow.y, sel), 0x01010101u, 0u));
+    if (!phelp) return 0;
+    if (!sp_is_fast(Q, pp.bx) || lut) {
+        const uint8_t *row = Q.P + (long long)min(pp.by + prow_idx, Q.ph - 1) * Q.pitch;
+        s = 0;
+#pragma unroll
+        for (int c = 0; c < 8; c++) {
+            const int p = sp_sample_at(row, Q, pp.bx, c, odd);
+            s += lut ? lut[p] : p;
+        }
+    }
+    return s;
+}
+
+template <int FMT, bool SP>
 __global__ void __launch_bounds__(kFdctThreads, H2J_FDCT_MIN_CTAS) fdct_quant_fmt_kernel(const uint8_t *__restrict__ frames, FrameLayout L,
                                                                          FrameState *__restrict__ state,
                                                                          const FrameTab *__restrict__ tabs,
@@ -63,15 +163,19 @@ __global__ void __launch_bounds__(kFdctThreads, H2J_FDCT_MIN_CTAS) fdct_quant_fm
     const int cls = comp ? 1 : 0;
     const uint8_t *lut = L.range_mode ? c_range_lut[cls] : nullptr;
     const bool phelp_lane = lane < 8;  // add one pixel row each of the block in front of the role's range
-    const PlaneRef R = plane_ref_fmt<FMT>(base, L, comp, k), Q = plane_ref_fmt<FMT>(base, L, comp, per_mcu - 1);
+    const PlaneRef R = plane_ref_fmt<FMT, SP>(base, L, comp, k), Q = plane_ref_fmt<FMT, SP>(base, L, comp, per_mcu - 1);
+    const bool spc = SP && comp != 0;  // this role reads the pair plane (role-uniform)
+    const int odd = comp - 1;          // (spc) the role's byte of a pair
 
     BlockFetch F;
+    PairHalves H;
     const uint8_t *safe = reinterpret_cast<const uint8_t *>(tabs);  // aligned, always readable: what skipped loads read
     BlockPos bp, pp;
     bp.init(tile0 * kTileMcus + mcu_l, R, L.mcu_w);
     pp.init(tile0 * kTileMcus + mcu_first - 1, Q, L.mcu_w);
     auto phelp_now = [&]() { return phelp_lane && pp.m >= 0 && pp.m < L.n_mcu; };
-    fetch_issue<false, false>(F, safe, R, bp, bp.m < L.n_mcu, Q, pp, phelp_now(), lane & 7);
+    if (spc) sp_fetch_issue(F, H, safe, R, bp, bp.m < L.n_mcu, Q, pp, phelp_now(), lane & 7);
+    else fetch_issue<false, false>(F, safe, R, bp, bp.m < L.n_mcu, Q, pp, phelp_now(), lane & 7);
 
     {
         const uint2 pk = reinterpret_cast<const uint2 *>(tabs[f].qpack)[lane];
@@ -92,7 +196,7 @@ __global__ void __launch_bounds__(kFdctThreads, H2J_FDCT_MIN_CTAS) fdct_quant_fm
         __syncwarp();
 
         // ---- predecessor DC of lane 0, from pixel sums ----
-        int psum = fetch_pred_rowsum<false>(F, Q, pp, phelp_now(), lane & 7, lut);
+        int psum = spc ? sp_pred_rowsum(F, H, Q, pp, phelp_now(), lane & 7, odd, lut) : fetch_pred_rowsum<false>(F, Q, pp, phelp_now(), lane & 7, lut);
         psum += __shfl_xor_sync(0xffffffffu, psum, 1);
         psum += __shfl_xor_sync(0xffffffffu, psum, 2);
         psum += __shfl_xor_sync(0xffffffffu, psum, 4);
@@ -105,7 +209,8 @@ __global__ void __launch_bounds__(kFdctThreads, H2J_FDCT_MIN_CTAS) fdct_quant_fm
         uint32_t *rec = img + lane * kBlkWords;
         if (valid) {
             int v[64];
-            fetch_consume<false>(F, R, bp, lut, v);
+            if (spc) sp_fetch_consume(F, H, R, bp, odd, lut, v);
+            else fetch_consume<false>(F, R, bp, lut, v);
             fdct_8x8(v);
             dc = quant_dc(v[0]);
 #pragma unroll
@@ -130,7 +235,8 @@ __global__ void __launch_bounds__(kFdctThreads, H2J_FDCT_MIN_CTAS) fdct_quant_fm
         if (tile + 1 < tile_end) {
             bp.advance(R, L.mcu_w);
             pp.advance(Q, L.mcu_w);
-            fetch_issue<false, false>(F, safe, R, bp, bp.m < L.n_mcu, Q, pp, phelp_now(), lane & 7);
+            if (spc) sp_fetch_issue(F, H, safe, R, bp, bp.m < L.n_mcu, Q, pp, phelp_now(), lane & 7);
+            else fetch_issue<false, false>(F, safe, R, bp, bp.m < L.n_mcu, Q, pp, phelp_now(), lane & 7);
         }
 
         // ---- DC difference to the previous block of the component (mjpegenc.c record_block) ----

@@ -137,9 +137,10 @@ __global__ void __launch_bounds__(128) convert_pad_kernel(const uint8_t *__restr
 }
 
 // ------------------------------------------------------------------------------------------------
-// NV12 (what hardware decoders produce: a luma plane and ONE plane of interleaved Cb/Cr pairs, both with a row pitch)
-// -> the tight I420 frames the pipeline reads.  grid (x, rows, frames): rows 0..h-1 copy luma, rows h..h+ch-1 split a
-// chroma row (kPlaneRowsPerCta rows per CTA: one row per CTA made 400 k CTAs of 120 busy threads for 256 frames).
+// NV12 / NV16 / NV24 (what hardware decoders produce: a luma plane and ONE plane of interleaved Cb/Cr pairs, both with a
+// row pitch) -> the tight planar frames the pipeline reads (I420 / 4:2:2 / 4:4:4 by L.fmt: c_pitch pairs per row, ch rows
+// of them).  grid (x, rows, frames): rows 0..h-1 copy luma, rows h..h+ch-1 split a chroma row (kPlaneRowsPerCta rows per
+// CTA: one row per CTA made 400 k CTAs of 120 busy threads for 256 frames).
 // 16 bytes per thread where pitch, base and width allow, bytes otherwise.
 // ------------------------------------------------------------------------------------------------
 constexpr int kPlaneRowsPerCta = 16;
@@ -149,7 +150,7 @@ __global__ void __launch_bounds__(128) nv12_to_i420_kernel(const uint8_t *__rest
     const int f = blockIdx.z;
     const uint8_t *S = src + (long long)f * src_stride;
     uint8_t *D = dst + (long long)f * L.frame_stride;
-    const int fch = (L.h + 1) >> 1;
+    const int fch = (L.h + fmt_vshift(L.fmt)) >> fmt_vshift(L.fmt);
     const int x0 = (blockIdx.x * blockDim.x + threadIdx.x) * 16;
     for (int row = blockIdx.y * kPlaneRowsPerCta; row < min((int)(blockIdx.y + 1) * kPlaneRowsPerCta, L.h + fch); row++)
     if (row < L.h) {
@@ -180,25 +181,27 @@ __global__ void __launch_bounds__(128) nv12_to_i420_kernel(const uint8_t *__rest
 }
 
 // ------------------------------------------------------------------------------------------------
-// Tight I420 frames whose rows do not start on 8-byte boundaries (odd widths such as 1918, or an unaligned base) ->
-// the same planes at a 16-byte row pitch, so that K1 and K2 take their vector-load paths (every block but the ones cut
-// by the right edge) instead of 64 byte loads per block.  grid (x, h + 2 * ceil(h/2), frames); a thread produces 16
-// output bytes from five aligned source words and four funnel shifts.  The padding bytes of a row are never read by
-// the pipeline (edges are replicated from the last real sample).
+// Planar frames whose rows do not start on 8-byte boundaries (odd widths such as 1918, an unaligned base, a caller's
+// pitches or plane offsets) -> the same planes at a 16-byte row pitch, so that K1 and K2 take their vector-load paths
+// (every block but the ones cut by the right edge) instead of 64 byte loads per block.  grid (x, h + 2 * ch, frames); a
+// thread produces 16 output bytes from five aligned source words and four funnel shifts.  A row copies the plane's
+// width, ceil-divided by the subsampling (not the source pitch); the padding bytes of a row are never read by the pipeline
+// (edges are replicated from the last real sample).
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) repitch_kernel(const uint8_t *__restrict__ src, FrameLayout T,  // tight layout of the source
+__global__ void __launch_bounds__(128) repitch_kernel(const uint8_t *__restrict__ src, FrameLayout T,  // layout of the source
                                                       int fch,                                         // rows of a chroma plane
                                                       uint8_t *__restrict__ dst, FrameLayout P,        // pitched layout of the copy
-                                                      const uint8_t *src_begin, const uint8_t *src_end)
+                                                      const uint8_t *src_begin, const uint8_t *src_end)  // what may be read
 {
     const int f = blockIdx.z;
+    const int fcw = (T.w + (1 << fmt_hshift(T.fmt)) - 1) >> fmt_hshift(T.fmt);  // (T.c_pitch of a tight source)
     for (int row = blockIdx.y * kPlaneRowsPerCta; row < min((int)(blockIdx.y + 1) * kPlaneRowsPerCta, T.h + 2 * fch); row++) {
     int pw, r;
     long long so, dof;
     int spitch, dpitch;
     if (row < T.h) { pw = T.w; r = row; so = 0; dof = 0; spitch = T.y_pitch; dpitch = P.y_pitch; }
-    else if (row < T.h + fch) { pw = T.c_pitch; r = row - T.h; so = T.u_off; dof = P.u_off; spitch = T.c_pitch; dpitch = P.c_pitch; }
-    else { pw = T.c_pitch; r = row - T.h - fch; so = T.v_off; dof = P.v_off; spitch = T.c_pitch; dpitch = P.c_pitch; }
+    else if (row < T.h + fch) { pw = fcw; r = row - T.h; so = T.u_off; dof = P.u_off; spitch = T.c_pitch; dpitch = P.c_pitch; }
+    else { pw = fcw; r = row - T.h - fch; so = T.v_off; dof = P.v_off; spitch = T.c_pitch; dpitch = P.c_pitch; }
     const int x0 = (blockIdx.x * blockDim.x + threadIdx.x) * 16;
     if (x0 >= pw) continue;
     const uint8_t *s = src + (long long)f * T.frame_stride + so + (long long)r * spitch + x0;

@@ -85,7 +85,8 @@ class FrameInfo(C.Structure):
 
 EXPORTS = [
     "h2j_default_settings", "h2j_create", "h2j_destroy", "h2j_last_error", "h2j_status_string", "h2j_abi_version",
-    "h2j_encode_frame", "h2j_submit_host", "h2j_submit_device", "h2j_submit_device_nv12", "h2j_collect", "h2j_collect_device", "h2j_wait",
+    "h2j_encode_frame", "h2j_submit_host", "h2j_submit_device", "h2j_submit_device_nv12",
+    "h2j_submit_device_semiplanar", "h2j_submit_device_pitched", "h2j_collect", "h2j_collect_device", "h2j_wait",
     "h2j_alloc_pinned", "h2j_free_pinned", "h2j_convert_pad", "h2j_debug_frame_info", "h2j_debug_coefficients",
     "h2j_slot_kernel_ms", "h2j_set_profile", "h2j_slot_total_ms", "h2j_kernel_launches", "h2j_slot_set_stream",
     "h2j_slot_wait_event", "h2j_device_count", "h2j_debug_set_knob", "h2j_debug_read_device", "h2j_stream_copy",
@@ -120,6 +121,8 @@ def load_library() -> C.CDLL:
     lib.h2j_submit_host.argtypes = [vp, ci, vp, sz, ci, ci, ci]
     lib.h2j_submit_device.argtypes = [vp, ci, vp, sz, ci, ci, ci]
     lib.h2j_submit_device_nv12.argtypes = [vp, ci, vp, sz, ci, sz, ci, ci, ci]
+    lib.h2j_submit_device_semiplanar.argtypes = [vp, ci, vp, sz, ci, sz, ci, ci, ci]
+    lib.h2j_submit_device_pitched.argtypes = [vp, ci, vp, sz, ci, ci, sz, sz, ci, ci, ci]
     lib.h2j_collect.argtypes = [vp, ci, vp, sz, C.POINTER(sz), C.POINTER(ci)]
     lib.h2j_collect_device.argtypes = [vp, ci, C.POINTER(vp), C.POINTER(sz), C.POINTER(sz), C.POINTER(ci)]
     lib.h2j_wait.argtypes = [vp, ci]
@@ -332,6 +335,21 @@ class Encoder:
                            width: int, height: int) -> None:
         """NV12 frames in device memory (luma plane + interleaved Cb/Cr plane, rows `pitch` apart)."""
         self._check(self._lib.h2j_submit_device_nv12(self._h, slot, d_frames_ptr, frame_stride, pitch, uv_offset, n, width, height))
+        self._n_in_slot[slot] = n
+
+    def submit_device_semiplanar(self, slot: int, d_frames_ptr: int, frame_stride: int, pitch: int, uv_offset: int, n: int,
+                                 width: int, height: int) -> None:
+        """Semi-planar frames in device memory by the encoder's chroma format: NV12 / NV16 / NV24 (luma plane + interleaved
+        Cb/Cr plane at `uv_offset`, rows `pitch` apart)."""
+        self._check(self._lib.h2j_submit_device_semiplanar(self._h, slot, d_frames_ptr, frame_stride, pitch, uv_offset, n, width, height))
+        self._n_in_slot[slot] = n
+
+    def submit_device_pitched(self, slot: int, d_frames_ptr: int, frame_stride: int, y_pitch: int, c_pitch: int, u_offset: int,
+                              v_offset: int, n: int, width: int, height: int) -> None:
+        """Planar frames in device memory at any layout: luma rows `y_pitch` apart at the frame's start, Cb / Cr planes at
+        `u_offset` / `v_offset` with rows `c_pitch` apart."""
+        self._check(self._lib.h2j_submit_device_pitched(self._h, slot, d_frames_ptr, frame_stride, y_pitch, c_pitch, u_offset, v_offset,
+                                                        n, width, height))
         self._n_in_slot[slot] = n
 
     def read_device(self, d_ptr: int, nbytes: int) -> bytes:

@@ -127,7 +127,7 @@ int h2j_encode_frame(h2j_encoder *e, const uint8_t *const planes[3], const int s
  * status[i] (optional, may be NULL) receives a per-frame h2j_status.
  *
  * Stream ordering of device inputs: the kernels of a slot run on the slot's own (non-blocking) stream, or on the stream
- * given with h2j_slot_set_stream.  h2j_submit_device / h2j_submit_device_nv12 read the caller's device memory on THAT
+ * given with h2j_slot_set_stream.  h2j_submit_device and the other h2j_submit_device_* read the caller's device memory on THAT
  * stream; nothing orders them behind work of other streams.  A caller whose frames are produced on another stream (a
  * decoder's, torch's current stream) must, before submitting, either synchronise that stream, or make the slot use it
  * (h2j_slot_set_stream), or record an event behind the producer and hand it to h2j_slot_wait_event.  The same holds
@@ -146,6 +146,26 @@ int h2j_submit_device(h2j_encoder *e, int slot, const uint8_t *d_frames, size_t 
  * libavcodec's software decoder, src/Decoder.cpp:183, :324-342).  Collect with h2j_collect / h2j_collect_device. */
 int h2j_submit_device_nv12(h2j_encoder *e, int slot, const uint8_t *d_frames, size_t frame_stride, int pitch,
                            size_t uv_offset, int n, int width, int height);
+/* Semi-planar frames in device memory, by the encoder's chroma_format: NV12 (4:2:0), NV16 (4:2:2), NV24 (4:4:4).
+ * Per frame: a luma plane of `height` rows; `uv_offset` bytes behind the frame's start, a plane of interleaved Cb/Cr pairs
+ * with ceil(width/2) pairs x ceil(height/2) rows (NV12), ceil(width/2) x height (NV16) or width x height (NV24).
+ * Both planes have rows `pitch` bytes apart; frames are `frame_stride` bytes apart.
+ * JPEGs: those of the equivalent planar frame.
+ * With the pointer, the stride, the pitch and uv_offset multiples of 8 the frames are read where they are; otherwise the
+ * pairs are first split into the slot's own planar frame buffer by one extra kernel.  At 4:2:0 this is
+ * h2j_submit_device_nv12.  H2J_ERR_INVALID_ARG: a pitch shorter than a luma row or a row of pairs, a pair plane that
+ * starts inside the luma plane, or a plane that reaches past frame_stride. */
+int h2j_submit_device_semiplanar(h2j_encoder *e, int slot, const uint8_t *d_frames, size_t frame_stride, int pitch,
+                                 size_t uv_offset, int n, int width, int height);
+/* Planar frames in device memory at any layout: luma rows `y_pitch` apart at the frame's start; Cb and Cr planes at
+ * `u_offset` / `v_offset` (any order, e.g. YV12's V before U), rows `c_pitch` apart.
+ * Plane sizes as for h2j_submit_device.
+ * A hardware decoder's 4:4:4 surface is y_pitch = c_pitch = pitch, u_offset = pitch * surface_height, v_offset =
+ * 2 * pitch * surface_height.  With the pointer, the stride, both pitches and both offsets multiples of 8 the frames are
+ * read where they are; otherwise one extra kernel copies them to a 16-byte pitch first.  H2J_ERR_INVALID_ARG: a pitch
+ * shorter than its plane's row, or a plane that reaches past frame_stride. */
+int h2j_submit_device_pitched(h2j_encoder *e, int slot, const uint8_t *d_frames, size_t frame_stride, int y_pitch,
+                              int c_pitch, size_t u_offset, size_t v_offset, int n, int width, int height);
 int h2j_collect(h2j_encoder *e, int slot, uint8_t *out, size_t out_capacity, size_t *offsets, int *status);
 int h2j_collect_device(h2j_encoder *e, int slot, const uint8_t **d_out, size_t *d_frame_capacity, size_t *sizes,
                        int *status);
@@ -199,7 +219,9 @@ int h2j_debug_coefficients(h2j_encoder *e, int slot, int frame, int16_t *out, si
 int h2j_debug_read_device(h2j_encoder *e, const void *d_src, void *dst, size_t bytes);
 /* Launch-shape overrides for tests that must reach code paths a small batch would not take on its own.  Results never
  * depend on a knob.  "fdct_tiles_per_cta": consecutive 16-MCU tiles one CTA of the FDCT kernel walks (0 = automatic:
- * 1 for small batches, up to 16 for large ones). */
+ * 1 for small batches, up to 16 for large ones).  "semiplanar_prepass": 1 = h2j_submit_device_semiplanar /
+ * h2j_submit_device_nv12 split the pairs into planes first even where the frames could be read in place (0 = by
+ * alignment). */
 int h2j_debug_set_knob(h2j_encoder *e, const char *name, int value);
 
 /* With settings.profile != 0: milliseconds each kernel of the slot's last batch took, measured with CUDA
