@@ -7,7 +7,6 @@
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <string>
 #include <vector>
@@ -85,8 +84,6 @@ struct h2j_encoder {
     int groups_cap = 0;           // K4b groups (64 units) per frame
     long long stage_cap_words = 0;
     int chunks_cap = 0;           // K5 chunks per frame
-    int stuff_ctas = 32;          // K5 CTAs per frame
-    int fdct_tiles_per_cta = 16;  // upper bound of consecutive K2 tiles one CTA walks
     int force_fdct_tiles = 0;     // h2j_debug_set_knob("fdct_tiles_per_cta"): exactly this many, whatever the batch size
     int force_sp_prepass = 0;     // h2j_debug_set_knob("semiplanar_prepass"): split semi-planar frames first even when aligned
     size_t frame_bytes_cap = 0;
@@ -238,8 +235,7 @@ int repitch_if_unaligned(h2j_encoder *e, Slot &sl, const uint8_t *d_src, const u
 {
     const int w = sl.L.w, h = sl.L.h;
     *pipe_src = d_src;
-    static const bool no_repitch = getenv("H2J_NO_REPITCH") != nullptr;  // measurement knob
-    if (sl.L.aligned8 || no_repitch) return H2J_OK;
+    if (sl.L.aligned8) return H2J_OK;
     if (!sl.d_pitched) {
         const size_t bytes = pitched_frame_bytes(e->s.max_width, e->s.max_height, e->s.chroma_format) * (size_t)e->s.max_batch;
         if (cudaMalloc(&sl.d_pitched, bytes) != cudaSuccess) {  // no room for the copy: the bytewise path still works
@@ -313,6 +309,9 @@ int enqueue_pack_and_sizes(h2j_encoder *e, Slot &sl, bool pack);
 enum TailMode { TAIL_SIZES = 0, TAIL_PACK = 1, TAIL_SINGLE = 2 };
 int enqueue_single_tail(h2j_encoder *e, Slot &sl);
 
+constexpr int kFdctMaxTilesPerCta = 16;  // K2: upper bound of consecutive tiles one CTA walks (h2j_debug_set_knob may force any)
+constexpr int kStuffCtas = 32;           // K5 CTAs per frame
+
 int launch_pipeline(h2j_encoder *e, Slot &sl, const uint8_t *d_frames, int n, int tail)
 {
     const FrameLayout &L = sl.L;
@@ -331,20 +330,15 @@ int launch_pipeline(h2j_encoder *e, Slot &sl, const uint8_t *d_frames, int n, in
     {
         ScopedTiming t(e, sl, "fdct_quant_kernel");
         // consecutive tiles per CTA: as many as keep the grid at four waves or more (amortises the per-CTA set-up
-        // and histogram flush), at most 16
-        int tiles_per_cta = (int)((long long)n_tiles * n * fmt_roles(L.fmt) / ((long long)e->sm_count * 16 * 4));
-        tiles_per_cta = tiles_per_cta < 1 ? 1 : (tiles_per_cta > e->fdct_tiles_per_cta ? e->fdct_tiles_per_cta : tiles_per_cta);
-        if (const char *env = getenv("H2J_FDCT_TILES_PER_CTA")) tiles_per_cta = atoi(env) > 0 ? atoi(env) : tiles_per_cta;  // tuning knob
+        // and histogram flush), at most kFdctMaxTilesPerCta
+        int tiles_per_cta = (int)((long long)n_tiles * n * fmt_roles(L.fmt) / ((long long)e->sm_count * kFdctMinCtas * 4));
+        tiles_per_cta = tiles_per_cta < 1 ? 1 : (tiles_per_cta > kFdctMaxTilesPerCta ? kFdctMaxTilesPerCta : tiles_per_cta);
         if (e->force_fdct_tiles > 0) tiles_per_cta = e->force_fdct_tiles;
-        // occupancy experiment knob (DESIGN.md section 4): extra dynamic shared memory limits the CTAs resident per SM
-        static const int extra_smem = getenv("H2J_K2_EXTRA_SMEM") ? atoi(getenv("H2J_K2_EXTRA_SMEM")) : 0;
         const dim3 grid(fmt_roles(L.fmt) * ((n_tiles + tiles_per_cta - 1) / tiles_per_cta), n);
-        if (L.fmt == kFmt422 && L.nv12) fdct_quant_fmt_kernel<kFmt422, true><<<grid, kFdctThreads, 0, st>>>(d_frames, L, sl.d_state, sl.d_tabs, sl.d_images, e->images_cap, tiles_per_cta);
-        else if (L.fmt == kFmt422) fdct_quant_fmt_kernel<kFmt422, false><<<grid, kFdctThreads, 0, st>>>(d_frames, L, sl.d_state, sl.d_tabs, sl.d_images, e->images_cap, tiles_per_cta);
-        else if (L.fmt == kFmt444 && L.nv12) fdct_quant_fmt_kernel<kFmt444, true><<<grid, kFdctThreads, 0, st>>>(d_frames, L, sl.d_state, sl.d_tabs, sl.d_images, e->images_cap, tiles_per_cta);
-        else if (L.fmt == kFmt444) fdct_quant_fmt_kernel<kFmt444, false><<<grid, kFdctThreads, 0, st>>>(d_frames, L, sl.d_state, sl.d_tabs, sl.d_images, e->images_cap, tiles_per_cta);
-        else if (L.nv12) fdct_quant_kernel<true><<<grid, kFdctThreads, extra_smem, st>>>(d_frames, L, sl.d_state, sl.d_tabs, sl.d_images, e->images_cap, tiles_per_cta);
-        else fdct_quant_kernel<false><<<grid, kFdctThreads, extra_smem, st>>>(d_frames, L, sl.d_state, sl.d_tabs, sl.d_images, e->images_cap, tiles_per_cta);
+        const auto k2 = L.fmt == kFmt422 ? (L.nv12 ? fdct_quant_fmt_kernel<kFmt422, true> : fdct_quant_fmt_kernel<kFmt422, false>)
+                        : L.fmt == kFmt444 ? (L.nv12 ? fdct_quant_fmt_kernel<kFmt444, true> : fdct_quant_fmt_kernel<kFmt444, false>)
+                                           : (L.nv12 ? fdct_quant_kernel<true> : fdct_quant_kernel<false>);
+        k2<<<grid, kFdctThreads, 0, st>>>(d_frames, L, sl.d_state, sl.d_tabs, sl.d_images, e->images_cap, tiles_per_cta);
         e->launches++;
     }
     {
@@ -355,16 +349,9 @@ int launch_pipeline(h2j_encoder *e, Slot &sl, const uint8_t *d_frames, int n, in
     }
     {
         ScopedTiming t(e, sl, "entropy_walk_kernel");
-        const dim3 grid(n_tiles, n);
-        if (L.fmt == kFmt422)
-            entropy_walk_kernel<kFmt422><<<grid, fmt_tile_blocks(kFmt422), ent_smem_bytes(kFmt422), st>>>(L, sl.d_tabs, sl.d_images, e->images_cap, sl.d_unit_info, e->units_cap,
-                                                                                                     sl.d_stage_alloc, sl.d_stage, e->stage_cap_words);
-        else if (L.fmt == kFmt444)
-            entropy_walk_kernel<kFmt444><<<grid, fmt_tile_blocks(kFmt444), ent_smem_bytes(kFmt444), st>>>(L, sl.d_tabs, sl.d_images, e->images_cap, sl.d_unit_info, e->units_cap,
-                                                                                                     sl.d_stage_alloc, sl.d_stage, e->stage_cap_words);
-        else
-            entropy_walk_kernel<kFmt420><<<grid, fmt_tile_blocks(kFmt420), ent_smem_bytes(kFmt420), st>>>(L, sl.d_tabs, sl.d_images, e->images_cap, sl.d_unit_info, e->units_cap,
-                                                                                                     sl.d_stage_alloc, sl.d_stage, e->stage_cap_words);
+        const auto k4a = L.fmt == kFmt420 ? entropy_walk_kernel<kFmt420> : L.fmt == kFmt422 ? entropy_walk_kernel<kFmt422> : entropy_walk_kernel<kFmt444>;
+        k4a<<<dim3(n_tiles, n), fmt_tile_blocks(L.fmt), ent_smem_bytes(L.fmt), st>>>(L, sl.d_tabs, sl.d_images, e->images_cap, sl.d_unit_info, e->units_cap,
+                                                                                     sl.d_stage_alloc, sl.d_stage, e->stage_cap_words);
         e->launches++;
     }
     {
@@ -384,9 +371,8 @@ int launch_pipeline(h2j_encoder *e, Slot &sl, const uint8_t *d_frames, int n, in
     }
     {
         ScopedTiming t(e, sl, "stuff_kernel");
-        static const int stuff_ctas_env = getenv("H2J_STUFF_CTAS") ? atoi(getenv("H2J_STUFF_CTAS")) : 0;  // tuning knob
-        stuff_kernel<<<dim3(stuff_ctas_env > 0 ? stuff_ctas_env : e->stuff_ctas, n), kStuffThreads, 0, st>>>(sl.d_tabs, sl.d_state, sl.d_scan, e->scan_cap_words, sl.d_chunk_ff,
-                                                                      e->chunks_cap, sl.d_out, (long long)e->out_cap, (long long)e->jpeg_cap);
+        stuff_kernel<<<dim3(kStuffCtas, n), kStuffThreads, 0, st>>>(sl.d_tabs, sl.d_state, sl.d_scan, e->scan_cap_words, sl.d_chunk_ff,
+                                                                    e->chunks_cap, sl.d_out, (long long)e->out_cap, (long long)e->jpeg_cap);
         e->launches++;
     }
     CU(e, cudaGetLastError());
@@ -635,7 +621,6 @@ int h2j_create(const h2j_settings *s, h2j_encoder **out)
         CUB(cudaMalloc(&e->d_comment, e->comment.size() + 1));
         CUB(cudaMemcpy(e->d_comment, e->comment.c_str(), e->comment.size() + 1, cudaMemcpyHostToDevice));
     }
-    if (getenv("H2J_K2_EXTRA_SMEM")) CUB(cudaFuncSetAttribute(fdct_quant_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
     CUB(cudaFuncSetAttribute(entropy_walk_kernel<kFmt420>, cudaFuncAttributeMaxDynamicSharedMemorySize, ent_smem_bytes(kFmt420)));
     CUB(cudaFuncSetAttribute(entropy_walk_kernel<kFmt422>, cudaFuncAttributeMaxDynamicSharedMemorySize, ent_smem_bytes(kFmt422)));
     CUB(cudaFuncSetAttribute(entropy_walk_kernel<kFmt444>, cudaFuncAttributeMaxDynamicSharedMemorySize, ent_smem_bytes(kFmt444)));
@@ -729,8 +714,7 @@ int h2j_submit_device_semiplanar(h2j_encoder *e, int slot, const uint8_t *d_fram
     // Rows on 8-byte boundaries (what decoders produce): the pipeline reads the frames where they are -- K1 only looks at
     // luma, K2's chroma roles fetch the pairs and keep their component in registers.  Otherwise the pairs are split into
     // the slot's planar frame buffer first (one more pass over the frame).
-    static const bool force_prepass = getenv("H2J_NV12_PREPASS") != nullptr;  // measurement knob
-    if (!force_prepass && !e->force_sp_prepass && (uintptr_t)d_frames % 8 == 0 && frame_stride % 8 == 0 && pitch % 8 == 0 && uv_offset % 8 == 0) {
+    if (!e->force_sp_prepass && (uintptr_t)d_frames % 8 == 0 && frame_stride % 8 == 0 && pitch % 8 == 0 && uv_offset % 8 == 0) {
         FrameLayout &L = sl.L;
         L.y_pitch = pitch;
         L.c_pitch = pitch;
@@ -987,8 +971,7 @@ int h2j_encode_frame(h2j_encoder *e, const uint8_t *const planes[3], const int s
             }
             return at.type == cudaMemoryTypeHost;
         };
-        static const bool no_direct = getenv("H2J_NO_DIRECT_UPLOAD") != nullptr;  // measurement knob
-        if (!no_direct && pinned(planes[0]) && pinned(planes[1]) && pinned(planes[2])) {
+        if (pinned(planes[0]) && pinned(planes[1]) && pinned(planes[2])) {
             CU(e, cudaMemcpy2DAsync(sl.d_frames, L.y_pitch, planes[0], strides[0], width, height, cudaMemcpyHostToDevice, sl.stream));
             CU(e, cudaMemcpy2DAsync(sl.d_frames + L.u_off, L.c_pitch, planes[1], strides[1], fcw, fch, cudaMemcpyHostToDevice, sl.stream));
             CU(e, cudaMemcpy2DAsync(sl.d_frames + L.v_off, L.c_pitch, planes[2], strides[2], fcw, fch, cudaMemcpyHostToDevice, sl.stream));

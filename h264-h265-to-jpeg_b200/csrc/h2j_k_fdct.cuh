@@ -25,17 +25,10 @@
 #pragma once
 #include "h2j_common.cuh"
 
-#ifndef H2J_K2_WALK
-#define H2J_K2_WALK 2  // positions the statistics walk takes per trip from the low end (0: the two-ended walk).  K2 per 2048 frames:
-                      // two-ended 5.538 ms, 2 per trip 5.511, 3 per trip 5.592, 4 per trip 5.626 (absent positions are predicated off)
-#endif
-#ifndef H2J_FDCT_MIN_CTAS
-#define H2J_FDCT_MIN_CTAS 16  // resident single-warp CTAs per SM the register allocation is bounded for (16 -> 128 registers)
-#endif
-
 namespace h2j {
 
-constexpr int kHistDummy = 257;  // s_hist: where the statistics walk counts a level that is not there (count_if)
+constexpr int kFdctMinCtas = 16;  // resident single-warp CTAs per SM the register allocation is bounded for (16 -> 128 registers)
+constexpr int kHistDummy = 257;   // s_hist: where the statistics walk counts a level that is not there (count_if)
 
 // What a thread needs to know about the plane its block lives in: fixed for the whole kernel.
 struct PlaneRef {
@@ -141,33 +134,43 @@ __device__ __forceinline__ void nv12_trade(BlockFetch &F, bool cr_lane)
     }
 }
 
-template <bool C>
-__device__ __forceinline__ void fetch_consume(const BlockFetch &F, const PlaneRef &R, const BlockPos &bp, const uint8_t *lut, int (&v)[64])
+// The block's 64 samples from its eight rows of eight bytes (`rows`, as fetched or with the component's bytes picked out),
+// then re-read bytewise with sample(row pointer, c) where the vector rows are not the block's (`fast` false), then through
+// the range LUT.
+template <class Sample>
+__device__ __forceinline__ void unpack_block(const uint2 (&rows)[8], bool fast, const PlaneRef &R, const BlockPos &bp, Sample sample,
+                                             const uint8_t *lut, int (&v)[64])
 {
 #pragma unroll
     for (int r = 0; r < 8; r++) {
         // one byte permute per sample (selector 4 = a zero byte of the second operand)
-        v[r * 8 + 0] = (int)__byte_perm(F.rows[r].x, 0u, 0x4440);
-        v[r * 8 + 1] = (int)__byte_perm(F.rows[r].x, 0u, 0x4441);
-        v[r * 8 + 2] = (int)__byte_perm(F.rows[r].x, 0u, 0x4442);
-        v[r * 8 + 3] = (int)__byte_perm(F.rows[r].x, 0u, 0x4443);
-        v[r * 8 + 4] = (int)__byte_perm(F.rows[r].y, 0u, 0x4440);
-        v[r * 8 + 5] = (int)__byte_perm(F.rows[r].y, 0u, 0x4441);
-        v[r * 8 + 6] = (int)__byte_perm(F.rows[r].y, 0u, 0x4442);
-        v[r * 8 + 7] = (int)__byte_perm(F.rows[r].y, 0u, 0x4443);
+        v[r * 8 + 0] = (int)__byte_perm(rows[r].x, 0u, 0x4440);
+        v[r * 8 + 1] = (int)__byte_perm(rows[r].x, 0u, 0x4441);
+        v[r * 8 + 2] = (int)__byte_perm(rows[r].x, 0u, 0x4442);
+        v[r * 8 + 3] = (int)__byte_perm(rows[r].x, 0u, 0x4443);
+        v[r * 8 + 4] = (int)__byte_perm(rows[r].y, 0u, 0x4440);
+        v[r * 8 + 5] = (int)__byte_perm(rows[r].y, 0u, 0x4441);
+        v[r * 8 + 6] = (int)__byte_perm(rows[r].y, 0u, 0x4442);
+        v[r * 8 + 7] = (int)__byte_perm(rows[r].y, 0u, 0x4443);
     }
-    if (!fetch_is_fast<C>(R, bp.bx)) {
+    if (!fast) {
 #pragma unroll
         for (int r = 0; r < 8; r++) {
             const uint8_t *row = R.P + (long long)min(bp.by + r, R.ph - 1) * R.pitch;
 #pragma unroll
-            for (int c = 0; c < 8; c++) v[r * 8 + c] = sample_at<C>(row, R, bp.bx, c);
+            for (int c = 0; c < 8; c++) v[r * 8 + c] = sample(row, c);
         }
     }
     if (lut) {
 #pragma unroll
         for (int i = 0; i < 64; i++) v[i] = lut[v[i]];
     }
+}
+
+template <bool C>
+__device__ __forceinline__ void fetch_consume(const BlockFetch &F, const PlaneRef &R, const BlockPos &bp, const uint8_t *lut, int (&v)[64])
+{
+    unpack_block(F.rows, fetch_is_fast<C>(R, bp.bx), R, bp, [&](const uint8_t *row, int c) { return sample_at<C>(row, R, bp.bx, c); }, lut, v);
 }
 
 // this lane's share (one pixel row) of the predecessor block's sample sum
@@ -189,13 +192,125 @@ __device__ __forceinline__ int fetch_pred_rowsum(const BlockFetch &F, const Plan
     return s;
 }
 
-#ifdef H2J_FDCT_MAXNREG  // experiment: an explicit register cap instead of the bound derived from resident CTAs
-#define H2J_FDCT_BOUNDS __maxnreg__(H2J_FDCT_MAXNREG)
-#else
-#define H2J_FDCT_BOUNDS __launch_bounds__(kFdctThreads, H2J_FDCT_MIN_CTAS)
-#endif
+// ---- the per-block core of both K2 kernels (fdct_quant_kernel, fdct_quant_fmt_kernel) ----
+
+// the frame's quantiser (set up once per frame by K1's last CTA) into shared memory, the CTA's statistics cleared
+__device__ __forceinline__ void k2_setup(const FrameTab &tab, int *s_q, int *s_bq, unsigned int *s_hist, unsigned int *s_dchist, int lane)
+{
+    const uint2 pk = reinterpret_cast<const uint2 *>(tab.qpack)[lane];
+    s_q[2 * lane] = (int)(pk.x & 0xffffu);
+    s_bq[2 * lane] = (int)(pk.x >> 16);
+    s_q[2 * lane + 1] = (int)(pk.y & 0xffffu);
+    s_bq[2 * lane + 1] = (int)(pk.y >> 16);
+#pragma unroll
+    for (int i = 0; i < 8; i++) s_hist[i * 32 + lane] = 0;
+    if (lane < 16) s_dchist[lane] = 0;
+    __syncwarp();
+}
+
+// Transform, quantise, zigzag and pack the block's samples into its record `rec` of the sub-image `img` (h2j_common.cuh).
+// Returns the quantised DC; its difference goes into the low half of word 0 later (count_block_symbols), the high half of
+// word 0 is left in word0_hi.
+__device__ __forceinline__ int quantise_record(int (&v)[64], const int *s_q, const int *s_bq, uint32_t *rec, uint32_t *img, int lane,
+                                               unsigned &mask_lo, unsigned &mask_hi, uint32_t &word0_hi)
+{
+    fdct_8x8(v);
+    const int dc = quant_dc(v[0]);
+    // quantise without the final >> 16: the level is the upper half of the 32-bit product, so two of them
+    // are packed into one record word with a single byte permute
+#pragma unroll
+    for (int i = 1; i < 64; i++) v[i] = quant_ac2_hi(v[i], s_q[i], s_bq[i]);
+    // zigzag; word j of the record holds levels j (low half) and j + 32 (high half), so that the non-zero
+    // flags of 32 levels fall out of 16 packed min(x, 1) results shifted into place (VIMNMX.U16x2)
+    unsigned fa = 0, fb = 0;
+#pragma unroll
+    for (int j = 0; j < 32; j++) {
+        const uint32_t w = j == 0 ? __byte_perm(0u, (uint32_t)v[zz_of(32)], 0x7610) : __byte_perm((uint32_t)v[zz_of(j)], (uint32_t)v[zz_of(j + 32)], 0x7632);
+        const unsigned t = __vminu2(w, 0x00010001u);
+        if (j < 16) fa += t << j;
+        else fb += t << (j - 16);
+        if (j == 0) word0_hi = w;  // the low half becomes the DC difference
+        else rec[j] = w;
+    }
+    mask_lo = ((fa & 0xffffu) | (fb << 16)) & ~1u;  // bit 0 is the DC position: always coded, never in the mask
+    mask_hi = (fa >> 16) | (fb & 0xffff0000u);
+    rec[kMaskLoWord] = mask_lo;
+    img[kSubMaskHiOff + lane] = mask_hi;
+    return dc;
+}
+
+// Completes the record with the DC difference to the previous block of the same component (mjpegenc.c encode_block) and
+// counts the block's DC and AC symbols (ff_mjpeg_encode_coef / record_block) into the CTA's histograms.
+__device__ __forceinline__ void count_block_symbols(uint32_t *rec, int diff, uint32_t word0_hi, unsigned mask_lo, unsigned mask_hi,
+                                                    unsigned int *s_hist, unsigned int *s_dchist)
+{
+    rec[0] = (uint32_t)(diff & 0xffff) | word0_hi;
+    atomicAdd(&s_dchist[mag_bits(diff)], 1u);
+    // The (run, size) symbol of a non-zero level needs only its position, the position of the non-zero level below it and
+    // its value, so the levels can be visited in any order.  Positions 1..31 (where nearly all of them are) are taken two
+    // at a time from the low end: two independent bit-scan -> load -> size -> atomic chains per trip instead of one, half
+    // the trips (three or four per trip, and two from opposite ends, measured slower: DESIGN.md section 4).
+    const int16_t *lv = reinterpret_cast<const int16_t *>(rec);
+    unsigned zrl = 0;  // 16-zero runs (symbol 0xF0): summed here, one update per block
+    auto count = [&](int k, int below, int val) {  // val != 0
+        const int run = k - below - 1;
+        unsigned top;  // size - 1: the + 1 rides in the address (size <= 15, no carry into the run nibble)
+        asm("bfind.u32 %0, %1;" : "=r"(top) : "r"(abs(val)));
+        zrl += (unsigned)run >> 4;
+        atomicAdd(&s_hist[1 + (((run & 15) << 4) | (int)top)], 1u);
+    };
+    // the same for a level a lane may not have, WITHOUT a branch: in a walking warp some lane has it, so the warp ran the
+    // branch's body anyway plus the branch and its reconvergence point (K2 5.458 -> 5.376 ms per 2048 frames); a lane
+    // without the level counts into a word nobody reads
+    auto count_if = [&](bool have, int k, int below, int val) {
+        const int run = k - below - 1;
+        unsigned top;
+        asm("bfind.u32 %0, %1;" : "=r"(top) : "r"(abs(val)));
+        zrl += have ? (unsigned)run >> 4 : 0u;
+        atomicAdd(&s_hist[have ? 1 + (((run & 15) << 4) | (int)top) : kHistDummy], 1u);
+    };
+    unsigned lo = mask_lo;
+    const int top_lo = lo ? 31 - __clz(lo) : 0;  // highest non-zero position below 32 (0: none but the DC)
+    int below = 0;
+    while (lo) {
+        const unsigned b0 = lo & (0u - lo);
+        lo ^= b0;
+        const unsigned b1 = lo & (0u - lo);
+        lo ^= b1;
+        const int k0 = 31 - __clz(b0), k1 = 31 - __clz(b1);  // k1 = -1: absent
+        const int v0 = (int)lv[2 * k0], v1 = (int)lv[2 * max(k1, 0)];
+        count(k0, below, v0);
+        count_if(b1 != 0, k1, k0, v1);
+        below = 31 - __clz(b0 | b1);
+    }
+    int prev = top_lo;
+    unsigned hi = mask_hi;
+    while (hi) {
+        const int bp = __ffs((int)hi) - 1, k = 32 + bp;
+        hi &= hi - 1;
+        count(k, prev, (int)lv[2 * bp + 1]);
+        prev = k;
+    }
+    if (prev < 63) atomicAdd(&s_hist[0], 1u);
+    if (zrl) atomicAdd(&s_hist[0xf0], zrl);
+}
+
+// the CTA's statistics into the frame's histograms (class 0 luma, 1 chroma)
+__device__ __forceinline__ void k2_flush(FrameState &st, int cls, const unsigned int *s_hist, const unsigned int *s_dchist, int lane)
+{
+#pragma unroll
+    for (int i = 0; i < 8; i++) {
+        const unsigned c = s_hist[i * 32 + lane];
+        if (c) atomicAdd(&st.hist[2 + cls][i * 32 + lane], c);
+    }
+    if (lane < 16) {
+        const unsigned c = s_dchist[lane];
+        if (c) atomicAdd(&st.hist[cls][lane], c);
+    }
+}
+
 template <bool NV12>
-__global__ void H2J_FDCT_BOUNDS fdct_quant_kernel(const uint8_t *__restrict__ frames, FrameLayout L,
+__global__ void __launch_bounds__(kFdctThreads, kFdctMinCtas) fdct_quant_kernel(const uint8_t *__restrict__ frames, FrameLayout L,
                                                                      FrameState *__restrict__ state,
                                                                      const FrameTab *__restrict__ tabs,
                                                                      uint32_t *__restrict__ images,  // [frame][images_cap] tile images
@@ -239,18 +354,7 @@ __global__ void H2J_FDCT_BOUNDS fdct_quant_kernel(const uint8_t *__restrict__ fr
     if (nvc) fetch_issue<true, true>(F, safe, R, bp, bp.m < L.n_mcu, Q, pp, phelp_at(tile0), lane & 7);
     else fetch_issue<false, false>(F, safe, R, bp, bp.m < L.n_mcu, Q, pp, phelp_at(tile0), lane & 7);
 
-    // ---- the frame's quantiser (set up once per frame by K1's last CTA), cleared statistics ----
-    {
-        const uint2 pk = reinterpret_cast<const uint2 *>(tabs[f].qpack)[lane];
-        s_q[2 * lane] = (int)(pk.x & 0xffffu);
-        s_bq[2 * lane] = (int)(pk.x >> 16);
-        s_q[2 * lane + 1] = (int)(pk.y & 0xffffu);
-        s_bq[2 * lane + 1] = (int)(pk.y >> 16);
-    }
-#pragma unroll
-    for (int i = 0; i < 8; i++) s_hist[i * 32 + lane] = 0;
-    if (lane < 16) s_dchist[lane] = 0;
-    __syncwarp();
+    k2_setup(tabs[f], s_q, s_bq, s_hist, s_dchist, lane);
 
     int chroma_carry = 128;  // chroma warp, lanes 0 / 16: DC of the previous tile's last Cb / Cr block
 
@@ -283,28 +387,7 @@ __global__ void H2J_FDCT_BOUNDS fdct_quant_kernel(const uint8_t *__restrict__ fr
             int v[64];
             if (nvc) fetch_consume<true>(F, R, bp, lut, v);
             else fetch_consume<false>(F, R, bp, lut, v);
-            fdct_8x8(v);
-            dc = quant_dc(v[0]);
-            // quantise without the final >> 16: the level is the upper half of the 32-bit product, so two of them
-            // are packed into one record word with a single byte permute
-#pragma unroll
-            for (int i = 1; i < 64; i++) v[i] = quant_ac2_hi(v[i], s_q[i], s_bq[i]);
-            // zigzag; word j of the record holds levels j (low half) and j + 32 (high half), so that the non-zero
-            // flags of 32 levels fall out of 16 packed min(x, 1) results shifted into place (VIMNMX.U16x2)
-            unsigned fa = 0, fb = 0;
-#pragma unroll
-            for (int j = 0; j < 32; j++) {
-                const uint32_t w = j == 0 ? __byte_perm(0u, (uint32_t)v[zz_of(32)], 0x7610) : __byte_perm((uint32_t)v[zz_of(j)], (uint32_t)v[zz_of(j + 32)], 0x7632);
-                const unsigned t = __vminu2(w, 0x00010001u);
-                if (j < 16) fa += t << j;
-                else fb += t << (j - 16);
-                if (j == 0) word0_hi = w;  // the low half becomes the DC difference below
-                else rec[j] = w;
-            }
-            mask_lo = ((fa & 0xffffu) | (fb << 16)) & ~1u;  // bit 0 is the DC position: always coded, never in the mask
-            mask_hi = (fa >> 16) | (fb & 0xffff0000u);
-            rec[kMaskLoWord] = mask_lo;
-            img[kSubMaskHiOff + lane] = mask_hi;
+            dc = quantise_record(v, s_q, s_bq, rec, img, lane, mask_lo, mask_hi, word0_hi);
         }
 
         // ---- request the next tile's pixels: nothing of this tile's 64-value block is live any more ----
@@ -320,88 +403,7 @@ __global__ void H2J_FDCT_BOUNDS fdct_quant_kernel(const uint8_t *__restrict__ fr
         const int pred = (luma ? lane == 0 : (lane & 15) == 0) ? pred_first : up;
         const int last = __shfl_sync(0xffffffffu, dc, (lane & 16) | 15);  // chroma: this tile's last Cb / Cr
         chroma_carry = last;
-        if (valid) {
-            const int diff = dc - pred;
-            rec[0] = (uint32_t)(diff & 0xffff) | word0_hi;
-            atomicAdd(&s_dchist[mag_bits(diff)], 1u);
-            // ---- AC symbol statistics (ff_mjpeg_encode_coef / record_block, AC part) ----
-            // The (run, size) symbol of a non-zero level needs only its position, the position of the non-zero level
-            // below it and its value, so the levels can be visited in any order.  Positions 1..31 (where nearly all of
-            // them are) are taken two at a time: two independent bit-scan -> load -> size -> atomic chains per
-            // iteration instead of one, half the trips.
-            const int16_t *lv = reinterpret_cast<const int16_t *>(rec);
-            unsigned int *hist = s_hist;
-            unsigned zrl = 0;  // 16-zero runs (symbol 0xF0): summed here, one update per block
-            auto count = [&](int k, int below, int val) {  // val != 0
-                const int run = k - below - 1;
-                unsigned top;  // size - 1: the + 1 rides in the address (size <= 15, no carry into the run nibble)
-                asm("bfind.u32 %0, %1;" : "=r"(top) : "r"(abs(val)));
-                zrl += (unsigned)run >> 4;
-                atomicAdd(&hist[1 + (((run & 15) << 4) | (int)top)], 1u);
-            };
-            // the same for a level a lane may not have, WITHOUT a branch: in a walking warp some lane has it, so the warp ran
-            // the branch's body anyway plus the branch and its reconvergence point (K2 5.458 -> 5.376 ms per 2048 frames); a lane
-            // without the level counts into a word nobody reads
-            auto count_if = [&](bool have, int k, int below, int val) {
-                const int run = k - below - 1;
-                unsigned top;
-                asm("bfind.u32 %0, %1;" : "=r"(top) : "r"(abs(val)));
-                zrl += have ? (unsigned)run >> 4 : 0u;
-                atomicAdd(&hist[have ? 1 + (((run & 15) << 4) | (int)top) : kHistDummy], 1u);
-            };
-            unsigned lo = mask_lo;
-            const int top_lo = lo ? 31 - __clz(lo) : 0;  // highest non-zero position below 32 (0: none but the DC)
-#if H2J_K2_WALK
-            // H2J_K2_WALK positions per trip, taken from the low end, without a branch inside: the chains (position -> level
-            // -> size -> histogram) are independent, the ones a lane does not have are predicated off
-            int below = 0;
-            while (lo) {
-                const unsigned b0 = lo & (0u - lo);
-                lo ^= b0;
-                const unsigned b1 = lo & (0u - lo);
-                lo ^= b1;
-                const unsigned b2 = H2J_K2_WALK >= 3 ? lo & (0u - lo) : 0u;
-                lo ^= b2;
-                const unsigned b3 = H2J_K2_WALK >= 4 ? lo & (0u - lo) : 0u;
-                lo ^= b3;
-                const int k0 = 31 - __clz(b0), k1 = 31 - __clz(b1), k2 = 31 - __clz(b2), k3 = 31 - __clz(b3);  // -1: absent
-                const int v0 = (int)lv[2 * k0], v1 = (int)lv[2 * max(k1, 0)];
-                count(k0, below, v0);
-                count_if(b1 != 0, k1, k0, v1);
-                if (H2J_K2_WALK >= 3) count_if(b2 != 0, k2, k1, (int)lv[2 * max(k2, 0)]);
-                if (H2J_K2_WALK >= 4) count_if(b3 != 0, k3, k2, (int)lv[2 * max(k3, 0)]);
-                below = 31 - __clz(b0 | b1 | b2 | b3);
-            }
-#else
-            int below_a = 0;   // ascending end: the non-zero position below the next one taken
-            int kb = top_lo;   // descending end: the highest position still in `lo`
-            while (lo) {
-                const unsigned bit_a = lo & (0u - lo);
-                const int ka = 31 - __clz(bit_a);
-                lo ^= bit_a;
-                const int val_a = (int)lv[2 * ka];
-                if (lo) {  // ka was not the last one: kb is a different position
-                    lo ^= 1u << kb;
-                    const int val_b = (int)lv[2 * kb];
-                    const int below_b = lo ? 31 - __clz(lo) : ka;  // next one down, or the one the other end just took
-                    count(kb, below_b, val_b);
-                    kb = below_b;
-                }
-                count(ka, below_a, val_a);
-                below_a = ka;
-            }
-#endif
-            int prev = top_lo;
-            unsigned hi = mask_hi;
-            while (hi) {
-                const int bp = __ffs((int)hi) - 1, k = 32 + bp;
-                hi &= hi - 1;
-                count(k, prev, (int)lv[2 * bp + 1]);
-                prev = k;
-            }
-            if (prev < 63) atomicAdd(&hist[0], 1u);
-            if (zrl) atomicAdd(&hist[0xf0], zrl);
-        }
+        if (valid) count_block_symbols(rec, dc - pred, word0_hi, mask_lo, mask_hi, s_hist, s_dchist);
 
         // ---- the warp's sub-image leaves with one bulk store ----
         fence_proxy_async_smem();
@@ -413,16 +415,7 @@ __global__ void H2J_FDCT_BOUNDS fdct_quant_kernel(const uint8_t *__restrict__ fr
     // kernel boundary orders them before K4a
     if (lane == 0) bulk_wait_read_all();
     __syncwarp();
-
-#pragma unroll
-    for (int i = 0; i < 8; i++) {
-        const unsigned c = s_hist[i * 32 + lane];
-        if (c) atomicAdd(&state[f].hist[2 + cls][i * 32 + lane], c);
-    }
-    if (lane < 16) {
-        const unsigned c = s_dchist[lane];
-        if (c) atomicAdd(&state[f].hist[cls][lane], c);
-    }
+    k2_flush(state[f], cls, s_hist, s_dchist, lane);
 }
 
 }  // namespace h2j

@@ -1,7 +1,8 @@
 // K2 for the encoder's other MCU geometries (DESIGN.md row f3): 4:2:2 and 4:4:4 frames (planar, as libavcodec's decoders
-// hand them over: yuv422p / yuv444p).  Same work per block as fdct_quant_kernel -- pixel load with edge replication (+ range
-// LUT), ff_fdct_sse2, quantise, zigzag, DC prediction by warp shuffle, symbol statistics, the role's sub-image of the tile
-// image sent with one bulk store -- and the same helpers (h2j_k_fdct.cuh); what differs is who does what:
+// hand them over: yuv422p / yuv444p).  The per-block work is fdct_quant_kernel's, with its helpers (h2j_k_fdct.cuh): the
+// planar fetch and unpack with edge replication (+ range LUT), the quantiser set-up, transform + quantise + zigzag into the
+// tile-image record (quantise_record), DC difference and symbol statistics (count_block_symbols), the histogram flush; the
+// role's sub-image of the tile image leaves with one bulk store.  What differs is who does what:
 //   4:2:2  16x16 MCUs of Y0 Y1 Y2 Y3 Cb0 Cb1 Cr0 Cr1; four roles per 16-MCU tile: luma of MCUs 0-7 (lane = mcu * 4 + n), luma
 //          of MCUs 8-15, Cb of the 16 MCUs (lane = mcu * 2 + n: top, bottom), Cr
 //   4:4:4   8x16 MCUs of Y0 Y1 Cb0 Cb1 Cr0 Cr1 (every component top, bottom); three roles: Y (lane = mcu * 2 + n), Cb, Cr
@@ -85,30 +86,10 @@ __device__ __forceinline__ void sp_fetch_consume(const BlockFetch &F, const Pair
                                                  const uint8_t *lut, int (&v)[64])
 {
     const unsigned sel = odd ? 0x7531u : 0x6420u;  // the Cr / Cb byte of four pairs
+    uint2 rows[8];
 #pragma unroll
-    for (int r = 0; r < 8; r++) {
-        const unsigned lo4 = __byte_perm(F.rows[r].x, F.rows[r].y, sel), hi4 = __byte_perm(H.hi[r].x, H.hi[r].y, sel);
-        v[r * 8 + 0] = (int)__byte_perm(lo4, 0u, 0x4440);
-        v[r * 8 + 1] = (int)__byte_perm(lo4, 0u, 0x4441);
-        v[r * 8 + 2] = (int)__byte_perm(lo4, 0u, 0x4442);
-        v[r * 8 + 3] = (int)__byte_perm(lo4, 0u, 0x4443);
-        v[r * 8 + 4] = (int)__byte_perm(hi4, 0u, 0x4440);
-        v[r * 8 + 5] = (int)__byte_perm(hi4, 0u, 0x4441);
-        v[r * 8 + 6] = (int)__byte_perm(hi4, 0u, 0x4442);
-        v[r * 8 + 7] = (int)__byte_perm(hi4, 0u, 0x4443);
-    }
-    if (!sp_is_fast(R, bp.bx)) {
-#pragma unroll
-        for (int r = 0; r < 8; r++) {
-            const uint8_t *row = R.P + (long long)min(bp.by + r, R.ph - 1) * R.pitch;
-#pragma unroll
-            for (int c = 0; c < 8; c++) v[r * 8 + c] = sp_sample_at(row, R, bp.bx, c, odd);
-        }
-    }
-    if (lut) {
-#pragma unroll
-        for (int i = 0; i < 64; i++) v[i] = lut[v[i]];
-    }
+    for (int r = 0; r < 8; r++) rows[r] = make_uint2(__byte_perm(F.rows[r].x, F.rows[r].y, sel), __byte_perm(H.hi[r].x, H.hi[r].y, sel));
+    unpack_block(rows, sp_is_fast(R, bp.bx), R, bp, [&](const uint8_t *row, int c) { return sp_sample_at(row, R, bp.bx, c, odd); }, lut, v);
 }
 
 // this lane's share (one pixel row) of the predecessor block's sample sum
@@ -131,7 +112,7 @@ __device__ __forceinline__ int sp_pred_rowsum(const BlockFetch &F, const PairHal
 }
 
 template <int FMT, bool SP>
-__global__ void __launch_bounds__(kFdctThreads, H2J_FDCT_MIN_CTAS) fdct_quant_fmt_kernel(const uint8_t *__restrict__ frames, FrameLayout L,
+__global__ void __launch_bounds__(kFdctThreads, kFdctMinCtas) fdct_quant_fmt_kernel(const uint8_t *__restrict__ frames, FrameLayout L,
                                                                          FrameState *__restrict__ state,
                                                                          const FrameTab *__restrict__ tabs,
                                                                          uint32_t *__restrict__ images,  // [frame][images_cap] tile images
@@ -177,17 +158,7 @@ __global__ void __launch_bounds__(kFdctThreads, H2J_FDCT_MIN_CTAS) fdct_quant_fm
     if (spc) sp_fetch_issue(F, H, safe, R, bp, bp.m < L.n_mcu, Q, pp, phelp_now(), lane & 7);
     else fetch_issue<false, false>(F, safe, R, bp, bp.m < L.n_mcu, Q, pp, phelp_now(), lane & 7);
 
-    {
-        const uint2 pk = reinterpret_cast<const uint2 *>(tabs[f].qpack)[lane];
-        s_q[2 * lane] = (int)(pk.x & 0xffffu);
-        s_bq[2 * lane] = (int)(pk.x >> 16);
-        s_q[2 * lane + 1] = (int)(pk.y & 0xffffu);
-        s_bq[2 * lane + 1] = (int)(pk.y >> 16);
-    }
-#pragma unroll
-    for (int i = 0; i < 8; i++) s_hist[i * 32 + lane] = 0;
-    if (lane < 16) s_dchist[lane] = 0;
-    __syncwarp();
+    k2_setup(tabs[f], s_q, s_bq, s_hist, s_dchist, lane);
 
     for (int tile = tile0; tile < tile_end; tile++) {
         uint32_t *img = s_img[(tile - tile0) & 1];
@@ -211,24 +182,7 @@ __global__ void __launch_bounds__(kFdctThreads, H2J_FDCT_MIN_CTAS) fdct_quant_fm
             int v[64];
             if (spc) sp_fetch_consume(F, H, R, bp, odd, lut, v);
             else fetch_consume<false>(F, R, bp, lut, v);
-            fdct_8x8(v);
-            dc = quant_dc(v[0]);
-#pragma unroll
-            for (int i = 1; i < 64; i++) v[i] = quant_ac2_hi(v[i], s_q[i], s_bq[i]);
-            unsigned fa = 0, fb = 0;
-#pragma unroll
-            for (int j = 0; j < 32; j++) {
-                const uint32_t w = j == 0 ? __byte_perm(0u, (uint32_t)v[zz_of(32)], 0x7610) : __byte_perm((uint32_t)v[zz_of(j)], (uint32_t)v[zz_of(j + 32)], 0x7632);
-                const unsigned t = __vminu2(w, 0x00010001u);
-                if (j < 16) fa += t << j;
-                else fb += t << (j - 16);
-                if (j == 0) word0_hi = w;
-                else rec[j] = w;
-            }
-            mask_lo = ((fa & 0xffffu) | (fb << 16)) & ~1u;
-            mask_hi = (fa >> 16) | (fb & 0xffff0000u);
-            rec[kMaskLoWord] = mask_lo;
-            img[kSubMaskHiOff + lane] = mask_hi;
+            dc = quantise_record(v, s_q, s_bq, rec, img, lane, mask_lo, mask_hi, word0_hi);
         }
 
         // ---- request the next tile's pixels ----
@@ -242,51 +196,7 @@ __global__ void __launch_bounds__(kFdctThreads, H2J_FDCT_MIN_CTAS) fdct_quant_fm
         // ---- DC difference to the previous block of the component (mjpegenc.c record_block) ----
         const int up = __shfl_up_sync(0xffffffffu, dc, 1);
         const int pred = lane == 0 ? pred_first : up;
-        if (valid) {
-            const int diff = dc - pred;
-            rec[0] = (uint32_t)(diff & 0xffff) | word0_hi;
-            atomicAdd(&s_dchist[mag_bits(diff)], 1u);
-            // ---- AC symbol statistics: as in fdct_quant_kernel, two positions per trip from the low end ----
-            const int16_t *lv = reinterpret_cast<const int16_t *>(rec);
-            unsigned zrl = 0;
-            auto count = [&](int kk, int below, int val) {
-                const int run = kk - below - 1;
-                unsigned top;
-                asm("bfind.u32 %0, %1;" : "=r"(top) : "r"(abs(val)));
-                zrl += (unsigned)run >> 4;
-                atomicAdd(&s_hist[1 + (((run & 15) << 4) | (int)top)], 1u);
-            };
-            unsigned lo = mask_lo;
-            const int top_lo = lo ? 31 - __clz(lo) : 0;
-            int below = 0;
-            while (lo) {
-                const unsigned b0 = lo & (0u - lo);
-                lo ^= b0;
-                const unsigned b1 = lo & (0u - lo);
-                lo ^= b1;
-                const int k0 = 31 - __clz(b0), k1 = 31 - __clz(b1);
-                const int v0 = (int)lv[2 * k0], v1 = (int)lv[2 * max(k1, 0)];
-                count(k0, below, v0);
-                {  // a level the lane may not have, without a branch (fdct_quant_kernel's count_if): counted into a word nobody reads
-                    const int run = k1 - k0 - 1;
-                    unsigned top;
-                    asm("bfind.u32 %0, %1;" : "=r"(top) : "r"(abs(v1)));
-                    zrl += b1 ? (unsigned)run >> 4 : 0u;
-                    atomicAdd(&s_hist[b1 ? 1 + (((run & 15) << 4) | (int)top) : kHistDummy], 1u);
-                }
-                below = 31 - __clz(b0 | b1);
-            }
-            int prev = top_lo;
-            unsigned hi = mask_hi;
-            while (hi) {
-                const int bpos = __ffs((int)hi) - 1, kk = 32 + bpos;
-                hi &= hi - 1;
-                count(kk, prev, (int)lv[2 * bpos + 1]);
-                prev = kk;
-            }
-            if (prev < 63) atomicAdd(&s_hist[0], 1u);
-            if (zrl) atomicAdd(&s_hist[0xf0], zrl);
-        }
+        if (valid) count_block_symbols(rec, dc - pred, word0_hi, mask_lo, mask_hi, s_hist, s_dchist);
 
         // ---- the role's sub-image leaves with one bulk store ----
         fence_proxy_async_smem();
@@ -296,16 +206,7 @@ __global__ void __launch_bounds__(kFdctThreads, H2J_FDCT_MIN_CTAS) fdct_quant_fm
     }
     if (lane == 0) bulk_wait_read_all();
     __syncwarp();
-
-#pragma unroll
-    for (int i = 0; i < 8; i++) {
-        const unsigned c = s_hist[i * 32 + lane];
-        if (c) atomicAdd(&state[f].hist[2 + cls][i * 32 + lane], c);
-    }
-    if (lane < 16) {
-        const unsigned c = s_dchist[lane];
-        if (c) atomicAdd(&state[f].hist[cls][lane], c);
-    }
+    k2_flush(state[f], cls, s_hist, s_dchist, lane);
 }
 
 }  // namespace h2j

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""Device-resident throughput of frames whose rows are not 8-byte aligned (1918x1078), with and without the copy to a
-16-byte row pitch (H2J_NO_REPITCH=1).  Run on the GPU box: python tools/oddsize_probe.py"""
+"""Device-resident throughput of frames whose rows are not 8-byte aligned (1918x1078); the library copies them to a
+16-byte row pitch first.  Run on the GPU box: python tools/oddsize_probe.py"""
 import os, sys, time, json
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path[:0] = [ROOT, os.path.join(ROOT, "h264-h265-to-jpeg_b200")]
@@ -18,4 +18,4 @@ with h2j_b200.Encoder(max_width=w, max_height=h, max_batch=n, n_slots=1) as e:
     for _ in range(5):
         e.submit_device(0, d.data_ptr(), stride, n, w, h); e.collect_device(0)
     torch.cuda.synchronize(); dt = (time.perf_counter() - t0) / 5
-print(json.dumps({"1918x1078_batch256_frames_per_s": round(n / dt), "no_repitch": bool(os.environ.get("H2J_NO_REPITCH"))}))
+print(json.dumps({"1918x1078_batch256_frames_per_s": round(n / dt)}))
