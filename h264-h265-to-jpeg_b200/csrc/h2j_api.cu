@@ -53,6 +53,8 @@ struct Slot {
     long long *h_sizes = nullptr;             // pinned (jpeg_bytes per frame)
     uint8_t *h_stage = nullptr;               // pinned staging for h2j_encode_frame / convert
     size_t h_stage_bytes = 0;
+    uint8_t *d_frames16 = nullptr;            // h2j_encode_frame16 (slot 0, allocated on its first call): the 16-bit planes ...
+    uint8_t *h_stage16 = nullptr;             // ... and their pinned staging
     unsigned char *h_tail = nullptr;          // pinned: status .. jpeg_bytes of frame 0's FrameTab (h2j_encode_frame)
     size_t spec_bytes = 384 * 1024;           // JPEG bytes h2j_encode_frame copies back before it knows the size
     bool busy = false;
@@ -263,6 +265,25 @@ int prepare_input(h2j_encoder *e, Slot &sl, const uint8_t *d_src, size_t src_str
     return repitch_if_unaligned(e, sl, d_src, src_end, n, pipe_src);
 }
 
+// High-bit-depth input: n frames at d_src (layout S; sp: semi-planar) -> 8-bit planar frames in the slot's frame buffer at
+// a 16-byte row pitch (frame_bytes_cap holds pitched_frame_bytes), in one launch for every layout and width.  On return
+// sl.L describes what the pipeline reads at sl.d_frames.
+int convert_depth(h2j_encoder *e, Slot &sl, const uint8_t *d_src, const Src16 &S, bool sp, int bit_depth, int n, int w, int h)
+{
+    int rc = make_layout(e, sl.d_frames, 0, w, h, &sl.L);
+    if (rc) return rc;
+    sl.L = pitched_layout(sl.L);
+    const int fch = chroma_h(h, sl.L.fmt);
+    const int row_words = sp ? std::max(w, 2 * chroma_w(w, sl.L.fmt)) : w;
+    const dim3 grid((row_words + 128 * 16 - 1) / (128 * 16), (h + (sp ? 1 : 2) * fch + kPlaneRowsPerCta - 1) / kPlaneRowsPerCta, n);
+    (sp ? depth_to_8_kernel<true> : depth_to_8_kernel<false>)<<<grid, 128, 0, sl.stream>>>(d_src, S, sl.d_frames, sl.L, bit_depth - 8);
+    e->launches++;
+    CU(e, cudaGetLastError());
+    return H2J_OK;
+}
+
+bool odd(size_t v) { return (v & 1) != 0; }
+
 struct ScopedTiming {
     Slot &sl;
     bool on;
@@ -471,11 +492,90 @@ int check_slot(h2j_encoder *e, int slot)
     return H2J_OK;
 }
 
+// Upload one picture's three planes (rows[i] rows of row_bytes[i] bytes, strides[i] apart in host memory) to dev + off[i]
+// at pitch[i] on the slot's stream.  Pageable planes go through `stage` (pinned, laid out as on the device) in pieces,
+// every piece uploaded as soon as it is in place, so that the DMA of one piece runs under the memcpy of the next.
+int upload_planes(h2j_encoder *e, Slot &sl, const uint8_t *const planes[3], const int strides[3], const int row_bytes[3], const int rows[3],
+                  const size_t off[3], const int pitch[3], uint8_t *dev, uint8_t *stage)
+{
+    constexpr int kMaxPieces = 96;
+    CopyPiece pieces[kMaxPieces];
+    int n_pieces = 0;
+    for (int p = 0; p < 3; p++) {
+        const int ph = rows[p];
+        // pieces of ~256 KiB, but never more than a third of the table per plane
+        int rows_per_piece = std::max(1, (256 * 1024) / pitch[p]);
+        rows_per_piece = std::max(rows_per_piece, (ph + kMaxPieces / 3 - 1) / (kMaxPieces / 3));
+        for (int r0 = 0; r0 < ph; r0 += rows_per_piece) {
+            const int r1 = std::min(ph, r0 + rows_per_piece);
+            CopyPiece &c = pieces[n_pieces++];
+            c.dst = stage + off[p] + (size_t)r0 * pitch[p];
+            c.src = planes[p] + (size_t)r0 * strides[p];
+            c.rows = r1 - r0;
+            c.row_bytes = row_bytes[p];
+            c.dst_pitch = pitch[p];
+            c.src_stride = strides[p];
+            c.dev_off = off[p] + (size_t)r0 * pitch[p];
+            c.dev_bytes = (size_t)(r1 - r0 - 1) * pitch[p] + row_bytes[p];
+        }
+    }
+    // Planes that already live in page-locked memory (h2j_alloc_pinned, cudaHostAlloc, cudaHostRegister by the caller -- a
+    // decoder whose frame buffers come from such a pool) are uploaded from where they are: no staging copy, one strided
+    // DMA per plane.  The host copy is three quarters of the call for pageable planes.
+    auto pinned = [](const void *p) {
+        cudaPointerAttributes at;
+        if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
+            cudaGetLastError();
+            return false;
+        }
+        return at.type == cudaMemoryTypeHost;
+    };
+    if (pinned(planes[0]) && pinned(planes[1]) && pinned(planes[2])) {
+        for (int p = 0; p < 3; p++)
+            CU(e, cudaMemcpy2DAsync(dev + off[p], pitch[p], planes[p], strides[p], row_bytes[p], rows[p], cudaMemcpyHostToDevice, sl.stream));
+        n_pieces = 0;
+    }
+    cudaError_t up_err = cudaSuccess;
+    for (int i = 0; i < n_pieces; i++) {
+        copy_piece(pieces[i]);
+        const cudaError_t ce = cudaMemcpyAsync(dev + pieces[i].dev_off, stage + pieces[i].dev_off, pieces[i].dev_bytes, cudaMemcpyHostToDevice, sl.stream);
+        if (ce != cudaSuccess && up_err == cudaSuccess) up_err = ce;
+    }
+    CU(e, up_err);
+    return H2J_OK;
+}
+
+// The single-picture pipeline (TAIL_SINGLE) is enqueued: wait for it and hand the JPEG over.
+int finish_single(h2j_encoder *e, Slot &sl, uint8_t *out, size_t out_capacity, size_t *out_size)
+{
+    CU(e, cudaStreamSynchronize(sl.stream));
+    int st = 0;
+    long long jpeg_bytes = 0;
+    memcpy(&st, sl.h_tail + (offsetof(FrameTab, status) - kTabTailOff), sizeof st);
+    memcpy(&jpeg_bytes, sl.h_tail + (offsetof(FrameTab, jpeg_bytes) - kTabTailOff), sizeof jpeg_bytes);
+    if (st != 0) return fail(e, st, "the frame failed: %s", h2j_status_string(st));
+    if (jpeg_bytes < 0 || (size_t)jpeg_bytes > e->jpeg_cap) return fail(e, H2J_ERR_OUTPUT_TOO_SMALL, "JPEG of %lld bytes exceeds max_jpeg_bytes", jpeg_bytes);
+    const size_t n_out = (size_t)jpeg_bytes;
+    *out_size = n_out;
+    if (n_out > out_capacity) return fail(e, H2J_ERR_OUTPUT_TOO_SMALL, "JPEG is %zu bytes, caller gave %zu", n_out, out_capacity);
+    const size_t spec = std::min(std::min(sl.spec_bytes, e->out_cap), sl.h_stage_bytes);
+    const size_t have = std::min(n_out, spec);
+    memcpy(out, sl.h_stage, have);
+    if (n_out > have) {  // the guess was short: the rest straight into the caller's buffer
+        CU(e, cudaMemcpy(out + have, sl.d_out + have, n_out - have, cudaMemcpyDeviceToHost));
+    }
+    // next guess: a quarter above this frame, in 64 KiB steps (consecutive frames of a stream are alike)
+    sl.spec_bytes = std::max<size_t>(64 * 1024, align_up(n_out + n_out / 4, 64 * 1024));
+    return H2J_OK;
+}
+
 void free_slot(Slot &sl)
 {
     if (sl.stream) cudaStreamSynchronize(sl.stream);
     cudaFree(sl.d_frames); cudaFree(sl.d_pitched); cudaFree(sl.d_images); cudaFree(sl.d_zero); cudaFree(sl.d_stage); cudaFree(sl.d_unit_info);
     cudaFree(sl.d_tabs); cudaFree(sl.d_scan); cudaFree(sl.d_out); cudaFree(sl.d_packed); cudaFree(sl.d_offsets); cudaFree(sl.d_status);
+    cudaFree(sl.d_frames16);
+    if (sl.h_stage16) cudaFreeHost(sl.h_stage16);
     if (sl.h_offsets) cudaFreeHost(sl.h_offsets);
     if (sl.h_status) cudaFreeHost(sl.h_status);
     if (sl.h_sizes) cudaFreeHost(sl.h_sizes);
@@ -794,6 +894,67 @@ int h2j_submit_device_pitched(h2j_encoder *e, int slot, const uint8_t *d_frames,
     return H2J_OK;
 }
 
+int h2j_submit_device_semiplanar16(h2j_encoder *e, int slot, const uint8_t *d_frames, size_t frame_stride, int pitch, size_t uv_offset,
+                                   int bit_depth, int n, int width, int height)
+{
+    int rc = check_slot(e, slot);
+    if (rc) return rc;
+    Slot &sl = e->slots[slot];
+    if (sl.busy) return fail(e, H2J_ERR_BUSY, "slot %d has a batch in flight", slot);
+    if (!d_frames || n < 1 || n > e->s.max_batch) return fail(e, H2J_ERR_INVALID_ARG, "bad frames pointer or batch size %d (max %d)", n, e->s.max_batch);
+    if (width < 2 || height < 2) return fail(e, H2J_ERR_UNSUPPORTED, "unsupported frame size %dx%d", width, height);
+    if (bit_depth < 9 || bit_depth > 16) return fail(e, H2J_ERR_INVALID_ARG, "bit_depth %d outside 9..16", bit_depth);
+    if (odd((uintptr_t)d_frames) || odd(frame_stride) || odd((size_t)pitch) || odd(uv_offset))
+        return fail(e, H2J_ERR_INVALID_ARG, "16-bit samples need even pointers, strides, pitches and offsets");
+    const int fmt = e->s.chroma_format;
+    const int fcw = chroma_w(width, fmt), fch = chroma_h(height, fmt);  // pairs per row, rows of the pair plane
+    if (pitch < 2 * std::max(width, 2 * fcw)) return fail(e, H2J_ERR_INVALID_ARG, "pitch %d smaller than a row of %d 16-bit words", pitch, std::max(width, 2 * fcw));
+    if (uv_offset < (size_t)pitch * height || frame_stride < uv_offset + (size_t)pitch * (fch - 1) + 4 * (size_t)fcw)
+        return fail(e, H2J_ERR_INVALID_ARG, "uv_offset / frame_stride do not hold a semi-planar frame of %dx%d at pitch %d", width, height, pitch);
+    ON_DEVICE(e);
+    sl.n = n;
+    CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
+    rc = convert_depth(e, sl, d_frames, Src16{(long long)frame_stride, (long long)uv_offset, (long long)uv_offset, pitch, pitch}, true, bit_depth, n,
+                       width, height);
+    if (rc) return rc;
+    rc = launch_pipeline(e, sl, sl.d_frames, n, TAIL_SIZES);
+    if (rc) return rc;
+    sl.busy = true;
+    return H2J_OK;
+}
+
+int h2j_submit_device_pitched16(h2j_encoder *e, int slot, const uint8_t *d_frames, size_t frame_stride, int y_pitch, int c_pitch,
+                                size_t u_offset, size_t v_offset, int bit_depth, int n, int width, int height)
+{
+    int rc = check_slot(e, slot);
+    if (rc) return rc;
+    Slot &sl = e->slots[slot];
+    if (sl.busy) return fail(e, H2J_ERR_BUSY, "slot %d has a batch in flight", slot);
+    if (!d_frames || n < 1 || n > e->s.max_batch) return fail(e, H2J_ERR_INVALID_ARG, "bad frames pointer or batch size %d (max %d)", n, e->s.max_batch);
+    if (width < 2 || height < 2) return fail(e, H2J_ERR_UNSUPPORTED, "unsupported frame size %dx%d", width, height);
+    if (bit_depth < 9 || bit_depth > 16) return fail(e, H2J_ERR_INVALID_ARG, "bit_depth %d outside 9..16", bit_depth);
+    if (odd((uintptr_t)d_frames) || odd(frame_stride) || odd((size_t)y_pitch) || odd((size_t)c_pitch) || odd(u_offset) || odd(v_offset))
+        return fail(e, H2J_ERR_INVALID_ARG, "16-bit samples need even pointers, strides, pitches and offsets");
+    const int fmt = e->s.chroma_format;
+    const int fcw = chroma_w(width, fmt), fch = chroma_h(height, fmt);
+    if (y_pitch < 2 * width || c_pitch < 2 * fcw)
+        return fail(e, H2J_ERR_INVALID_ARG, "pitches %d / %d smaller than rows of %d / %d 16-bit words", y_pitch, c_pitch, width, fcw);
+    const size_t y_end = (size_t)y_pitch * (height - 1) + 2 * (size_t)width;
+    const size_t u_end = u_offset + (size_t)c_pitch * (fch - 1) + 2 * (size_t)fcw, v_end = v_offset + (size_t)c_pitch * (fch - 1) + 2 * (size_t)fcw;
+    if (y_end > frame_stride || u_end > frame_stride || v_end > frame_stride)
+        return fail(e, H2J_ERR_INVALID_ARG, "a plane of the %dx%d frame reaches past frame_stride %zu", width, height, frame_stride);
+    ON_DEVICE(e);
+    sl.n = n;
+    CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
+    rc = convert_depth(e, sl, d_frames, Src16{(long long)frame_stride, (long long)u_offset, (long long)v_offset, y_pitch, c_pitch}, false, bit_depth,
+                       n, width, height);
+    if (rc) return rc;
+    rc = launch_pipeline(e, sl, sl.d_frames, n, TAIL_SIZES);
+    if (rc) return rc;
+    sl.busy = true;
+    return H2J_OK;
+}
+
 int h2j_submit_host(h2j_encoder *e, int slot, const uint8_t *frames, size_t frame_stride, int n, int width, int height)
 {
     int rc = check_slot(e, slot);
@@ -937,78 +1098,58 @@ int h2j_encode_frame(h2j_encoder *e, const uint8_t *const planes[3], const int s
     sl.n = 1;
     CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
     {
-        constexpr int kMaxPieces = 96;
-        CopyPiece pieces[kMaxPieces];
-        int n_pieces = 0;
-        auto plane = [&](const uint8_t *src, int stride, size_t off, int pw, int pitch, int ph) {
-            // pieces of ~256 KiB, but never more than a third of the table per plane
-            int rows_per_piece = std::max(1, (256 * 1024) / pitch);
-            rows_per_piece = std::max(rows_per_piece, (ph + kMaxPieces / 3 - 1) / (kMaxPieces / 3));
-            for (int r0 = 0; r0 < ph; r0 += rows_per_piece) {
-                const int r1 = std::min(ph, r0 + rows_per_piece);
-                CopyPiece &c = pieces[n_pieces++];
-                c.dst = sl.h_stage + off + (size_t)r0 * pitch;
-                c.src = src + (size_t)r0 * stride;
-                c.rows = r1 - r0;
-                c.row_bytes = pw;
-                c.dst_pitch = pitch;
-                c.src_stride = stride;
-                c.dev_off = off + (size_t)r0 * pitch;
-                c.dev_bytes = (size_t)(r1 - r0 - 1) * pitch + pw;
-            }
-        };
-        plane(planes[0], strides[0], 0, width, L.y_pitch, height);
-        plane(planes[1], strides[1], (size_t)L.u_off, fcw, L.c_pitch, fch);
-        plane(planes[2], strides[2], (size_t)L.v_off, fcw, L.c_pitch, fch);
-        // Planes that already live in page-locked memory (h2j_alloc_pinned, cudaHostAlloc, cudaHostRegister by the caller -- a
-        // decoder whose frame buffers come from such a pool) are uploaded from where they are: no staging copy, one strided
-        // DMA per plane.  The host copy is three quarters of the call for pageable planes.
-        auto pinned = [](const void *p) {
-            cudaPointerAttributes at;
-            if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
-                cudaGetLastError();
-                return false;
-            }
-            return at.type == cudaMemoryTypeHost;
-        };
-        if (pinned(planes[0]) && pinned(planes[1]) && pinned(planes[2])) {
-            CU(e, cudaMemcpy2DAsync(sl.d_frames, L.y_pitch, planes[0], strides[0], width, height, cudaMemcpyHostToDevice, sl.stream));
-            CU(e, cudaMemcpy2DAsync(sl.d_frames + L.u_off, L.c_pitch, planes[1], strides[1], fcw, fch, cudaMemcpyHostToDevice, sl.stream));
-            CU(e, cudaMemcpy2DAsync(sl.d_frames + L.v_off, L.c_pitch, planes[2], strides[2], fcw, fch, cudaMemcpyHostToDevice, sl.stream));
-            n_pieces = 0;
-        }
-        cudaError_t up_err = cudaSuccess;
-        auto upload = [&](int i) {
-            const cudaError_t ce = cudaMemcpyAsync(sl.d_frames + pieces[i].dev_off, sl.h_stage + pieces[i].dev_off, pieces[i].dev_bytes, cudaMemcpyHostToDevice, sl.stream);
-            if (ce != cudaSuccess && up_err == cudaSuccess) up_err = ce;
-        };
-        for (int i = 0; i < n_pieces; i++) {
-            copy_piece(pieces[i]);
-            upload(i);
-        }
-        CU(e, up_err);
+        const int row_bytes[3] = {width, fcw, fcw}, rows[3] = {height, fch, fch}, pitch[3] = {L.y_pitch, L.c_pitch, L.c_pitch};
+        const size_t off[3] = {0, (size_t)L.u_off, (size_t)L.v_off};
+        rc = upload_planes(e, sl, planes, strides, row_bytes, rows, off, pitch, sl.d_frames, sl.h_stage);
+        if (rc) return rc;
     }
     rc = launch_pipeline(e, sl, sl.d_frames, 1, TAIL_SINGLE);
     if (rc) return rc;
-    CU(e, cudaStreamSynchronize(sl.stream));
-    int st = 0;
-    long long jpeg_bytes = 0;
-    memcpy(&st, sl.h_tail + (offsetof(FrameTab, status) - kTabTailOff), sizeof st);
-    memcpy(&jpeg_bytes, sl.h_tail + (offsetof(FrameTab, jpeg_bytes) - kTabTailOff), sizeof jpeg_bytes);
-    if (st != 0) return fail(e, st, "the frame failed: %s", h2j_status_string(st));
-    if (jpeg_bytes < 0 || (size_t)jpeg_bytes > e->jpeg_cap) return fail(e, H2J_ERR_OUTPUT_TOO_SMALL, "JPEG of %lld bytes exceeds max_jpeg_bytes", jpeg_bytes);
-    const size_t n_out = (size_t)jpeg_bytes;
-    *out_size = n_out;
-    if (n_out > out_capacity) return fail(e, H2J_ERR_OUTPUT_TOO_SMALL, "JPEG is %zu bytes, caller gave %zu", n_out, out_capacity);
-    const size_t spec = std::min(std::min(sl.spec_bytes, e->out_cap), sl.h_stage_bytes);
-    const size_t have = std::min(n_out, spec);
-    memcpy(out, sl.h_stage, have);
-    if (n_out > have) {  // the guess was short: the rest straight into the caller's buffer
-        CU(e, cudaMemcpy(out + have, sl.d_out + have, n_out - have, cudaMemcpyDeviceToHost));
+    return finish_single(e, sl, out, out_capacity, out_size);
+}
+
+int h2j_encode_frame16(h2j_encoder *e, const uint8_t *const planes[3], const int strides[3], int bit_depth, int width, int height,
+                       uint8_t *out, size_t out_capacity, size_t *out_size)
+{
+    if (!e) return H2J_ERR_INVALID_ARG;
+    if (!planes || !strides || !planes[0] || !planes[1] || !planes[2] || !out || !out_size)
+        return fail(e, H2J_ERR_INVALID_ARG, "null plane/out pointer");
+    if (bit_depth < 9 || bit_depth > 16) return fail(e, H2J_ERR_INVALID_ARG, "bit_depth %d outside 9..16", bit_depth);
+    if (width < 2 || height < 2 || width > e->s.max_width || height > e->s.max_height)
+        return fail(e, H2J_ERR_UNSUPPORTED, "frame %dx%d outside 2x2 .. %dx%d", width, height, e->s.max_width, e->s.max_height);
+    Slot &sl = e->slots[0];
+    if (sl.busy) return fail(e, H2J_ERR_BUSY, "slot 0 has a batch in flight");
+    const int fmt = e->s.chroma_format;
+    const int fcw = chroma_w(width, fmt), fch = chroma_h(height, fmt);
+    for (int p = 0; p < 3; p++)
+        if (odd((uintptr_t)planes[p]) || odd((size_t)strides[p])) return fail(e, H2J_ERR_INVALID_ARG, "plane %d: odd pointer or stride", p);
+    if (strides[0] < 2 * width || strides[1] < 2 * fcw || strides[2] < 2 * fcw) return fail(e, H2J_ERR_INVALID_ARG, "stride smaller than the row");
+    ON_DEVICE(e);
+    // the 16-bit planes go to the device at 16-byte aligned row pitches, so that the conversion reads them with vector loads
+    const int yp = (int)align_up((size_t)2 * width, 16), cp = (int)align_up((size_t)2 * fcw, 16);
+    if (!sl.d_frames16) {
+        const int mcw = chroma_w(e->s.max_width, fmt), mch = chroma_h(e->s.max_height, fmt);
+        const size_t bytes = align_up((size_t)2 * e->s.max_width, 16) * e->s.max_height + 2 * align_up((size_t)2 * mcw, 16) * mch;
+        if (cudaMalloc(&sl.d_frames16, bytes) != cudaSuccess || cudaHostAlloc(&sl.h_stage16, bytes, cudaHostAllocDefault) != cudaSuccess) {
+            cudaGetLastError();
+            cudaFree(sl.d_frames16);
+            sl.d_frames16 = nullptr;
+            sl.h_stage16 = nullptr;
+            return fail(e, H2J_ERR_NOMEM, "no room for the 16-bit staging of a %dx%d picture", e->s.max_width, e->s.max_height);
+        }
     }
-    // next guess: a quarter above this frame, in 64 KiB steps (consecutive frames of a stream are alike)
-    sl.spec_bytes = std::max<size_t>(64 * 1024, align_up(n_out + n_out / 4, 64 * 1024));
-    return H2J_OK;
+    sl.n = 1;
+    CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
+    const Src16 S{0, (long long)yp * height, (long long)yp * height + (long long)cp * fch, yp, cp};
+    const int row_bytes[3] = {2 * width, 2 * fcw, 2 * fcw}, rows[3] = {height, fch, fch}, pitch[3] = {yp, cp, cp};
+    const size_t off[3] = {0, (size_t)S.u_off, (size_t)S.v_off};
+    int rc = upload_planes(e, sl, planes, strides, row_bytes, rows, off, pitch, sl.d_frames16, sl.h_stage16);
+    if (rc) return rc;
+    rc = convert_depth(e, sl, sl.d_frames16, S, false, bit_depth, 1, width, height);
+    if (rc) return rc;
+    rc = launch_pipeline(e, sl, sl.d_frames, 1, TAIL_SINGLE);
+    if (rc) return rc;
+    return finish_single(e, sl, out, out_capacity, out_size);
 }
 
 int h2j_convert_pad(h2j_encoder *e, const uint8_t *const planes[3], const int strides[3], int width, int height, int range_mode,

@@ -220,4 +220,70 @@ __global__ void __launch_bounds__(128) repitch_kernel(const uint8_t *__restrict_
     }
 }
 
+// ------------------------------------------------------------------------------------------------
+// High-bit-depth frames (P010 / P016, P210 / P216, a decoder's 16-bit 4:4:4 surface, yuv420p10le ...) -> 8-bit planar frames
+// at the 16-byte row pitch of pitched_layout(), which the pipeline then reads with its vector loads.  Every sample is a
+// little-endian 16-bit word whose low `bit_depth` bits hold the value; the 8-bit sample is bits [bit_depth - 8, bit_depth)
+// of the word (truncation: no rounding, no dither; bits above bit_depth never reach the picture).  All offsets and pitches
+// of Src16 are in bytes.
+// SP: a luma plane and one plane of interleaved Cb/Cr word pairs (rows h .. h + ch - 1 of the grid split one row of pairs),
+// otherwise three planes (rows h .. h + 2 ch - 1: Cb, then Cr).  grid (x, rows / kPlaneRowsPerCta, frames) as
+// nv12_to_i420_kernel; a thread converts 16 words of a source row: two 128-bit loads where that row is 16-byte aligned and
+// holds all 16 words, 16-bit loads otherwise.  No word past a row's last sample is read.
+// ------------------------------------------------------------------------------------------------
+struct Src16 {
+    long long frame_stride, u_off, v_off;  // SP: u_off = v_off = the pair plane
+    int y_pitch, c_pitch;
+};
+
+template <bool SP>
+__global__ void __launch_bounds__(128) depth_to_8_kernel(const uint8_t *__restrict__ src, Src16 S, uint8_t *__restrict__ dst, FrameLayout P,
+                                                         int shift)  // bit_depth - 8
+{
+    const int f = blockIdx.z;
+    const int fcw = (P.w + (1 << fmt_hshift(P.fmt)) - 1) >> fmt_hshift(P.fmt), fch = (P.h + fmt_vshift(P.fmt)) >> fmt_vshift(P.fmt);
+    const int x0 = (blockIdx.x * blockDim.x + threadIdx.x) * 16;  // first word of the row this thread converts
+    const uint8_t *F = src + (long long)f * S.frame_stride;
+    uint8_t *D = dst + (long long)f * P.frame_stride;
+    for (int row = blockIdx.y * kPlaneRowsPerCta; row < min((int)(blockIdx.y + 1) * kPlaneRowsPerCta, P.h + (SP ? 1 : 2) * fch); row++) {
+        int n;  // words in the row
+        const uint8_t *s;
+        uint8_t *d;
+        if (row < P.h) { n = P.w; s = F + (long long)row * S.y_pitch; d = D + (long long)row * P.y_pitch + x0; }
+        else if (SP) { const int r = row - P.h; n = 2 * fcw; s = F + S.u_off + (long long)r * S.c_pitch; d = D + P.u_off + (long long)r * P.c_pitch + (x0 >> 1); }
+        else {
+            const int r = row - P.h - (row >= P.h + fch ? fch : 0);
+            n = fcw;
+            s = F + (row >= P.h + fch ? S.v_off : S.u_off) + (long long)r * S.c_pitch;
+            d = D + (row >= P.h + fch ? P.v_off : P.u_off) + (long long)r * P.c_pitch + x0;
+        }
+        if (x0 >= n) continue;
+        s += 2 * x0;
+        unsigned t[8];  // word 2k in the low half of t[k], word 2k + 1 in the high half
+        if (x0 + 16 <= n && ((uintptr_t)s & 15u) == 0) {
+            const uint4 a = ldg128(s), b = ldg128(s + 16);
+            t[0] = a.x; t[1] = a.y; t[2] = a.z; t[3] = a.w; t[4] = b.x; t[5] = b.y; t[6] = b.z; t[7] = b.w;
+        } else {
+            const unsigned short *s16 = reinterpret_cast<const unsigned short *>(s);
+#pragma unroll
+            for (int k = 0; k < 8; k++)
+                t[k] = (x0 + 2 * k < n ? (unsigned)__ldg(s16 + 2 * k) : 0u) | (x0 + 2 * k + 1 < n ? (unsigned)__ldg(s16 + 2 * k + 1) << 16 : 0u);
+        }
+        // after the shift, bytes 0 and 2 of t[k] are bits [shift, shift + 8) of its two words: the high word's low bits only
+        // reach bits 8..15, and nothing above bit_depth is in either byte
+#pragma unroll
+        for (int k = 0; k < 8; k++) t[k] >>= shift;
+        const unsigned p0 = __byte_perm(t[0], t[1], 0x6420), p1 = __byte_perm(t[2], t[3], 0x6420), p2 = __byte_perm(t[4], t[5], 0x6420),
+                       p3 = __byte_perm(t[6], t[7], 0x6420);
+        // rows of the copy are 16-byte aligned and at least 16 bytes (8 per chroma component of a pair row) past x0
+        if (SP && row >= P.h) {
+            const long long cr = P.v_off - P.u_off;
+            *reinterpret_cast<uint2 *>(d) = make_uint2(__byte_perm(p0, p1, 0x6420), __byte_perm(p2, p3, 0x6420));       // Cb
+            *reinterpret_cast<uint2 *>(d + cr) = make_uint2(__byte_perm(p0, p1, 0x7531), __byte_perm(p2, p3, 0x7531));  // Cr
+        } else {
+            *reinterpret_cast<uint4 *>(d) = make_uint4(p0, p1, p2, p3);
+        }
+    }
+}
+
 }  // namespace h2j

@@ -90,6 +90,7 @@ EXPORTS = [
     "h2j_alloc_pinned", "h2j_free_pinned", "h2j_convert_pad", "h2j_debug_frame_info", "h2j_debug_coefficients",
     "h2j_slot_kernel_ms", "h2j_set_profile", "h2j_slot_total_ms", "h2j_kernel_launches", "h2j_slot_set_stream",
     "h2j_slot_wait_event", "h2j_device_count", "h2j_debug_set_knob", "h2j_debug_read_device", "h2j_stream_copy",
+    "h2j_submit_device_semiplanar16", "h2j_submit_device_pitched16", "h2j_encode_frame16",
 ]
 
 _lib = None
@@ -123,6 +124,9 @@ def load_library() -> C.CDLL:
     lib.h2j_submit_device_nv12.argtypes = [vp, ci, vp, sz, ci, sz, ci, ci, ci]
     lib.h2j_submit_device_semiplanar.argtypes = [vp, ci, vp, sz, ci, sz, ci, ci, ci]
     lib.h2j_submit_device_pitched.argtypes = [vp, ci, vp, sz, ci, ci, sz, sz, ci, ci, ci]
+    lib.h2j_submit_device_semiplanar16.argtypes = [vp, ci, vp, sz, ci, sz, ci, ci, ci, ci]
+    lib.h2j_submit_device_pitched16.argtypes = [vp, ci, vp, sz, ci, ci, sz, sz, ci, ci, ci, ci]
+    lib.h2j_encode_frame16.argtypes = [vp, C.POINTER(vp), C.POINTER(ci), ci, ci, ci, vp, sz, C.POINTER(sz)]
     lib.h2j_collect.argtypes = [vp, ci, vp, sz, C.POINTER(sz), C.POINTER(ci)]
     lib.h2j_collect_device.argtypes = [vp, ci, C.POINTER(vp), C.POINTER(sz), C.POINTER(sz), C.POINTER(ci)]
     lib.h2j_wait.argtypes = [vp, ci]
@@ -308,6 +312,21 @@ class Encoder:
         self._check(self._lib.h2j_encode_frame(self._h, planes, strides, w, h, out.ctypes.data, out.size, C.byref(n)))
         return out[: n.value].tobytes()
 
+    def yuv2jpeg16(self, y: np.ndarray, u: np.ndarray, v: np.ndarray, bit_depth: int) -> bytes:
+        """One high-bit-depth frame (2-D uint16 planes, any row stride; `bit_depth`-bit values in the low bits of each
+        little-endian word, 16 for MSB-aligned data) -> JPEG bytes of its truncated 8-bit frame (h2j_encode_frame16)."""
+        for p in (y, u, v):
+            if p.dtype != np.uint16 or p.ndim != 2 or p.strides[1] != 2:
+                raise H2JError(ERR_INVALID_ARG, "planes must be 2-D uint16 arrays with contiguous rows")
+        h, w = y.shape
+        self._check_chroma(w, h, u, v)
+        planes = (C.c_void_p * 3)(y.ctypes.data, u.ctypes.data, v.ctypes.data)
+        strides = (C.c_int * 3)(y.strides[0], u.strides[0], v.strides[0])
+        out = np.empty(self.out_capacity, np.uint8)
+        n = C.c_size_t(0)
+        self._check(self._lib.h2j_encode_frame16(self._h, planes, strides, bit_depth, w, h, out.ctypes.data, out.size, C.byref(n)))
+        return out[: n.value].tobytes()
+
     def yuv2jpeg_into(self, y: np.ndarray, u: np.ndarray, v: np.ndarray, out: Optional[np.ndarray] = None) -> int:
         """Same call, JPEG bytes into a caller buffer (or a buffer kept by this object: ``self.last_out``); returns the
         size.  Nothing is allocated per call -- the form to time."""
@@ -350,6 +369,21 @@ class Encoder:
         `u_offset` / `v_offset` with rows `c_pitch` apart."""
         self._check(self._lib.h2j_submit_device_pitched(self._h, slot, d_frames_ptr, frame_stride, y_pitch, c_pitch, u_offset, v_offset,
                                                         n, width, height))
+        self._n_in_slot[slot] = n
+
+    def submit_device_semiplanar16(self, slot: int, d_frames_ptr: int, frame_stride: int, pitch: int, uv_offset: int, bit_depth: int,
+                                   n: int, width: int, height: int) -> None:
+        """Semi-planar frames of 16-bit words in device memory (P010 / P016, P210 / P216, ... by the encoder's chroma
+        format); pitch and offsets in bytes, `bit_depth`-bit values in the low bits of each word (16 for MSB-aligned)."""
+        self._check(self._lib.h2j_submit_device_semiplanar16(self._h, slot, d_frames_ptr, frame_stride, pitch, uv_offset, bit_depth, n,
+                                                             width, height))
+        self._n_in_slot[slot] = n
+
+    def submit_device_pitched16(self, slot: int, d_frames_ptr: int, frame_stride: int, y_pitch: int, c_pitch: int, u_offset: int,
+                                v_offset: int, bit_depth: int, n: int, width: int, height: int) -> None:
+        """Planar frames of 16-bit words in device memory at any layout (pitches and offsets in bytes)."""
+        self._check(self._lib.h2j_submit_device_pitched16(self._h, slot, d_frames_ptr, frame_stride, y_pitch, c_pitch, u_offset, v_offset,
+                                                          bit_depth, n, width, height))
         self._n_in_slot[slot] = n
 
     def read_device(self, d_ptr: int, nbytes: int) -> bytes:

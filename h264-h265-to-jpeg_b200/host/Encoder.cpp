@@ -34,6 +34,15 @@ namespace {
 
 constexpr int kSlotsPerDevice = 2;  // batches in flight per device: the upload of one runs under the kernels of the other
 
+// What libavcodec's HEVC decoder produces for Main10 / Main12 4:2:0: 16-bit little-endian words holding 10 / 12-bit values.
+#ifdef H2J_WITH_LIBAV
+constexpr int kFmtYuv420p10le = AV_PIX_FMT_YUV420P10LE, kFmtYuv420p12le = AV_PIX_FMT_YUV420P12LE;
+static_assert(AV_PIX_FMT_YUV420P == 0 && AV_PIX_FMT_YUVJ420P == 12 && kFmtYuv420p10le == 64 && kFmtYuv420p12le == 125,
+              "H2JFrameView callers pass the AVPixelFormat numbers of libavutil 56");
+#else
+constexpr int kFmtYuv420p10le = 64, kFmtYuv420p12le = 125;  // AV_PIX_FMT_YUV420P10LE / AV_PIX_FMT_YUV420P12LE (libavutil 56)
+#endif
+
 size_t i420_bytes(int w, int h) { return (size_t)w * h + 2 * (size_t)((w + 1) >> 1) * ((h + 1) >> 1); }
 
 // reference src/Encoder.cpp:338-361 saveJpegtoFile: same open mode, same log lines, same false on error
@@ -506,9 +515,12 @@ bool Encoder::yuv2Jpeg(AVFrame *)
 bool Encoder::yuv2Jpeg(const H2JFrameView &f)
 {
     // The reference feeds whatever the decoder produced to an encoder opened as YUVJ420P (src/Encoder.cpp:162);
-    // anything but 8-bit 4:2:0 planar would be read as garbage there.  Here it is refused.
-    if (f.format != 0 /* AV_PIX_FMT_YUV420P */ && f.format != 12 /* AV_PIX_FMT_YUVJ420P */) {
-        LOG("%s line=%d | unsupported pixel format %d (need yuv420p / yuvj420p)", __PRETTY_FUNCTION__, __LINE__, f.format);
+    // anything but 8-bit 4:2:0 planar would be read as garbage there.  Here 10 / 12-bit 4:2:0 (Main10 / Main12 streams) is
+    // encoded from its 8-bit truncation (include/h2j_b200.h, h2j_encode_frame16); everything else is refused.
+    const int bit_depth = f.format == kFmtYuv420p10le ? 10 : (f.format == kFmtYuv420p12le ? 12 : 8);
+    if (bit_depth == 8 && f.format != 0 /* AV_PIX_FMT_YUV420P */ && f.format != 12 /* AV_PIX_FMT_YUVJ420P */) {
+        LOG("%s line=%d | unsupported pixel format %d (need yuv420p / yuvj420p / yuv420p10le / yuv420p12le)", __PRETTY_FUNCTION__, __LINE__,
+            f.format);
         release();
         return false;
     }
@@ -523,7 +535,7 @@ bool Encoder::yuv2Jpeg(const H2JFrameView &f)
     int range_mode;
     {
         std::unique_lock<std::mutex> lock(H.mu);
-        if (H.batching) {
+        if (H.batching && bit_depth == 8) {  // (high-bit-depth pictures take the synchronous path below)
             // batch scope: the picture is queued; it is encoded and its file written when its batch is complete or the scope ends
             if (this->outputFilePath == nullptr || strlen(this->outputFilePath) == 0) {
                 LOG("Jpeg 文件路径为空，请核查！");
@@ -565,9 +577,10 @@ bool Encoder::yuv2Jpeg(const H2JFrameView &f)
     const uint8_t *planes[3] = {f.data[0], f.data[1], f.data[2]};
     const int strides[3] = {f.linesize[0], f.linesize[1], f.linesize[2]};
     jpegSize_ = 0;
-    const int rc = h2j_encode_frame(D->sync_box.enc, planes, strides, f.width, f.height, jpeg_.get(), jpegCap_, &jpegSize_);
+    const int rc = bit_depth == 8 ? h2j_encode_frame(D->sync_box.enc, planes, strides, f.width, f.height, jpeg_.get(), jpegCap_, &jpegSize_)
+                                  : h2j_encode_frame16(D->sync_box.enc, planes, strides, bit_depth, f.width, f.height, jpeg_.get(), jpegCap_, &jpegSize_);
     if (rc != H2J_OK) {
-        LOG("h2j_encode_frame failed, rc=%d (%s), error=%s", rc, h2j_status_string(rc), h2j_last_error(D->sync_box.enc));
+        LOG("h2j_encode_frame%s failed, rc=%d (%s), error=%s", bit_depth == 8 ? "" : "16", rc, h2j_status_string(rc), h2j_last_error(D->sync_box.enc));
         release();
         return false;
     }

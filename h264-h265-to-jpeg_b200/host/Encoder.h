@@ -47,7 +47,9 @@ struct H2JFrameView {
     const uint8_t *data[3];
     int linesize[3];
     int width, height;
-    int format;  // AVPixelFormat: 0 = AV_PIX_FMT_YUV420P, 12 = AV_PIX_FMT_YUVJ420P
+    int format;  // AVPixelFormat (libavutil 56): 0 = AV_PIX_FMT_YUV420P, 12 = AV_PIX_FMT_YUVJ420P, and the 16-bit little-endian
+                 // 64 = AV_PIX_FMT_YUV420P10LE, 125 = AV_PIX_FMT_YUV420P12LE (linesize in bytes, as AVFrame's), which are
+                 // encoded from their 8-bit truncation (h2j_encode_frame16 in include/h2j_b200.h)
 };
 
 class Encoder {
@@ -90,6 +92,8 @@ extern "C" void h2j_host_configure(int cuda_device, int range_mode);
 // per device so that the upload of one runs under the kernels of the other), which also writes the JPEG files, while
 // the callers already fill the next batch.  h2j_host_batch_end() drains everything and returns the number of files
 // written (-1 outside a scope); *failed receives the number of pictures that could not be encoded or saved.
+// High-bit-depth pictures (yuv420p10le / yuv420p12le) are not queued: inside a scope they take the synchronous path, so
+// their file exists when yuv2Jpeg returns, and they do not count in h2j_host_batch_end's result.
 extern "C" int h2j_host_batch_begin(int max_frames);
 extern "C" int h2j_host_batch_end(int *failed);
 // Devices that currently hold GPU state for this process (inspection).

@@ -166,6 +166,37 @@ int h2j_submit_device_semiplanar(h2j_encoder *e, int slot, const uint8_t *d_fram
  * shorter than its plane's row, or a plane that reaches past frame_stride. */
 int h2j_submit_device_pitched(h2j_encoder *e, int slot, const uint8_t *d_frames, size_t frame_stride, int y_pitch,
                               int c_pitch, size_t u_offset, size_t v_offset, int n, int width, int height);
+
+/*
+ * High-bit-depth frames (H.265 Main10 / Main12 and the like).  Every sample is a little-endian 16-bit word that holds a
+ * `bit_depth`-bit value (9..16) in its low bits.  MSB-aligned formats -- P010 / P016, P210 / P216 and a hardware decoder's
+ * 16-bit 4:4:4 surface -- are bit_depth 16.  The 8-bit sample the encoder uses is
+ *     (word & ((1 << bit_depth) - 1)) >> (bit_depth - 8)
+ * i.e. truncation: bits above bit_depth are ignored, there is no rounding and no dither.  The JPEG is byte-identical to
+ * the one this encoder writes for the 8-bit planar frame of those samples, with the same range_mode and fixed_qscale
+ * (H2J_RANGE_LIMITED_TO_FULL maps 10-bit limited range, 64..940 -> 16..235, exactly as 8-bit).  No colour-space or transfer
+ * conversion is done: BT.2020 / PQ content is encoded as it stands, as the reference ignores colour metadata.
+ * All pitches, strides and offsets are in BYTES (as AVFrame.linesize); pointers, pitches, strides and offsets must be even.
+ * Each device submit converts the batch into the slot's own 8-bit frame buffer with one extra kernel, then runs the
+ * usual pipeline; collect with h2j_collect / h2j_collect_device.
+ *
+ * h2j_submit_device_semiplanar16: as h2j_submit_device_semiplanar with 16-bit words: P010 / P016 (4:2:0), P210 / P216
+ *   (4:2:2) or the 4:4:4 equivalent, by the encoder's chroma_format.  A row of pairs is 2 * pair count words.
+ * h2j_submit_device_pitched16: as h2j_submit_device_pitched with 16-bit words (a decoder's 16-bit 4:4:4 surface,
+ *   yuv420p10le frames in device memory ...).
+ * h2j_encode_frame16: as h2j_encode_frame with 16-bit planes (libavcodec's yuv420p10le / yuv420p12le are bit_depth 10 /
+ *   12).  Its device buffer and pinned staging are allocated on its first call (H2J_ERR_NOMEM if that fails; the encoder
+ *   stays usable) and freed by h2j_destroy.
+ * H2J_ERR_INVALID_ARG: bit_depth outside 9..16, an odd pointer / pitch / stride / offset, a pitch or stride shorter than
+ * two bytes per sample of its row (semi-planar: 2 * max(width, 2 * pairs per row)), a pair plane that starts inside the
+ * luma plane, or a plane that reaches past frame_stride.  H2J_ERR_UNSUPPORTED: a size above the encoder's maximum.
+ */
+int h2j_submit_device_semiplanar16(h2j_encoder *e, int slot, const uint8_t *d_frames, size_t frame_stride, int pitch,
+                                   size_t uv_offset, int bit_depth, int n, int width, int height);
+int h2j_submit_device_pitched16(h2j_encoder *e, int slot, const uint8_t *d_frames, size_t frame_stride, int y_pitch,
+                                int c_pitch, size_t u_offset, size_t v_offset, int bit_depth, int n, int width, int height);
+int h2j_encode_frame16(h2j_encoder *e, const uint8_t *const planes[3], const int strides[3], int bit_depth, int width,
+                       int height, uint8_t *out, size_t out_capacity, size_t *out_size);
 int h2j_collect(h2j_encoder *e, int slot, uint8_t *out, size_t out_capacity, size_t *offsets, int *status);
 int h2j_collect_device(h2j_encoder *e, int slot, const uint8_t **d_out, size_t *d_frame_capacity, size_t *sizes,
                        int *status);
