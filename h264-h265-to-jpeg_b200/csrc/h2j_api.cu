@@ -62,6 +62,12 @@ struct Slot {
     bool packed = false;      // pack_kernel already ran for the batch in flight
     int n = 0;
     FrameLayout L{};
+    // list batches (h2j_submit_device_list / h2j_submit_host_list): descs[i] is frame i as the pipeline reads it, descs[n + i]
+    // the source a copy kernel reads it from (base nullptr: no copy).  The pinned mirror is filled by the submit and uploaded
+    // with one copy on the slot's stream; a busy slot refuses a submit, so it is never rewritten while that copy is pending.
+    bool list = false;
+    FrameDesc *d_desc = nullptr;  // [2 * max_batch]
+    FrameDesc *h_desc = nullptr;  // pinned mirror
     std::vector<KernelTiming> timings;
     std::vector<cudaEvent_t> events;
     int timings_used = 0, events_used = 0;
@@ -333,9 +339,34 @@ int enqueue_single_tail(h2j_encoder *e, Slot &sl);
 constexpr int kFdctMaxTilesPerCta = 16;  // K2: upper bound of consecutive tiles one CTA walks (h2j_debug_set_knob may force any)
 constexpr int kStuffCtas = 32;           // K5 CTAs per frame
 
-int launch_pipeline(h2j_encoder *e, Slot &sl, const uint8_t *d_frames, int n, int tail)
+// the K2 instantiation for the layout kind (chroma format, semi-planar chroma read in place) and the batch kind
+template <bool LIST>
+decltype(&fdct_quant_kernel<false, false>) k2_kernel(const FrameLayout &L)
 {
-    const FrameLayout &L = sl.L;
+    return L.fmt == kFmt422 ? (L.nv12 ? fdct_quant_fmt_kernel<kFmt422, true, LIST> : fdct_quant_fmt_kernel<kFmt422, false, LIST>)
+           : L.fmt == kFmt444 ? (L.nv12 ? fdct_quant_fmt_kernel<kFmt444, true, LIST> : fdct_quant_fmt_kernel<kFmt444, false, LIST>)
+                              : (L.nv12 ? fdct_quant_kernel<true, LIST> : fdct_quant_kernel<false, LIST>);
+}
+
+// list: the frames are sl.h_desc[0 .. n) (already uploaded to sl.d_desc); the grids are sized for the largest of them
+int launch_pipeline(h2j_encoder *e, Slot &sl, const uint8_t *d_frames, int n, int tail, bool list = false)
+{
+    sl.list = list;
+    const FrameLayout &L = list ? sl.h_desc[0].L : sl.L;  // (what all frames share: chroma format, nv12)
+    const FrameDesc *D = list ? sl.d_desc : nullptr;
+    int mcu_h = L.mcu_h, n_tiles = (L.n_mcu + kTileMcus - 1) / kTileMcus, n_units = (L.n_blocks + kUnitBlocks - 1) / kUnitBlocks;
+    long long total_tiles = (long long)n_tiles * n;
+    if (list) {
+        total_tiles = 0;
+        for (int i = 0; i < n; i++) {
+            const FrameLayout &Li = sl.h_desc[i].L;
+            const int t = (Li.n_mcu + kTileMcus - 1) / kTileMcus;
+            mcu_h = std::max(mcu_h, Li.mcu_h);
+            n_tiles = std::max(n_tiles, t);
+            n_units = std::max(n_units, (Li.n_blocks + kUnitBlocks - 1) / kUnitBlocks);
+            total_tiles += t;
+        }
+    }
     cudaStream_t st = sl.stream;
     sl.timings_used = 0;
     sl.events_used = 0;
@@ -344,50 +375,47 @@ int launch_pipeline(h2j_encoder *e, Slot &sl, const uint8_t *d_frames, int n, in
     CU(e, cudaMemsetAsync(sl.d_zero, 0, sl.zero_bytes, st));
     {
         ScopedTiming t(e, sl, "mbvar_kernel");
-        mbvar_kernel<<<dim3(L.mcu_h, n), 128, 0, st>>>(d_frames, L, sl.d_state, e->d_qscale_lut, sl.d_tabs);
+        (list ? mbvar_kernel<true> : mbvar_kernel<false>)<<<dim3(mcu_h, n), 128, 0, st>>>(d_frames, L, sl.d_state, e->d_qscale_lut, sl.d_tabs, D);
         e->launches++;
     }
-    const int n_tiles = (L.n_mcu + kTileMcus - 1) / kTileMcus;
     {
         ScopedTiming t(e, sl, "fdct_quant_kernel");
         // consecutive tiles per CTA: as many as keep the grid at four waves or more (amortises the per-CTA set-up
         // and histogram flush), at most kFdctMaxTilesPerCta
-        int tiles_per_cta = (int)((long long)n_tiles * n * fmt_roles(L.fmt) / ((long long)e->sm_count * kFdctMinCtas * 4));
+        int tiles_per_cta = (int)(total_tiles * fmt_roles(L.fmt) / ((long long)e->sm_count * kFdctMinCtas * 4));
         tiles_per_cta = tiles_per_cta < 1 ? 1 : (tiles_per_cta > kFdctMaxTilesPerCta ? kFdctMaxTilesPerCta : tiles_per_cta);
         if (e->force_fdct_tiles > 0) tiles_per_cta = e->force_fdct_tiles;
         const dim3 grid(fmt_roles(L.fmt) * ((n_tiles + tiles_per_cta - 1) / tiles_per_cta), n);
-        const auto k2 = L.fmt == kFmt422 ? (L.nv12 ? fdct_quant_fmt_kernel<kFmt422, true> : fdct_quant_fmt_kernel<kFmt422, false>)
-                        : L.fmt == kFmt444 ? (L.nv12 ? fdct_quant_fmt_kernel<kFmt444, true> : fdct_quant_fmt_kernel<kFmt444, false>)
-                                           : (L.nv12 ? fdct_quant_kernel<true> : fdct_quant_kernel<false>);
-        k2<<<grid, kFdctThreads, 0, st>>>(d_frames, L, sl.d_state, sl.d_tabs, sl.d_images, e->images_cap, tiles_per_cta);
+        const auto k2 = list ? k2_kernel<true>(L) : k2_kernel<false>(L);
+        k2<<<grid, kFdctThreads, 0, st>>>(d_frames, L, sl.d_state, sl.d_tabs, sl.d_images, e->images_cap, tiles_per_cta, D);
         e->launches++;
     }
     {
         ScopedTiming t(e, sl, "huffman_kernel");
-        huffman_kernel<<<4 * n, kHuffGroup, 0, st>>>(L, sl.d_tabs, sl.d_state, n, sl.d_out, (long long)e->out_cap, (long long)e->jpeg_cap,
-                                                                       e->d_comment, (int)e->comment.size());
+        (list ? huffman_kernel<true> : huffman_kernel<false>)<<<4 * n, kHuffGroup, 0, st>>>(L, sl.d_tabs, sl.d_state, n, sl.d_out, (long long)e->out_cap,
+                                                                                        (long long)e->jpeg_cap, e->d_comment, (int)e->comment.size(), D);
         e->launches++;
     }
     {
         ScopedTiming t(e, sl, "entropy_walk_kernel");
-        const auto k4a = L.fmt == kFmt420 ? entropy_walk_kernel<kFmt420> : L.fmt == kFmt422 ? entropy_walk_kernel<kFmt422> : entropy_walk_kernel<kFmt444>;
+        const auto k4a = list ? (L.fmt == kFmt420 ? entropy_walk_kernel<kFmt420, true> : L.fmt == kFmt422 ? entropy_walk_kernel<kFmt422, true> : entropy_walk_kernel<kFmt444, true>)
+                              : (L.fmt == kFmt420 ? entropy_walk_kernel<kFmt420, false> : L.fmt == kFmt422 ? entropy_walk_kernel<kFmt422, false> : entropy_walk_kernel<kFmt444, false>);
         k4a<<<dim3(n_tiles, n), fmt_tile_blocks(L.fmt), ent_smem_bytes(L.fmt), st>>>(L, sl.d_tabs, sl.d_images, e->images_cap, sl.d_unit_info, e->units_cap,
-                                                                                     sl.d_stage_alloc, sl.d_stage, e->stage_cap_words);
+                                                                                     sl.d_stage_alloc, sl.d_stage, e->stage_cap_words, D);
         e->launches++;
     }
     {
         ScopedTiming t(e, sl, "scan_place_kernel");
-        const int n_units = (L.n_blocks + kUnitBlocks - 1) / kUnitBlocks;
         const int groups_per_frame = (n_units + kPlaceGroupUnits - 1) / kPlaceGroupUnits;
         // fewer groups than two per SM: every group on four times as many warps
         if ((long long)groups_per_frame * n < 2LL * e->sm_count)
-            scan_place_kernel<8><<<groups_per_frame * n, kPlaceGroupUnits / 8 * 32, 0, st>>>(L, sl.d_tabs, sl.d_state, sl.d_unit_info, e->units_cap, sl.d_stage,
-                                                                                   e->stage_cap_words, sl.d_descs, groups_per_frame, sl.d_ticket, sl.d_scan,
-                                                                                   e->scan_cap_words, sl.d_chunk_ff, e->chunks_cap);
+            (list ? scan_place_kernel<8, true> : scan_place_kernel<8, false>)<<<groups_per_frame * n, kPlaceGroupUnits / 8 * 32, 0, st>>>(
+                L, sl.d_tabs, sl.d_state, sl.d_unit_info, e->units_cap, sl.d_stage, e->stage_cap_words, sl.d_descs, groups_per_frame, sl.d_ticket,
+                sl.d_scan, e->scan_cap_words, sl.d_chunk_ff, e->chunks_cap, D);
         else
-            scan_place_kernel<32><<<groups_per_frame * n, kPlaceThreads, 0, st>>>(L, sl.d_tabs, sl.d_state, sl.d_unit_info, e->units_cap, sl.d_stage,
-                                                                              e->stage_cap_words, sl.d_descs, groups_per_frame, sl.d_ticket, sl.d_scan,
-                                                                              e->scan_cap_words, sl.d_chunk_ff, e->chunks_cap);
+            (list ? scan_place_kernel<32, true> : scan_place_kernel<32, false>)<<<groups_per_frame * n, kPlaceThreads, 0, st>>>(
+                L, sl.d_tabs, sl.d_state, sl.d_unit_info, e->units_cap, sl.d_stage, e->stage_cap_words, sl.d_descs, groups_per_frame, sl.d_ticket,
+                sl.d_scan, e->scan_cap_words, sl.d_chunk_ff, e->chunks_cap, D);
         e->launches++;
     }
     {
@@ -569,12 +597,17 @@ int finish_single(h2j_encoder *e, Slot &sl, uint8_t *out, size_t out_capacity, s
     return H2J_OK;
 }
 
+// the layout of frame `frame` of the slot's last batch
+const FrameLayout &frame_layout(const Slot &sl, int frame) { return sl.list ? sl.h_desc[frame].L : sl.L; }
+
 void free_slot(Slot &sl)
 {
     if (sl.stream) cudaStreamSynchronize(sl.stream);
     cudaFree(sl.d_frames); cudaFree(sl.d_pitched); cudaFree(sl.d_images); cudaFree(sl.d_zero); cudaFree(sl.d_stage); cudaFree(sl.d_unit_info);
     cudaFree(sl.d_tabs); cudaFree(sl.d_scan); cudaFree(sl.d_out); cudaFree(sl.d_packed); cudaFree(sl.d_offsets); cudaFree(sl.d_status);
     cudaFree(sl.d_frames16);
+    cudaFree(sl.d_desc);
+    if (sl.h_desc) cudaFreeHost(sl.h_desc);
     if (sl.h_stage16) cudaFreeHost(sl.h_stage16);
     if (sl.h_offsets) cudaFreeHost(sl.h_offsets);
     if (sl.h_status) cudaFreeHost(sl.h_status);
@@ -721,9 +754,12 @@ int h2j_create(const h2j_settings *s, h2j_encoder **out)
         CUB(cudaMalloc(&e->d_comment, e->comment.size() + 1));
         CUB(cudaMemcpy(e->d_comment, e->comment.c_str(), e->comment.size() + 1, cudaMemcpyHostToDevice));
     }
-    CUB(cudaFuncSetAttribute(entropy_walk_kernel<kFmt420>, cudaFuncAttributeMaxDynamicSharedMemorySize, ent_smem_bytes(kFmt420)));
-    CUB(cudaFuncSetAttribute(entropy_walk_kernel<kFmt422>, cudaFuncAttributeMaxDynamicSharedMemorySize, ent_smem_bytes(kFmt422)));
-    CUB(cudaFuncSetAttribute(entropy_walk_kernel<kFmt444>, cudaFuncAttributeMaxDynamicSharedMemorySize, ent_smem_bytes(kFmt444)));
+    CUB(cudaFuncSetAttribute(entropy_walk_kernel<kFmt420, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ent_smem_bytes(kFmt420)));
+    CUB(cudaFuncSetAttribute(entropy_walk_kernel<kFmt422, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ent_smem_bytes(kFmt422)));
+    CUB(cudaFuncSetAttribute(entropy_walk_kernel<kFmt444, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ent_smem_bytes(kFmt444)));
+    CUB(cudaFuncSetAttribute(entropy_walk_kernel<kFmt420, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ent_smem_bytes(kFmt420)));
+    CUB(cudaFuncSetAttribute(entropy_walk_kernel<kFmt422, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ent_smem_bytes(kFmt422)));
+    CUB(cudaFuncSetAttribute(entropy_walk_kernel<kFmt444, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ent_smem_bytes(kFmt444)));
 
     const int B = s->max_batch;
     e->slots.resize(s->n_slots);
@@ -755,6 +791,8 @@ int h2j_create(const h2j_settings *s, h2j_encoder **out)
         CUB(cudaHostAlloc(&sl.h_offsets, sizeof(unsigned long long) * (B + 1), cudaHostAllocDefault));
         CUB(cudaHostAlloc(&sl.h_status, sizeof(int) * B, cudaHostAllocDefault));
         CUB(cudaHostAlloc(&sl.h_sizes, sizeof(long long) * B, cudaHostAllocDefault));
+        CUB(cudaMalloc(&sl.d_desc, sizeof(FrameDesc) * 2 * B));
+        CUB(cudaHostAlloc(&sl.h_desc, sizeof(FrameDesc) * 2 * B, cudaHostAllocDefault));
     }
     // single-frame staging (slot 0 only): planes in, JPEG / padded planes out
     {
@@ -978,6 +1016,173 @@ int h2j_submit_host(h2j_encoder *e, int slot, const uint8_t *frames, size_t fram
     rc = prepare_input(e, sl, sl.d_frames, dstride, n, width, height, &pipe_src);
     if (rc) return rc;
     rc = launch_pipeline(e, sl, pipe_src, n, TAIL_PACK);
+    if (rc) return rc;
+    sl.busy = true;
+    return H2J_OK;
+}
+
+int h2j_submit_device_list(h2j_encoder *e, int slot, int layout, const h2j_frame_desc *frames, int n)
+{
+    int rc = check_slot(e, slot);
+    if (rc) return rc;
+    Slot &sl = e->slots[slot];
+    if (sl.busy) return fail(e, H2J_ERR_BUSY, "slot %d has a batch in flight", slot);
+    if (!frames || n < 1 || n > e->s.max_batch) return fail(e, H2J_ERR_INVALID_ARG, "bad frames pointer or batch size %d (max %d)", n, e->s.max_batch);
+    if (layout != H2J_LAYOUT_PLANAR && layout != H2J_LAYOUT_SEMIPLANAR) return fail(e, H2J_ERR_INVALID_ARG, "bad layout %d", layout);
+    const bool sp = layout == H2J_LAYOUT_SEMIPLANAR;
+    const int fmt = e->s.chroma_format;
+    // every frame is checked before anything is enqueued or the slot's table is touched (a rejected call leaves the previous
+    // batch's table as it was); tab[i] is what the pipeline reads, tab[n + i] the copy's source
+    std::vector<FrameDesc> tab(2 * (size_t)n);
+    bool in_place = !e->force_sp_prepass;  // (semi-planar: every frame on 8-byte boundaries)
+    bool copies = false;
+    for (int i = 0; i < n; i++) {
+        const h2j_frame_desc &F = frames[i];
+        if (!F.data) return fail(e, H2J_ERR_INVALID_ARG, "frame %d: null data", i);
+        FrameLayout L;
+        rc = make_layout(e, F.data, 0, F.width, F.height, &L);
+        if (rc) return rc;
+        const int fcw = chroma_w(F.width, fmt), fch = chroma_h(F.height, fmt);
+        const int c_row = sp ? 2 * fcw : fcw;  // bytes in a chroma row
+        if (F.y_pitch < F.width || F.c_pitch < c_row)
+            return fail(e, H2J_ERR_INVALID_ARG, "frame %d: pitches %d / %d shorter than rows of %d / %d bytes", i, F.y_pitch, F.c_pitch, F.width, c_row);
+        if (sp && F.u_offset < (size_t)F.y_pitch * F.height)
+            return fail(e, H2J_ERR_INVALID_ARG, "frame %d: the pair plane starts inside the luma plane", i);
+        L.y_pitch = F.y_pitch;
+        L.c_pitch = F.c_pitch;
+        L.u_off = (long long)F.u_offset;
+        L.v_off = (long long)(sp ? F.u_offset : F.v_offset);
+        set_alignment(&L, F.data);
+        FrameDesc &src = tab[n + i];
+        src.L = L;
+        src.base = nullptr;
+        src.extent = (long long)std::max((size_t)F.y_pitch * (F.height - 1) + F.width,
+                                         std::max((size_t)L.u_off, (size_t)L.v_off) + (size_t)F.c_pitch * (fch - 1) + c_row);
+        tab[i].L = L;
+        tab[i].base = F.data;
+        tab[i].extent = 0;
+        if (sp) {
+            if ((uintptr_t)F.data % 8 || F.y_pitch % 8 || F.c_pitch % 8 || F.u_offset % 8) in_place = false;
+        } else if (!L.aligned8) {
+            copies = true;
+        }
+    }
+    memcpy(sl.h_desc, tab.data(), sizeof(FrameDesc) * 2 * n);
+    sl.list = true;  // the debug hooks answer from this table from here on
+    sl.n = n;
+    ON_DEVICE(e);
+    sl.n = n;
+    CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
+    // planar frames with rows off 8-byte boundaries are copied to a 16-byte pitch, all in one launch; the others are read
+    // where they are
+    if (copies && !sl.d_pitched) {
+        const size_t bytes = pitched_frame_bytes(e->s.max_width, e->s.max_height, fmt) * (size_t)e->s.max_batch;
+        if (cudaMalloc(&sl.d_pitched, bytes) != cudaSuccess) {  // no room for the copies: the bytewise path still works
+            cudaGetLastError();
+            sl.d_pitched = nullptr;
+            copies = false;
+        }
+    }
+    if (sp) copies = !in_place;  // a semi-planar batch is read in place or split completely
+    int copy_w = 0, copy_rows = 0;
+    for (int i = 0; i < n; i++) {
+        FrameDesc &d = sl.h_desc[i];
+        const int fch = chroma_h(d.L.h, fmt);
+        if (sp && in_place) {
+            d.L.aligned8 = 1;
+            d.L.aligned16 = ((uintptr_t)d.base % 16 == 0 && d.L.y_pitch % 16 == 0) ? 1 : 0;
+            d.L.nv12 = 1;
+        } else if (sp || (copies && !d.L.aligned8)) {
+            FrameDesc &src = sl.h_desc[n + i];
+            src.base = d.base;
+            src.L.aligned16 = ((uintptr_t)d.base % 16 == 0 && d.L.y_pitch % 16 == 0 && d.L.c_pitch % 16 == 0) ? 1 : 0;
+            d.L = pitched_layout(d.L);
+            d.L.frame_stride = 0;
+            d.base = sp ? sl.d_frames + (size_t)i * e->frame_bytes_cap
+                        : sl.d_pitched + (size_t)i * pitched_frame_bytes(e->s.max_width, e->s.max_height, fmt);
+            copy_w = std::max(copy_w, sp ? std::max(d.L.w, 2 * chroma_w(d.L.w, fmt)) : d.L.w);
+            copy_rows = std::max(copy_rows, d.L.h + (sp ? 1 : 2) * fch);
+        }
+    }
+    CU(e, cudaMemcpyAsync(sl.d_desc, sl.h_desc, sizeof(FrameDesc) * (copies ? 2 * n : n), cudaMemcpyHostToDevice, sl.stream));
+    if (copies) {
+        const dim3 grid((copy_w + 128 * 16 - 1) / (128 * 16), (copy_rows + kPlaneRowsPerCta - 1) / kPlaneRowsPerCta, n);
+        (sp ? nv12_to_i420_list_kernel : repitch_list_kernel)<<<grid, 128, 0, sl.stream>>>(sl.d_desc, n);
+        e->launches++;
+        CU(e, cudaGetLastError());
+    }
+    rc = launch_pipeline(e, sl, nullptr, n, TAIL_SIZES, true);
+    if (rc) return rc;
+    sl.busy = true;
+    return H2J_OK;
+}
+
+int h2j_submit_host_list(h2j_encoder *e, int slot, const uint8_t *const *frames, const int *widths, const int *heights, int n)
+{
+    int rc = check_slot(e, slot);
+    if (rc) return rc;
+    Slot &sl = e->slots[slot];
+    if (sl.busy) return fail(e, H2J_ERR_BUSY, "slot %d has a batch in flight", slot);
+    if (!frames || !widths || !heights || n < 1 || n > e->s.max_batch)
+        return fail(e, H2J_ERR_INVALID_ARG, "bad frames / sizes pointer or batch size %d (max %d)", n, e->s.max_batch);
+    const int fmt = e->s.chroma_format;
+    std::vector<FrameDesc> tab(2 * (size_t)n);  // (checked before the slot's table is touched, as h2j_submit_device_list)
+    bool copies = false;
+    for (int i = 0; i < n; i++) {
+        if (!frames[i]) return fail(e, H2J_ERR_INVALID_ARG, "frame %d: null pointer", i);
+        // frame i goes to its own place of the slot's frame buffer, sized for a tight frame at the maximum geometry
+        uint8_t *dev = sl.d_frames + (size_t)i * e->frame_bytes_cap;
+        FrameDesc &d = tab[i];
+        rc = make_layout(e, dev, 0, widths[i], heights[i], &d.L);
+        if (rc) return rc;
+        d.base = dev;
+        d.extent = 0;
+        FrameDesc &src = tab[n + i];
+        src.base = nullptr;
+        if (!d.L.aligned8) {  // odd widths: copied once more, to a 16-byte pitch
+            copies = true;
+            src.L = d.L;
+            src.base = dev;
+            src.extent = (long long)tight_frame_bytes(widths[i], heights[i], fmt);
+            d.L = pitched_layout(d.L);
+            d.L.frame_stride = 0;
+        }
+    }
+    memcpy(sl.h_desc, tab.data(), sizeof(FrameDesc) * 2 * n);
+    sl.list = true;  // the debug hooks answer from this table from here on
+    sl.n = n;
+    ON_DEVICE(e);
+    if (copies && !sl.d_pitched) {
+        const size_t bytes = pitched_frame_bytes(e->s.max_width, e->s.max_height, fmt) * (size_t)e->s.max_batch;
+        if (cudaMalloc(&sl.d_pitched, bytes) != cudaSuccess) {  // no room for the copies: the bytewise path still works
+            cudaGetLastError();
+            sl.d_pitched = nullptr;
+            copies = false;
+            for (int i = 0; i < n; i++)
+                if (sl.h_desc[n + i].base) sl.h_desc[i].L = sl.h_desc[n + i].L;
+        }
+    }
+    int copy_w = 0, copy_rows = 0;
+    for (int i = 0; copies && i < n; i++) {
+        FrameDesc &d = sl.h_desc[i];
+        if (!sl.h_desc[n + i].base) continue;
+        d.base = sl.d_pitched + (size_t)i * pitched_frame_bytes(e->s.max_width, e->s.max_height, fmt);
+        copy_w = std::max(copy_w, d.L.w);
+        copy_rows = std::max(copy_rows, d.L.h + 2 * chroma_h(d.L.h, fmt));
+    }
+    sl.n = n;
+    CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
+    for (int i = 0; i < n; i++)
+        CU(e, cudaMemcpyAsync(sl.d_frames + (size_t)i * e->frame_bytes_cap, frames[i], tight_frame_bytes(widths[i], heights[i], fmt),
+                              cudaMemcpyHostToDevice, sl.stream));
+    CU(e, cudaMemcpyAsync(sl.d_desc, sl.h_desc, sizeof(FrameDesc) * (copies ? 2 * n : n), cudaMemcpyHostToDevice, sl.stream));
+    if (copies) {
+        const dim3 grid((copy_w + 128 * 16 - 1) / (128 * 16), (copy_rows + kPlaneRowsPerCta - 1) / kPlaneRowsPerCta, n);
+        repitch_list_kernel<<<grid, 128, 0, sl.stream>>>(sl.d_desc, n);
+        e->launches++;
+        CU(e, cudaGetLastError());
+    }
+    rc = launch_pipeline(e, sl, nullptr, n, TAIL_PACK, true);
     if (rc) return rc;
     sl.busy = true;
     return H2J_OK;
@@ -1208,8 +1413,9 @@ int h2j_debug_frame_info(h2j_encoder *e, int slot, int frame, h2j_frame_info *in
     memset(info, 0, sizeof *info);
     info->qscale = t.qscale;
     info->mb_var_sum = t.mb_var_sum;
-    info->mcu_w = sl.L.mcu_w;
-    info->mcu_h = sl.L.mcu_h;
+    const FrameLayout &L = frame_layout(sl, frame);
+    info->mcu_w = L.mcu_w;
+    info->mcu_h = L.mcu_h;
     info->header_bytes = t.header_bytes;
     info->scan_bits = t.scan_bits;
     info->stuffed_ff = t.stuffed_ff;
@@ -1227,19 +1433,20 @@ int h2j_debug_coefficients(h2j_encoder *e, int slot, int frame, int16_t *out, si
     if (rc) return rc;
     Slot &sl = e->slots[slot];
     if (!out || frame < 0 || frame >= sl.n) return fail(e, H2J_ERR_INVALID_ARG, "bad frame index %d", frame);
-    const size_t need = (size_t)sl.L.n_blocks * 64;
+    const FrameLayout &L = frame_layout(sl, frame);
+    const size_t need = (size_t)L.n_blocks * 64;
     if (out_elems < need) return fail(e, H2J_ERR_OUTPUT_TOO_SMALL, "need %zu int16 elements", need);
     ON_DEVICE(e);
     CU(e, cudaStreamSynchronize(sl.stream));
     // tile images -> dense blocks; halfword 0 of a record is the DC difference, so the levels are rebuilt by
     // running the encoder's predictors (one per component, reset to 128) over the blocks in coding order
-    const int fmt = sl.L.fmt, tile_blocks = fmt_tile_blocks(fmt), tile_words = fmt_tile_image_words(fmt);
-    const int n_tiles = (sl.L.n_mcu + kTileMcus - 1) / kTileMcus;
+    const int fmt = L.fmt, tile_blocks = fmt_tile_blocks(fmt), tile_words = fmt_tile_image_words(fmt);
+    const int n_tiles = (L.n_mcu + kTileMcus - 1) / kTileMcus;
     std::vector<int16_t> img((size_t)n_tiles * tile_words * 2);
     CU(e, cudaMemcpy(img.data(), sl.d_images + (size_t)frame * e->images_cap * tile_words, img.size() * sizeof(int16_t),
                      cudaMemcpyDeviceToHost));
     int last_dc[3] = {128, 128, 128};
-    for (int b = 0; b < sl.L.n_blocks; b++) {
+    for (int b = 0; b < L.n_blocks; b++) {
         const TileRec tr = tile_rec_fmt(fmt, b % tile_blocks);
         const int16_t *rec = img.data() + ((size_t)(b / tile_blocks) * tile_words + (size_t)tr.sub * kSubImageWords + (size_t)tr.idx * kBlkWords) * 2;
         const int comp = block_component(fmt, b % fmt_mcu_blocks(fmt));

@@ -36,6 +36,16 @@ struct FrameLayout {
     int mb_w;          // 16x16 luma macroblocks per row (= mcu_w except at 4:4:4, whose MCUs are 8 wide): what K1 walks
 };
 
+// One frame of a list batch (h2j_submit_device_list / h2j_submit_host_list), where every frame has its own address and
+// size.  The *_list_kernel forms read their frame's entry of a per-slot table at blockIdx instead of taking one layout for
+// the whole batch by value; their grids are sized for the batch's largest frame, and CTAs past their own frame's extent
+// return before they touch any shared state.
+struct FrameDesc {
+    FrameLayout L;         // frame_stride unused (0)
+    const uint8_t *base;   // the frame's first luma byte
+    long long extent;      // copy sources (repitch / semi-planar split): bytes from base that may be read
+};
+
 // ---- chroma formats ------------------------------------------------------------------------------
 // libavcodec's mjpeg encoder codes (mjpegenc.c ff_mjpeg_encode_mb, mjpegenc_common.c ff_mjpeg_init_hvsample)
 //   4:2:0  16x16 MCUs of Y0 Y1 Y2 Y3 Cb Cr               (6 blocks; Y 2x2, chroma 1x1)      -- the reference's format

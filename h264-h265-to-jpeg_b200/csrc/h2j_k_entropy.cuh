@@ -223,12 +223,14 @@ static_assert(offsetof(FrameTab, hcode) % 16 == 0 && sizeof(FrameTab) % 16 == 0 
 
 // grid (tiles_per_frame, frames); FMT = the chroma format (h2j_common.cuh): a tile is 96 blocks (three units) at 4:2:0 and
 // 4:4:4, 128 blocks (four units) at 4:2:2; one thread per block, one warp per unit
-template <int FMT>
-__global__ void __launch_bounds__(fmt_tile_blocks(FMT)) entropy_walk_kernel(FrameLayout L, FrameTab *__restrict__ tabs,
+// LIST: a list batch (h2j_common.cuh FrameDesc); the grid has the largest frame's tiles, the ones past this frame's return
+template <int FMT, bool LIST>
+__global__ void __launch_bounds__(fmt_tile_blocks(FMT)) entropy_walk_kernel(FrameLayout L_, FrameTab *__restrict__ tabs,
                                                                    const uint32_t *__restrict__ images, long long images_cap,
                                                                    unsigned long long *__restrict__ unit_info, int units_cap,
                                                                    unsigned int *__restrict__ stage_alloc,  // [frame] words handed out
-                                                                   uint32_t *__restrict__ stage, long long stage_cap_words)
+                                                                   uint32_t *__restrict__ stage, long long stage_cap_words,
+                                                                   const FrameDesc *__restrict__ descs)
 {
     constexpr int kWarps = fmt_roles(FMT), kThreads = fmt_tile_blocks(FMT);       // units per tile = roles per tile
     constexpr int kImageWords = kWarps * kSubImageWords, kImageBytes = kImageWords * 4;
@@ -242,6 +244,8 @@ __global__ void __launch_bounds__(fmt_tile_blocks(FMT)) entropy_walk_kernel(Fram
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int f = blockIdx.y, tile = blockIdx.x;
+    const FrameLayout &L = LIST ? descs[f].L : L_;
+    if (LIST && tile * kThreads >= L.n_blocks) return;
     if (tid == 0) {
         mbar_init(&s_bar, 1);
         const uint32_t *src = images + ((long long)f * images_cap + tile) * kImageWords;
@@ -391,13 +395,16 @@ __global__ void __launch_bounds__(fmt_tile_blocks(FMT)) entropy_walk_kernel(Fram
 // UPW = units a warp concatenates: 32 (256 threads, throughput form) or 8 (1024 threads: the same group spread over four
 // times as many warps, for batches too small to fill the GPU with groups -- one 1080p frame is six groups, and a warp that
 // walks 32 units one after the other takes ~19 us).
-template <int UPW>
-__global__ void __launch_bounds__(kPlaceGroupUnits / UPW * 32) scan_place_kernel(FrameLayout L, FrameTab *__restrict__ tabs, FrameState *__restrict__ state,
+// LIST: a list batch (h2j_common.cuh FrameDesc); groups_per_frame is the largest frame's, and a ticket past its frame's groups
+// returns at once (nobody waits for it: the look-back only reads earlier groups of the same frame)
+template <int UPW, bool LIST>
+__global__ void __launch_bounds__(kPlaceGroupUnits / UPW * 32) scan_place_kernel(FrameLayout L_, FrameTab *__restrict__ tabs, FrameState *__restrict__ state,
                                                                    const unsigned long long *__restrict__ unit_info, int units_cap,
                                                                    const uint32_t *__restrict__ stage, long long stage_cap_words,
                                                                    unsigned long long *__restrict__ descs, int groups_per_frame,
                                                                    unsigned int *__restrict__ ticket, uint32_t *__restrict__ scan,
-                                                                   long long scan_cap_words, unsigned int *__restrict__ chunk_ff, int chunks_cap)
+                                                                   long long scan_cap_words, unsigned int *__restrict__ chunk_ff, int chunks_cap,
+                                                                   const FrameDesc *__restrict__ fdescs)
 {
     static_assert(kPlaceGroupUnits == kPlaceThreads, "one unit per thread in the scan (the first 256 threads)");
     static_assert(UPW == 32 || UPW == 8, "units per warp");
@@ -413,8 +420,10 @@ __global__ void __launch_bounds__(kPlaceGroupUnits / UPW * 32) scan_place_kernel
     __syncthreads();
     const int f = (int)(s_ticket / (unsigned)groups_per_frame);
     const int g = (int)(s_ticket % (unsigned)groups_per_frame);
+    const FrameLayout &L = LIST ? fdescs[f].L : L_;
     const int n_units = (L.n_blocks + kUnitBlocks - 1) / kUnitBlocks;
     const int u0 = g * kPlaceGroupUnits;
+    if (LIST && u0 >= n_units) return;
     const int n_here = min(kPlaceGroupUnits, n_units - u0);  // >= 1 by construction of groups_per_frame
     const unsigned long long *info = unit_info + (long long)f * units_cap;
 

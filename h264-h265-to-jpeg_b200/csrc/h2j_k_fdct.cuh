@@ -309,12 +309,15 @@ __device__ __forceinline__ void k2_flush(FrameState &st, int cls, const unsigned
     }
 }
 
-template <bool NV12>
-__global__ void __launch_bounds__(kFdctThreads, kFdctMinCtas) fdct_quant_kernel(const uint8_t *__restrict__ frames, FrameLayout L,
+// LIST: a list batch (h2j_common.cuh FrameDesc): the frame's layout and address come from descs[blockIdx.y], and the grid is
+// sized for the batch's largest frame (the CTAs past this frame's tiles return at the tile0 test)
+template <bool NV12, bool LIST>
+__global__ void __launch_bounds__(kFdctThreads, kFdctMinCtas) fdct_quant_kernel(const uint8_t *__restrict__ frames, FrameLayout L_,
                                                                      FrameState *__restrict__ state,
                                                                      const FrameTab *__restrict__ tabs,
                                                                      uint32_t *__restrict__ images,  // [frame][images_cap] tile images
-                                                                     long long images_cap, int tiles_per_cta)
+                                                                     long long images_cap, int tiles_per_cta,
+                                                                     const FrameDesc *__restrict__ descs)
 {
     __shared__ __align__(128) uint32_t s_img[2][kSubImageWords];
     __shared__ __align__(16) int s_q[64];
@@ -325,7 +328,8 @@ __global__ void __launch_bounds__(kFdctThreads, kFdctMinCtas) fdct_quant_kernel(
     const int f = blockIdx.y;
     const int lane = threadIdx.x;
     const int group = blockIdx.x / 3, warp = blockIdx.x - group * 3;  // `warp` = the role of this single-warp CTA
-    const uint8_t *base = frames + (long long)f * L.frame_stride;
+    const FrameLayout &L = LIST ? descs[f].L : L_;
+    const uint8_t *base = LIST ? descs[f].base : frames + (long long)f * L.frame_stride;
     const int n_tiles = (L.n_mcu + kTileMcus - 1) / kTileMcus;
     const int tile0 = group * tiles_per_cta;
     if (tile0 >= n_tiles) return;

@@ -111,12 +111,14 @@ __device__ __forceinline__ int sp_pred_rowsum(const BlockFetch &F, const PairHal
     return s;
 }
 
-template <int FMT, bool SP>
-__global__ void __launch_bounds__(kFdctThreads, kFdctMinCtas) fdct_quant_fmt_kernel(const uint8_t *__restrict__ frames, FrameLayout L,
+// LIST: a list batch, as fdct_quant_kernel
+template <int FMT, bool SP, bool LIST>
+__global__ void __launch_bounds__(kFdctThreads, kFdctMinCtas) fdct_quant_fmt_kernel(const uint8_t *__restrict__ frames, FrameLayout L_,
                                                                          FrameState *__restrict__ state,
                                                                          const FrameTab *__restrict__ tabs,
                                                                          uint32_t *__restrict__ images,  // [frame][images_cap] tile images
-                                                                         long long images_cap, int tiles_per_cta)
+                                                                         long long images_cap, int tiles_per_cta,
+                                                                         const FrameDesc *__restrict__ descs)
 {
     constexpr int kRoles = fmt_roles(FMT);
     __shared__ __align__(128) uint32_t s_img[2][kSubImageWords];
@@ -128,7 +130,8 @@ __global__ void __launch_bounds__(kFdctThreads, kFdctMinCtas) fdct_quant_fmt_ker
     const int f = blockIdx.y;
     const int lane = threadIdx.x;
     const int group = blockIdx.x / kRoles, role = blockIdx.x - group * kRoles;
-    const uint8_t *base = frames + (long long)f * L.frame_stride;
+    const FrameLayout &L = LIST ? descs[f].L : L_;
+    const uint8_t *base = LIST ? descs[f].base : frames + (long long)f * L.frame_stride;
     const int n_tiles = (L.n_mcu + kTileMcus - 1) / kTileMcus;
     const int tile0 = group * tiles_per_cta;
     if (tile0 >= n_tiles) return;

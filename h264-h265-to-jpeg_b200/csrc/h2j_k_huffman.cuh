@@ -396,9 +396,13 @@ __device__ uint8_t header_byte(int i, const HeaderPlan &h, const FrameTab *T, co
 // allowed two CTAs per SM, and 512 frames needed two waves of them).  The frame's CTA that finishes last writes the header.
 // Frame f's output starts at out + f * out_cap; jpeg_cap (<= out_cap) is the largest JPEG allowed, and no byte at or past
 // it is written.
+// LIST: a list batch; the SOF segment gets the frame's own size, descs[f].L.  (The defaults keep callers that launch K3 on its
+// own with the batch form's arguments -- tests/support/k3_shim.cu, tools/microbench/k3_phases.cu -- compiling unchanged.)
+template <bool LIST = false>
 __global__ void __launch_bounds__(kHuffGroup) huffman_kernel(FrameLayout L, FrameTab *__restrict__ tabs, FrameState *__restrict__ state,
                                                              int n_frames, uint8_t *__restrict__ out, long long out_cap, long long jpeg_cap,
-                                                             const char *__restrict__ comment, int comment_len)
+                                                             const char *__restrict__ comment, int comment_len,
+                                                             const FrameDesc *__restrict__ descs = nullptr)
 {
     __shared__ HuffScratch scratch;
     __shared__ int s_last;
@@ -425,7 +429,7 @@ __global__ void __launch_bounds__(kHuffGroup) huffman_kernel(FrameLayout L, Fram
     const HeaderPlan h = header_plan(nvals, comment_len);
     uint8_t *o = out + (long long)f * out_cap;
     for (int i = tid; i < h.total; i += kHuffGroup)
-        if (i < jpeg_cap) o[i] = header_byte(i, h, T, L, comment, comment_len);
+        if (i < jpeg_cap) o[i] = header_byte(i, h, T, LIST ? descs[f].L : L, comment, comment_len);
     if (tid == 0) {
         T->header_bytes = h.total;
         if (h.total > jpeg_cap) T->status = -4;

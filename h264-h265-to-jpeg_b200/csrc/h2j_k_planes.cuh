@@ -10,12 +10,16 @@ namespace h2j {
 // ------------------------------------------------------------------------------------------------
 // The CTA that finishes a frame last (completion counter) turns the sum into the frame's qscale (ratecontrol.c first
 // I picture) and publishes the quantiser tables (mpegvideo_enc.c encode_picture + ff_convert_matrix) for K2.
-__global__ void __launch_bounds__(128) mbvar_kernel(const uint8_t *__restrict__ frames, FrameLayout L,
+// LIST: a list batch (h2j_common.cuh FrameDesc): the grid has the largest frame's mcu_h, rows past this frame's return
+template <bool LIST>
+__global__ void __launch_bounds__(128) mbvar_kernel(const uint8_t *__restrict__ frames, FrameLayout L_,
                                                     FrameState *__restrict__ state, const uint8_t *__restrict__ qscale_lut,
-                                                    FrameTab *__restrict__ tabs)
+                                                    FrameTab *__restrict__ tabs, const FrameDesc *__restrict__ descs)
 {
     const int f = blockIdx.y, my = blockIdx.x;
-    const uint8_t *Y = frames + (long long)f * L.frame_stride;
+    const FrameLayout &L = LIST ? descs[f].L : L_;
+    if (LIST && my >= L.mcu_h) return;
+    const uint8_t *Y = LIST ? descs[f].base : frames + (long long)f * L.frame_stride;
     int local = 0;
     for (int mx = threadIdx.x; mx < L.mb_w; mx += blockDim.x) {  // 16x16 macroblocks (= MCUs except at 4:4:4)
         unsigned sum = 0, norm = 0;
@@ -61,7 +65,7 @@ __global__ void __launch_bounds__(128) mbvar_kernel(const uint8_t *__restrict__ 
         atomicAdd(&state[f].var_sum, (unsigned long long)t);
         __threadfence();
         const unsigned done = atomicAdd(&state[f].k1_done, 1u);
-        s_last = done == gridDim.x - 1;
+        s_last = done == (LIST ? (unsigned)L.mcu_h : gridDim.x) - 1;
         if (s_last) {
             __threadfence();
             const long long var = (long long)atomicAdd(&state[f].var_sum, 0ull);  // every CTA's share is in
@@ -143,9 +147,10 @@ __global__ void __launch_bounds__(128) convert_pad_kernel(const uint8_t *__restr
 // CTA: one row per CTA made 400 k CTAs of 120 busy threads for 256 frames).
 // 16 bytes per thread where pitch, base and width allow, bytes otherwise.
 // ------------------------------------------------------------------------------------------------
+// `pairs`: Cb/Cr pairs per chroma row (L.c_pitch of a tight copy; a list batch writes a 16-byte row pitch, wider than that)
 constexpr int kPlaneRowsPerCta = 16;
-__global__ void __launch_bounds__(128) nv12_to_i420_kernel(const uint8_t *__restrict__ src, long long src_stride, int pitch, long long uv_off,
-                                                           uint8_t *__restrict__ dst, FrameLayout L, int src_aligned16)
+__device__ __forceinline__ void nv12_to_i420_body(const uint8_t *__restrict__ src, long long src_stride, int pitch, int uv_pitch, long long uv_off,
+                                                  uint8_t *__restrict__ dst, const FrameLayout &L, int src_aligned16, int pairs)
 {
     const int f = blockIdx.z;
     const uint8_t *S = src + (long long)f * src_stride;
@@ -162,22 +167,36 @@ __global__ void __launch_bounds__(128) nv12_to_i420_kernel(const uint8_t *__rest
             for (int i = 0; i < 16 && x0 + i < L.w; i++) d[i] = s[i];
     } else if (row < L.h + fch) {
         const int r = row - L.h;
-        if (x0 >= 2 * L.c_pitch) continue;  // c_pitch = ceil(w / 2) pairs per row
-        const uint8_t *s = S + uv_off + (long long)r * pitch + x0;
+        if (x0 >= 2 * pairs) continue;
+        const uint8_t *s = S + uv_off + (long long)r * uv_pitch + x0;
         uint8_t *du = D + L.u_off + (long long)r * L.c_pitch + (x0 >> 1), *dv = D + L.v_off + (long long)r * L.c_pitch + (x0 >> 1);
-        if (src_aligned16 && (uv_off & 15) == 0 && L.aligned8 && x0 + 16 <= 2 * L.c_pitch) {
+        if (src_aligned16 && (uv_off & 15) == 0 && L.aligned8 && x0 + 16 <= 2 * pairs) {
             const uint4 v = ldg128(s);
             const unsigned u0 = __byte_perm(v.x, v.y, 0x6420), u1 = __byte_perm(v.z, v.w, 0x6420);
             const unsigned w0 = __byte_perm(v.x, v.y, 0x7531), w1 = __byte_perm(v.z, v.w, 0x7531);
             *reinterpret_cast<uint2 *>(du) = make_uint2(u0, u1);
             *reinterpret_cast<uint2 *>(dv) = make_uint2(w0, w1);
         } else {
-            for (int i = 0; i < 8 && (x0 >> 1) + i < L.c_pitch; i++) {
+            for (int i = 0; i < 8 && (x0 >> 1) + i < pairs; i++) {
                 du[i] = s[2 * i];
                 dv[i] = s[2 * i + 1];
             }
         }
     }
+}
+__global__ void __launch_bounds__(128) nv12_to_i420_kernel(const uint8_t *__restrict__ src, long long src_stride, int pitch, long long uv_off,
+                                                           uint8_t *__restrict__ dst, FrameLayout L, int src_aligned16)
+{
+    nv12_to_i420_body(src, src_stride, pitch, pitch, uv_off, dst, L, src_aligned16, L.c_pitch);
+}
+// a list batch: descs[f] is where the pipeline reads frame f (planar, pitched_layout), descs[n + f] the semi-planar source
+// (L.y_pitch / L.c_pitch: its pitches, L.u_off: its pair plane, L.aligned16: base and pitches are 16-byte aligned); grid
+// sized for the largest frame
+__global__ void __launch_bounds__(128) nv12_to_i420_list_kernel(const FrameDesc *__restrict__ descs, int n)
+{
+    const FrameDesc &d = descs[blockIdx.z], &s = descs[n + blockIdx.z];
+    const int fcw = (d.L.w + (1 << fmt_hshift(d.L.fmt)) - 1) >> fmt_hshift(d.L.fmt);
+    nv12_to_i420_body(s.base, 0, s.L.y_pitch, s.L.c_pitch, s.L.u_off, const_cast<uint8_t *>(d.base), d.L, s.L.aligned16, fcw);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -188,10 +207,10 @@ __global__ void __launch_bounds__(128) nv12_to_i420_kernel(const uint8_t *__rest
 // width, ceil-divided by the subsampling (not the source pitch); the padding bytes of a row are never read by the pipeline
 // (edges are replicated from the last real sample).
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) repitch_kernel(const uint8_t *__restrict__ src, FrameLayout T,  // layout of the source
-                                                      int fch,                                         // rows of a chroma plane
-                                                      uint8_t *__restrict__ dst, FrameLayout P,        // pitched layout of the copy
-                                                      const uint8_t *src_begin, const uint8_t *src_end)  // what may be read
+__device__ __forceinline__ void repitch_body(const uint8_t *__restrict__ src, const FrameLayout &T,  // the source frames, their layout
+                                             int fch,                                               // rows of a chroma plane
+                                             uint8_t *__restrict__ dst, const FrameLayout &P,       // the copies, their pitched layout
+                                             const uint8_t *src_begin, const uint8_t *src_end)      // what may be read
 {
     const int f = blockIdx.z;
     const int fcw = (T.w + (1 << fmt_hshift(T.fmt)) - 1) >> fmt_hshift(T.fmt);  // (T.c_pitch of a tight source)
@@ -218,6 +237,20 @@ __global__ void __launch_bounds__(128) repitch_kernel(const uint8_t *__restrict_
         for (int i = 0; i < 16 && x0 + i < pw; i++) d[i] = s[i];
     }
     }
+}
+__global__ void __launch_bounds__(128) repitch_kernel(const uint8_t *__restrict__ src, FrameLayout T, int fch, uint8_t *__restrict__ dst,
+                                                      FrameLayout P, const uint8_t *src_begin, const uint8_t *src_end)
+{
+    repitch_body(src, T, fch, dst, P, src_begin, src_end);
+}
+// a list batch: descs[f] is the copy the pipeline reads, descs[n + f] the source; frames read in place have no source
+// (base == nullptr) and return at once.  Grid sized for the largest frame that is copied.
+__global__ void __launch_bounds__(128) repitch_list_kernel(const FrameDesc *__restrict__ descs, int n)
+{
+    const FrameDesc &d = descs[blockIdx.z], &s = descs[n + blockIdx.z];
+    if (!s.base) return;
+    const int fch = (s.L.h + fmt_vshift(s.L.fmt)) >> fmt_vshift(s.L.fmt);
+    repitch_body(s.base, s.L, fch, const_cast<uint8_t *>(d.base), d.L, s.base, s.base + s.extent);
 }
 
 // ------------------------------------------------------------------------------------------------

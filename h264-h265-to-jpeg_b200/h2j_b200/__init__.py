@@ -66,6 +66,23 @@ class Settings(C.Structure):
     ]
 
 
+LAYOUT_PLANAR = 0
+LAYOUT_SEMIPLANAR = 1
+
+
+class FrameDesc(C.Structure):
+    """h2j_frame_desc: one device frame of a list submit (pitches and offsets in bytes)"""
+    _fields_ = [
+        ("data", C.c_void_p),
+        ("width", C.c_int),
+        ("height", C.c_int),
+        ("y_pitch", C.c_int),
+        ("c_pitch", C.c_int),
+        ("u_offset", C.c_size_t),
+        ("v_offset", C.c_size_t),
+    ]
+
+
 class FrameInfo(C.Structure):
     _fields_ = [
         ("qscale", C.c_int),
@@ -90,7 +107,8 @@ EXPORTS = [
     "h2j_alloc_pinned", "h2j_free_pinned", "h2j_convert_pad", "h2j_debug_frame_info", "h2j_debug_coefficients",
     "h2j_slot_kernel_ms", "h2j_set_profile", "h2j_slot_total_ms", "h2j_kernel_launches", "h2j_slot_set_stream",
     "h2j_slot_wait_event", "h2j_device_count", "h2j_debug_set_knob", "h2j_debug_read_device", "h2j_stream_copy",
-    "h2j_submit_device_semiplanar16", "h2j_submit_device_pitched16", "h2j_encode_frame16",
+    "h2j_submit_device_semiplanar16", "h2j_submit_device_pitched16", "h2j_encode_frame16", "h2j_submit_device_list",
+    "h2j_submit_host_list",
 ]
 
 _lib = None
@@ -127,6 +145,8 @@ def load_library() -> C.CDLL:
     lib.h2j_submit_device_semiplanar16.argtypes = [vp, ci, vp, sz, ci, sz, ci, ci, ci, ci]
     lib.h2j_submit_device_pitched16.argtypes = [vp, ci, vp, sz, ci, ci, sz, sz, ci, ci, ci, ci]
     lib.h2j_encode_frame16.argtypes = [vp, C.POINTER(vp), C.POINTER(ci), ci, ci, ci, vp, sz, C.POINTER(sz)]
+    lib.h2j_submit_device_list.argtypes = [vp, ci, ci, C.POINTER(FrameDesc), ci]
+    lib.h2j_submit_host_list.argtypes = [vp, ci, C.POINTER(vp), C.POINTER(ci), C.POINTER(ci), ci]
     lib.h2j_collect.argtypes = [vp, ci, vp, sz, C.POINTER(sz), C.POINTER(ci)]
     lib.h2j_collect_device.argtypes = [vp, ci, C.POINTER(vp), C.POINTER(sz), C.POINTER(sz), C.POINTER(ci)]
     lib.h2j_wait.argtypes = [vp, ci]
@@ -384,6 +404,21 @@ class Encoder:
         """Planar frames of 16-bit words in device memory at any layout (pitches and offsets in bytes)."""
         self._check(self._lib.h2j_submit_device_pitched16(self._h, slot, d_frames_ptr, frame_stride, y_pitch, c_pitch, u_offset, v_offset,
                                                           bit_depth, n, width, height))
+        self._n_in_slot[slot] = n
+
+    def submit_device_list(self, slot: int, layout: int, descs: Sequence[FrameDesc]) -> None:
+        """Device frames each at its own address and of its own size (LAYOUT_PLANAR or LAYOUT_SEMIPLANAR for all)."""
+        arr = (FrameDesc * max(1, len(descs)))(*descs)
+        self._check(self._lib.h2j_submit_device_list(self._h, slot, layout, arr, len(descs)))
+        self._n_in_slot[slot] = len(descs)
+
+    def submit_host_list(self, slot: int, frames: Sequence[int], sizes: Sequence[Tuple[int, int]]) -> None:
+        """Tight planar frames in host memory (addresses, as from ndarray.ctypes.data), each of its own (width, height)."""
+        n = len(frames)
+        ptrs = (C.c_void_p * max(1, n))(*frames)
+        ws = (C.c_int * max(1, n))(*[w for w, _ in sizes])
+        hs = (C.c_int * max(1, n))(*[h for _, h in sizes])
+        self._check(self._lib.h2j_submit_host_list(self._h, slot, ptrs, ws, hs, n))
         self._n_in_slot[slot] = n
 
     def read_device(self, d_ptr: int, nbytes: int) -> bytes:

@@ -11,6 +11,7 @@
 // CUDA context and its buffers are far too expensive for that, so Encoder objects are thin and share the Hub.
 #include "Encoder.h"
 
+#include <algorithm>
 #include <cerrno>
 #include <condition_variable>
 #include <cstdio>
@@ -84,14 +85,16 @@ void copy_planes(uint8_t *p, const H2JFrameView &f)
     }
 }
 
-// One batch on its way: pinned staging for up to `cap_frames` same-sized pictures, their output paths, pinned output.
+// One batch on its way: pinned staging for up to `cap_frames` pictures of any sizes, each tight at its own offset, their
+// output paths, pinned output.
 struct Job {
     uint8_t *in = nullptr;
     size_t in_bytes = 0;
+    size_t used = 0;           // bytes of `in` reserved by pictures so far
+    std::vector<size_t> at;    // where picture k starts in `in`
+    std::vector<int> ws, hs;   // its size
     uint8_t *out = nullptr;
     size_t out_bytes = 0;
-    size_t slot_bytes = 0;  // distance between two pictures in `in`
-    int w = 0, h = 0;
     int cap_frames = 0;
     int reserved = 0;  // pictures that have a place in this job
     int filled = 0;    // ... and whose planes have been copied in
@@ -130,6 +133,8 @@ struct Hub {
     // batch scope
     bool batching = false;
     int batch_frames = 0;
+    size_t room = 0;           // pinned bytes per picture a new job gets: the largest picture of the scope so far
+    int batches = 0;           // jobs handed to a GPU since h2j_host_batch_begin
     std::vector<std::unique_ptr<Job>> jobs;
     Job *filling = nullptr;
     int written = 0, failed = 0;
@@ -262,19 +267,24 @@ void worker_main(Hub *Hp, DeviceCtx *Dp)
             }
         }
         if (j) {
+            int jw = 0, jh = 0;  // the encoder is sized for the job's largest picture
+            for (int k = 0; k < j->reserved; k++) {
+                jw = std::max(jw, j->ws[k]);
+                jh = std::max(jh, j->hs[k]);
+            }
             // a geometry or batch size the encoder was not built for (or new settings): everything in flight leaves first
-            const bool fits = !stale && D.batch_box.enc && j->w <= D.batch_box.max_w && j->h <= D.batch_box.max_h && j->cap_frames <= D.batch_box.max_batch;
+            const bool fits = !stale && D.batch_box.enc && jw <= D.batch_box.max_w && jh <= D.batch_box.max_h && j->cap_frames <= D.batch_box.max_batch;
             if (!fits)
                 while (!running.empty()) finish_oldest();
             if (stale) drop_box(D.batch_box);
-            bool ok = ensure_box(D.batch_box, D.device, H.range_mode, j->w, j->h, j->cap_frames, kSlotsPerDevice);
+            bool ok = ensure_box(D.batch_box, D.device, H.range_mode, jw, jh, j->cap_frames, kSlotsPerDevice);
             // pinned room for the batch's JPEGs: 4 bits per pixel to start with (camera pictures at the reference's settings
             // come to about 1 bit); a batch that needs more is collected again into a buffer of exactly its size (finish_job)
-            size_t per_picture = (size_t)j->w * j->h / 2 + 65536;
-            if (per_picture > D.batch_box.cap) per_picture = D.batch_box.cap;
-            if (ok && j->out_bytes < per_picture * (size_t)j->cap_frames) {
+            size_t out_guess = 0;
+            for (int k = 0; k < j->reserved; k++) out_guess += std::min((size_t)j->ws[k] * j->hs[k] / 2 + 65536, D.batch_box.cap);
+            if (ok && j->out_bytes < out_guess) {
                 if (j->out) h2j_free_pinned(j->out);
-                j->out_bytes = per_picture * (size_t)j->cap_frames;
+                j->out_bytes = out_guess;
                 j->out = static_cast<uint8_t *>(h2j_alloc_pinned(j->out_bytes));
                 if (!j->out) {
                     LOG("%s line=%d | pinned allocation of %zu bytes failed", __PRETTY_FUNCTION__, __LINE__, j->out_bytes);
@@ -284,7 +294,9 @@ void worker_main(Hub *Hp, DeviceCtx *Dp)
             }
             const int slot = next_slot;
             if (ok) {
-                const int rc = h2j_submit_host(D.batch_box.enc, slot, j->in, j->slot_bytes, j->reserved, j->w, j->h);
+                std::vector<const uint8_t *> pics(j->reserved);
+                for (int k = 0; k < j->reserved; k++) pics[k] = j->in + j->at[k];
+                const int rc = h2j_submit_host_list(D.batch_box.enc, slot, pics.data(), j->ws.data(), j->hs.data(), j->reserved);
                 if (rc != H2J_OK) {
                     LOG("h2j_submit_host of %d frames failed, rc=%d (%s), error=%s", j->reserved, rc, h2j_status_string(rc), h2j_last_error(D.batch_box.enc));
                     ok = false;
@@ -323,6 +335,7 @@ void route_job(Hub &H, Job *j)
         }
     }
     DeviceCtx &D = *H.devices[best];
+    H.batches++;
     D.queue.push_back(j);
     D.inflight++;
     H.cv_queue.notify_all();
@@ -342,16 +355,32 @@ void seal_job(Hub &H, Job *j)
     }
 }
 
-// (lock held on entry and exit) a job with room for a w x h picture: the one being filled, or a free one (re-cut if it was
-// made for smaller pictures), or a new one while fewer than two per device plus one exist; otherwise wait for one
-Job *job_for(Hub &H, std::unique_lock<std::mutex> &lock, int w, int h)
+// (lock held) give a job that is being filled room for `cap_frames` pictures of H.room bytes.  Only while no copy into it is
+// in progress (filled == reserved): the pictures already in are moved over.
+bool grow_job(Hub &H, Job *j)
 {
-    const size_t need = (i420_bytes(w, h) + 255) / 256 * 256;
+    const size_t bytes = H.room * (size_t)j->cap_frames;
+    if (j->filled != j->reserved || bytes <= j->in_bytes) return false;
+    uint8_t *p = static_cast<uint8_t *>(h2j_alloc_pinned(bytes));
+    if (!p) return false;
+    if (j->used) memcpy(p, j->in, j->used);
+    h2j_free_pinned(j->in);
+    j->in = p;
+    j->in_bytes = bytes;
+    return true;
+}
+
+// (lock held on entry and exit) a job with room for a w x h picture: the one being filled (pictures of any sizes share a
+// job), or a free one (re-cut if it was made for smaller pictures), or a new one while fewer than two per device plus one
+// exist; otherwise wait for one
+Job *job_for(Hub &H, std::unique_lock<std::mutex> &lock, int w, int h, size_t need)
+{
+    if (need > H.room) H.room = need;
     for (;;) {
         if (H.filling) {
             Job *j = H.filling;
-            if (j->w == w && j->h == h && j->reserved < j->cap_frames) return j;
-            seal_job(H, j);  // another size: it goes as it is
+            if (j->used + need <= j->in_bytes || grow_job(H, j)) return j;
+            seal_job(H, j);  // no pinned room left for this picture: it goes as it is
         }
         Job *free_job = nullptr;
         for (auto &jp : H.jobs)
@@ -370,9 +399,9 @@ Job *job_for(Hub &H, std::unique_lock<std::mutex> &lock, int w, int h)
         }
         Job *j = free_job;
         j->busy = true;
-        if (j->in_bytes < need * (size_t)H.batch_frames) {
+        if (j->in_bytes < H.room * (size_t)H.batch_frames) {
             if (j->in) h2j_free_pinned(j->in);
-            j->in_bytes = need * (size_t)H.batch_frames;
+            j->in_bytes = H.room * (size_t)H.batch_frames;
             j->in = static_cast<uint8_t *>(h2j_alloc_pinned(j->in_bytes));
             if (!j->in) {
                 LOG("%s line=%d | pinned allocation of %zu bytes failed", __PRETTY_FUNCTION__, __LINE__, j->in_bytes);
@@ -381,9 +410,10 @@ Job *job_for(Hub &H, std::unique_lock<std::mutex> &lock, int w, int h)
                 return nullptr;
             }
         }
-        j->slot_bytes = need;
-        j->w = w;
-        j->h = h;
+        j->used = 0;
+        j->at.clear();
+        j->ws.clear();
+        j->hs.clear();
         j->cap_frames = H.batch_frames;
         j->reserved = j->filled = 0;
         j->sealed = false;
@@ -399,16 +429,22 @@ bool enqueue_frame(Hub &H, const H2JFrameView &f, const char *path)
 {
     std::unique_lock<std::mutex> lock(H.mu);
     if (!H.batching) return false;
-    Job *j = job_for(H, lock, f.width, f.height);
+    const size_t need = (i420_bytes(f.width, f.height) + 255) / 256 * 256;
+    Job *j = job_for(H, lock, f.width, f.height, need);
     if (!j) return false;
-    const int k = j->reserved++;
+    j->reserved++;
+    const size_t at = j->used;
+    j->used += need;
+    j->at.push_back(at);
+    j->ws.push_back(f.width);
+    j->hs.push_back(f.height);
     j->paths.emplace_back(path);
     if (j->reserved == j->cap_frames) {  // full: the next picture opens another job
         j->sealed = true;
         H.filling = nullptr;
     }
     lock.unlock();
-    copy_planes(j->in + (size_t)k * j->slot_bytes, f);
+    copy_planes(j->in + at, f);
     lock.lock();
     j->filled++;
     if (j->sealed && j->filled == j->reserved) route_job(H, j);
@@ -436,6 +472,8 @@ extern "C" int h2j_host_batch_begin(int max_frames)
     H.batching = true;
     H.batch_frames = max_frames;
     H.written = H.failed = 0;
+    H.room = 0;
+    H.batches = 0;
     return 0;
 }
 
@@ -465,6 +503,13 @@ extern "C" void h2j_host_configure(int cuda_device, int range_mode)
     }
     H.only_device = cuda_device >= 0 ? cuda_device : -1;
     H.range_mode = range_mode;
+}
+
+extern "C" int h2j_host_batches_submitted(void)
+{
+    Hub &H = hub();
+    std::lock_guard<std::mutex> lock(H.mu);
+    return H.batches;
 }
 
 extern "C" int h2j_host_devices_in_use(void)

@@ -87,8 +87,9 @@ extern "C" void h2j_host_configure(int cuda_device, int range_mode);
 // Batch scope for services that convert many pictures (the reference has no such call: a loop over
 // IDecoder::H265ToJpeg is what it offers, main.cpp:37-65).  Between begin and end, yuv2Jpeg() -- and therefore the
 // unchanged IDecoder::H265ToJpeg() that calls it (reference src/Decoder.cpp:349) -- only copies the decoded planes into
-// pinned staging and returns true; it may be called from any number of threads.  Runs of equal-sized pictures are
-// encoded `max_frames` at a time: a full batch goes to a GPU worker thread (one per device in use, two batches in flight
+// pinned staging and returns true; it may be called from any number of threads.  Pictures of any sizes, in any order, are
+// encoded `max_frames` at a time (each gets pinned room for its own size; a picture that no longer fits the batch's room
+// closes it early): a full batch goes to a GPU worker thread (one per device in use, two batches in flight
 // per device so that the upload of one runs under the kernels of the other), which also writes the JPEG files, while
 // the callers already fill the next batch.  h2j_host_batch_end() drains everything and returns the number of files
 // written (-1 outside a scope); *failed receives the number of pictures that could not be encoded or saved.
@@ -98,5 +99,7 @@ extern "C" int h2j_host_batch_begin(int max_frames);
 extern "C" int h2j_host_batch_end(int *failed);
 // Devices that currently hold GPU state for this process (inspection).
 extern "C" int h2j_host_devices_in_use(void);
+// Batches the scope has handed to a GPU since h2j_host_batch_begin (inspection).
+extern "C" int h2j_host_batches_submitted(void);
 
 #endif  // H265TOJPEG_ENCODER_H

@@ -32,6 +32,8 @@
 extern "C" {
 #endif
 
+/* Bumped when an existing entry point or struct changes.  Additions (the semi-planar, pitched, 16-bit and list submits)
+ * leave it as it is: a caller built against an older header keeps working unchanged. */
 #define H2J_ABI_VERSION 3
 
 typedef enum h2j_status {
@@ -197,6 +199,40 @@ int h2j_submit_device_pitched16(h2j_encoder *e, int slot, const uint8_t *d_frame
                                 int c_pitch, size_t u_offset, size_t v_offset, int bit_depth, int n, int width, int height);
 int h2j_encode_frame16(h2j_encoder *e, const uint8_t *const planes[3], const int strides[3], int bit_depth, int width,
                        int height, uint8_t *out, size_t out_capacity, size_t *out_size);
+
+/*
+ * Lists of frames, each at its own address and of its own size (at most max_width x max_height): frames of several
+ * streams at different resolutions in one batch, or a decoder's surfaces where they are, without gathering them into one
+ * strided buffer first.  One layout kind per call; chroma format, range_mode and fixed_qscale are the encoder's.  Frame i's
+ * JPEG is byte-identical to the one h2j_submit_device writes for that frame alone.  Collect with h2j_collect /
+ * h2j_collect_device as for the other submits.  The device frames are read on the slot's stream, under the stream-ordering
+ * rule above.
+ * h2j_submit_device_list: n device frames.  H2J_LAYOUT_PLANAR: luma rows y_pitch apart from data, Cb and Cr planes at
+ *   u_offset / v_offset with rows c_pitch apart; frames whose rows are not all on 8-byte boundaries are copied to a 16-byte
+ *   pitch (one extra kernel for all of them), the others are read where they are.  H2J_LAYOUT_SEMIPLANAR: NV12 / NV16 /
+ *   NV24 by the encoder's chroma format, the pair plane at u_offset with rows c_pitch apart (v_offset unused); read in
+ *   place when every frame's pointer, pitches and offset are multiples of 8, otherwise the whole batch is split into
+ *   planes first by one extra kernel.
+ * h2j_submit_host_list: n tight planar frames in host memory (the layout of h2j_submit_host); frame i is uploaded with
+ *   one copy.
+ * H2J_ERR_INVALID_ARG: a null pointer, n < 1 or n > max_batch, a pitch shorter than its plane's row (semi-planar chroma:
+ * 2 * pairs per row), or a pair plane that starts inside the luma plane.  H2J_ERR_UNSUPPORTED: a frame outside 2..65500 or
+ * above the encoder's maximum.  H2J_ERR_BUSY: the slot has a batch in flight.
+ */
+typedef enum h2j_layout { H2J_LAYOUT_PLANAR = 0, H2J_LAYOUT_SEMIPLANAR = 1 } h2j_layout;
+
+typedef struct h2j_frame_desc {
+    const uint8_t *data;   /* device address of the frame's first luma byte */
+    int width, height;
+    int y_pitch;           /* bytes between luma rows */
+    int c_pitch;           /* bytes between chroma rows (semi-planar: rows of Cb/Cr pairs) */
+    size_t u_offset;       /* bytes from data to the Cb plane (semi-planar: to the pair plane) */
+    size_t v_offset;       /* bytes from data to the Cr plane (semi-planar: unused) */
+} h2j_frame_desc;
+
+int h2j_submit_device_list(h2j_encoder *e, int slot, int layout, const h2j_frame_desc *frames, int n);
+int h2j_submit_host_list(h2j_encoder *e, int slot, const uint8_t *const *frames, const int *widths, const int *heights, int n);
+
 int h2j_collect(h2j_encoder *e, int slot, uint8_t *out, size_t out_capacity, size_t *offsets, int *status);
 int h2j_collect_device(h2j_encoder *e, int slot, const uint8_t **d_out, size_t *d_frame_capacity, size_t *sizes,
                        int *status);
