@@ -338,6 +338,7 @@ int enqueue_single_tail(h2j_encoder *e, Slot &sl);
 
 constexpr int kFdctMaxTilesPerCta = 16;  // K2: upper bound of consecutive tiles one CTA walks (h2j_debug_set_knob may force any)
 constexpr int kStuffCtas = 32;           // K5 CTAs per frame
+constexpr size_t kMaxCommentBytes = 65535 - 3;  // settings.comment: a COM segment's length field counts the text, its NUL and itself
 
 // the K2 instantiation for the layout kind (chroma format, semi-planar chroma read in place) and the batch kind
 template <bool LIST>
@@ -700,6 +701,8 @@ int h2j_create(const h2j_settings *s, h2j_encoder **out)
         s->chroma_format < H2J_CHROMA_420 || s->chroma_format > H2J_CHROMA_444 ||
         s->max_jpeg_bytes > ((size_t)256 << 20))  // bit positions inside a frame's scan are 32-bit
         return fail(nullptr, H2J_ERR_INVALID_ARG, "bad settings");
+    if (s->comment && strlen(s->comment) > kMaxCommentBytes)
+        return fail(nullptr, H2J_ERR_INVALID_ARG, "comment of %zu bytes: at most %zu fit a COM segment", strlen(s->comment), kMaxCommentBytes);
     int ndev = 0;
     cudaError_t ce = cudaGetDeviceCount(&ndev);
     if (ce != cudaSuccess || ndev == 0)

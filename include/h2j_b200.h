@@ -80,7 +80,9 @@ typedef struct h2j_settings {
     size_t max_jpeg_bytes; /* largest JPEG a frame may have, exactly (a larger one fails with H2J_ERR_OUTPUT_TOO_SMALL);
                               0 = 2 MiB, the reference's HEAP_SIZE; at most 256 MiB */
     const char *comment;   /* COM segment payload; NULL = "Lavc58.117.101", the LIBAVCODEC_IDENT of the
-                              ffmpeg build the reference links on x86-64 (lib/ffmpeg/x86_64_shared) */
+                              ffmpeg build the reference links on x86-64 (lib/ffmpeg/x86_64_shared); at most
+                              65,532 bytes, the most a COM segment's 16-bit length (text + NUL + the field's own two
+                              bytes) can hold -- a longer one fails with H2J_ERR_INVALID_ARG */
     int profile;           /* non-zero: bracket every kernel with CUDA events (see h2j_slot_kernel_ms) */
     int chroma_format;     /* h2j_chroma_format of every frame this encoder is given (default H2J_CHROMA_420) */
 } h2j_settings;

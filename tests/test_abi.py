@@ -52,6 +52,10 @@ def test_bad_settings_rejected():
     with pytest.raises(h2j_b200.H2JError) as ei:
         h2j_b200.Encoder(max_width=1, max_height=1)
     assert ei.value.status == h2j_b200.ERR_INVALID_ARG
+    # a comment whose COM segment length (text + NUL + 2) does not fit 16 bits; checked before any device is looked for
+    with pytest.raises(h2j_b200.H2JError) as ei:
+        h2j_b200.Encoder(comment=b"c" * 65533)
+    assert ei.value.status == h2j_b200.ERR_INVALID_ARG and "COM segment" in str(ei.value)
 
 
 def test_no_gpu_means_loud_failure():

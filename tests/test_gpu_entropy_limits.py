@@ -15,6 +15,7 @@ import numpy as np
 import pytest
 
 from tests.support import histograms as H
+from tests.support.scan_model import block_bits, coding_order, frame_from_blocks
 
 pytestmark = pytest.mark.gpu
 
@@ -168,36 +169,6 @@ FIB_SYMBOLS = [0x12, 0x13, 0x23, 0x32, 0x14, 0x24, 0x33, 0x43, 0x52, 0x62, 0x72,
 DEEP = (0x99, 0xD9)  # size 9 after runs of 9 and 13
 
 
-def coding_order(chroma_format, h):
-    """(plane, block row, block column) of every block of a W x h frame in the order the encoder codes them (mjpegenc.c
-    ff_mjpeg_encode_mb, see oracle/mjpeg_oracle.c): plane 0 is Y, 1 Cb, 2 Cr"""
-    out = []
-    for my in range(h // 16):
-        for mx in range(W // 16):
-            y = [(0, 2 * my + r, 2 * mx + c) for r in range(2) for c in range(2)]
-            if chroma_format == 0:
-                out += y + [(1, my, mx), (2, my, mx)]
-            elif chroma_format == 1:
-                out += y + [(1, 2 * my, mx), (1, 2 * my + 1, mx), (2, 2 * my, mx), (2, 2 * my + 1, mx)]
-            else:  # two 8x16 MCUs per macroblock, every component 1x2
-                for c in range(2):
-                    out += [(pl, 2 * my + r, 2 * mx + c) for pl in range(3) for r in range(2)]
-    return out
-
-
-def frame_from_blocks(chroma_format, h, blocks):
-    """planes of a W x h frame whose coded blocks are blocks[i] (coding order; None or missing: flat)"""
-    orc = _tools()[0]
-    ch, cw = orc.chroma_shape(W, h, chroma_format)
-    planes = [np.full((h, W), 128, np.uint8), np.full((ch, cw), 128, np.uint8), np.full((ch, cw), 128, np.uint8)]
-    order = coding_order(chroma_format, h)
-    assert len(blocks) <= len(order), "frame too small for its blocks"
-    for (pl, r, c), px in zip(order, blocks):
-        if px is not None:
-            planes[pl][8 * r: 8 * r + 8, 8 * c: 8 * c + 8] = px
-    return tuple(planes)
-
-
 PATHS = ("slot", "direct", "clip")
 
 
@@ -210,7 +181,7 @@ def deep_frame(chroma_format, path, h=1536):
     The rest is flat but for single-level blocks whose counts make a Fibonacci spread in each table: that, and the heavy
     blocks using only a few frequent symbols, keeps the tree 16 levels deep under DEEP."""
     rng = np.random.default_rng(9 + PATHS.index(path))
-    order = coding_order(chroma_format, h)
+    order = coding_order(chroma_format, W, h)
     cls = [min(pl, 1) for pl, _, _ in order]
     deep = [single_level(s) for s in DEEP]
     pos0 = next(p for p in range(1, 64) if levels(deep[0])[p])
@@ -243,7 +214,7 @@ def deep_frame(chroma_format, path, h=1536):
         assert len(at) >= len(todo), "frame too small for the spread"
         for i, px in zip(at, todo):
             blocks[i] = px
-    return frame_from_blocks(chroma_format, h, blocks)
+    return frame_from_blocks(chroma_format, W, h, blocks)
 
 
 def _lengths(dbg, t):
@@ -305,27 +276,12 @@ def test_every_symbol_both_signs_and_zrl_chains(orc, chroma_format):
     assert any([s >> 4 for s, _ in syms] == [15, 15, 15, 14] for syms in per_block)
 
 
-def block_bits(dbg, coefs, chroma_format, h):
-    """bits K4a emits for every block in coding order, from the oracle's tables; and the class (0 luma, 1 chroma) of each"""
-    dc_len, ac_len = [_lengths(dbg, 0), _lengths(dbg, 1)], [_lengths(dbg, 2), _lengths(dbg, 3)]
-    last = [128] * 3  # mjpegenc's DC predictors start at 128 (1024 >> 3)
-    bits, classes = [], []
-    for (pl, _, _), z in zip(coding_order(chroma_format, h), coefs):
-        c = min(pl, 1)
-        diff = int(z[0]) - last[pl]
-        last[pl] = int(z[0])
-        size = abs(diff).bit_length()
-        bits.append(dc_len[c][size] + size + sum(ac_len[c][s] + (s & 15) for s, _ in ac_symbols(z)))
-        classes.append(c)
-    return bits, classes
-
-
 def test_coding_order_matches_the_encoder(orc):
     rng = np.random.default_rng(3)
     for fmt in FORMATS:
-        n = len(coding_order(fmt, 32))
+        n = len(coding_order(fmt, W, 32))
         blocks = [rng.integers(0, 256, (8, 8)).astype(np.uint8) for _ in range(n)]
-        _, _, coefs = orc.oracle_encode(*frame_from_blocks(fmt, 32, blocks), fixed_qscale=QSCALE, want_coefs=True, chroma_format=fmt)
+        _, _, coefs = orc.oracle_encode(*frame_from_blocks(fmt, W, 32, blocks), fixed_qscale=QSCALE, want_coefs=True, chroma_format=fmt)
         assert all((coefs[i][1:] == levels(px)[1:]).all() for i, px in enumerate(blocks)), fmt
 
 
@@ -340,7 +296,7 @@ def test_25_bit_items_on_every_k4a_path(orc, chroma_format, path):
     for t in (2, 3):
         L = _lengths(dbg, t)
         assert L[DEEP[0]] == 16 and (path != "slot" or L[DEEP[1]] == 16), (t, {hex(s): L.get(s) for s in DEEP})
-    bits, classes = block_bits(dbg, coefs, chroma_format, h)
+    bits, classes = block_bits(dbg, coefs, chroma_format, W, h)
     assert sum(bits) == dbg.scan_bits
     unit_bits = [sum(bits[i: i + 32]) for i in range(0, len(bits), 32)]  # entropy_walk_kernel: unit u = blocks 32u .. 32u + 31
     seen = set()
