@@ -188,10 +188,11 @@ void set_alignment(FrameLayout *L, const uint8_t *base)
     L->aligned16 = ((uintptr_t)base % 16) == 0 && (L->frame_stride % 16) == 0 && (L->y_pitch % 16) == 0 ? 1 : 0;
 }
 
-int make_layout(h2j_encoder *e, const uint8_t *base, size_t frame_stride, int w, int h, FrameLayout *L)
+// within_max = false: a frame the encoder does not encode at this size (the source of a downscaled submit)
+int make_layout(h2j_encoder *e, const uint8_t *base, size_t frame_stride, int w, int h, FrameLayout *L, bool within_max = true)
 {
     if (w < 2 || h < 2 || w > 65500 || h > 65500) return fail(e, H2J_ERR_UNSUPPORTED, "unsupported frame size %dx%d", w, h);
-    if (w > e->s.max_width || h > e->s.max_height)
+    if (within_max && (w > e->s.max_width || h > e->s.max_height))
         return fail(e, H2J_ERR_UNSUPPORTED, "frame %dx%d exceeds the configured maximum %dx%d", w, h, e->s.max_width, e->s.max_height);
     const int fmt = e->s.chroma_format;
     const int fcw = chroma_w(w, fmt), fch = chroma_h(h, fmt);
@@ -622,6 +623,42 @@ void free_slot(Slot &sl)
     sl = Slot{};
 }
 
+// The checks of a device list submit's arguments (h2j_submit_device_list, h2j_submit_device_downscaled), all made before
+// anything is enqueued or the slot's table is touched.
+int check_device_list(h2j_encoder *e, int slot, int layout, const h2j_frame_desc *frames, int n)
+{
+    int rc = check_slot(e, slot);
+    if (rc) return rc;
+    if (e->slots[slot].busy) return fail(e, H2J_ERR_BUSY, "slot %d has a batch in flight", slot);
+    if (!frames || n < 1 || n > e->s.max_batch) return fail(e, H2J_ERR_INVALID_ARG, "bad frames pointer or batch size %d (max %d)", n, e->s.max_batch);
+    if (layout != H2J_LAYOUT_PLANAR && layout != H2J_LAYOUT_SEMIPLANAR) return fail(e, H2J_ERR_INVALID_ARG, "bad layout %d", layout);
+    return H2J_OK;
+}
+
+// Caller frame i of a device list submit -> its layout where it is (semi-planar: the pair plane at u_off = v_off) and the
+// bytes from its base that may be read.  within_max: the frame is encoded at this size, so it must fit the encoder.
+int device_frame_layout(h2j_encoder *e, int i, const h2j_frame_desc &F, bool sp, bool within_max, FrameLayout *L, long long *extent)
+{
+    const int fmt = e->s.chroma_format;
+    if (!F.data) return fail(e, H2J_ERR_INVALID_ARG, "frame %d: null data", i);
+    int rc = make_layout(e, F.data, 0, F.width, F.height, L, within_max);
+    if (rc) return rc;
+    const int fcw = chroma_w(F.width, fmt), fch = chroma_h(F.height, fmt);
+    const int c_row = sp ? 2 * fcw : fcw;  // bytes in a chroma row
+    if (F.y_pitch < F.width || F.c_pitch < c_row)
+        return fail(e, H2J_ERR_INVALID_ARG, "frame %d: pitches %d / %d shorter than rows of %d / %d bytes", i, F.y_pitch, F.c_pitch, F.width, c_row);
+    if (sp && F.u_offset < (size_t)F.y_pitch * F.height)
+        return fail(e, H2J_ERR_INVALID_ARG, "frame %d: the pair plane starts inside the luma plane", i);
+    L->y_pitch = F.y_pitch;
+    L->c_pitch = F.c_pitch;
+    L->u_off = (long long)F.u_offset;
+    L->v_off = (long long)(sp ? F.u_offset : F.v_offset);
+    set_alignment(L, F.data);
+    *extent = (long long)std::max((size_t)F.y_pitch * (F.height - 1) + F.width,
+                                  std::max((size_t)L->u_off, (size_t)L->v_off) + (size_t)F.c_pitch * (fch - 1) + c_row);
+    return H2J_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1026,12 +1063,9 @@ int h2j_submit_host(h2j_encoder *e, int slot, const uint8_t *frames, size_t fram
 
 int h2j_submit_device_list(h2j_encoder *e, int slot, int layout, const h2j_frame_desc *frames, int n)
 {
-    int rc = check_slot(e, slot);
+    int rc = check_device_list(e, slot, layout, frames, n);
     if (rc) return rc;
     Slot &sl = e->slots[slot];
-    if (sl.busy) return fail(e, H2J_ERR_BUSY, "slot %d has a batch in flight", slot);
-    if (!frames || n < 1 || n > e->s.max_batch) return fail(e, H2J_ERR_INVALID_ARG, "bad frames pointer or batch size %d (max %d)", n, e->s.max_batch);
-    if (layout != H2J_LAYOUT_PLANAR && layout != H2J_LAYOUT_SEMIPLANAR) return fail(e, H2J_ERR_INVALID_ARG, "bad layout %d", layout);
     const bool sp = layout == H2J_LAYOUT_SEMIPLANAR;
     const int fmt = e->s.chroma_format;
     // every frame is checked before anything is enqueued or the slot's table is touched (a rejected call leaves the previous
@@ -1041,26 +1075,14 @@ int h2j_submit_device_list(h2j_encoder *e, int slot, int layout, const h2j_frame
     bool copies = false;
     for (int i = 0; i < n; i++) {
         const h2j_frame_desc &F = frames[i];
-        if (!F.data) return fail(e, H2J_ERR_INVALID_ARG, "frame %d: null data", i);
         FrameLayout L;
-        rc = make_layout(e, F.data, 0, F.width, F.height, &L);
+        long long extent = 0;
+        rc = device_frame_layout(e, i, F, sp, true, &L, &extent);
         if (rc) return rc;
-        const int fcw = chroma_w(F.width, fmt), fch = chroma_h(F.height, fmt);
-        const int c_row = sp ? 2 * fcw : fcw;  // bytes in a chroma row
-        if (F.y_pitch < F.width || F.c_pitch < c_row)
-            return fail(e, H2J_ERR_INVALID_ARG, "frame %d: pitches %d / %d shorter than rows of %d / %d bytes", i, F.y_pitch, F.c_pitch, F.width, c_row);
-        if (sp && F.u_offset < (size_t)F.y_pitch * F.height)
-            return fail(e, H2J_ERR_INVALID_ARG, "frame %d: the pair plane starts inside the luma plane", i);
-        L.y_pitch = F.y_pitch;
-        L.c_pitch = F.c_pitch;
-        L.u_off = (long long)F.u_offset;
-        L.v_off = (long long)(sp ? F.u_offset : F.v_offset);
-        set_alignment(&L, F.data);
         FrameDesc &src = tab[n + i];
         src.L = L;
         src.base = nullptr;
-        src.extent = (long long)std::max((size_t)F.y_pitch * (F.height - 1) + F.width,
-                                         std::max((size_t)L.u_off, (size_t)L.v_off) + (size_t)F.c_pitch * (fch - 1) + c_row);
+        src.extent = extent;
         tab[i].L = L;
         tab[i].base = F.data;
         tab[i].extent = 0;
@@ -1115,6 +1137,73 @@ int h2j_submit_device_list(h2j_encoder *e, int slot, int layout, const h2j_frame
         CU(e, cudaGetLastError());
     }
     rc = launch_pipeline(e, sl, nullptr, n, TAIL_SIZES, true);
+    if (rc) return rc;
+    sl.busy = true;
+    return H2J_OK;
+}
+
+int h2j_submit_device_downscaled(h2j_encoder *e, int slot, int layout, const h2j_frame_desc *frames, int n, int factor)
+{
+    int rc = check_device_list(e, slot, layout, frames, n);
+    if (rc) return rc;
+    if (factor != 2 && factor != 4 && factor != 8) return fail(e, H2J_ERR_INVALID_ARG, "factor %d is not 2, 4 or 8", factor);
+    Slot &sl = e->slots[slot];
+    const bool sp = layout == H2J_LAYOUT_SEMIPLANAR;
+    const int fmt = e->s.chroma_format;
+    // tab[i]: the downscaled frame the pipeline reads, planar at a 16-byte row pitch in the slot's frame buffer; tab[n + i]:
+    // the caller's frame.  Only the downscaled size is held to the encoder's maximum.  (Checked before the slot's table is
+    // touched, as h2j_submit_device_list.)
+    std::vector<FrameDesc> tab(2 * (size_t)n);
+    bool uniform = true;
+    int cols = 0, rows = 0;  // the largest destination: 16-byte columns of a row (SP chroma: 8 pairs), rows of all planes
+    for (int i = 0; i < n; i++) {
+        const h2j_frame_desc &F = frames[i];
+        FrameDesc &src = tab[n + i];
+        rc = device_frame_layout(e, i, F, sp, false, &src.L, &src.extent);
+        if (rc) return rc;
+        src.base = F.data;
+        const int w = (F.width + factor - 1) / factor, h = (F.height + factor - 1) / factor;
+        if (w < 2 || h < 2)
+            return fail(e, H2J_ERR_UNSUPPORTED, "frame %d: %dx%d at 1/%d is %dx%d, smaller than 2x2", i, F.width, F.height, factor, w, h);
+        FrameDesc &d = tab[i];
+        uint8_t *dev = sl.d_frames + (size_t)i * e->frame_bytes_cap;
+        rc = make_layout(e, dev, 0, w, h, &d.L);
+        if (rc) return rc;
+        d.L = pitched_layout(d.L);
+        d.L.frame_stride = 0;
+        d.base = dev;
+        d.extent = 0;
+        uniform = uniform && w == tab[0].L.w && h == tab[0].L.h;
+        const int fcw = chroma_w(w, fmt), fch = chroma_h(h, fmt);
+        cols = std::max(cols, std::max((w + 15) / 16, sp ? (fcw + 7) / 8 : (fcw + 15) / 16));
+        rows = std::max(rows, h + (sp ? 1 : 2) * fch);
+    }
+    memcpy(sl.h_desc, tab.data(), sizeof(FrameDesc) * 2 * n);
+    sl.list = true;  // the debug hooks answer from this table from here on (the batch form below answers from sl.L)
+    sl.n = n;
+    ON_DEVICE(e);
+    CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
+    CU(e, cudaMemcpyAsync(sl.d_desc, sl.h_desc, sizeof(FrameDesc) * 2 * n, cudaMemcpyHostToDevice, sl.stream));
+    // every layout is read where it is: no repitch or split in front
+    {
+        const int rows_per_cta = kDownWarps * 16 / factor;
+        const dim3 grid((cols + 31) / 32, (rows + rows_per_cta - 1) / rows_per_cta, n);
+        decltype(&downscale_list_kernel<2, false>) k;
+        if (factor == 2) k = sp ? downscale_list_kernel<2, true> : downscale_list_kernel<2, false>;
+        else if (factor == 4) k = sp ? downscale_list_kernel<4, true> : downscale_list_kernel<4, false>;
+        else k = sp ? downscale_list_kernel<8, true> : downscale_list_kernel<8, false>;
+        k<<<grid, 32 * kDownWarps, 0, sl.stream>>>(sl.d_desc, n);
+        e->launches++;
+        CU(e, cudaGetLastError());
+    }
+    // frames of one size go through the batch form of the pipeline (the list form costs 0.92x on uniform input)
+    if (uniform) {
+        sl.L = sl.h_desc[0].L;
+        sl.L.frame_stride = (long long)e->frame_bytes_cap;
+        rc = launch_pipeline(e, sl, sl.d_frames, n, TAIL_SIZES);
+    } else {
+        rc = launch_pipeline(e, sl, nullptr, n, TAIL_SIZES, true);
+    }
     if (rc) return rc;
     sl.busy = true;
     return H2J_OK;

@@ -319,4 +319,153 @@ __global__ void __launch_bounds__(128) depth_to_8_kernel(const uint8_t *__restri
     }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Downscaled frames (h2j_submit_device_downscaled): every plane of the caller's frame, at its decoder size pw x ph, box-
+// filtered by K (2, 4, 8) to ceil(pw/K) x ceil(ph/K): out[y][x] = (S + c/2) / c, S the sum of the c source samples of the
+// box (K*K, fewer in the partial boxes at the right and bottom edges), semi-planar Cb and Cr averaged separately.  The
+// result is the planar frame the pipeline reads, at pitched_layout() of the downscaled size in the slot's d_frames.
+// descs[f] is that destination, descs[n + f] the source (L: its size, pitches and plane offsets; SP: the pair plane at
+// u_off).  grid (x, y, frames): a warp per output row (kDownRowsPerWarp of them, one after the other), a lane per 16 output
+// bytes of the row (SP chroma: 8 Cb + 8 Cr of a row of pairs), so 16 * K source bytes per source row; grid sized for the
+// largest destination, CTAs past their frame's extent return.  A source row is summed into the 16 accumulators as soon as
+// it is loaded (dp4a).  16-byte aligned segments take 128-bit loads (the lane cut by the row's end: the chunks inside the
+// row), others aligned 32-bit words and funnel shifts; only words an end of the row cuts are read byte by byte, so no
+// byte past a row's last sample is read.
+// ------------------------------------------------------------------------------------------------
+template <int K>
+constexpr int kDownRowsPerWarp = 16 / K;  // 16 source rows per warp whatever K
+constexpr int kDownWarps = 4;
+
+// the 16 * K bytes of a source row at row + x0 as 4 * K little-endian words; bytes at or past `bytes` (the row's end) are 0
+template <int K>
+__device__ __forceinline__ void down_fetch(const uint8_t *__restrict__ row, int x0, int bytes, unsigned (&w)[4 * K])
+{
+    constexpr int kWords = 4 * K;
+    const uint8_t *s = row + x0;
+    const int a = (int)((uintptr_t)s & 3u);
+    const uint32_t *q = reinterpret_cast<const uint32_t *>(s - a);
+    // aligned word j holds bytes [x0 - a + 4j, + 4) of the row: loaded whole where it lies inside the row, byte by byte
+    // where an end of the row cuts it, without the bytes outside
+    auto word = [&](int j) {
+        const int p = x0 - a + 4 * j;
+        if (p >= 0 && p + 4 <= bytes) return __ldg(q + j);
+        unsigned v = 0;
+#pragma unroll
+        for (int b = 0; b < 4; b++)
+            if (p + b >= 0 && p + b < bytes) v |= (unsigned)row[p + b] << (8 * b);
+        return v;
+    };
+    if (((uintptr_t)s & 15u) == 0) {  // 16-byte chunks: whole inside the row, 0 past its end, by words where the end cuts one
+#pragma unroll
+        for (int i = 0; i < K; i++) {
+            uint4 v = make_uint4(0, 0, 0, 0);
+            if (x0 + 16 * i + 16 <= bytes) v = ldg128(s + 16 * i);
+            else if (x0 + 16 * i < bytes) v = make_uint4(word(4 * i), word(4 * i + 1), word(4 * i + 2), word(4 * i + 3));
+            w[4 * i] = v.x; w[4 * i + 1] = v.y; w[4 * i + 2] = v.z; w[4 * i + 3] = v.w;
+        }
+        return;
+    }
+    unsigned prev = word(0);
+#pragma unroll
+    for (int i = 0; i < kWords; i++) {
+        const unsigned next = (i + 1 < kWords || a) ? word(i + 1) : 0u;
+        w[i] = __funnelshift_r(prev, next, a * 8);
+        prev = next;
+    }
+}
+
+// (S + c/2) / c of the box of output x (its first source sample k * x), rh rows high, of a row of pw samples; full boxes by a
+// shift, outputs past the row's end 0
+template <int K>
+__device__ __forceinline__ unsigned down_avg(unsigned s, int x, int pw, int rh, bool full)
+{
+    constexpr int kShift = K == 2 ? 2 : (K == 4 ? 4 : 6);
+    if (full) return (s + K * K / 2) >> kShift;
+    const int c = min(K, pw - K * x) * rh;
+    return c > 0 ? (s + (unsigned)(c >> 1)) / (unsigned)c : 0u;
+}
+
+template <int K, bool SP>
+__global__ void __launch_bounds__(32 * kDownWarps, K == 2 ? 6 : 4) downscale_list_kernel(const FrameDesc *__restrict__ descs, int n)
+{
+    static_assert(K == 2 || K == 4 || K == 8, "box factors 2, 4, 8");
+    constexpr int kWords = 4 * K;
+    const int f = blockIdx.z;
+    const FrameDesc &d = descs[f], &s = descs[n + f];
+    const FrameLayout &D = d.L, &S = s.L;
+    const int hs = fmt_hshift(S.fmt), vs = fmt_vshift(S.fmt);
+    const int scw = (S.w + (1 << hs) - 1) >> hs, sch = (S.h + (1 << vs) - 1) >> vs;  // source chroma plane
+    const int dch = (D.h + (1 << vs) - 1) >> vs;                                     // = ceil(sch / K) rows
+    const int rows = D.h + (SP ? 1 : 2) * dch;
+    const int lane = threadIdx.x & 31;
+    const int x16 = blockIdx.x * 32 + lane;  // this lane's 16 output bytes of a row (SP chroma: its 8 pairs)
+    const int row0 = (blockIdx.y * kDownWarps + (threadIdx.x >> 5)) * kDownRowsPerWarp<K>;
+    for (int row = row0; row < min(row0 + kDownRowsPerWarp<K>, rows); row++) {
+        int r, pw, ph, spitch;  // output row in its plane, source plane samples per row (SP chroma: pairs) and rows, pitch
+        long long so;
+        uint8_t *o;
+        bool pairs = false;
+        if (row < D.h) {
+            r = row; pw = S.w; ph = S.h; spitch = S.y_pitch; so = 0;
+            o = const_cast<uint8_t *>(d.base) + (long long)r * D.y_pitch;
+        } else if (SP) {
+            r = row - D.h; pw = scw; ph = sch; spitch = S.c_pitch; so = S.u_off; pairs = true;
+            o = const_cast<uint8_t *>(d.base) + D.u_off + (long long)r * D.c_pitch;
+        } else {
+            const bool cr = row >= D.h + dch;
+            r = row - D.h - (cr ? dch : 0); pw = scw; ph = sch; spitch = S.c_pitch; so = cr ? S.v_off : S.u_off;
+            o = const_cast<uint8_t *>(d.base) + (cr ? D.v_off : D.u_off) + (long long)r * D.c_pitch;
+        }
+        const int per = pairs ? 8 : 16;  // outputs per lane and component
+        const int ox = x16 * per;        // first of them
+        if (K * ox >= pw) continue;
+        const int bytes = pairs ? 2 * pw : pw;  // of a source row
+        const int x0 = 16 * K * x16;            // first source byte of the lane's segment
+        const int rh = min(K, ph - K * r);
+        const uint8_t *src = s.base + so + (long long)K * r * spitch;
+        unsigned acc[16];  // planar: output ox + i; SP: Cb of pair ox + i (0..7), Cr (8..15)
+#pragma unroll
+        for (int i = 0; i < 16; i++) acc[i] = 0;
+#pragma unroll
+        for (int j = 0; j < K; j++) {
+            if (j >= rh) break;
+            unsigned w[kWords];
+            down_fetch<K>(src + (long long)j * spitch, x0, bytes, w);
+            if (pairs) {  // Cb Cr Cb Cr: K / 2 words per output pair
+#pragma unroll
+                for (int i = 0; i < kWords; i++) {
+                    acc[i / (K / 2)] = __dp4a(w[i], 0x00010001u, acc[i / (K / 2)]);
+                    acc[8 + i / (K / 2)] = __dp4a(w[i], 0x01000100u, acc[8 + i / (K / 2)]);
+                }
+            } else if constexpr (K == 2) {  // two outputs per word
+#pragma unroll
+                for (int i = 0; i < kWords; i++) {
+                    acc[2 * i] = __dp4a(w[i], 0x00000101u, acc[2 * i]);
+                    acc[2 * i + 1] = __dp4a(w[i], 0x01010000u, acc[2 * i + 1]);
+                }
+            } else {  // K / 4 words per output
+#pragma unroll
+                for (int i = 0; i < kWords; i++) acc[i / (K / 4)] = __dp4a(w[i], 0x01010101u, acc[i / (K / 4)]);
+            }
+        }
+        const bool full = rh == K && x0 + 16 * K <= bytes;
+        unsigned p[4] = {0, 0, 0, 0};
+        if (pairs) {
+            unsigned q[4] = {0, 0, 0, 0};
+#pragma unroll
+            for (int i = 0; i < 8; i++) {
+                p[i >> 2] |= down_avg<K>(acc[i], ox + i, pw, rh, full) << (8 * (i & 3));
+                q[i >> 2] |= down_avg<K>(acc[8 + i], ox + i, pw, rh, full) << (8 * (i & 3));
+            }
+            // rows of the destination are 16-byte aligned and hold at least 8 bytes from ox
+            *reinterpret_cast<uint2 *>(o + ox) = make_uint2(p[0], p[1]);
+            *reinterpret_cast<uint2 *>(o + (D.v_off - D.u_off) + ox) = make_uint2(q[0], q[1]);
+        } else {
+#pragma unroll
+            for (int i = 0; i < 16; i++) p[i >> 2] |= down_avg<K>(acc[i], ox + i, pw, rh, full) << (8 * (i & 3));
+            *reinterpret_cast<uint4 *>(o + ox) = make_uint4(p[0], p[1], p[2], p[3]);
+        }
+    }
+}
+
 }  // namespace h2j

@@ -108,7 +108,7 @@ EXPORTS = [
     "h2j_slot_kernel_ms", "h2j_set_profile", "h2j_slot_total_ms", "h2j_kernel_launches", "h2j_slot_set_stream",
     "h2j_slot_wait_event", "h2j_device_count", "h2j_debug_set_knob", "h2j_debug_read_device", "h2j_stream_copy",
     "h2j_submit_device_semiplanar16", "h2j_submit_device_pitched16", "h2j_encode_frame16", "h2j_submit_device_list",
-    "h2j_submit_host_list",
+    "h2j_submit_host_list", "h2j_submit_device_downscaled",
 ]
 
 _lib = None
@@ -147,6 +147,7 @@ def load_library() -> C.CDLL:
     lib.h2j_encode_frame16.argtypes = [vp, C.POINTER(vp), C.POINTER(ci), ci, ci, ci, vp, sz, C.POINTER(sz)]
     lib.h2j_submit_device_list.argtypes = [vp, ci, ci, C.POINTER(FrameDesc), ci]
     lib.h2j_submit_host_list.argtypes = [vp, ci, C.POINTER(vp), C.POINTER(ci), C.POINTER(ci), ci]
+    lib.h2j_submit_device_downscaled.argtypes = [vp, ci, ci, C.POINTER(FrameDesc), ci, ci]
     lib.h2j_collect.argtypes = [vp, ci, vp, sz, C.POINTER(sz), C.POINTER(ci)]
     lib.h2j_collect_device.argtypes = [vp, ci, C.POINTER(vp), C.POINTER(sz), C.POINTER(sz), C.POINTER(ci)]
     lib.h2j_wait.argtypes = [vp, ci]
@@ -175,6 +176,13 @@ def frame_bytes(width: int, height: int, chroma_format: int = CHROMA_420) -> int
     """Bytes of one tightly packed planar frame (Y, U, V; I420 by default)."""
     ch, cw = chroma_shape(width, height, chroma_format)
     return width * height + 2 * cw * ch
+
+
+def downscaled_size(width: int, height: int, factor: int) -> Tuple[int, int]:
+    """(width, height) of the frame h2j_submit_device_downscaled encodes for a width x height source at 1/factor"""
+    if factor not in (2, 4, 8):
+        raise ValueError(f"factor {factor} is not 2, 4 or 8")
+    return (width + factor - 1) // factor, (height + factor - 1) // factor
 
 
 def split_planes(frame: np.ndarray, width: int, height: int, chroma_format: int = CHROMA_420) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
@@ -410,6 +418,13 @@ class Encoder:
         """Device frames each at its own address and of its own size (LAYOUT_PLANAR or LAYOUT_SEMIPLANAR for all)."""
         arr = (FrameDesc * max(1, len(descs)))(*descs)
         self._check(self._lib.h2j_submit_device_list(self._h, slot, layout, arr, len(descs)))
+        self._n_in_slot[slot] = len(descs)
+
+    def submit_device_downscaled(self, slot: int, layout: int, descs: Sequence[FrameDesc], factor: int) -> None:
+        """Device frames as for submit_device_list, each encoded box-filtered to 1/factor (2, 4 or 8) of its size
+        (downscaled_size); only the downscaled frames must fit the encoder's maximum."""
+        arr = (FrameDesc * max(1, len(descs)))(*descs)
+        self._check(self._lib.h2j_submit_device_downscaled(self._h, slot, layout, arr, len(descs), factor))
         self._n_in_slot[slot] = len(descs)
 
     def submit_host_list(self, slot: int, frames: Sequence[int], sizes: Sequence[Tuple[int, int]]) -> None:

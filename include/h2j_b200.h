@@ -235,6 +235,28 @@ typedef struct h2j_frame_desc {
 int h2j_submit_device_list(h2j_encoder *e, int slot, int layout, const h2j_frame_desc *frames, int n);
 int h2j_submit_host_list(h2j_encoder *e, int slot, const uint8_t *const *frames, const int *widths, const int *heights, int n);
 
+/*
+ * Downscaled device frames: thumbnails and previews of decoder surfaces, encoded without a full-size pass.  `layout` and
+ * `frames` are those of h2j_submit_device_list (planar at any pitches and plane offsets, or NV12 / NV16 / NV24 by the
+ * encoder's chroma format; any alignment; each frame of its own size).  `factor` is 2, 4 or 8.  Frame i's JPEG is
+ * byte-identical to the one h2j_submit_device writes, with the same encoder settings, for the planar frame D_k(frame i):
+ *   every plane, at its decoder size pw x ph (chroma ceil-divided as for the other submits), becomes a plane of
+ *   ceil(pw/k) x ceil(ph/k) samples, out[y][x] = (S + c/2) / c in integers (rounded half up), where S is the sum of the
+ *   c source samples P[j][i] with k*x <= i < min(k*x + k, pw) and k*y <= j < min(k*y + k, ph) -- c = k*k except in the
+ *   partial boxes at the right and bottom edges.  Semi-planar Cb and Cr are averaged separately.
+ * The downscaled frame is ceil(w/k) x ceil(h/k), and its chroma planes are exactly that frame's chroma size
+ * (ceil(ceil(w/2)/k) == ceil(ceil(w/k)/2)).  Range conversion (range_mode) applies to the downscaled samples.
+ * Sources may be up to 65500 on a side whatever max_width / max_height; only the downscaled frame must fit the encoder (an
+ * encoder created for 480x272 takes 1920x1080 sources at factor 4).  One kernel writes the downscaled frames into the slot's
+ * own frame buffer, then the usual pipeline runs on them.  Collect with h2j_collect / h2j_collect_device; the inspection
+ * calls answer for the downscaled frames; the device frames are read on the slot's stream, under the stream-ordering
+ * rule above.
+ * H2J_ERR_INVALID_ARG: as h2j_submit_device_list, or a factor other than 2, 4, 8.  H2J_ERR_UNSUPPORTED: a source outside
+ * 2..65500, or a downscaled frame smaller than 2 on a side or larger than the encoder's maximum.  H2J_ERR_BUSY: the slot has
+ * a batch in flight.  Every frame is checked before anything is enqueued: a rejected call leaves the previous batch as it was.
+ */
+int h2j_submit_device_downscaled(h2j_encoder *e, int slot, int layout, const h2j_frame_desc *frames, int n, int factor);
+
 int h2j_collect(h2j_encoder *e, int slot, uint8_t *out, size_t out_capacity, size_t *offsets, int *status);
 int h2j_collect_device(h2j_encoder *e, int slot, const uint8_t **d_out, size_t *d_frame_capacity, size_t *sizes,
                        int *status);
