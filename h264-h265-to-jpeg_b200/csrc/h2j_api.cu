@@ -30,7 +30,7 @@ struct KernelTiming {
 struct Slot {
     cudaStream_t stream = nullptr;
     cudaEvent_t ev_begin = nullptr, ev_done = nullptr;
-    uint8_t *d_frames = nullptr;  // staging for host submits
+    uint8_t *d_frames = nullptr;  // staging for host submits; the input stage's split, converted and downscaled frames
     uint8_t *d_pitched = nullptr; // copies of frames with unaligned rows at a 16-byte pitch (allocated on first need)
     uint32_t *d_images = nullptr;  // [max_batch][images_cap] tile images (h2j_common.cuh)
     uint8_t *d_zero = nullptr;    // FrameState[max_batch] | descs | ticket | chunk_ff — zeroed every batch
@@ -61,11 +61,11 @@ struct Slot {
     bool own_stream = true;
     bool packed = false;      // pack_kernel already ran for the batch in flight
     int n = 0;
-    FrameLayout L{};
-    // list batches (h2j_submit_device_list / h2j_submit_host_list): descs[i] is frame i as the pipeline reads it, descs[n + i]
-    // the source a copy kernel reads it from (base nullptr: no copy).  The pinned mirror is filled by the submit and uploaded
-    // with one copy on the slot's stream; a busy slot refuses a submit, so it is never rewritten while that copy is pending.
-    bool list = false;
+    // the batch (every submit), m entry pairs (h2j_common.cuh FrameDesc): descs[i] is frame i as the pipeline reads it,
+    // descs[m + i] the source a copy kernel reads it from (base nullptr: no copy).  m = n, or 1 for n frames of one layout at
+    // one stride.  The pinned mirror is filled by the submit and, when a kernel reads the table, uploaded with one copy on the
+    // slot's stream; a busy slot refuses a submit, so it is never rewritten while that copy is pending.
+    int m = 0;
     FrameDesc *d_desc = nullptr;  // [2 * max_batch]
     FrameDesc *h_desc = nullptr;  // pinned mirror
     std::vector<KernelTiming> timings;
@@ -177,19 +177,20 @@ int chroma_w(int w, int fmt) { return (w + (1 << fmt_hshift(fmt)) - 1) >> fmt_hs
 int chroma_h(int h, int fmt) { return (h + (1 << fmt_vshift(fmt)) - 1) >> fmt_vshift(fmt); }
 size_t tight_frame_bytes(int w, int h, int fmt) { return (size_t)w * h + 2 * (size_t)chroma_w(w, fmt) * chroma_h(h, fmt); }
 
-// the vector-load flags of a planar layout whose frames start at `base`
-void set_alignment(FrameLayout *L, const uint8_t *base)
+// the vector-load flags of a planar layout whose frames start at `base`, `frame_stride` apart
+void set_alignment(FrameLayout *L, const uint8_t *base, size_t frame_stride = 0)
 {
     auto al = [&](int a) {
-        return ((uintptr_t)base % a) == 0 && (L->frame_stride % a) == 0 && (L->u_off % a) == 0 && (L->v_off % a) == 0 &&
+        return ((uintptr_t)base % a) == 0 && (frame_stride % a) == 0 && (L->u_off % a) == 0 && (L->v_off % a) == 0 &&
                (L->y_pitch % a) == 0 && (L->c_pitch % a) == 0;
     };
     L->aligned8 = al(8) ? 1 : 0;
-    L->aligned16 = ((uintptr_t)base % 16) == 0 && (L->frame_stride % 16) == 0 && (L->y_pitch % 16) == 0 ? 1 : 0;
+    L->aligned16 = ((uintptr_t)base % 16) == 0 && (frame_stride % 16) == 0 && (L->y_pitch % 16) == 0 ? 1 : 0;
 }
 
-// within_max = false: a frame the encoder does not encode at this size (the source of a downscaled submit)
-int make_layout(h2j_encoder *e, const uint8_t *base, size_t frame_stride, int w, int h, FrameLayout *L, bool within_max = true)
+// A tight planar frame at `base`.  within_max = false: a frame the encoder does not encode at this size (the source of a
+// downscaled submit)
+int make_layout(h2j_encoder *e, const uint8_t *base, int w, int h, FrameLayout *L, bool within_max = true)
 {
     if (w < 2 || h < 2 || w > 65500 || h > 65500) return fail(e, H2J_ERR_UNSUPPORTED, "unsupported frame size %dx%d", w, h);
     if (within_max && (w > e->s.max_width || h > e->s.max_height))
@@ -203,7 +204,7 @@ int make_layout(h2j_encoder *e, const uint8_t *base, size_t frame_stride, int w,
     L->y_pitch = w; L->c_pitch = fcw;
     L->u_off = (long long)w * h;
     L->v_off = L->u_off + (long long)fcw * fch;
-    L->frame_stride = (long long)frame_stride;
+    L->frame_stride = 0;
     L->mb_w = (w + 15) >> 4;
     L->mcu_w = (w + fmt_mcu_px_w(fmt) - 1) / fmt_mcu_px_w(fmt); L->mcu_h = (h + 15) >> 4;
     L->n_mcu = L->mcu_w * L->mcu_h;
@@ -215,9 +216,8 @@ int make_layout(h2j_encoder *e, const uint8_t *base, size_t frame_stride, int w,
     return H2J_OK;
 }
 
-// Rows that do not start on 8-byte boundaries would send every block of K1 / K2 down the bytewise path: such batches are
+// Rows that do not start on 8-byte boundaries would send every block of K1 / K2 down the bytewise path: such frames are
 // copied once to a 16-byte row pitch (repitch_kernel, ~1 us per 1080p frame) and the pipeline reads the copy.
-// On return sl.L describes what the pipeline reads and *pipe_src is where it reads it.
 size_t pitched_frame_bytes(int w, int h, int fmt)
 {
     const int fcw = chroma_w(w, fmt), fch = chroma_h(h, fmt);
@@ -233,60 +233,17 @@ FrameLayout pitched_layout(const FrameLayout &T)
     P.c_pitch = (int)align_up((size_t)fcw, 16);
     P.u_off = (long long)P.y_pitch * T.h;
     P.v_off = P.u_off + (long long)P.c_pitch * fch;
-    P.frame_stride = (long long)pitched_frame_bytes(T.w, T.h, T.fmt);
     P.aligned8 = 1;
     P.aligned16 = 1;
     return P;
 }
 
-// sl.L describes the n frames at d_src (any planar layout); src_end is the end of the last one's last plane
-int repitch_if_unaligned(h2j_encoder *e, Slot &sl, const uint8_t *d_src, const uint8_t *src_end, int n, const uint8_t **pipe_src)
+// the h2j_frame_desc of a tight planar frame at `base`
+h2j_frame_desc tight_frame(const uint8_t *base, int w, int h, int fmt)
 {
-    const int w = sl.L.w, h = sl.L.h;
-    *pipe_src = d_src;
-    if (sl.L.aligned8) return H2J_OK;
-    if (!sl.d_pitched) {
-        const size_t bytes = pitched_frame_bytes(e->s.max_width, e->s.max_height, e->s.chroma_format) * (size_t)e->s.max_batch;
-        if (cudaMalloc(&sl.d_pitched, bytes) != cudaSuccess) {  // no room for the copy: the bytewise path still works
-            cudaGetLastError();
-            sl.d_pitched = nullptr;
-            return H2J_OK;
-        }
-    }
-    const FrameLayout T = sl.L;
-    const FrameLayout P = pitched_layout(T);
-    const int fch = chroma_h(h, T.fmt);
-    repitch_kernel<<<dim3((w + 128 * 16 - 1) / (128 * 16), (h + 2 * fch + kPlaneRowsPerCta - 1) / kPlaneRowsPerCta, n), 128, 0, sl.stream>>>(d_src, T, fch, sl.d_pitched, P, d_src, src_end);
-    e->launches++;
-    CU(e, cudaGetLastError());
-    sl.L = P;
-    *pipe_src = sl.d_pitched;
-    return H2J_OK;
-}
-
-int prepare_input(h2j_encoder *e, Slot &sl, const uint8_t *d_src, size_t src_stride, int n, int w, int h, const uint8_t **pipe_src)
-{
-    int rc = make_layout(e, d_src, src_stride, w, h, &sl.L);
-    if (rc) return rc;
-    const uint8_t *src_end = d_src + (size_t)(n - 1) * src_stride + tight_frame_bytes(w, h, sl.L.fmt);
-    return repitch_if_unaligned(e, sl, d_src, src_end, n, pipe_src);
-}
-
-// High-bit-depth input: n frames at d_src (layout S; sp: semi-planar) -> 8-bit planar frames in the slot's frame buffer at
-// a 16-byte row pitch (frame_bytes_cap holds pitched_frame_bytes), in one launch for every layout and width.  On return
-// sl.L describes what the pipeline reads at sl.d_frames.
-int convert_depth(h2j_encoder *e, Slot &sl, const uint8_t *d_src, const Src16 &S, bool sp, int bit_depth, int n, int w, int h)
-{
-    int rc = make_layout(e, sl.d_frames, 0, w, h, &sl.L);
-    if (rc) return rc;
-    sl.L = pitched_layout(sl.L);
-    const int fch = chroma_h(h, sl.L.fmt);
-    const int row_words = sp ? std::max(w, 2 * chroma_w(w, sl.L.fmt)) : w;
-    const dim3 grid((row_words + 128 * 16 - 1) / (128 * 16), (h + (sp ? 1 : 2) * fch + kPlaneRowsPerCta - 1) / kPlaneRowsPerCta, n);
-    (sp ? depth_to_8_kernel<true> : depth_to_8_kernel<false>)<<<grid, 128, 0, sl.stream>>>(d_src, S, sl.d_frames, sl.L, bit_depth - 8);
-    e->launches++;
-    CU(e, cudaGetLastError());
-    return H2J_OK;
+    const int fcw = chroma_w(w, fmt);
+    const size_t u_off = (size_t)w * h;
+    return h2j_frame_desc{base, w, h, w, fcw, u_off, u_off + (size_t)fcw * chroma_h(h, fmt)};
 }
 
 bool odd(size_t v) { return (v & 1) != 0; }
@@ -350,24 +307,43 @@ decltype(&fdct_quant_kernel<false, false>) k2_kernel(const FrameLayout &L)
                               : (L.nv12 ? fdct_quant_kernel<true, LIST> : fdct_quant_kernel<false, LIST>);
 }
 
-// list: the frames are sl.h_desc[0 .. n) (already uploaded to sl.d_desc); the grids are sized for the largest of them
-int launch_pipeline(h2j_encoder *e, Slot &sl, const uint8_t *d_frames, int n, int tail, bool list = false)
+// frame f of the slot's batch as the pipeline reads it (a table of one pair: the pair's layout, for every frame)
+const FrameDesc &frame_desc(const Slot &sl, int f) { return sl.h_desc[f < sl.m ? f : 0]; }
+
+// The batch form of the pipeline takes one layout and reads frame f at base + f * frame_stride: it runs when the frames of the
+// slot's table all have the same layout and are evenly spaced (the list form costs 0.92x on uniform input).  false: a list.
+bool batch_stride(const Slot &sl, long long *frame_stride)
 {
-    sl.list = list;
-    const FrameLayout &L = list ? sl.h_desc[0].L : sl.L;  // (what all frames share: chroma format, nv12)
+    const FrameDesc *D = sl.h_desc;
+    const int m = sl.m;
+    const long long stride = m > 1 ? (long long)((uintptr_t)D[1].base - (uintptr_t)D[0].base) : D[0].L.frame_stride;
+    for (int i = 1; i < m; i++)
+        if (memcmp(&D[i].L, &D[0].L, offsetof(FrameLayout, mb_w) + sizeof(int)) != 0 ||  // (every field, not the tail padding)
+            (uintptr_t)D[i].base != (uintptr_t)D[0].base + (uintptr_t)(i * stride))
+            return false;
+    *frame_stride = stride;
+    return true;
+}
+
+// The pipeline for the slot's batch; the list form reads it from sl.d_desc (uploaded by run_batch), its grids sized for the
+// largest frame
+int launch_pipeline(h2j_encoder *e, Slot &sl, int n, int tail)
+{
+    long long stride = 0;
+    const bool list = !batch_stride(sl, &stride);
+    FrameLayout L = sl.h_desc[0].L;  // (list: what all frames share: chroma format, nv12)
+    L.frame_stride = stride;
+    const uint8_t *d_frames = list ? nullptr : sl.h_desc[0].base;
     const FrameDesc *D = list ? sl.d_desc : nullptr;
-    int mcu_h = L.mcu_h, n_tiles = (L.n_mcu + kTileMcus - 1) / kTileMcus, n_units = (L.n_blocks + kUnitBlocks - 1) / kUnitBlocks;
-    long long total_tiles = (long long)n_tiles * n;
-    if (list) {
-        total_tiles = 0;
-        for (int i = 0; i < n; i++) {
-            const FrameLayout &Li = sl.h_desc[i].L;
-            const int t = (Li.n_mcu + kTileMcus - 1) / kTileMcus;
-            mcu_h = std::max(mcu_h, Li.mcu_h);
-            n_tiles = std::max(n_tiles, t);
-            n_units = std::max(n_units, (Li.n_blocks + kUnitBlocks - 1) / kUnitBlocks);
-            total_tiles += t;
-        }
+    int mcu_h = 0, n_tiles = 0, n_units = 0;
+    long long total_tiles = 0;
+    for (int i = 0; i < n; i++) {
+        const FrameLayout &Li = frame_desc(sl, i).L;
+        const int t = (Li.n_mcu + kTileMcus - 1) / kTileMcus;
+        mcu_h = std::max(mcu_h, Li.mcu_h);
+        n_tiles = std::max(n_tiles, t);
+        n_units = std::max(n_units, (Li.n_blocks + kUnitBlocks - 1) / kUnitBlocks);
+        total_tiles += t;
     }
     cudaStream_t st = sl.stream;
     sl.timings_used = 0;
@@ -599,9 +575,6 @@ int finish_single(h2j_encoder *e, Slot &sl, uint8_t *out, size_t out_capacity, s
     return H2J_OK;
 }
 
-// the layout of frame `frame` of the slot's last batch
-const FrameLayout &frame_layout(const Slot &sl, int frame) { return sl.list ? sl.h_desc[frame].L : sl.L; }
-
 void free_slot(Slot &sl)
 {
     if (sl.stream) cudaStreamSynchronize(sl.stream);
@@ -623,30 +596,40 @@ void free_slot(Slot &sl)
     sl = Slot{};
 }
 
-// The checks of a device list submit's arguments (h2j_submit_device_list, h2j_submit_device_downscaled), all made before
-// anything is enqueued or the slot's table is touched.
-int check_device_list(h2j_encoder *e, int slot, int layout, const h2j_frame_desc *frames, int n)
+// The preamble of every batch submit: a slot that exists and has no batch in flight, a frames pointer, 1 .. max_batch frames.
+// Every check of a submit is made before anything is enqueued or the slot's table is touched: a rejected call leaves the
+// previous batch collectable and inspectable.
+int check_submit(h2j_encoder *e, int slot, const void *frames, int n)
 {
     int rc = check_slot(e, slot);
     if (rc) return rc;
     if (e->slots[slot].busy) return fail(e, H2J_ERR_BUSY, "slot %d has a batch in flight", slot);
     if (!frames || n < 1 || n > e->s.max_batch) return fail(e, H2J_ERR_INVALID_ARG, "bad frames pointer or batch size %d (max %d)", n, e->s.max_batch);
+    return H2J_OK;
+}
+
+// the preamble of a device list submit (h2j_submit_device_list, h2j_submit_device_downscaled)
+int check_device_list(h2j_encoder *e, int slot, int layout, const h2j_frame_desc *frames, int n)
+{
+    int rc = check_submit(e, slot, frames, n);
+    if (rc) return rc;
     if (layout != H2J_LAYOUT_PLANAR && layout != H2J_LAYOUT_SEMIPLANAR) return fail(e, H2J_ERR_INVALID_ARG, "bad layout %d", layout);
     return H2J_OK;
 }
 
-// Caller frame i of a device list submit -> its layout where it is (semi-planar: the pair plane at u_off = v_off) and the
-// bytes from its base that may be read.  within_max: the frame is encoded at this size, so it must fit the encoder.
-int device_frame_layout(h2j_encoder *e, int i, const h2j_frame_desc &F, bool sp, bool within_max, FrameLayout *L, long long *extent)
+// Caller frame i of a device submit -> its layout where it is (semi-planar: the pair plane at u_off = v_off) and the bytes
+// from its base that may be read.  bps: bytes per sample (2: 16-bit words; the layout's pitches and offsets stay in bytes).
+// within_max: the frame is encoded at this size, so it must fit the encoder.
+int device_frame_layout(h2j_encoder *e, int i, const h2j_frame_desc &F, bool sp, int bps, bool within_max, FrameLayout *L, long long *extent)
 {
     const int fmt = e->s.chroma_format;
     if (!F.data) return fail(e, H2J_ERR_INVALID_ARG, "frame %d: null data", i);
-    int rc = make_layout(e, F.data, 0, F.width, F.height, L, within_max);
+    int rc = make_layout(e, F.data, F.width, F.height, L, within_max);
     if (rc) return rc;
     const int fcw = chroma_w(F.width, fmt), fch = chroma_h(F.height, fmt);
-    const int c_row = sp ? 2 * fcw : fcw;  // bytes in a chroma row
-    if (F.y_pitch < F.width || F.c_pitch < c_row)
-        return fail(e, H2J_ERR_INVALID_ARG, "frame %d: pitches %d / %d shorter than rows of %d / %d bytes", i, F.y_pitch, F.c_pitch, F.width, c_row);
+    const int y_row = bps * F.width, c_row = bps * (sp ? 2 * fcw : fcw);  // bytes in a luma / chroma row
+    if (F.y_pitch < y_row || F.c_pitch < c_row)
+        return fail(e, H2J_ERR_INVALID_ARG, "frame %d: pitches %d / %d shorter than rows of %d / %d bytes", i, F.y_pitch, F.c_pitch, y_row, c_row);
     if (sp && F.u_offset < (size_t)F.y_pitch * F.height)
         return fail(e, H2J_ERR_INVALID_ARG, "frame %d: the pair plane starts inside the luma plane", i);
     L->y_pitch = F.y_pitch;
@@ -654,8 +637,97 @@ int device_frame_layout(h2j_encoder *e, int i, const h2j_frame_desc &F, bool sp,
     L->u_off = (long long)F.u_offset;
     L->v_off = (long long)(sp ? F.u_offset : F.v_offset);
     set_alignment(L, F.data);
-    *extent = (long long)std::max((size_t)F.y_pitch * (F.height - 1) + F.width,
+    *extent = (long long)std::max((size_t)F.y_pitch * (F.height - 1) + y_row,
                                   std::max((size_t)L->u_off, (size_t)L->v_off) + (size_t)F.c_pitch * (fch - 1) + c_row);
+    return H2J_OK;
+}
+
+// A batch of frames of one layout F, frame i at F.data + i * frame_stride: checked as frame 0 of a device submit, with every
+// plane inside frame_stride.  Then the slot's table is one pair that describes the frames, read in place.
+int describe_batch(h2j_encoder *e, Slot &sl, const h2j_frame_desc &F, size_t frame_stride, bool sp, int bps)
+{
+    FrameDesc d;
+    int rc = device_frame_layout(e, 0, F, sp, bps, true, &d.L, &d.extent);
+    if (rc) return rc;
+    if ((size_t)d.extent > frame_stride)
+        return fail(e, H2J_ERR_INVALID_ARG, "a plane of the %dx%d frame reaches past frame_stride %zu", F.width, F.height, frame_stride);
+    set_alignment(&d.L, F.data, frame_stride);  // the vector-load flags hold for every frame of the batch
+    d.L.frame_stride = (long long)frame_stride;
+    d.base = F.data;
+    sl.h_desc[0] = sl.h_desc[1] = d;
+    return H2J_OK;
+}
+
+// What a batch's sources are
+struct Input {
+    bool sp = false;    // semi-planar: the Cb/Cr pairs in one plane at u_off (= v_off)
+    int bit_depth = 8;  // 9 .. 16: 16-bit words, converted to 8-bit planar frames
+    int factor = 1;     // 2, 4, 8: box-filtered to 1/factor
+};
+
+// The input stage of every submit, then the pipeline, for n frames described by m entry pairs (m = n, or 1: see Slot).  On
+// entry sl.h_desc[m + i] is the source of frame i where it lies, and sl.h_desc[i] the frame the pipeline encodes (at its
+// size: a downscaled frame's is smaller), read in place.  A frame is read
+// where it is unless it has to be copied:
+//   - 16-bit and downscaled frames are converted (depth_to_8_kernel, downscale_list_kernel);
+//   - a semi-planar batch is read in place when every frame's rows start on 8-byte boundaries (K1 only looks at luma, K2's
+//     chroma roles fetch the pairs and keep their component in registers); otherwise, or with semiplanar_prepass, all of it
+//     is split into planes (nv12_to_i420_kernel);
+//   - planar frames whose rows do not all start on 8-byte boundaries are copied to a 16-byte row pitch (repitch_kernel), when
+//     the slot has room for the copies; otherwise the pipeline's bytewise path reads them where they are.
+// Copies are planar at pitched_layout(), the repitched ones in d_pitched, the others in the slot's frame buffer; one kernel
+// makes all of them.  A table of pairs is uploaded when that kernel or the list form of the pipeline reads it; a batch of one
+// layout at one stride is one pair, which the kernel takes by value.
+int run_batch(h2j_encoder *e, Slot &sl, int n, int m, const Input &in, int tail)
+{
+    FrameDesc *D = sl.h_desc, *S = sl.h_desc + m;
+    const int fmt = e->s.chroma_format;
+    const bool convert = in.bit_depth > 8 || in.factor > 1;
+    bool unaligned = false;
+    for (int i = 0; i < m; i++) unaligned = unaligned || !S[i].L.aligned8;
+    const bool split = in.sp && (unaligned || e->force_sp_prepass);
+    const size_t pitched_cap = pitched_frame_bytes(e->s.max_width, e->s.max_height, fmt);
+    if (!convert && !in.sp && unaligned && !sl.d_pitched && cudaMalloc(&sl.d_pitched, pitched_cap * e->s.max_batch) != cudaSuccess) {
+        cudaGetLastError();  // no room for the copies: the bytewise path still works
+        sl.d_pitched = nullptr;
+    }
+    int cols = 0, rows = 0;  // the largest copy: 16-byte columns of its widest row (semi-planar: of pairs), rows of all planes
+    for (int i = 0; i < m; i++) {
+        if (!convert && !split && (in.sp || S[i].L.aligned8 || !sl.d_pitched)) {
+            S[i].base = nullptr;
+            D[i].L.nv12 = in.sp ? 1 : 0;
+            continue;
+        }
+        const size_t spacing = convert || in.sp ? e->frame_bytes_cap : pitched_cap;
+        D[i].L = pitched_layout(D[i].L);
+        D[i].L.frame_stride = (long long)spacing;
+        D[i].base = (convert || in.sp ? sl.d_frames : sl.d_pitched) + (size_t)i * spacing;
+        const int w = D[i].L.w, h = D[i].L.h;
+        cols = std::max(cols, (std::max(w, (in.sp ? 2 : 1) * chroma_w(w, fmt)) + 15) / 16);
+        rows = std::max(rows, h + (in.sp ? 1 : 2) * chroma_h(h, fmt));
+    }
+    sl.n = n;
+    sl.m = m;
+    long long stride;
+    if (m > 1 && (rows || !batch_stride(sl, &stride)))  // (a table of one pair goes to the copy kernel by value)
+        CU(e, cudaMemcpyAsync(sl.d_desc, sl.h_desc, sizeof(FrameDesc) * (rows ? 2 * m : m), cudaMemcpyHostToDevice, sl.stream));
+    if (rows) {
+        static_assert(32 * kDownWarps == 128, "every copy kernel runs CTAs of 128 threads");
+        const int rows_per_cta = in.factor > 1 ? kDownWarps * 16 / in.factor : kPlaneRowsPerCta;
+        const dim3 grid(in.factor > 1 ? (cols + 31) / 32 : (cols + 127) / 128, (rows + rows_per_cta - 1) / rows_per_cta, n);
+        decltype(&repitch_kernel) k = in.sp ? nv12_to_i420_kernel : repitch_kernel;
+        if (in.factor == 2) k = in.sp ? downscale_list_kernel<2, true> : downscale_list_kernel<2, false>;
+        else if (in.factor == 4) k = in.sp ? downscale_list_kernel<4, true> : downscale_list_kernel<4, false>;
+        else if (in.factor == 8) k = in.sp ? downscale_list_kernel<8, true> : downscale_list_kernel<8, false>;
+        const CopyTable t{sl.d_desc, m, D[0], S[0]};
+        if (in.bit_depth > 8) (in.sp ? depth_to_8_kernel<true> : depth_to_8_kernel<false>)<<<grid, 128, 0, sl.stream>>>(t, in.bit_depth - 8);
+        else k<<<grid, 128, 0, sl.stream>>>(t);
+        e->launches++;
+        CU(e, cudaGetLastError());
+    }
+    int rc = launch_pipeline(e, sl, n, tail);
+    if (rc) return rc;
+    if (tail != TAIL_SINGLE) sl.busy = true;
     return H2J_OK;
 }
 
@@ -849,87 +921,34 @@ int h2j_create(const h2j_settings *s, h2j_encoder **out)
 
 int h2j_submit_device(h2j_encoder *e, int slot, const uint8_t *d_frames, size_t frame_stride, int n, int width, int height)
 {
-    int rc = check_slot(e, slot);
+    int rc = check_submit(e, slot, d_frames, n);
     if (rc) return rc;
     Slot &sl = e->slots[slot];
-    if (sl.busy) return fail(e, H2J_ERR_BUSY, "slot %d has a batch in flight", slot);
-    if (!d_frames || n < 1 || n > e->s.max_batch) return fail(e, H2J_ERR_INVALID_ARG, "bad frames pointer or batch size %d (max %d)", n, e->s.max_batch);
-    if (frame_stride < tight_frame_bytes(width, height, e->s.chroma_format)) return fail(e, H2J_ERR_INVALID_ARG, "frame_stride smaller than one frame");
+    rc = describe_batch(e, sl, tight_frame(d_frames, width, height, e->s.chroma_format), frame_stride, false, 1);
+    if (rc) return rc;
     ON_DEVICE(e);
-    sl.n = n;
     CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
-    const uint8_t *pipe_src = nullptr;
-    rc = prepare_input(e, sl, d_frames, frame_stride, n, width, height, &pipe_src);
-    if (rc) return rc;
-    rc = launch_pipeline(e, sl, pipe_src, n, TAIL_SIZES);
-    if (rc) return rc;
-    sl.busy = true;
-    return H2J_OK;
+    return run_batch(e, sl, n, 1, Input{}, TAIL_SIZES);
 }
 
 int h2j_submit_device_semiplanar(h2j_encoder *e, int slot, const uint8_t *d_frames, size_t frame_stride, int pitch, size_t uv_offset,
                                  int n, int width, int height)
 {
-    int rc = check_slot(e, slot);
+    int rc = check_submit(e, slot, d_frames, n);
     if (rc) return rc;
     Slot &sl = e->slots[slot];
-    if (sl.busy) return fail(e, H2J_ERR_BUSY, "slot %d has a batch in flight", slot);
-    if (!d_frames || n < 1 || n > e->s.max_batch) return fail(e, H2J_ERR_INVALID_ARG, "bad frames pointer or batch size %d (max %d)", n, e->s.max_batch);
-    if (width < 2 || height < 2) return fail(e, H2J_ERR_UNSUPPORTED, "unsupported frame size %dx%d", width, height);
-    const int fmt = e->s.chroma_format;
-    const int fcw = chroma_w(width, fmt), fch = chroma_h(height, fmt);  // pairs per row, rows of the pair plane
-    if (pitch < width || pitch < 2 * fcw) return fail(e, H2J_ERR_INVALID_ARG, "pitch %d smaller than a row of %d samples", pitch, width);
-    if (uv_offset < (size_t)pitch * height || frame_stride < uv_offset + (size_t)pitch * (fch - 1) + 2 * (size_t)fcw)
-        return fail(e, H2J_ERR_INVALID_ARG, "uv_offset / frame_stride do not hold a semi-planar frame of %dx%d at pitch %d", width, height, pitch);
-    const size_t fb = tight_frame_bytes(width, height, fmt);
-    const size_t dstride = align_up(fb, 256);
-    if (dstride > e->frame_bytes_cap) return fail(e, H2J_ERR_UNSUPPORTED, "frame %dx%d exceeds the configured maximum", width, height);
+    rc = describe_batch(e, sl, h2j_frame_desc{d_frames, width, height, pitch, pitch, uv_offset, uv_offset}, frame_stride, true, 1);
+    if (rc) return rc;
     ON_DEVICE(e);
-    rc = make_layout(e, sl.d_frames, dstride, width, height, &sl.L);
-    if (rc) return rc;
-    sl.n = n;
     CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
-    // Rows on 8-byte boundaries (what decoders produce): the pipeline reads the frames where they are -- K1 only looks at
-    // luma, K2's chroma roles fetch the pairs and keep their component in registers.  Otherwise the pairs are split into
-    // the slot's planar frame buffer first (one more pass over the frame).
-    if (!e->force_sp_prepass && (uintptr_t)d_frames % 8 == 0 && frame_stride % 8 == 0 && pitch % 8 == 0 && uv_offset % 8 == 0) {
-        FrameLayout &L = sl.L;
-        L.y_pitch = pitch;
-        L.c_pitch = pitch;
-        L.u_off = (long long)uv_offset;
-        L.v_off = (long long)uv_offset;
-        L.frame_stride = (long long)frame_stride;
-        L.aligned8 = 1;
-        L.aligned16 = ((uintptr_t)d_frames % 16 == 0 && frame_stride % 16 == 0 && pitch % 16 == 0) ? 1 : 0;
-        L.nv12 = 1;
-        rc = launch_pipeline(e, sl, d_frames, n, TAIL_SIZES);
-        if (rc) return rc;
-        sl.busy = true;
-        return H2J_OK;
-    }
-    const int src_aligned16 = ((uintptr_t)d_frames % 16) == 0 && (frame_stride % 16) == 0 && (pitch % 16) == 0 ? 1 : 0;
-    const int row_bytes = width > 2 * fcw ? width : 2 * fcw;
-    nv12_to_i420_kernel<<<dim3((row_bytes + 128 * 16 - 1) / (128 * 16), (height + fch + kPlaneRowsPerCta - 1) / kPlaneRowsPerCta, n), 128, 0, sl.stream>>>(
-        d_frames, (long long)frame_stride, pitch, (long long)uv_offset, sl.d_frames, sl.L, src_aligned16);
-    e->launches++;
-    CU(e, cudaGetLastError());
-    const uint8_t *pipe_src = nullptr;
-    rc = prepare_input(e, sl, sl.d_frames, dstride, n, width, height, &pipe_src);  // (odd widths: once more, to a 16-byte pitch)
-    if (rc) return rc;
-    rc = launch_pipeline(e, sl, pipe_src, n, TAIL_SIZES);
-    if (rc) return rc;
-    sl.busy = true;
-    return H2J_OK;
+    return run_batch(e, sl, n, 1, Input{true}, TAIL_SIZES);
 }
 
 int h2j_submit_device_nv12(h2j_encoder *e, int slot, const uint8_t *d_frames, size_t frame_stride, int pitch, size_t uv_offset, int n,
                            int width, int height)
 {
-    int rc = check_slot(e, slot);
+    int rc = check_submit(e, slot, d_frames, n);
     if (rc) return rc;
-    if (e->slots[slot].busy) return fail(e, H2J_ERR_BUSY, "slot %d has a batch in flight", slot);
-    if (!d_frames || n < 1 || n > e->s.max_batch) return fail(e, H2J_ERR_INVALID_ARG, "bad frames pointer or batch size %d (max %d)", n, e->s.max_batch);
-    if (width < 2 || height < 2) return fail(e, H2J_ERR_UNSUPPORTED, "unsupported frame size %dx%d", width, height);
     if (e->s.chroma_format != H2J_CHROMA_420) return fail(e, H2J_ERR_UNSUPPORTED, "NV12 is a 4:2:0 layout; this encoder was created for another chroma format");
     return h2j_submit_device_semiplanar(e, slot, d_frames, frame_stride, pitch, uv_offset, n, width, height);
 }
@@ -937,128 +956,65 @@ int h2j_submit_device_nv12(h2j_encoder *e, int slot, const uint8_t *d_frames, si
 int h2j_submit_device_pitched(h2j_encoder *e, int slot, const uint8_t *d_frames, size_t frame_stride, int y_pitch, int c_pitch,
                               size_t u_offset, size_t v_offset, int n, int width, int height)
 {
-    int rc = check_slot(e, slot);
+    int rc = check_submit(e, slot, d_frames, n);
     if (rc) return rc;
     Slot &sl = e->slots[slot];
-    if (sl.busy) return fail(e, H2J_ERR_BUSY, "slot %d has a batch in flight", slot);
-    if (!d_frames || n < 1 || n > e->s.max_batch) return fail(e, H2J_ERR_INVALID_ARG, "bad frames pointer or batch size %d (max %d)", n, e->s.max_batch);
-    if (width < 2 || height < 2) return fail(e, H2J_ERR_UNSUPPORTED, "unsupported frame size %dx%d", width, height);
-    const int fmt = e->s.chroma_format;
-    const int fcw = chroma_w(width, fmt), fch = chroma_h(height, fmt);
-    if (y_pitch < width || c_pitch < fcw) return fail(e, H2J_ERR_INVALID_ARG, "pitches %d / %d smaller than rows of %d / %d samples", y_pitch, c_pitch, width, fcw);
-    const size_t y_end = (size_t)y_pitch * (height - 1) + width;
-    const size_t u_end = u_offset + (size_t)c_pitch * (fch - 1) + fcw, v_end = v_offset + (size_t)c_pitch * (fch - 1) + fcw;
-    if (y_end > frame_stride || u_end > frame_stride || v_end > frame_stride)
-        return fail(e, H2J_ERR_INVALID_ARG, "a plane of the %dx%d frame reaches past frame_stride %zu", width, height, frame_stride);
+    rc = describe_batch(e, sl, h2j_frame_desc{d_frames, width, height, y_pitch, c_pitch, u_offset, v_offset}, frame_stride, false, 1);
+    if (rc) return rc;
     ON_DEVICE(e);
-    rc = make_layout(e, d_frames, frame_stride, width, height, &sl.L);
-    if (rc) return rc;
-    FrameLayout &L = sl.L;
-    L.y_pitch = y_pitch;
-    L.c_pitch = c_pitch;
-    L.u_off = (long long)u_offset;
-    L.v_off = (long long)v_offset;
-    set_alignment(&L, d_frames);
-    sl.n = n;
     CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
-    // rows on 8-byte boundaries: the pipeline reads the frames where they are; otherwise one copy to a 16-byte pitch
-    const uint8_t *pipe_src = nullptr;
-    const uint8_t *src_end = d_frames + (size_t)(n - 1) * frame_stride + std::max(y_end, std::max(u_end, v_end));
-    rc = repitch_if_unaligned(e, sl, d_frames, src_end, n, &pipe_src);
-    if (rc) return rc;
-    rc = launch_pipeline(e, sl, pipe_src, n, TAIL_SIZES);
-    if (rc) return rc;
-    sl.busy = true;
-    return H2J_OK;
+    return run_batch(e, sl, n, 1, Input{}, TAIL_SIZES);
 }
 
 int h2j_submit_device_semiplanar16(h2j_encoder *e, int slot, const uint8_t *d_frames, size_t frame_stride, int pitch, size_t uv_offset,
                                    int bit_depth, int n, int width, int height)
 {
-    int rc = check_slot(e, slot);
+    int rc = check_submit(e, slot, d_frames, n);
     if (rc) return rc;
-    Slot &sl = e->slots[slot];
-    if (sl.busy) return fail(e, H2J_ERR_BUSY, "slot %d has a batch in flight", slot);
-    if (!d_frames || n < 1 || n > e->s.max_batch) return fail(e, H2J_ERR_INVALID_ARG, "bad frames pointer or batch size %d (max %d)", n, e->s.max_batch);
-    if (width < 2 || height < 2) return fail(e, H2J_ERR_UNSUPPORTED, "unsupported frame size %dx%d", width, height);
     if (bit_depth < 9 || bit_depth > 16) return fail(e, H2J_ERR_INVALID_ARG, "bit_depth %d outside 9..16", bit_depth);
     if (odd((uintptr_t)d_frames) || odd(frame_stride) || odd((size_t)pitch) || odd(uv_offset))
         return fail(e, H2J_ERR_INVALID_ARG, "16-bit samples need even pointers, strides, pitches and offsets");
-    const int fmt = e->s.chroma_format;
-    const int fcw = chroma_w(width, fmt), fch = chroma_h(height, fmt);  // pairs per row, rows of the pair plane
-    if (pitch < 2 * std::max(width, 2 * fcw)) return fail(e, H2J_ERR_INVALID_ARG, "pitch %d smaller than a row of %d 16-bit words", pitch, std::max(width, 2 * fcw));
-    if (uv_offset < (size_t)pitch * height || frame_stride < uv_offset + (size_t)pitch * (fch - 1) + 4 * (size_t)fcw)
-        return fail(e, H2J_ERR_INVALID_ARG, "uv_offset / frame_stride do not hold a semi-planar frame of %dx%d at pitch %d", width, height, pitch);
+    Slot &sl = e->slots[slot];
+    rc = describe_batch(e, sl, h2j_frame_desc{d_frames, width, height, pitch, pitch, uv_offset, uv_offset}, frame_stride, true, 2);
+    if (rc) return rc;
     ON_DEVICE(e);
-    sl.n = n;
     CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
-    rc = convert_depth(e, sl, d_frames, Src16{(long long)frame_stride, (long long)uv_offset, (long long)uv_offset, pitch, pitch}, true, bit_depth, n,
-                       width, height);
-    if (rc) return rc;
-    rc = launch_pipeline(e, sl, sl.d_frames, n, TAIL_SIZES);
-    if (rc) return rc;
-    sl.busy = true;
-    return H2J_OK;
+    return run_batch(e, sl, n, 1, Input{true, bit_depth}, TAIL_SIZES);
 }
 
 int h2j_submit_device_pitched16(h2j_encoder *e, int slot, const uint8_t *d_frames, size_t frame_stride, int y_pitch, int c_pitch,
                                 size_t u_offset, size_t v_offset, int bit_depth, int n, int width, int height)
 {
-    int rc = check_slot(e, slot);
+    int rc = check_submit(e, slot, d_frames, n);
     if (rc) return rc;
-    Slot &sl = e->slots[slot];
-    if (sl.busy) return fail(e, H2J_ERR_BUSY, "slot %d has a batch in flight", slot);
-    if (!d_frames || n < 1 || n > e->s.max_batch) return fail(e, H2J_ERR_INVALID_ARG, "bad frames pointer or batch size %d (max %d)", n, e->s.max_batch);
-    if (width < 2 || height < 2) return fail(e, H2J_ERR_UNSUPPORTED, "unsupported frame size %dx%d", width, height);
     if (bit_depth < 9 || bit_depth > 16) return fail(e, H2J_ERR_INVALID_ARG, "bit_depth %d outside 9..16", bit_depth);
     if (odd((uintptr_t)d_frames) || odd(frame_stride) || odd((size_t)y_pitch) || odd((size_t)c_pitch) || odd(u_offset) || odd(v_offset))
         return fail(e, H2J_ERR_INVALID_ARG, "16-bit samples need even pointers, strides, pitches and offsets");
-    const int fmt = e->s.chroma_format;
-    const int fcw = chroma_w(width, fmt), fch = chroma_h(height, fmt);
-    if (y_pitch < 2 * width || c_pitch < 2 * fcw)
-        return fail(e, H2J_ERR_INVALID_ARG, "pitches %d / %d smaller than rows of %d / %d 16-bit words", y_pitch, c_pitch, width, fcw);
-    const size_t y_end = (size_t)y_pitch * (height - 1) + 2 * (size_t)width;
-    const size_t u_end = u_offset + (size_t)c_pitch * (fch - 1) + 2 * (size_t)fcw, v_end = v_offset + (size_t)c_pitch * (fch - 1) + 2 * (size_t)fcw;
-    if (y_end > frame_stride || u_end > frame_stride || v_end > frame_stride)
-        return fail(e, H2J_ERR_INVALID_ARG, "a plane of the %dx%d frame reaches past frame_stride %zu", width, height, frame_stride);
+    Slot &sl = e->slots[slot];
+    rc = describe_batch(e, sl, h2j_frame_desc{d_frames, width, height, y_pitch, c_pitch, u_offset, v_offset}, frame_stride, false, 2);
+    if (rc) return rc;
     ON_DEVICE(e);
-    sl.n = n;
     CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
-    rc = convert_depth(e, sl, d_frames, Src16{(long long)frame_stride, (long long)u_offset, (long long)v_offset, y_pitch, c_pitch}, false, bit_depth,
-                       n, width, height);
-    if (rc) return rc;
-    rc = launch_pipeline(e, sl, sl.d_frames, n, TAIL_SIZES);
-    if (rc) return rc;
-    sl.busy = true;
-    return H2J_OK;
+    return run_batch(e, sl, n, 1, Input{false, bit_depth}, TAIL_SIZES);
 }
 
 int h2j_submit_host(h2j_encoder *e, int slot, const uint8_t *frames, size_t frame_stride, int n, int width, int height)
 {
-    int rc = check_slot(e, slot);
+    int rc = check_submit(e, slot, frames, n);
     if (rc) return rc;
     Slot &sl = e->slots[slot];
-    if (sl.busy) return fail(e, H2J_ERR_BUSY, "slot %d has a batch in flight", slot);
-    if (!frames || n < 1 || n > e->s.max_batch) return fail(e, H2J_ERR_INVALID_ARG, "bad frames pointer or batch size %d (max %d)", n, e->s.max_batch);
     const size_t fb = tight_frame_bytes(width, height, e->s.chroma_format);
     if (frame_stride < fb) return fail(e, H2J_ERR_INVALID_ARG, "frame_stride smaller than one frame");
-    ON_DEVICE(e);
     // device copy keeps frames at a 256-byte aligned stride so the vector-load paths apply
     const size_t dstride = align_up(fb, 256);
     if (dstride > e->frame_bytes_cap) return fail(e, H2J_ERR_UNSUPPORTED, "frame %dx%d exceeds the configured maximum", width, height);
-    rc = make_layout(e, sl.d_frames, dstride, width, height, &sl.L);
+    rc = describe_batch(e, sl, tight_frame(sl.d_frames, width, height, e->s.chroma_format), dstride, false, 1);
     if (rc) return rc;
-    sl.n = n;
+    ON_DEVICE(e);
     CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
     if (frame_stride == dstride) CU(e, cudaMemcpyAsync(sl.d_frames, frames, dstride * (n - 1) + fb, cudaMemcpyHostToDevice, sl.stream));
     else CU(e, cudaMemcpy2DAsync(sl.d_frames, dstride, frames, frame_stride, fb, n, cudaMemcpyHostToDevice, sl.stream));
-    const uint8_t *pipe_src = nullptr;
-    rc = prepare_input(e, sl, sl.d_frames, dstride, n, width, height, &pipe_src);
-    if (rc) return rc;
-    rc = launch_pipeline(e, sl, pipe_src, n, TAIL_PACK);
-    if (rc) return rc;
-    sl.busy = true;
-    return H2J_OK;
+    return run_batch(e, sl, n, 1, Input{}, TAIL_PACK);
 }
 
 int h2j_submit_device_list(h2j_encoder *e, int slot, int layout, const h2j_frame_desc *frames, int n)
@@ -1067,79 +1023,16 @@ int h2j_submit_device_list(h2j_encoder *e, int slot, int layout, const h2j_frame
     if (rc) return rc;
     Slot &sl = e->slots[slot];
     const bool sp = layout == H2J_LAYOUT_SEMIPLANAR;
-    const int fmt = e->s.chroma_format;
-    // every frame is checked before anything is enqueued or the slot's table is touched (a rejected call leaves the previous
-    // batch's table as it was); tab[i] is what the pipeline reads, tab[n + i] the copy's source
-    std::vector<FrameDesc> tab(2 * (size_t)n);
-    bool in_place = !e->force_sp_prepass;  // (semi-planar: every frame on 8-byte boundaries)
-    bool copies = false;
+    std::vector<FrameDesc> tab(n);  // (every frame is checked before the slot's table is touched)
     for (int i = 0; i < n; i++) {
-        const h2j_frame_desc &F = frames[i];
-        FrameLayout L;
-        long long extent = 0;
-        rc = device_frame_layout(e, i, F, sp, true, &L, &extent);
+        rc = device_frame_layout(e, i, frames[i], sp, 1, true, &tab[i].L, &tab[i].extent);
         if (rc) return rc;
-        FrameDesc &src = tab[n + i];
-        src.L = L;
-        src.base = nullptr;
-        src.extent = extent;
-        tab[i].L = L;
-        tab[i].base = F.data;
-        tab[i].extent = 0;
-        if (sp) {
-            if ((uintptr_t)F.data % 8 || F.y_pitch % 8 || F.c_pitch % 8 || F.u_offset % 8) in_place = false;
-        } else if (!L.aligned8) {
-            copies = true;
-        }
+        tab[i].base = frames[i].data;
     }
-    memcpy(sl.h_desc, tab.data(), sizeof(FrameDesc) * 2 * n);
-    sl.list = true;  // the debug hooks answer from this table from here on
-    sl.n = n;
+    for (int i = 0; i < n; i++) sl.h_desc[i] = sl.h_desc[n + i] = tab[i];
     ON_DEVICE(e);
-    sl.n = n;
     CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
-    // planar frames with rows off 8-byte boundaries are copied to a 16-byte pitch, all in one launch; the others are read
-    // where they are
-    if (copies && !sl.d_pitched) {
-        const size_t bytes = pitched_frame_bytes(e->s.max_width, e->s.max_height, fmt) * (size_t)e->s.max_batch;
-        if (cudaMalloc(&sl.d_pitched, bytes) != cudaSuccess) {  // no room for the copies: the bytewise path still works
-            cudaGetLastError();
-            sl.d_pitched = nullptr;
-            copies = false;
-        }
-    }
-    if (sp) copies = !in_place;  // a semi-planar batch is read in place or split completely
-    int copy_w = 0, copy_rows = 0;
-    for (int i = 0; i < n; i++) {
-        FrameDesc &d = sl.h_desc[i];
-        const int fch = chroma_h(d.L.h, fmt);
-        if (sp && in_place) {
-            d.L.aligned8 = 1;
-            d.L.aligned16 = ((uintptr_t)d.base % 16 == 0 && d.L.y_pitch % 16 == 0) ? 1 : 0;
-            d.L.nv12 = 1;
-        } else if (sp || (copies && !d.L.aligned8)) {
-            FrameDesc &src = sl.h_desc[n + i];
-            src.base = d.base;
-            src.L.aligned16 = ((uintptr_t)d.base % 16 == 0 && d.L.y_pitch % 16 == 0 && d.L.c_pitch % 16 == 0) ? 1 : 0;
-            d.L = pitched_layout(d.L);
-            d.L.frame_stride = 0;
-            d.base = sp ? sl.d_frames + (size_t)i * e->frame_bytes_cap
-                        : sl.d_pitched + (size_t)i * pitched_frame_bytes(e->s.max_width, e->s.max_height, fmt);
-            copy_w = std::max(copy_w, sp ? std::max(d.L.w, 2 * chroma_w(d.L.w, fmt)) : d.L.w);
-            copy_rows = std::max(copy_rows, d.L.h + (sp ? 1 : 2) * fch);
-        }
-    }
-    CU(e, cudaMemcpyAsync(sl.d_desc, sl.h_desc, sizeof(FrameDesc) * (copies ? 2 * n : n), cudaMemcpyHostToDevice, sl.stream));
-    if (copies) {
-        const dim3 grid((copy_w + 128 * 16 - 1) / (128 * 16), (copy_rows + kPlaneRowsPerCta - 1) / kPlaneRowsPerCta, n);
-        (sp ? nv12_to_i420_list_kernel : repitch_list_kernel)<<<grid, 128, 0, sl.stream>>>(sl.d_desc, n);
-        e->launches++;
-        CU(e, cudaGetLastError());
-    }
-    rc = launch_pipeline(e, sl, nullptr, n, TAIL_SIZES, true);
-    if (rc) return rc;
-    sl.busy = true;
-    return H2J_OK;
+    return run_batch(e, sl, n, n, Input{sp}, TAIL_SIZES);
 }
 
 int h2j_submit_device_downscaled(h2j_encoder *e, int slot, int layout, const h2j_frame_desc *frames, int n, int factor)
@@ -1149,135 +1042,50 @@ int h2j_submit_device_downscaled(h2j_encoder *e, int slot, int layout, const h2j
     if (factor != 2 && factor != 4 && factor != 8) return fail(e, H2J_ERR_INVALID_ARG, "factor %d is not 2, 4 or 8", factor);
     Slot &sl = e->slots[slot];
     const bool sp = layout == H2J_LAYOUT_SEMIPLANAR;
-    const int fmt = e->s.chroma_format;
-    // tab[i]: the downscaled frame the pipeline reads, planar at a 16-byte row pitch in the slot's frame buffer; tab[n + i]:
-    // the caller's frame.  Only the downscaled size is held to the encoder's maximum.  (Checked before the slot's table is
-    // touched, as h2j_submit_device_list.)
+    // tab[i]: the downscaled frame the pipeline encodes, tab[n + i]: the caller's frame.  Only the downscaled size is held to
+    // the encoder's maximum.
     std::vector<FrameDesc> tab(2 * (size_t)n);
-    bool uniform = true;
-    int cols = 0, rows = 0;  // the largest destination: 16-byte columns of a row (SP chroma: 8 pairs), rows of all planes
     for (int i = 0; i < n; i++) {
         const h2j_frame_desc &F = frames[i];
         FrameDesc &src = tab[n + i];
-        rc = device_frame_layout(e, i, F, sp, false, &src.L, &src.extent);
+        rc = device_frame_layout(e, i, F, sp, 1, false, &src.L, &src.extent);
         if (rc) return rc;
         src.base = F.data;
         const int w = (F.width + factor - 1) / factor, h = (F.height + factor - 1) / factor;
         if (w < 2 || h < 2)
             return fail(e, H2J_ERR_UNSUPPORTED, "frame %d: %dx%d at 1/%d is %dx%d, smaller than 2x2", i, F.width, F.height, factor, w, h);
-        FrameDesc &d = tab[i];
-        uint8_t *dev = sl.d_frames + (size_t)i * e->frame_bytes_cap;
-        rc = make_layout(e, dev, 0, w, h, &d.L);
+        rc = make_layout(e, nullptr, w, h, &tab[i].L);
         if (rc) return rc;
-        d.L = pitched_layout(d.L);
-        d.L.frame_stride = 0;
-        d.base = dev;
-        d.extent = 0;
-        uniform = uniform && w == tab[0].L.w && h == tab[0].L.h;
-        const int fcw = chroma_w(w, fmt), fch = chroma_h(h, fmt);
-        cols = std::max(cols, std::max((w + 15) / 16, sp ? (fcw + 7) / 8 : (fcw + 15) / 16));
-        rows = std::max(rows, h + (sp ? 1 : 2) * fch);
     }
     memcpy(sl.h_desc, tab.data(), sizeof(FrameDesc) * 2 * n);
-    sl.list = true;  // the debug hooks answer from this table from here on (the batch form below answers from sl.L)
-    sl.n = n;
     ON_DEVICE(e);
     CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
-    CU(e, cudaMemcpyAsync(sl.d_desc, sl.h_desc, sizeof(FrameDesc) * 2 * n, cudaMemcpyHostToDevice, sl.stream));
-    // every layout is read where it is: no repitch or split in front
-    {
-        const int rows_per_cta = kDownWarps * 16 / factor;
-        const dim3 grid((cols + 31) / 32, (rows + rows_per_cta - 1) / rows_per_cta, n);
-        decltype(&downscale_list_kernel<2, false>) k;
-        if (factor == 2) k = sp ? downscale_list_kernel<2, true> : downscale_list_kernel<2, false>;
-        else if (factor == 4) k = sp ? downscale_list_kernel<4, true> : downscale_list_kernel<4, false>;
-        else k = sp ? downscale_list_kernel<8, true> : downscale_list_kernel<8, false>;
-        k<<<grid, 32 * kDownWarps, 0, sl.stream>>>(sl.d_desc, n);
-        e->launches++;
-        CU(e, cudaGetLastError());
-    }
-    // frames of one size go through the batch form of the pipeline (the list form costs 0.92x on uniform input)
-    if (uniform) {
-        sl.L = sl.h_desc[0].L;
-        sl.L.frame_stride = (long long)e->frame_bytes_cap;
-        rc = launch_pipeline(e, sl, sl.d_frames, n, TAIL_SIZES);
-    } else {
-        rc = launch_pipeline(e, sl, nullptr, n, TAIL_SIZES, true);
-    }
-    if (rc) return rc;
-    sl.busy = true;
-    return H2J_OK;
+    return run_batch(e, sl, n, n, Input{sp, 8, factor}, TAIL_SIZES);
 }
 
 int h2j_submit_host_list(h2j_encoder *e, int slot, const uint8_t *const *frames, const int *widths, const int *heights, int n)
 {
-    int rc = check_slot(e, slot);
+    int rc = check_submit(e, slot, widths && heights ? frames : nullptr, n);
     if (rc) return rc;
     Slot &sl = e->slots[slot];
-    if (sl.busy) return fail(e, H2J_ERR_BUSY, "slot %d has a batch in flight", slot);
-    if (!frames || !widths || !heights || n < 1 || n > e->s.max_batch)
-        return fail(e, H2J_ERR_INVALID_ARG, "bad frames / sizes pointer or batch size %d (max %d)", n, e->s.max_batch);
     const int fmt = e->s.chroma_format;
-    std::vector<FrameDesc> tab(2 * (size_t)n);  // (checked before the slot's table is touched, as h2j_submit_device_list)
-    bool copies = false;
+    std::vector<FrameDesc> tab(n);  // (every frame is checked before the slot's table is touched)
     for (int i = 0; i < n; i++) {
         if (!frames[i]) return fail(e, H2J_ERR_INVALID_ARG, "frame %d: null pointer", i);
         // frame i goes to its own place of the slot's frame buffer, sized for a tight frame at the maximum geometry
         uint8_t *dev = sl.d_frames + (size_t)i * e->frame_bytes_cap;
-        FrameDesc &d = tab[i];
-        rc = make_layout(e, dev, 0, widths[i], heights[i], &d.L);
+        rc = make_layout(e, dev, widths[i], heights[i], &tab[i].L);
         if (rc) return rc;
-        d.base = dev;
-        d.extent = 0;
-        FrameDesc &src = tab[n + i];
-        src.base = nullptr;
-        if (!d.L.aligned8) {  // odd widths: copied once more, to a 16-byte pitch
-            copies = true;
-            src.L = d.L;
-            src.base = dev;
-            src.extent = (long long)tight_frame_bytes(widths[i], heights[i], fmt);
-            d.L = pitched_layout(d.L);
-            d.L.frame_stride = 0;
-        }
+        tab[i].base = dev;
+        tab[i].extent = (long long)tight_frame_bytes(widths[i], heights[i], fmt);
     }
-    memcpy(sl.h_desc, tab.data(), sizeof(FrameDesc) * 2 * n);
-    sl.list = true;  // the debug hooks answer from this table from here on
-    sl.n = n;
+    for (int i = 0; i < n; i++) sl.h_desc[i] = sl.h_desc[n + i] = tab[i];
     ON_DEVICE(e);
-    if (copies && !sl.d_pitched) {
-        const size_t bytes = pitched_frame_bytes(e->s.max_width, e->s.max_height, fmt) * (size_t)e->s.max_batch;
-        if (cudaMalloc(&sl.d_pitched, bytes) != cudaSuccess) {  // no room for the copies: the bytewise path still works
-            cudaGetLastError();
-            sl.d_pitched = nullptr;
-            copies = false;
-            for (int i = 0; i < n; i++)
-                if (sl.h_desc[n + i].base) sl.h_desc[i].L = sl.h_desc[n + i].L;
-        }
-    }
-    int copy_w = 0, copy_rows = 0;
-    for (int i = 0; copies && i < n; i++) {
-        FrameDesc &d = sl.h_desc[i];
-        if (!sl.h_desc[n + i].base) continue;
-        d.base = sl.d_pitched + (size_t)i * pitched_frame_bytes(e->s.max_width, e->s.max_height, fmt);
-        copy_w = std::max(copy_w, d.L.w);
-        copy_rows = std::max(copy_rows, d.L.h + 2 * chroma_h(d.L.h, fmt));
-    }
-    sl.n = n;
     CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
     for (int i = 0; i < n; i++)
         CU(e, cudaMemcpyAsync(sl.d_frames + (size_t)i * e->frame_bytes_cap, frames[i], tight_frame_bytes(widths[i], heights[i], fmt),
                               cudaMemcpyHostToDevice, sl.stream));
-    CU(e, cudaMemcpyAsync(sl.d_desc, sl.h_desc, sizeof(FrameDesc) * (copies ? 2 * n : n), cudaMemcpyHostToDevice, sl.stream));
-    if (copies) {
-        const dim3 grid((copy_w + 128 * 16 - 1) / (128 * 16), (copy_rows + kPlaneRowsPerCta - 1) / kPlaneRowsPerCta, n);
-        repitch_list_kernel<<<grid, 128, 0, sl.stream>>>(sl.d_desc, n);
-        e->launches++;
-        CU(e, cudaGetLastError());
-    }
-    rc = launch_pipeline(e, sl, nullptr, n, TAIL_PACK, true);
-    if (rc) return rc;
-    sl.busy = true;
-    return H2J_OK;
+    return run_batch(e, sl, n, n, Input{}, TAIL_PACK);
 }
 
 int h2j_slot_set_stream(h2j_encoder *e, int slot, void *cuda_stream)
@@ -1386,13 +1194,13 @@ int h2j_encode_frame(h2j_encoder *e, const uint8_t *const planes[3], const int s
     const size_t fb = tight_frame_bytes(width, height, e->s.chroma_format);
     const size_t dstride = align_up(fb, 256);
     if (dstride > e->frame_bytes_cap) return fail(e, H2J_ERR_UNSUPPORTED, "frame %dx%d exceeds the configured maximum", width, height);
-    int rc = make_layout(e, sl.d_frames, dstride, width, height, &sl.L);
+    FrameLayout L;
+    int rc = make_layout(e, sl.d_frames, width, height, &L);
     if (rc) return rc;
     // rows that would not start on 8-byte boundaries (odd widths) are staged at a 16-byte pitch right here: the rows are
     // copied one by one anyway, and the kernels keep their vector loads without a second pass over the frame
-    if (!sl.L.aligned8) sl.L = pitched_layout(sl.L);
-    const FrameLayout &L = sl.L;
-    sl.n = 1;
+    if (!L.aligned8) L = pitched_layout(L);
+    sl.h_desc[0] = sl.h_desc[1] = FrameDesc{L, sl.d_frames, 0};
     CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
     {
         const int row_bytes[3] = {width, fcw, fcw}, rows[3] = {height, fch, fch}, pitch[3] = {L.y_pitch, L.c_pitch, L.c_pitch};
@@ -1400,7 +1208,7 @@ int h2j_encode_frame(h2j_encoder *e, const uint8_t *const planes[3], const int s
         rc = upload_planes(e, sl, planes, strides, row_bytes, rows, off, pitch, sl.d_frames, sl.h_stage);
         if (rc) return rc;
     }
-    rc = launch_pipeline(e, sl, sl.d_frames, 1, TAIL_SINGLE);
+    rc = run_batch(e, sl, 1, 1, Input{}, TAIL_SINGLE);
     if (rc) return rc;
     return finish_single(e, sl, out, out_capacity, out_size);
 }
@@ -1435,16 +1243,16 @@ int h2j_encode_frame16(h2j_encoder *e, const uint8_t *const planes[3], const int
             return fail(e, H2J_ERR_NOMEM, "no room for the 16-bit staging of a %dx%d picture", e->s.max_width, e->s.max_height);
         }
     }
-    sl.n = 1;
+    // a batch of one frame: the planes as staged on the device, converted by the input stage
+    const h2j_frame_desc F{sl.d_frames16, width, height, yp, cp, (size_t)yp * height, (size_t)yp * height + (size_t)cp * fch};
+    int rc = describe_batch(e, sl, F, (size_t)yp * height + 2 * (size_t)cp * fch, false, 2);
+    if (rc) return rc;
     CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
-    const Src16 S{0, (long long)yp * height, (long long)yp * height + (long long)cp * fch, yp, cp};
     const int row_bytes[3] = {2 * width, 2 * fcw, 2 * fcw}, rows[3] = {height, fch, fch}, pitch[3] = {yp, cp, cp};
-    const size_t off[3] = {0, (size_t)S.u_off, (size_t)S.v_off};
-    int rc = upload_planes(e, sl, planes, strides, row_bytes, rows, off, pitch, sl.d_frames16, sl.h_stage16);
+    const size_t off[3] = {0, F.u_offset, F.v_offset};
+    rc = upload_planes(e, sl, planes, strides, row_bytes, rows, off, pitch, sl.d_frames16, sl.h_stage16);
     if (rc) return rc;
-    rc = convert_depth(e, sl, sl.d_frames16, S, false, bit_depth, 1, width, height);
-    if (rc) return rc;
-    rc = launch_pipeline(e, sl, sl.d_frames, 1, TAIL_SINGLE);
+    rc = run_batch(e, sl, 1, 1, Input{false, bit_depth}, TAIL_SINGLE);
     if (rc) return rc;
     return finish_single(e, sl, out, out_capacity, out_size);
 }
@@ -1472,7 +1280,7 @@ int h2j_convert_pad(h2j_encoder *e, const uint8_t *const planes[3], const int st
     }
     const size_t fb = tight_frame_bytes(width, height, e->s.chroma_format);
     FrameLayout L;
-    int rc = make_layout(e, sl.d_frames, align_up(fb, 256), width, height, &L);
+    int rc = make_layout(e, sl.d_frames, width, height, &L);
     if (rc) return rc;
     CU(e, cudaMemcpyAsync(sl.d_frames, sl.h_stage, fb, cudaMemcpyHostToDevice, sl.stream));
     const int pw = L.mcu_w * 16, ph = L.mcu_h * 16;
@@ -1505,7 +1313,7 @@ int h2j_debug_frame_info(h2j_encoder *e, int slot, int frame, h2j_frame_info *in
     memset(info, 0, sizeof *info);
     info->qscale = t.qscale;
     info->mb_var_sum = t.mb_var_sum;
-    const FrameLayout &L = frame_layout(sl, frame);
+    const FrameLayout &L = frame_desc(sl, frame).L;
     info->mcu_w = L.mcu_w;
     info->mcu_h = L.mcu_h;
     info->header_bytes = t.header_bytes;
@@ -1525,7 +1333,7 @@ int h2j_debug_coefficients(h2j_encoder *e, int slot, int frame, int16_t *out, si
     if (rc) return rc;
     Slot &sl = e->slots[slot];
     if (!out || frame < 0 || frame >= sl.n) return fail(e, H2J_ERR_INVALID_ARG, "bad frame index %d", frame);
-    const FrameLayout &L = frame_layout(sl, frame);
+    const FrameLayout &L = frame_desc(sl, frame).L;
     const size_t need = (size_t)L.n_blocks * 64;
     if (out_elems < need) return fail(e, H2J_ERR_OUTPUT_TOO_SMALL, "need %zu int16 elements", need);
     ON_DEVICE(e);

@@ -1,6 +1,9 @@
 // Device side of h2j_b200: the YUV -> JPEG stage of the reference (src/Encoder.cpp:104-308, i.e. libavcodec's
-// mjpeg encoder as the reference configures it) as sm_100a kernels.  One launch handles a batch of same-sized
-// frames; frames never interact, so the batch index is simply a grid dimension.
+// mjpeg encoder as the reference configures it) as sm_100a kernels.  One launch handles a batch of frames; frames never
+// interact, so the batch index is simply a grid dimension.  Every submit describes its batch by a per-frame table (FrameDesc);
+// an input stage copies the frames the pipeline cannot read where they are (repitch, semi-planar split, 16-bit conversion,
+// downscale: one launch), then the pipeline runs in its batch form (one layout by value, frames evenly spaced) or, for
+// frames of different layouts, its list form (each CTA reads its frame's table entry).
 //
 //   K1  mbvar_kernel         luma 16x16 variance sums -> rate-control input              (HBM bound, 1 B/px read)
 //   K2  fdct_quant_kernel    qscale + quantiser set-up, (range convert +) edge replicate + FDCT + quantise +
@@ -36,12 +39,13 @@ struct FrameLayout {
     int mb_w;          // 16x16 luma macroblocks per row (= mcu_w except at 4:4:4, whose MCUs are 8 wide): what K1 walks
 };
 
-// One frame of a list batch (h2j_submit_device_list / h2j_submit_host_list), where every frame has its own address and
-// size.  The *_list_kernel forms read their frame's entry of a per-slot table at blockIdx instead of taking one layout for
-// the whole batch by value; their grids are sized for the batch's largest frame, and CTAs past their own frame's extent
-// return before they touch any shared state.
+// One frame of a batch.  A slot's table holds m pairs of them for n frames: entry f is frame f as the pipeline reads it,
+// entry m + f the source a copy kernel makes it from (base nullptr: frame f is read in place).  m = n, or m = 1 for n frames of
+// one layout at one stride: that pair stands for every frame, frame f at base + f * L.frame_stride.  The copy kernels and
+// the LIST forms of K1-K4b (m = n only) read their frame's entry at blockIdx; their grids are sized for the batch's largest
+// frame, and CTAs past their own frame's extent return before they touch any shared state.
 struct FrameDesc {
-    FrameLayout L;         // frame_stride unused (0)
+    FrameLayout L;         // frame_stride: with m = 1, bytes between the frames' bases
     const uint8_t *base;   // the frame's first luma byte
     long long extent;      // copy sources (repitch / semi-planar split): bytes from base that may be read
 };

@@ -141,79 +141,95 @@ __global__ void __launch_bounds__(128) convert_pad_kernel(const uint8_t *__restr
 }
 
 // ------------------------------------------------------------------------------------------------
-// NV12 / NV16 / NV24 (what hardware decoders produce: a luma plane and ONE plane of interleaved Cb/Cr pairs, both with a
-// row pitch) -> the tight planar frames the pipeline reads (I420 / 4:2:2 / 4:4:4 by L.fmt: c_pitch pairs per row, ch rows
-// of them).  grid (x, rows, frames): rows 0..h-1 copy luma, rows h..h+ch-1 split a chroma row (kPlaneRowsPerCta rows per
-// CTA: one row per CTA made 400 k CTAs of 120 busy threads for 256 frames).
-// 16 bytes per thread where pitch, base and width allow, bytes otherwise.
+// The copy kernels of the input stage.  Each reads the slot's FrameDesc table of m entry pairs (h2j_common.cuh): frame f as
+// the pipeline reads it (planar, at the 16-byte row pitch of pitched_layout()) and the source it is made from (base nullptr:
+// frame f is read in place, no copy).  grid (x, rows / kPlaneRowsPerCta, frames), sized for the largest frame that is
+// copied: rows of a frame are its luma rows, then its chroma rows (kPlaneRowsPerCta rows per CTA: one row per CTA made 400 k
+// CTAs of 120 busy threads for 256 frames); CTAs past their frame's extent do nothing.  A thread writes 16 bytes of a row.
 // ------------------------------------------------------------------------------------------------
-// `pairs`: Cb/Cr pairs per chroma row (L.c_pitch of a tight copy; a list batch writes a 16-byte row pitch, wider than that)
 constexpr int kPlaneRowsPerCta = 16;
-__device__ __forceinline__ void nv12_to_i420_body(const uint8_t *__restrict__ src, long long src_stride, int pitch, int uv_pitch, long long uv_off,
-                                                  uint8_t *__restrict__ dst, const FrameLayout &L, int src_aligned16, int pairs)
+
+// What a copy kernel reads: the slot's uploaded table of m pairs, or with m = 1 the one pair itself, by value (a batch of
+// one layout at one stride costs no upload)
+struct CopyTable {
+    const FrameDesc *descs;
+    int m;
+    FrameDesc d, s;  // m = 1
+};
+
+// frame f's pair: its own entries, or the one pair of a uniform batch with both bases moved on f frame strides
+__device__ __forceinline__ void frame_pair(const CopyTable &t, int f, FrameDesc &d, FrameDesc &s)
 {
-    const int f = blockIdx.z;
-    const uint8_t *S = src + (long long)f * src_stride;
-    uint8_t *D = dst + (long long)f * L.frame_stride;
+    if (t.m > 1) {
+        d = t.descs[f];
+        s = t.descs[t.m + f];
+        return;
+    }
+    d = t.d;
+    s = t.s;
+    d.base += (long long)f * d.L.frame_stride;
+    if (s.base) s.base += (long long)f * s.L.frame_stride;
+}
+
+// NV12 / NV16 / NV24 (what hardware decoders produce: a luma plane and ONE plane of interleaved Cb/Cr pairs, both with a row
+// pitch; the source's L.y_pitch / L.c_pitch, the pair plane at L.u_off) -> planar frames (I420 / 4:2:2 / 4:4:4 by L.fmt).
+// Rows h .. h + ch - 1 split a row of pairs.  128-bit loads where the source row segment is 16-byte aligned, bytes otherwise.
+__global__ void __launch_bounds__(128) nv12_to_i420_kernel(const __grid_constant__ CopyTable t)
+{
+    FrameDesc d, s;
+    frame_pair(t, blockIdx.z, d, s);
+    const FrameLayout &L = d.L;
+    uint8_t *D = const_cast<uint8_t *>(d.base);
+    const int pairs = (L.w + (1 << fmt_hshift(L.fmt)) - 1) >> fmt_hshift(L.fmt);  // per chroma row
     const int fch = (L.h + fmt_vshift(L.fmt)) >> fmt_vshift(L.fmt);
     const int x0 = (blockIdx.x * blockDim.x + threadIdx.x) * 16;
     for (int row = blockIdx.y * kPlaneRowsPerCta; row < min((int)(blockIdx.y + 1) * kPlaneRowsPerCta, L.h + fch); row++)
     if (row < L.h) {
         if (x0 >= L.w) continue;
-        const uint8_t *s = S + (long long)row * pitch + x0;
-        uint8_t *d = D + (long long)row * L.y_pitch + x0;
-        if (src_aligned16 && L.aligned16 && x0 + 16 <= L.w) *reinterpret_cast<uint4 *>(d) = ldg128(s);
+        const uint8_t *src = s.base + (long long)row * s.L.y_pitch + x0;
+        uint8_t *dst = D + (long long)row * L.y_pitch + x0;
+        if (x0 + 16 <= L.w && ((uintptr_t)src & 15u) == 0) *reinterpret_cast<uint4 *>(dst) = ldg128(src);
         else
-            for (int i = 0; i < 16 && x0 + i < L.w; i++) d[i] = s[i];
-    } else if (row < L.h + fch) {
+            for (int i = 0; i < 16 && x0 + i < L.w; i++) dst[i] = src[i];
+    } else {
         const int r = row - L.h;
         if (x0 >= 2 * pairs) continue;
-        const uint8_t *s = S + uv_off + (long long)r * uv_pitch + x0;
+        const uint8_t *src = s.base + s.L.u_off + (long long)r * s.L.c_pitch + x0;
         uint8_t *du = D + L.u_off + (long long)r * L.c_pitch + (x0 >> 1), *dv = D + L.v_off + (long long)r * L.c_pitch + (x0 >> 1);
-        if (src_aligned16 && (uv_off & 15) == 0 && L.aligned8 && x0 + 16 <= 2 * pairs) {
-            const uint4 v = ldg128(s);
+        if (x0 + 16 <= 2 * pairs && ((uintptr_t)src & 15u) == 0) {
+            const uint4 v = ldg128(src);
             const unsigned u0 = __byte_perm(v.x, v.y, 0x6420), u1 = __byte_perm(v.z, v.w, 0x6420);
             const unsigned w0 = __byte_perm(v.x, v.y, 0x7531), w1 = __byte_perm(v.z, v.w, 0x7531);
             *reinterpret_cast<uint2 *>(du) = make_uint2(u0, u1);
             *reinterpret_cast<uint2 *>(dv) = make_uint2(w0, w1);
         } else {
             for (int i = 0; i < 8 && (x0 >> 1) + i < pairs; i++) {
-                du[i] = s[2 * i];
-                dv[i] = s[2 * i + 1];
+                du[i] = src[2 * i];
+                dv[i] = src[2 * i + 1];
             }
         }
     }
 }
-__global__ void __launch_bounds__(128) nv12_to_i420_kernel(const uint8_t *__restrict__ src, long long src_stride, int pitch, long long uv_off,
-                                                           uint8_t *__restrict__ dst, FrameLayout L, int src_aligned16)
-{
-    nv12_to_i420_body(src, src_stride, pitch, pitch, uv_off, dst, L, src_aligned16, L.c_pitch);
-}
-// a list batch: descs[f] is where the pipeline reads frame f (planar, pitched_layout), descs[n + f] the semi-planar source
-// (L.y_pitch / L.c_pitch: its pitches, L.u_off: its pair plane, L.aligned16: base and pitches are 16-byte aligned); grid
-// sized for the largest frame
-__global__ void __launch_bounds__(128) nv12_to_i420_list_kernel(const FrameDesc *__restrict__ descs, int n)
-{
-    const FrameDesc &d = descs[blockIdx.z], &s = descs[n + blockIdx.z];
-    const int fcw = (d.L.w + (1 << fmt_hshift(d.L.fmt)) - 1) >> fmt_hshift(d.L.fmt);
-    nv12_to_i420_body(s.base, 0, s.L.y_pitch, s.L.c_pitch, s.L.u_off, const_cast<uint8_t *>(d.base), d.L, s.L.aligned16, fcw);
-}
 
-// ------------------------------------------------------------------------------------------------
 // Planar frames whose rows do not start on 8-byte boundaries (odd widths such as 1918, an unaligned base, a caller's
 // pitches or plane offsets) -> the same planes at a 16-byte row pitch, so that K1 and K2 take their vector-load paths
-// (every block but the ones cut by the right edge) instead of 64 byte loads per block.  grid (x, h + 2 * ch, frames); a
-// thread produces 16 output bytes from five aligned source words and four funnel shifts.  A row copies the plane's
-// width, ceil-divided by the subsampling (not the source pitch); the padding bytes of a row are never read by the pipeline
-// (edges are replicated from the last real sample).
-// ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void repitch_body(const uint8_t *__restrict__ src, const FrameLayout &T,  // the source frames, their layout
-                                             int fch,                                               // rows of a chroma plane
-                                             uint8_t *__restrict__ dst, const FrameLayout &P,       // the copies, their pitched layout
-                                             const uint8_t *src_begin, const uint8_t *src_end)      // what may be read
+// (every block but the ones cut by the right edge) instead of 64 byte loads per block.  Rows h .. h + 2 ch - 1 are Cb, then
+// Cr.  A thread produces 16 output bytes from five aligned source words and four funnel shifts; it reads nothing outside
+// the source's extent.  A row copies the plane's width, ceil-divided by the subsampling (not the source pitch); the padding
+// bytes of a row are never read by the pipeline (edges are replicated from the last real sample).
+__global__ void __launch_bounds__(128) repitch_kernel(const __grid_constant__ CopyTable t)
 {
-    const int f = blockIdx.z;
-    const int fcw = (T.w + (1 << fmt_hshift(T.fmt)) - 1) >> fmt_hshift(T.fmt);  // (T.c_pitch of a tight source)
+    FrameDesc d, s;
+    frame_pair(t, blockIdx.z, d, s);
+    if (!s.base) return;
+    const FrameLayout &T = s.L, &P = d.L;  // the source's layout, the copy's
+    const uint8_t *sbase = s.base;
+    uint8_t *dbase = const_cast<uint8_t *>(d.base);
+    const int fcw = (T.w + (1 << fmt_hshift(T.fmt)) - 1) >> fmt_hshift(T.fmt), fch = (T.h + fmt_vshift(T.fmt)) >> fmt_vshift(T.fmt);
+    // what may be read: the frame, or for a batch of one layout at one stride (m = 1) every frame of the caller's buffer, so
+    // that only the batch's last frame ends in the bytewise path
+    const uint8_t *src_begin = t.m > 1 ? sbase : t.s.base;
+    const uint8_t *src_end = t.m > 1 ? sbase + s.extent : t.s.base + (long long)(gridDim.z - 1) * T.frame_stride + s.extent;
     for (int row = blockIdx.y * kPlaneRowsPerCta; row < min((int)(blockIdx.y + 1) * kPlaneRowsPerCta, T.h + 2 * fch); row++) {
     int pw, r;
     long long so, dof;
@@ -223,61 +239,40 @@ __device__ __forceinline__ void repitch_body(const uint8_t *__restrict__ src, co
     else { pw = fcw; r = row - T.h - fch; so = T.v_off; dof = P.v_off; spitch = T.c_pitch; dpitch = P.c_pitch; }
     const int x0 = (blockIdx.x * blockDim.x + threadIdx.x) * 16;
     if (x0 >= pw) continue;
-    const uint8_t *s = src + (long long)f * T.frame_stride + so + (long long)r * spitch + x0;
-    uint8_t *d = dst + (long long)f * P.frame_stride + dof + (long long)r * dpitch + x0;  // 16-byte aligned, x0 + 16 <= dpitch
-    const unsigned a = (unsigned)((uintptr_t)s & 3u);
-    const uint8_t *s4 = s - a;
+    const uint8_t *sp = sbase + so + (long long)r * spitch + x0;
+    uint8_t *dp = dbase + dof + (long long)r * dpitch + x0;  // 16-byte aligned, x0 + 16 <= dpitch
+    const unsigned a = (unsigned)((uintptr_t)sp & 3u);
+    const uint8_t *s4 = sp - a;
     if (s4 >= src_begin && s4 + 20 <= src_end) {
         const uint32_t *q = reinterpret_cast<const uint32_t *>(s4);
         const unsigned w0 = __ldg(q), w1 = __ldg(q + 1), w2 = __ldg(q + 2), w3 = __ldg(q + 3), w4 = a ? __ldg(q + 4) : 0u;
         const unsigned sh = a * 8;
-        *reinterpret_cast<uint4 *>(d) = make_uint4(__funnelshift_r(w0, w1, sh), __funnelshift_r(w1, w2, sh), __funnelshift_r(w2, w3, sh),
-                                                   __funnelshift_r(w3, w4, sh));
+        *reinterpret_cast<uint4 *>(dp) = make_uint4(__funnelshift_r(w0, w1, sh), __funnelshift_r(w1, w2, sh), __funnelshift_r(w2, w3, sh),
+                                                    __funnelshift_r(w3, w4, sh));
     } else {
-        for (int i = 0; i < 16 && x0 + i < pw; i++) d[i] = s[i];
+        for (int i = 0; i < 16 && x0 + i < pw; i++) dp[i] = sp[i];
     }
     }
 }
-__global__ void __launch_bounds__(128) repitch_kernel(const uint8_t *__restrict__ src, FrameLayout T, int fch, uint8_t *__restrict__ dst,
-                                                      FrameLayout P, const uint8_t *src_begin, const uint8_t *src_end)
-{
-    repitch_body(src, T, fch, dst, P, src_begin, src_end);
-}
-// a list batch: descs[f] is the copy the pipeline reads, descs[n + f] the source; frames read in place have no source
-// (base == nullptr) and return at once.  Grid sized for the largest frame that is copied.
-__global__ void __launch_bounds__(128) repitch_list_kernel(const FrameDesc *__restrict__ descs, int n)
-{
-    const FrameDesc &d = descs[blockIdx.z], &s = descs[n + blockIdx.z];
-    if (!s.base) return;
-    const int fch = (s.L.h + fmt_vshift(s.L.fmt)) >> fmt_vshift(s.L.fmt);
-    repitch_body(s.base, s.L, fch, const_cast<uint8_t *>(d.base), d.L, s.base, s.base + s.extent);
-}
 
-// ------------------------------------------------------------------------------------------------
-// High-bit-depth frames (P010 / P016, P210 / P216, a decoder's 16-bit 4:4:4 surface, yuv420p10le ...) -> 8-bit planar frames
-// at the 16-byte row pitch of pitched_layout(), which the pipeline then reads with its vector loads.  Every sample is a
-// little-endian 16-bit word whose low `bit_depth` bits hold the value; the 8-bit sample is bits [bit_depth - 8, bit_depth)
-// of the word (truncation: no rounding, no dither; bits above bit_depth never reach the picture).  All offsets and pitches
-// of Src16 are in bytes.
-// SP: a luma plane and one plane of interleaved Cb/Cr word pairs (rows h .. h + ch - 1 of the grid split one row of pairs),
-// otherwise three planes (rows h .. h + 2 ch - 1: Cb, then Cr).  grid (x, rows / kPlaneRowsPerCta, frames) as
-// nv12_to_i420_kernel; a thread converts 16 words of a source row: two 128-bit loads where that row is 16-byte aligned and
-// holds all 16 words, 16-bit loads otherwise.  No word past a row's last sample is read.
-// ------------------------------------------------------------------------------------------------
-struct Src16 {
-    long long frame_stride, u_off, v_off;  // SP: u_off = v_off = the pair plane
-    int y_pitch, c_pitch;
-};
-
+// High-bit-depth frames (P010 / P016, P210 / P216, a decoder's 16-bit 4:4:4 surface, yuv420p10le ...) -> 8-bit planar frames.
+// Every sample is a little-endian 16-bit word whose low `bit_depth` bits hold the value; the 8-bit sample is bits
+// [bit_depth - 8, bit_depth) of the word (truncation: no rounding, no dither; bits above bit_depth never reach the picture).
+// The source's L.w / L.h count samples, its pitches and offsets are in bytes.
+// SP: a luma plane and one plane of interleaved Cb/Cr word pairs at L.u_off (rows h .. h + ch - 1 of the grid split one row
+// of pairs), otherwise three planes (rows h .. h + 2 ch - 1: Cb, then Cr).  A thread converts 16 words of a source row: two
+// 128-bit loads where that row is 16-byte aligned and holds all 16 words, 16-bit loads otherwise.  No word past a row's last
+// sample is read.
 template <bool SP>
-__global__ void __launch_bounds__(128) depth_to_8_kernel(const uint8_t *__restrict__ src, Src16 S, uint8_t *__restrict__ dst, FrameLayout P,
-                                                         int shift)  // bit_depth - 8
+__global__ void __launch_bounds__(128) depth_to_8_kernel(const __grid_constant__ CopyTable t, int shift)  // shift: bit_depth - 8
 {
-    const int f = blockIdx.z;
+    FrameDesc d, s;
+    frame_pair(t, blockIdx.z, d, s);
+    const FrameLayout &S = s.L, &P = d.L;
     const int fcw = (P.w + (1 << fmt_hshift(P.fmt)) - 1) >> fmt_hshift(P.fmt), fch = (P.h + fmt_vshift(P.fmt)) >> fmt_vshift(P.fmt);
     const int x0 = (blockIdx.x * blockDim.x + threadIdx.x) * 16;  // first word of the row this thread converts
-    const uint8_t *F = src + (long long)f * S.frame_stride;
-    uint8_t *D = dst + (long long)f * P.frame_stride;
+    const uint8_t *F = s.base;
+    uint8_t *D = const_cast<uint8_t *>(d.base);
     for (int row = blockIdx.y * kPlaneRowsPerCta; row < min((int)(blockIdx.y + 1) * kPlaneRowsPerCta, P.h + (SP ? 1 : 2) * fch); row++) {
         int n;  // words in the row
         const uint8_t *s;
@@ -386,12 +381,13 @@ __device__ __forceinline__ unsigned down_avg(unsigned s, int x, int pw, int rh, 
 }
 
 template <int K, bool SP>
-__global__ void __launch_bounds__(32 * kDownWarps, K == 2 ? 6 : 4) downscale_list_kernel(const FrameDesc *__restrict__ descs, int n)
+__global__ void __launch_bounds__(32 * kDownWarps, K == 2 ? 6 : 4) downscale_list_kernel(const __grid_constant__ CopyTable t)
 {
     static_assert(K == 2 || K == 4 || K == 8, "box factors 2, 4, 8");
     constexpr int kWords = 4 * K;
     const int f = blockIdx.z;
-    const FrameDesc &d = descs[f], &s = descs[n + f];
+    // a list (m = n): a table of one pair is frame 0's
+    const FrameDesc &d = t.m > 1 ? t.descs[f] : t.d, &s = t.m > 1 ? t.descs[t.m + f] : t.s;
     const FrameLayout &D = d.L, &S = s.L;
     const int hs = fmt_hshift(S.fmt), vs = fmt_vshift(S.fmt);
     const int scw = (S.w + (1 << hs) - 1) >> hs, sch = (S.h + (1 << vs) - 1) >> vs;  // source chroma plane

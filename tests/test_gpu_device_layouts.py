@@ -58,12 +58,6 @@ def upload(frames, stride, shift=0):
     return d, d.data_ptr() + shift
 
 
-def tight_aligned8(w, h, fmt):
-    """what the pipeline needs to read the slot's tight planar copy with vector loads (else: one repitch pass)"""
-    ch, cw = chroma_dims(w, h, fmt)
-    return w % 8 == 0 and cw % 8 == 0 and (w * h) % 8 == 0 and (w * h + cw * ch) % 8 == 0
-
-
 def pipeline_launches(e):
     """launches of a planar submit that needs no copy: the pipeline plus the pack at collect"""
     import torch
@@ -91,7 +85,7 @@ def run(e, submit, n):
 
 @pytest.mark.parametrize("layout", ["decoder", "tight", "unaligned"])
 @pytest.mark.parametrize("fmt", [1, 2])
-def test_semiplanar_matches_planar(orc, fmt, layout):
+def test_semiplanar_matches_planar_split_in_one_launch(orc, fmt, layout):
     import h2j_b200
 
     with h2j_b200.Encoder(max_width=1920, max_height=1088, max_batch=2, n_slots=1, chroma_format=fmt, max_jpeg_bytes=BIG_JPEG) as e:
@@ -112,13 +106,13 @@ def test_semiplanar_matches_planar(orc, fmt, layout):
             for k in range(2):
                 assert got[k] == want[k], f"fmt {fmt} {layout} {w}x{h} frame {k}: JPEG differs from the oracle's planar JPEG"
             in_place = layout != "unaligned" and pitch % 8 == 0 and uv_off % 8 == 0
-            expect = P if in_place else P + 1 + (0 if tight_aligned8(w, h, fmt) else 1)
+            expect = P if in_place else P + 1
             assert launches == expect, f"fmt {fmt} {layout} {w}x{h}: {launches} launches, expected {expect} (in place: {in_place})"
 
 
 @pytest.mark.parametrize("fmt,w,h", [(1, 641, 479), (2, 641, 479), (1, 330, 225), (2, 330, 225), (1, 330, 241), (2, 330, 241),
                                      (1, 2562, 1442), (2, 2562, 1442)])
-def test_semiplanar_batches_across_tiles(orc, fmt, w, h):
+def test_semiplanar_batches_across_tiles_split_in_one_launch(orc, fmt, w, h):
     """partial tiles, partial units and the predecessor DC across tiles: several tiles per CTA, both paths"""
     import h2j_b200
 
@@ -137,7 +131,7 @@ def test_semiplanar_batches_across_tiles(orc, fmt, w, h):
             for tpc in (0, 2, 5, 16):
                 e.set_knob("fdct_tiles_per_cta", tpc)
                 got, launches = run(e, lambda: e.submit_device_semiplanar(0, ptr, size, pitch, uv_off, n, w, h), n)
-                assert launches == (P + 1 + (0 if tight_aligned8(w, h, fmt) else 1) if prepass else P)
+                assert launches == (P + 1 if prepass else P)
                 for i in range(n):
                     assert got[i] == want[i], f"fmt {fmt} {w}x{h}, prepass {prepass}, {tpc} tiles per CTA, frame {i}"
 
