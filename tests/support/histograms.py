@@ -6,6 +6,8 @@ exact ties between a symbol and a package sum), Zipf-like AC tables, all 256 byt
 TEST INFRASTRUCTURE ONLY."""
 from __future__ import annotations
 
+import ctypes as C
+
 import numpy as np
 
 MAX_LEN = 16
@@ -213,3 +215,13 @@ def check_table(hist, bits, vals, nvals):
     if cost != opt:
         bad.append(f"sum count*length {cost} != optimum {opt}")
     return bad
+
+
+def oracle_table(orc, hist):
+    """(BITS, HUFFVAL, number of values) of the oracle's table builder (orc_huffman_table) on `hist`"""
+    bits = np.zeros(17, np.uint8)
+    vals = np.zeros(256, np.uint8)
+    nv = C.c_int(0)
+    h = np.ascontiguousarray(hist, np.uint32)
+    orc.oracle().orc_huffman_table(h.ctypes.data, bits.ctypes.data, vals.ctypes.data, C.byref(nv))
+    return bits, vals, nv.value

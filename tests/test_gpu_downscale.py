@@ -4,12 +4,10 @@ allocations surrounded by 0xA5 padding, and pitch and surface gaps are 0xA5 too:
 would change the JPEG."""
 import random
 
-import numpy as np
 import pytest
 
 from tests.support.downscale import FACTORS, downscale_planar
-from tests.test_gpu_formats import CASES
-from tests.test_gpu_mixed_batch import PAD, Frames, align, encoder, planes
+from tests.support.layouts import CASES, Frames, align, desc, encoder, place, planar, semiplanar, upload
 
 pytestmark = pytest.mark.gpu
 
@@ -22,7 +20,7 @@ _planes = {}
 def source(orc, w, h, fmt, kind="textured", amp=40, seed=0):
     key = (w, h, fmt, kind, amp, seed)
     if key not in _planes:
-        _planes[key] = planes(orc, w, h, fmt, kind, seed=seed, amp=amp)
+        _planes[key] = orc.synth_planes_fmt(w, h, fmt, kind, seed=seed, amp=amp)
     return _planes[key]
 
 
@@ -32,34 +30,6 @@ def want_jpeg(orc, y, u, v, k, fmt, **kw):
 
 def fits(w, h, k):
     return -(-w // k) >= 2 and -(-h // k) >= 2
-
-
-def planar_at(h2j, fr, y, u, v, y_pitch=None, c_pitch=None, surf_rows=0, shift=0):
-    """planar frame, luma rows y_pitch apart, Cb and Cr planes behind `surf_rows` extra rows of each plane"""
-    h, w = y.shape
-    ch, cw = u.shape
-    y_pitch = y_pitch or w
-    c_pitch = c_pitch or cw
-    u_off = y_pitch * (h + surf_rows)
-    v_off = u_off + c_pitch * (ch + surf_rows)
-    buf = np.full(v_off + c_pitch * (ch - 1) + cw, PAD, np.uint8)
-    buf[: y_pitch * (h - 1) + w] = np.pad(y, ((0, 0), (0, y_pitch - w)), constant_values=PAD).ravel()[: y_pitch * (h - 1) + w]
-    for off, p in ((u_off, u), (v_off, v)):
-        buf[off: off + c_pitch * (ch - 1) + cw] = np.pad(p, ((0, 0), (0, c_pitch - cw)), constant_values=PAD).ravel()[: c_pitch * (ch - 1) + cw]
-    return h2j.FrameDesc(fr.put(buf, shift), w, h, y_pitch, c_pitch, u_off, v_off)
-
-
-def semiplanar_at(h2j, fr, y, u, v, pitch, surf_rows=0, shift=0):
-    h, w = y.shape
-    ch, cw = u.shape
-    uv_off = pitch * (h + surf_rows)
-    buf = np.full(uv_off + pitch * (ch - 1) + 2 * cw, PAD, np.uint8)
-    buf[: pitch * (h - 1) + w] = np.pad(y, ((0, 0), (0, pitch - w)), constant_values=PAD).ravel()[: pitch * (h - 1) + w]
-    uv = np.full((ch, pitch), PAD, np.uint8)
-    uv[:, 0: 2 * cw: 2] = u
-    uv[:, 1: 2 * cw: 2] = v
-    buf[uv_off:] = uv.ravel()[: pitch * (ch - 1) + 2 * cw]
-    return h2j.FrameDesc(fr.put(buf, shift), w, h, pitch, pitch, uv_off, 0)
 
 
 def odd_pitch(n, j):
@@ -72,11 +42,11 @@ def layouts(h2j, fr, y, u, v, i):
     ch, cw = u.shape
     sp_row = max(w, 2 * cw)
     return [
-        ("planar tight", h2j.LAYOUT_PLANAR, planar_at(h2j, fr, y, u, v)),
-        ("planar decoder", h2j.LAYOUT_PLANAR, planar_at(h2j, fr, y, u, v, align(w, 256), align(cw, 256), align(h, 16) - h + 16)),
-        ("planar shifted", h2j.LAYOUT_PLANAR, planar_at(h2j, fr, y, u, v, odd_pitch(w, i % 3), odd_pitch(cw, i % 2), i % 3, 1 + i % 15)),
-        ("semi-planar aligned", h2j.LAYOUT_SEMIPLANAR, semiplanar_at(h2j, fr, y, u, v, align(sp_row, 64), align(h, 16) - h)),
-        ("semi-planar unaligned", h2j.LAYOUT_SEMIPLANAR, semiplanar_at(h2j, fr, y, u, v, odd_pitch(sp_row, i % 2), 1, 1 + (i + 4) % 15)),
+        ("planar tight", h2j.LAYOUT_PLANAR, desc(fr, y, u, v, *planar(y, u))),
+        ("planar decoder", h2j.LAYOUT_PLANAR, desc(fr, y, u, v, *planar(y, u, align(w, 256), align(cw, 256), align(h, 16) - h + 16))),
+        ("planar shifted", h2j.LAYOUT_PLANAR, desc(fr, y, u, v, *planar(y, u, odd_pitch(w, i % 3), odd_pitch(cw, i % 2), i % 3), shift=1 + i % 15)),
+        ("semi-planar aligned", h2j.LAYOUT_SEMIPLANAR, desc(fr, y, u, v, *semiplanar(y, align(sp_row, 64), align(h, 16) - h))),
+        ("semi-planar unaligned", h2j.LAYOUT_SEMIPLANAR, desc(fr, y, u, v, *semiplanar(y, odd_pitch(sp_row, i % 2), 1), shift=1 + (i + 4) % 15)),
     ]
 
 
@@ -117,11 +87,11 @@ def test_uniform_list_runs_the_batch_form(orc, fmt, k):
     fr = Frames()
     srcs = [source(orc, w, h, fmt, "noise" if i % 2 else "textured", 30, seed=300 + i) for i in range(n)]
     outs = [orc.oracle_encode(*downscale_planar(*p, k), chroma_format=fmt, want_coefs=True) for p in srcs]
-    planar = [planar_at(h2j, fr, *p, y_pitch=odd_pitch(w, i), shift=i) for i, p in enumerate(srcs)]
-    semi = [semiplanar_at(h2j, fr, *p, pitch=align(max(w, 2 * p[1].shape[1]), 256), surf_rows=13) for p in srcs]
+    flat = [desc(fr, y, u, v, *planar(y, u, odd_pitch(w, i)), shift=i) for i, (y, u, v) in enumerate(srcs)]
+    semi = [desc(fr, y, u, v, *semiplanar(y, align(max(w, 2 * u.shape[1]), 256), 13)) for y, u, v in srcs]
     torch.cuda.synchronize()
     with encoder(fmt, n, max_width=MAX_W, max_height=MAX_H) as e:
-        for layout, descs in ((h2j.LAYOUT_PLANAR, planar), (h2j.LAYOUT_SEMIPLANAR, semi)):
+        for layout, descs in ((h2j.LAYOUT_PLANAR, flat), (h2j.LAYOUT_SEMIPLANAR, semi)):
             e.submit_device_downscaled(0, layout, descs, k)
             for i, (_, dbg, coefs) in enumerate(outs):
                 info = e.frame_info(0, i)
@@ -142,7 +112,7 @@ def test_debug_hooks_answer_for_the_downscaled_frame_of_a_mixed_list(orc):
     for i, (w, h) in enumerate(sizes):
         y, u, v = source(orc, w, h, 0, seed=400 + i)
         outs.append(orc.oracle_encode(*downscale_planar(y, u, v, 2), want_coefs=True))
-        descs.append(planar_at(h2j, fr, y, u, v, shift=i))
+        descs.append(desc(fr, y, u, v, *planar(y, u), shift=i))
     torch.cuda.synchronize()
     with encoder(0, len(sizes)) as e:
         e.submit_device_downscaled(0, h2j.LAYOUT_PLANAR, descs, 2)
@@ -165,7 +135,7 @@ def test_range_conversion_and_fixed_qscale(orc, fmt, kw):
     fr = Frames()
     geoms = [(322, 242), (1918, 1078), (131, 77)]
     srcs = [source(orc, w, h, fmt, "textured", 70, seed=500 + i) for i, (w, h) in enumerate(geoms)]
-    descs = [semiplanar_at(h2j, fr, *p, pitch=odd_pitch(max(p[0].shape[1], 2 * p[1].shape[1]), i), shift=i) for i, p in enumerate(srcs)]
+    descs = [desc(fr, y, u, v, *semiplanar(y, odd_pitch(max(y.shape[1], 2 * u.shape[1]), i)), shift=i) for i, (y, u, v) in enumerate(srcs)]
     torch.cuda.synchronize()
     with encoder(fmt, len(geoms), **kw) as e:
         for k in (2, 4):
@@ -184,11 +154,12 @@ def test_one_launch_more_than_the_pipeline(orc, layout):
     fr = Frames()
     sizes = [(1280, 720), (1279, 719), (640, 360)]
     srcs = [source(orc, w, h, 0, seed=600 + i) for i, (w, h) in enumerate(sizes)]
-    small = [planar_at(h2j, fr, *downscale_planar(*srcs[0], 2))] * 3
+    y, u, v = downscale_planar(*srcs[0], 2)
+    small = [desc(fr, y, u, v, *planar(y, u))] * 3
     if layout == h2j.LAYOUT_PLANAR:
-        descs = [planar_at(h2j, fr, *p, shift=3) for p in srcs]
+        descs = [desc(fr, y, u, v, *planar(y, u), shift=3) for y, u, v in srcs]
     else:
-        descs = [semiplanar_at(h2j, fr, *p, pitch=1283, shift=5) for p in srcs]
+        descs = [desc(fr, y, u, v, *semiplanar(y, 1283), shift=5) for y, u, v in srcs]
     torch.cuda.synchronize()
     with encoder(0, 3) as e:
         l0 = e.kernel_launches
@@ -212,8 +183,9 @@ def test_thumbnail_encoder_and_refusals(orc):
 
     fr = Frames()
     y, u, v = source(orc, 1920, 1080, 0, seed=700)
-    src = semiplanar_at(h2j, fr, y, u, v, pitch=2048, surf_rows=8)
-    tiny = planar_at(h2j, fr, *source(orc, 4, 4, 0, seed=701))
+    src = desc(fr, y, u, v, *semiplanar(y, 2048, 8))
+    ty, tu, tv = source(orc, 4, 4, 0, seed=701)
+    tiny = desc(fr, ty, tu, tv, *planar(ty, tu))
     torch.cuda.synchronize()
     with encoder(0, 2, max_width=480, max_height=272) as e:
         for k in (4, 8):
@@ -259,7 +231,7 @@ def test_full_size_and_thumbnail_from_the_same_surfaces_on_two_slots(orc):
     fr = Frames()
     n = 4
     srcs = [source(orc, 1920, 1080, 0, "textured" if i % 2 else "noise", 30, seed=800 + i) for i in range(n)]
-    descs = [semiplanar_at(h2j, fr, *p, pitch=2048, surf_rows=8) for p in srcs]
+    descs = [desc(fr, y, u, v, *semiplanar(y, 2048, 8)) for y, u, v in srcs]
     torch.cuda.synchronize()
     with h2j.Encoder(max_width=1920, max_height=1088, max_batch=n, n_slots=2, max_jpeg_bytes=8 * 1024 * 1024) as e:
         e.submit_device_list(0, h2j.LAYOUT_SEMIPLANAR, descs)
@@ -273,8 +245,6 @@ def test_full_size_and_thumbnail_from_the_same_surfaces_on_two_slots(orc):
 @pytest.mark.parametrize("k", FACTORS)
 def test_64_decoder_layout_nv12_frames(orc, k):
     """64 x 1080p NV12 at a hardware decoder's layout (pitch 2048, pair plane behind 1088 rows) in one allocation"""
-    import torch
-
     import h2j_b200 as h2j
 
     n, pitch, surf = 64, 2048, 1088
@@ -282,17 +252,9 @@ def test_64_decoder_layout_nv12_frames(orc, k):
     bases = [source(orc, 1920, 1080, 0, "textured" if i % 2 else "noise", 20 + 5 * i, seed=900 + i) for i in range(8)]
     rng = random.Random(k)
     pick = [rng.randrange(8) for _ in range(n)]
-    host = np.full(n * frame_bytes, PAD, np.uint8)
-    for i in range(n):
-        y, u, v = bases[pick[i]]
-        f = host[i * frame_bytes: (i + 1) * frame_bytes]
-        f[: pitch * surf].reshape(surf, pitch)[:1080, :1920] = y
-        uv = f[pitch * surf:].reshape(surf // 2, pitch)
-        uv[:540, 0:1920:2] = u
-        uv[:540, 1:1920:2] = v
-    d = torch.from_numpy(host).cuda()
-    torch.cuda.synchronize()
-    descs = [h2j.FrameDesc(d.data_ptr() + i * frame_bytes, 1920, 1080, pitch, pitch, pitch * surf, 0) for i in range(n)]
+    placed = [place(y, u, v, *semiplanar(y, pitch, surf - 1080), size=frame_bytes) for y, u, v in bases]
+    d, ptr = upload([placed[i] for i in pick], frame_bytes)
+    descs = [h2j.FrameDesc(ptr + i * frame_bytes, 1920, 1080, pitch, pitch, pitch * surf, 0) for i in range(n)]
     check = sorted({0, n - 1} | set(rng.sample(range(1, n - 1), 6)))
     w, h = h2j.downscaled_size(1920, 1080, k)
     with h2j.Encoder(max_width=w, max_height=h, max_batch=n, n_slots=1) as e:

@@ -9,13 +9,11 @@ import os
 import numpy as np
 import pytest
 
+from tests.support.layouts import CASES, upload
+
 pytestmark = pytest.mark.gpu
 
 G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-
-CASES = [(16, 16, "textured", 40), (2, 2, "noise", 100), (17, 17, "noise", 60), (33, 47, "blocks", 30), (64, 64, "binary", 0), (131, 77, "textured", 80),
-         (322, 242, "textured", 40), (641, 479, "noise", 20), (8, 16, "noise", 50), (9, 31, "noise", 50), (1280, 720, "textured", 30),
-         (1918, 1078, "textured", 40), (1920, 1080, "ff", 0)]
 
 
 @pytest.mark.parametrize("fmt", [1, 2])
@@ -62,8 +60,6 @@ def test_golden_digests_of_libavcodec_at_422_and_444(orc):
 
 @pytest.mark.parametrize("fmt,w,h", [(1, 641, 479), (2, 641, 479), (1, 330, 225), (2, 330, 225), (2, 1918, 1078), (1, 2562, 1442)])
 def test_batches_with_several_tiles_per_cta_and_partial_tiles(orc, fmt, w, h):
-    import torch
-
     import h2j_b200
 
     n = 6
@@ -72,14 +68,11 @@ def test_batches_with_several_tiles_per_cta_and_partial_tiles(orc, fmt, w, h):
     frames = np.stack([orc.pack_i420(*p) for p in planes])
     assert frames.shape[1] == h2j_b200.frame_bytes(w, h, fmt)
     stride = (frames.shape[1] + 255) // 256 * 256
-    host = np.zeros((n, stride), np.uint8)
-    host[:, : frames.shape[1]] = frames
-    d = torch.from_numpy(host).cuda()
-    torch.cuda.synchronize()
+    d, ptr = upload(frames, stride)
     with h2j_b200.Encoder(max_width=w, max_height=h, max_batch=n, n_slots=1, chroma_format=fmt, max_jpeg_bytes=8 * 1024 * 1024) as e:
         for tpc in (0, 2, 5, 16):
             e.set_knob("fdct_tiles_per_cta", tpc)
-            e.submit_device(0, d.data_ptr(), stride, n, w, h)
+            e.submit_device(0, ptr, stride, n, w, h)
             res = e.collect(0)
             assert res.status == [0] * n
             for i in range(n):

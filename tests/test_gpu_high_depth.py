@@ -11,13 +11,11 @@ import os
 import numpy as np
 import pytest
 
-from tests.test_gpu_device_layouts import align, chroma_dims, pipeline_launches, run, upload
-from tests.test_gpu_formats import CASES
+from tests.support.layouts import BIG_JPEG, CASES, align, pipeline_launches, place, run, upload
 
 pytestmark = pytest.mark.gpu
 
 PAD16 = 0xA5A5
-BIG_JPEG = 8 * 1024 * 1024
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HOST_SO = os.path.join(ROOT, "h264-h265-to-jpeg_b200", "lib", "libh2j_host.so")
 YUV420P10LE, YUV420P12LE, YUV420P10BE = 64, 125, 63  # AVPixelFormat of libavutil 56
@@ -31,35 +29,11 @@ def widen(p, d, rng):
     return w
 
 
-def words(nbytes):
-    return np.full(nbytes // 2, PAD16, np.uint16)
-
-
-def sp16(y, u, v, pitch, uv_off, size):
-    """16-bit semi-planar frame (pitch, offsets in bytes) as bytes"""
-    h, w = y.shape
-    ch, cw = u.shape
-    buf = words(size)
-    buf[: pitch // 2 * h].reshape(h, pitch // 2)[:, :w] = y
-    uv = buf[uv_off // 2: uv_off // 2 + pitch // 2 * ch].reshape(ch, pitch // 2)
-    uv[:, 0: 2 * cw: 2] = u
-    uv[:, 1: 2 * cw: 2] = v
-    return buf.view(np.uint8)
-
-
-def pl16(y, u, v, y_pitch, c_pitch, u_off, v_off, size):
-    h, w = y.shape
-    ch, cw = u.shape
-    buf = words(size)
-    buf[: y_pitch // 2 * h].reshape(h, y_pitch // 2)[:, :w] = y
-    buf[u_off // 2: u_off // 2 + c_pitch // 2 * ch].reshape(ch, c_pitch // 2)[:, :cw] = u
-    buf[v_off // 2: v_off // 2 + c_pitch // 2 * ch].reshape(ch, c_pitch // 2)[:, :cw] = v
-    return buf.view(np.uint8)
-
-
 def sp_layout(w, h, fmt, layout):
     """(pitch, uv_off, size, base shift) in bytes"""
-    ch, cw = chroma_dims(w, h, fmt)
+    import h2j_b200
+
+    ch, cw = h2j_b200.chroma_shape(w, h, fmt)
     row = 2 * max(w, 2 * cw)
     if layout == "decoder":  # pitch rounded to 256, pair plane behind luma rows padded to a multiple of 16
         pitch = align(row, 256)
@@ -74,7 +48,9 @@ def sp_layout(w, h, fmt, layout):
 
 def pl_layouts(w, h, fmt):
     """name -> (y_pitch, c_pitch, u_off, v_off, size, base shift), bytes"""
-    ch, cw = chroma_dims(w, h, fmt)
+    import h2j_b200
+
+    ch, cw = h2j_b200.chroma_shape(w, h, fmt)
     out = {"tight": (2 * w, 2 * cw, 2 * w * h, 2 * w * h + 2 * cw * ch, 2 * (w * h + 2 * cw * ch), 0)}
     p, sh = align(2 * w, 256), align(h, 16)  # a decoder's 16-bit surface: one pitch, planes at multiples of pitch * surface height
     out["decoder"] = (p, p, p * sh, 2 * p * sh, 2 * p * sh + p * ch, 0)
@@ -100,7 +76,7 @@ def test_semiplanar16_matches_oracle(orc, fmt, depth, layout):
             stride = align(size, 256)
             planes = [orc.synth_planes_fmt(w, h, fmt, kind, seed=300 + 2 * i + s, amp=amp) for s in range(2)]
             want = [orc.oracle_encode(*p, chroma_format=fmt)[0] for p in planes]
-            d, ptr = upload([sp16(*(widen(x, depth, rng) for x in p), pitch, uv_off, size) for p in planes], stride, shift)
+            d, ptr = upload([place(*(widen(x, depth, rng) for x in p), pitch, pitch, uv_off, size=size) for p in planes], stride, shift)
             got, launches = run(e, lambda: e.submit_device_semiplanar16(0, ptr, stride, pitch, uv_off, depth, 2, w, h), 2)
             for k in range(2):
                 assert got[k] == want[k], f"fmt {fmt} depth {depth} {layout} {w}x{h} frame {k}: JPEG differs from the oracle's"
@@ -125,7 +101,7 @@ def test_pitched16_matches_oracle(orc, fmt):
             for depth in (9, 10, 12, 16):
                 for name, (yp, cp, uo, vo, size, shift) in pl_layouts(w, h, fmt).items():
                     stride = align(size, 256)
-                    d, ptr = upload([pl16(*(widen(x, depth, rng) for x in p), yp, cp, uo, vo, size) for p in planes], stride, shift)
+                    d, ptr = upload([place(*(widen(x, depth, rng) for x in p), yp, cp, uo, vo, size) for p in planes], stride, shift)
                     got, launches = run(e, lambda: e.submit_device_pitched16(0, ptr, stride, yp, cp, uo, vo, depth, n, w, h), n)
                     assert got == want, f"fmt {fmt} depth {depth} {w}x{h} {name}"
                     assert launches == P + 1, f"fmt {fmt} {w}x{h} {name}: {launches} launches"
@@ -138,24 +114,16 @@ def test_p010_equals_nv12_of_high_bytes(orc):
 
     rng = np.random.default_rng(5)
     for (w, h) in ((1920, 1080), (330, 241), (17, 9)):
-        cw, ch = (w + 1) // 2, (h + 1) // 2
+        ch = (h + 1) // 2
         planes = [orc.synth_planes(w, h, "textured", seed=90 + s) for s in range(2)]
         wide = [[widen(x, 16, rng) for x in p] for p in planes]
         high = [[(x >> 8).astype(np.uint8) for x in p] for p in wide]
         pitch, uv_off, size, _ = sp_layout(w, h, 0, "decoder")
         stride = align(size, 256)
-        d16, p16 = upload([sp16(*p, pitch, uv_off, size) for p in wide], stride)
+        d16, p16 = upload([place(*p, pitch, pitch, uv_off, size=size) for p in wide], stride)
         npitch, nuv = pitch // 2, pitch // 2 * align(h, 16)
         nsize = nuv + npitch * ch
-        nv = []
-        for y, u, v in high:
-            buf = np.full(nsize, 0xA5, np.uint8)
-            buf[: npitch * h].reshape(h, npitch)[:, :w] = y
-            uv = buf[nuv: nuv + npitch * ch].reshape(ch, npitch)
-            uv[:, 0: 2 * cw: 2] = u
-            uv[:, 1: 2 * cw: 2] = v
-            nv.append(buf)
-        d8, p8 = upload(nv, align(nsize, 256))
+        d8, p8 = upload([place(*p, npitch, npitch, nuv, size=nsize) for p in high], align(nsize, 256))
         with h2j_b200.Encoder(max_width=w, max_height=h, max_batch=2, n_slots=1) as e:
             got, _ = run(e, lambda: e.submit_device_semiplanar16(0, p16, stride, pitch, uv_off, 16, 2, w, h), 2)
             for prepass in (0, 1):  # both paths of the 8-bit entry
@@ -177,7 +145,7 @@ def test_batches_across_tiles(orc, fmt, w, h, n):
     want = [orc.oracle_encode(*p, chroma_format=fmt)[0] for p in planes]
     pitch, uv_off, size, _ = sp_layout(w, h, fmt, "decoder")
     stride = align(size, 256)
-    d, ptr = upload([sp16(*(widen(x, 10, rng) for x in p), pitch, uv_off, size) for p in planes], stride)
+    d, ptr = upload([place(*(widen(x, 10, rng) for x in p), pitch, pitch, uv_off, size=size) for p in planes], stride)
     with h2j_b200.Encoder(max_width=w, max_height=h, max_batch=n, n_slots=1, chroma_format=fmt, max_jpeg_bytes=64 << 20) as e:
         for tpc in (0, 2, 16):
             e.set_knob("fdct_tiles_per_cta", tpc)
@@ -196,9 +164,9 @@ def test_range_conversion_and_fixed_qscale(orc, fmt):
     w, h = 322, 242
     y, u, v = orc.synth_planes_fmt(w, h, fmt, "textured", seed=77, amp=70)
     pitch, uv_off, size, _ = sp_layout(w, h, fmt, "tight")
-    ds, ps = upload([sp16(*(widen(x, 10, rng) for x in (y, u, v)), pitch, uv_off, size)], size)
+    ds, ps = upload([place(*(widen(x, 10, rng) for x in (y, u, v)), pitch, pitch, uv_off, size=size)], size)
     yp, cp, uo, vo, psize, _ = pl_layouts(w, h, fmt)["decoder"]
-    dp, pp = upload([pl16(*(widen(x, 12, rng) for x in (y, u, v)), yp, cp, uo, vo, psize)], align(psize, 256))
+    dp, pp = upload([place(*(widen(x, 12, rng) for x in (y, u, v)), yp, cp, uo, vo, psize)], align(psize, 256))
     for kw in ({"range_mode": 1}, {"fixed_qscale": 1}, {"fixed_qscale": 31}):
         want = orc.oracle_encode(y, u, v, chroma_format=fmt, **kw)[0]
         with h2j_b200.Encoder(max_width=w, max_height=h, max_batch=1, n_slots=1, chroma_format=fmt, max_jpeg_bytes=BIG_JPEG, **kw) as e:
@@ -287,77 +255,3 @@ def test_host_class_high_depth_inside_a_batch_scope(orc, tmp_path):
     finally:
         failed = C.c_int(-1)
         assert lib.h2j_host_batch_end(C.byref(failed)) == 0 and failed.value == 0
-
-
-# ---- argument checks ----------------------------------------------------------------------------------------------
-
-def test_argument_checks():
-    import torch
-
-    import h2j_b200
-
-    INVALID, UNSUPPORTED, BUSY = h2j_b200.ERR_INVALID_ARG, h2j_b200.ERR_UNSUPPORTED, h2j_b200.ERR_BUSY
-    d = torch.zeros(1 << 20, dtype=torch.uint8, device="cuda")
-    torch.cuda.synchronize()
-    p = d.data_ptr()
-
-    def status(call):
-        with pytest.raises(h2j_b200.H2JError) as ei:
-            call()
-        return ei.value.status
-
-    w, h = 64, 32
-    with h2j_b200.Encoder(max_width=w, max_height=h, max_batch=1, n_slots=1, chroma_format=2) as e:  # 4:4:4: 128-word pair rows
-        sp = e.submit_device_semiplanar16  # pitch 256 bytes, pair plane at 256 * 32, frame 256 * 64 bytes
-        assert status(lambda: sp(0, p, 256 * 64, 256, 256 * 32, 8, 1, w, h)) == INVALID           # bit_depth below 9
-        assert status(lambda: sp(0, p, 256 * 64, 256, 256 * 32, 17, 1, w, h)) == INVALID          # bit_depth above 16
-        assert status(lambda: sp(0, p + 1, 256 * 64, 256, 256 * 32, 10, 1, w, h)) == INVALID      # odd base pointer
-        assert status(lambda: sp(0, p, 256 * 64 + 1, 256, 256 * 32, 10, 1, w, h)) == INVALID      # odd frame_stride
-        assert status(lambda: sp(0, p, 258 * 64, 257, 258 * 32, 10, 1, w, h)) == INVALID          # odd pitch
-        assert status(lambda: sp(0, p, 256 * 64, 256, 256 * 32 + 1, 10, 1, w, h)) == INVALID      # odd uv_offset
-        assert status(lambda: sp(0, p, 256 * 64, 254, 256 * 32, 10, 1, w, h)) == INVALID          # pitch shorter than a row of pairs
-        assert status(lambda: sp(0, p, 256 * 64, 256, 256 * 16, 10, 1, w, h)) == INVALID          # pair plane inside the luma plane
-        assert status(lambda: sp(0, p, 256 * 64 - 2, 256, 256 * 32, 10, 1, w, h)) == INVALID      # pair plane past frame_stride
-        assert status(lambda: sp(0, p, 512 * 64, 512, 512 * 32, 10, 1, 2 * w, h)) == UNSUPPORTED  # wider than the maximum
-        sp(0, p, 256 * 64, 256, 256 * 32, 10, 1, w, h)
-        assert status(lambda: sp(0, p, 256 * 64, 256, 256 * 32, 10, 1, w, h)) == BUSY            # slot in flight
-        assert e.collect(0).status == [0]
-
-        pt = e.submit_device_pitched16  # 4:4:4 planes of 64 x 32 words: 128-byte rows, 4096-byte planes
-        assert status(lambda: pt(0, p, 12288, 128, 128, 4096, 8192, 8, 1, w, h)) == INVALID       # bit_depth below 9
-        assert status(lambda: pt(0, p + 1, 12288, 128, 128, 4096, 8192, 10, 1, w, h)) == INVALID  # odd base pointer
-        assert status(lambda: pt(0, p, 12289, 128, 128, 4096, 8192, 10, 1, w, h)) == INVALID      # odd frame_stride
-        assert status(lambda: pt(0, p, 12288, 129, 128, 4160, 8192, 10, 1, w, h)) == INVALID      # odd luma pitch
-        assert status(lambda: pt(0, p, 12288, 128, 129, 4096, 8192, 10, 1, w, h)) == INVALID      # odd chroma pitch
-        assert status(lambda: pt(0, p, 12288, 128, 128, 4097, 8192, 10, 1, w, h)) == INVALID      # odd Cb offset
-        assert status(lambda: pt(0, p, 12288, 128, 128, 4096, 8193, 10, 1, w, h)) == INVALID      # odd Cr offset
-        assert status(lambda: pt(0, p, 12288, 126, 128, 4096, 8192, 10, 1, w, h)) == INVALID      # luma pitch shorter than a row
-        assert status(lambda: pt(0, p, 12288, 128, 126, 4096, 8192, 10, 1, w, h)) == INVALID      # chroma pitch shorter than a row
-        assert status(lambda: pt(0, p, 4094, 128, 128, 0, 0, 10, 1, w, h)) == INVALID             # luma plane past frame_stride
-        assert status(lambda: pt(0, p, 12288, 128, 128, 8194, 4096, 10, 1, w, h)) == INVALID      # Cb plane past frame_stride
-        assert status(lambda: pt(0, p, 12288, 128, 128, 4096, 8194, 10, 1, w, h)) == INVALID      # Cr plane past frame_stride
-        assert status(lambda: pt(0, p, 4 * 12288, 256, 256, 16384, 32768, 10, 1, 2 * w, h)) == UNSUPPORTED
-        pt(0, p, 12288, 128, 128, 4096, 8192, 16, 1, w, h)
-        assert status(lambda: pt(0, p, 12288, 128, 128, 4096, 8192, 16, 1, w, h)) == BUSY
-        # the host entry shares slot 0
-        z = np.zeros((h, w), np.uint16)
-        assert status(lambda: e.yuv2jpeg16(z, z, z, 10)) == BUSY
-        assert e.collect(0).status == [0]
-
-        f16 = e._lib.h2j_encode_frame16
-        out = np.empty(1 << 16, np.uint8)
-        n = C.c_size_t(0)
-        raw = np.zeros(2 * w * h + 2, np.uint8)
-
-        def enc16(ptrs, strides, depth, ww=w):
-            rc = f16(e._h, (C.c_void_p * 3)(*ptrs), (C.c_int * 3)(*strides), depth, ww, h, out.ctypes.data, out.size, C.byref(n))
-            return rc
-
-        base = raw.ctypes.data + (raw.ctypes.data & 1)
-        assert enc16([base] * 3, [128] * 3, 8) == INVALID                  # bit_depth below 9
-        assert enc16([base] * 3, [128] * 3, 17) == INVALID                 # bit_depth above 16
-        assert enc16([base + 1, base, base], [128] * 3, 10) == INVALID     # odd plane pointer
-        assert enc16([base] * 3, [128, 129, 128], 10) == INVALID           # odd stride
-        assert enc16([base] * 3, [126, 128, 128], 10) == INVALID           # stride shorter than a row
-        assert enc16([base] * 3, [256] * 3, 10, 2 * w) == UNSUPPORTED      # wider than the maximum
-        assert enc16([base] * 3, [128] * 3, 10) == 0

@@ -11,7 +11,6 @@ import numpy as np
 import pytest
 
 from tests.support import histograms as H
-from tests.test_huffman_tables import oracle_table
 
 pytestmark = pytest.mark.gpu
 
@@ -80,7 +79,7 @@ def test_k3_tables_equal_the_oracle(run, orc):
     n = hist.shape[0]
     assert (out["status"] == 0).all()
     for f in range(n):
-        want = [oracle_table(orc, hist[f, t]) for t in range(4)]
+        want = [H.oracle_table(orc, hist[f, t]) for t in range(4)]
         for t in range(4):
             what = (f, t, kinds[f, t])
             bits, vals, nv = want[t]

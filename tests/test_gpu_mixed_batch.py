@@ -7,71 +7,13 @@ import random
 import numpy as np
 import pytest
 
-from tests.test_gpu_formats import CASES
+from tests.support.layouts import CASES, Frames, align, desc, encoder, planar, semiplanar
 
 pytestmark = pytest.mark.gpu
-
-PAD = 0xA5
-GUARD = 64
-BIG_JPEG = 8 * 1024 * 1024
-
-
-def align(x, a):
-    return (x + a - 1) // a * a
 
 
 def planes(orc, w, h, fmt, kind="textured", seed=0, amp=40):
     return orc.synth_planes_fmt(w, h, fmt, kind, seed=seed, amp=amp)
-
-
-class Frames:
-    """frames in their own device allocations, GUARD bytes of padding on both sides plus `shift` bytes in front"""
-
-    def __init__(self):
-        self.keep = []
-
-    def put(self, buf: np.ndarray, shift: int = 0) -> int:
-        import torch
-
-        host = np.full(GUARD + shift + buf.size + GUARD, PAD, np.uint8)
-        host[GUARD + shift: GUARD + shift + buf.size] = buf
-        t = torch.from_numpy(host).cuda()
-        self.keep.append(t)
-        return t.data_ptr() + GUARD + shift
-
-
-def planar_desc(h2j, fr, y, u, v, y_pitch=None, c_pitch=None, shift=0):
-    h, w = y.shape
-    ch, cw = u.shape
-    y_pitch = y_pitch or w
-    c_pitch = c_pitch or cw
-    u_off = y_pitch * h
-    v_off = u_off + c_pitch * ch
-    buf = np.full(v_off + c_pitch * ch, PAD, np.uint8)
-    buf[: y_pitch * h].reshape(h, y_pitch)[:, :w] = y
-    buf[u_off: u_off + c_pitch * ch].reshape(ch, c_pitch)[:, :cw] = u
-    buf[v_off: v_off + c_pitch * ch].reshape(ch, c_pitch)[:, :cw] = v
-    return h2j.FrameDesc(fr.put(buf, shift), w, h, y_pitch, c_pitch, u_off, v_off)
-
-
-def semiplanar_desc(h2j, fr, y, u, v, pitch, shift=0):
-    h, w = y.shape
-    ch, cw = u.shape
-    uv_off = pitch * h
-    buf = np.full(uv_off + pitch * ch, PAD, np.uint8)
-    buf[: pitch * h].reshape(h, pitch)[:, :w] = y
-    uv = buf[uv_off:].reshape(ch, pitch)
-    uv[:, 0: 2 * cw: 2] = u
-    uv[:, 1: 2 * cw: 2] = v
-    return h2j.FrameDesc(fr.put(buf, shift), w, h, pitch, pitch, uv_off, 0)
-
-
-def encoder(fmt, max_batch, **kw):
-    import h2j_b200
-
-    kw.setdefault("max_jpeg_bytes", BIG_JPEG)
-    return h2j_b200.Encoder(max_width=kw.pop("max_width", 1920), max_height=kw.pop("max_height", 1088), max_batch=max_batch, n_slots=1,
-                            chroma_format=fmt, **kw)
 
 
 def collect_jpegs(e, n):
@@ -94,7 +36,7 @@ def test_all_sizes_in_one_batch(orc, fmt, order):
     for i, (w, h, kind, amp) in enumerate(cases):
         y, u, v = planes(orc, w, h, fmt, kind, seed=30 + i, amp=amp)
         want.append(orc.oracle_encode(y, u, v, chroma_format=fmt)[0])
-        descs.append(planar_desc(h2j, fr, y, u, v))
+        descs.append(desc(fr, y, u, v, *planar(y, u)))
     with encoder(fmt, len(cases)) as e:
         e.submit_device_list(0, h2j.LAYOUT_PLANAR, descs)
         got = collect_jpegs(e, len(cases))
@@ -113,7 +55,7 @@ def test_uniform_list_equals_submit_device(orc, fmt):
     tight = np.concatenate([np.concatenate([p.ravel() for p in f]) for f in frames])
     fb = tight.size // n
     fr = Frames()
-    descs = [planar_desc(h2j, fr, *f) for f in frames]
+    descs = [desc(fr, y, u, v, *planar(y, u)) for y, u, v in frames]
     with encoder(fmt, n) as e:
         d = torch.from_numpy(tight).cuda()
         e.submit_device(0, d.data_ptr(), fb, n, w, h)
@@ -137,7 +79,7 @@ def test_frame_info_and_coefficients_answer_for_the_frame(orc):
         y, u, v = planes(orc, w, h, 0, seed=60 + i)
         _, dbg, coefs = orc.oracle_encode(y, u, v, want_coefs=True)
         dbgs.append((dbg, coefs))
-        descs.append(planar_desc(h2j, fr, y, u, v))
+        descs.append(desc(fr, y, u, v, *planar(y, u)))
     with encoder(0, len(sizes)) as e:
         e.submit_device_list(0, h2j.LAYOUT_PLANAR, descs)
         for i, (dbg, coefs) in enumerate(dbgs):
@@ -158,7 +100,8 @@ def test_pitched_aligned_and_unaligned_mixed(orc, fmt):
     for i, (w, h, yp, cp, shift) in enumerate(specs):
         y, u, v = planes(orc, w, h, fmt, seed=70 + i)
         want.append(orc.oracle_encode(y, u, v, chroma_format=fmt)[0])
-        descs.append(planar_desc(h2j, fr, y, u, v, yp, cp, shift))
+        y_pitch, c_pitch, u_off, v_off = planar(y, u, yp, cp)
+        descs.append(desc(fr, y, u, v, y_pitch, c_pitch, u_off, v_off, size=v_off + c_pitch * u.shape[0], shift=shift))
     aligned = [d for d, s in zip(descs, specs) if s[0] in (1920, 1280) or s[2] == 704]
     with encoder(fmt, len(specs)) as e:
         l0 = e.kernel_launches
@@ -183,9 +126,11 @@ def test_semiplanar_in_place_and_split(orc, fmt):
     for i, (w, h) in enumerate(sizes):
         y, u, v = planes(orc, w, h, fmt, seed=80 + i)
         want.append(orc.oracle_encode(y, u, v, chroma_format=fmt)[0])
-        descs.append(semiplanar_desc(h2j, fr, y, u, v, align(max(w, 2 * u.shape[1]), 64)))
+        pitch = align(max(w, 2 * u.shape[1]), 64)
+        descs.append(desc(fr, y, u, v, *semiplanar(y, pitch), size=pitch * (h + u.shape[0])))
     y, u, v = planes(orc, 131, 77, fmt, seed=89)
-    odd = semiplanar_desc(h2j, fr, y, u, v, 2 * u.shape[1] + 3, shift=5)
+    pitch = 2 * u.shape[1] + 3
+    odd = desc(fr, y, u, v, *semiplanar(y, pitch), size=pitch * (77 + u.shape[0]), shift=5)
     want_odd = orc.oracle_encode(y, u, v, chroma_format=fmt)[0]
     with encoder(fmt, len(sizes) + 1) as e:
         l0 = e.kernel_launches
@@ -210,7 +155,7 @@ def test_several_tiles_per_cta(orc, fmt, tiles):
     for i, (w, h) in enumerate(sizes):
         y, u, v = planes(orc, w, h, fmt, "noise", seed=90 + i, amp=30)
         want.append(orc.oracle_encode(y, u, v, chroma_format=fmt)[0])
-        descs.append(planar_desc(h2j, fr, y, u, v))
+        descs.append(desc(fr, y, u, v, *planar(y, u)))
     with encoder(fmt, len(sizes), max_width=2562, max_height=4098) as e:
         e.set_knob("fdct_tiles_per_cta", tiles)
         e.submit_device_list(0, h2j.LAYOUT_PLANAR, descs)
@@ -231,7 +176,8 @@ def test_both_scan_place_widths(orc):
             if (w, h) not in want:
                 y, u, v = planes(orc, w, h, 0, seed=100 + len(want))
                 want[(w, h)] = (orc.oracle_encode(y, u, v)[0], (y, u, v))
-            descs.append(planar_desc(h2j, fr, *want[(w, h)][1]))
+            y, u, v = want[(w, h)][1]
+            descs.append(desc(fr, y, u, v, *planar(y, u)))
         with encoder(0, len(sizes)) as e:
             e.set_profile(True)
             e.submit_device_list(0, h2j.LAYOUT_PLANAR, descs)
@@ -248,7 +194,7 @@ def test_one_frame_over_the_limit_fails_alone(orc):
     for i, (w, h, kind, amp) in enumerate(sizes):
         y, u, v = planes(orc, w, h, 0, kind, seed=110 + i, amp=amp)
         want.append(orc.oracle_encode(y, u, v)[0])
-        descs.append(planar_desc(h2j, fr, y, u, v))
+        descs.append(desc(fr, y, u, v, *planar(y, u)))
     limit = max(len(want[0]), len(want[2])) + 16
     assert len(want[1]) > limit
     with encoder(0, len(sizes), max_width=640, max_height=480, max_jpeg_bytes=limit) as e:
@@ -256,49 +202,6 @@ def test_one_frame_over_the_limit_fails_alone(orc):
         r = e.collect(0, strict=False)
         assert r.status[1] != 0 and r.status[0] == 0 and r.status[2] == 0
         assert r.jpegs[0] == want[0] and r.jpegs[2] == want[2]
-
-
-def test_argument_errors(orc):
-    import h2j_b200 as h2j
-
-    fr = Frames()
-    y, u, v = planes(orc, 64, 48, 0)
-    good = planar_desc(h2j, fr, y, u, v)
-    sp = semiplanar_desc(h2j, fr, y, u, v, 64)
-
-    def with_(d, **kw):
-        x = h2j.FrameDesc(d.data, d.width, d.height, d.y_pitch, d.c_pitch, d.u_offset, d.v_offset)
-        for k, val in kw.items():
-            setattr(x, k, val)
-        return x
-
-    with encoder(0, 2, max_width=128, max_height=128) as e:
-        def status(layout, descs):
-            with pytest.raises(h2j.H2JError) as ex:
-                e.submit_device_list(0, layout, descs)
-            return ex.value.status
-
-        assert status(h2j.LAYOUT_PLANAR, []) == h2j.ERR_INVALID_ARG
-        assert status(h2j.LAYOUT_PLANAR, [good] * 3) == h2j.ERR_INVALID_ARG
-        assert status(2, [good]) == h2j.ERR_INVALID_ARG
-        assert status(h2j.LAYOUT_PLANAR, [good, with_(good, data=None)]) == h2j.ERR_INVALID_ARG
-        assert status(h2j.LAYOUT_PLANAR, [with_(good, y_pitch=63)]) == h2j.ERR_INVALID_ARG
-        assert status(h2j.LAYOUT_PLANAR, [with_(good, c_pitch=31)]) == h2j.ERR_INVALID_ARG
-        assert status(h2j.LAYOUT_SEMIPLANAR, [with_(sp, c_pitch=63)]) == h2j.ERR_INVALID_ARG
-        assert status(h2j.LAYOUT_SEMIPLANAR, [with_(sp, u_offset=64 * 47)]) == h2j.ERR_INVALID_ARG
-        assert status(h2j.LAYOUT_PLANAR, [with_(good, width=1)]) == h2j.ERR_UNSUPPORTED
-        assert status(h2j.LAYOUT_PLANAR, [with_(good, height=129)]) == h2j.ERR_UNSUPPORTED
-        assert status(h2j.LAYOUT_PLANAR, [with_(good, width=70000)]) == h2j.ERR_UNSUPPORTED
-        for bad in ([None], None):
-            with pytest.raises(h2j.H2JError) as ex:
-                if bad is None:
-                    e._check(e._lib.h2j_submit_host_list(e._h, 0, None, None, None, 1))
-                else:
-                    e.submit_host_list(0, [0], [(64, 48)])
-            assert ex.value.status == h2j.ERR_INVALID_ARG
-        e.submit_device_list(0, h2j.LAYOUT_PLANAR, [good])
-        assert status(h2j.LAYOUT_PLANAR, [good]) == h2j.ERR_BUSY
-        e.collect(0)
 
 
 def test_large_mixed_batch(orc):
@@ -312,7 +215,7 @@ def test_large_mixed_batch(orc):
         y, u, v = planes(orc, *s, 0, seed=120 + i)
         base[s] = (y, u, v)
     fr = Frames()
-    descs = [planar_desc(h2j, fr, *base[s]) for s in sizes]
+    descs = [desc(fr, y, u, v, *planar(y, u)) for y, u, v in (base[s] for s in sizes)]
     check = sorted({0, 255} | set(rng.sample(range(256), 6)))
     with encoder(0, 256, max_width=3840, max_height=2160) as e:
         e.submit_device_list(0, h2j.LAYOUT_PLANAR, descs)

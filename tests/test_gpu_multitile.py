@@ -9,18 +9,9 @@ read in place, every JPEG compared with the oracle byte for byte.  Then the benc
 import numpy as np
 import pytest
 
+from tests.support.layouts import place, upload
+
 pytestmark = pytest.mark.gpu
-
-
-def _nv12(y, u, v, pitch):
-    h, w = y.shape
-    ch, cw = u.shape
-    buf = np.full(pitch * (h + ch), 0x5A, np.uint8)
-    buf[: pitch * h].reshape(h, pitch)[:, :w] = y
-    uv = buf[pitch * h:].reshape(ch, pitch)
-    uv[:, 0: 2 * cw: 2] = u
-    uv[:, 1: 2 * cw: 2] = v
-    return buf
 
 
 # (w, h): MCUs -> tiles.  641x479: 41x30 = 1230 -> 76.9 (last tile 14 MCUs, last unit 20 blocks); 330x225: 21x15 = 315 ->
@@ -28,8 +19,6 @@ def _nv12(y, u, v, pitch):
 # eight MCU rows, the last one holds 2 MCUs); 2562x1442: 161x91 = 14651 -> 915.7
 @pytest.mark.parametrize("w,h", [(641, 479), (330, 225), (330, 241), (17, 4098), (2562, 1442)])
 def test_multi_tile_ctas_on_partial_tiles(orc, w, h):
-    import torch
-
     import h2j_b200
 
     n = 8
@@ -37,26 +26,21 @@ def test_multi_tile_ctas_on_partial_tiles(orc, w, h):
     want = [orc.oracle_encode(*p)[0] for p in planes]
     frames = np.stack([orc.pack_i420(*p) for p in planes])
     stride = (frames.shape[1] + 255) // 256 * 256
-    host = np.zeros((n, stride), np.uint8)
-    host[:, : frames.shape[1]] = frames
-    d = torch.from_numpy(host).cuda()
+    d, ptr = upload(frames, stride)
     cw = (w + 1) // 2
     pitch = (max(w, 2 * cw) + 63) // 64 * 64
-    nv = np.stack([_nv12(*p, pitch) for p in planes])
-    nstride = (nv.shape[1] + 255) // 256 * 256
-    nhost = np.zeros((n, nstride), np.uint8)
-    nhost[:, : nv.shape[1]] = nv
-    dn = torch.from_numpy(nhost).cuda()
-    torch.cuda.synchronize()
+    nv = [place(*p, pitch, pitch, pitch * h, size=pitch * (h + p[1].shape[0]), pad=0x5A) for p in planes]
+    nstride = (len(nv[0]) + 255) // 256 * 256
+    dn, nptr = upload(nv, nstride)
     with h2j_b200.Encoder(max_width=w, max_height=h, max_batch=n, n_slots=1) as e:
         for tpc in (2, 5, 16):
             e.set_knob("fdct_tiles_per_cta", tpc)
-            e.submit_device(0, d.data_ptr(), stride, n, w, h)
+            e.submit_device(0, ptr, stride, n, w, h)
             res = e.collect(0)
             assert res.status == [0] * n
             for i in range(n):
                 assert res.jpegs[i] == want[i], f"{w}x{h}, {tpc} tiles per CTA, planar frame {i}"
-            e.submit_device_nv12(0, dn.data_ptr(), nstride, pitch, pitch * h, n, w, h)
+            e.submit_device_nv12(0, nptr, nstride, pitch, pitch * h, n, w, h)
             res = e.collect(0)
             for i in range(n):
                 assert res.jpegs[i] == want[i], f"{w}x{h}, {tpc} tiles per CTA, NV12 frame {i}"

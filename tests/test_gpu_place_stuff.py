@@ -12,6 +12,7 @@ import numpy as np
 import pytest
 
 from tests.support import scan_model as M
+from tests.support.layouts import Frames, desc, planar
 
 pytestmark = pytest.mark.gpu
 
@@ -90,8 +91,6 @@ def test_k4b_cases_in_one_list_batch(orc, form):
     past their own groups return at once"""
     import h2j_b200 as h2j
 
-    from tests.test_gpu_mixed_batch import Frames, planar_desc
-
     base = [M.case(k) for k in M.K4B_EDGES + M.SIZE_EDGES]
     groups = max(c.scan.groups for c in base)
     assert len({c.scan.groups for c in base}) >= 3
@@ -99,7 +98,7 @@ def test_k4b_cases_in_one_list_batch(orc, form):
     cases = base * reps
     assert (groups * len(cases) < 2 * _sm_count()) == (form == 8)
     fr = Frames()
-    descs = [planar_desc(h2j, fr, *c.planes) for c in cases]
+    descs = [desc(fr, y, u, v, *planar(y, u)) for y, u, v in (c.planes for c in cases)]
     w, h = max(c.size[0] for c in base), max(c.size[1] for c in base)
     with h2j.Encoder(max_width=w, max_height=h, max_batch=len(cases), n_slots=1, fixed_qscale=M.QSCALE,
                      max_jpeg_bytes=_cap([c.scan.jpeg for c in base])) as e:

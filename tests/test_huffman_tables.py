@@ -1,8 +1,6 @@
 """CPU suite: the oracle's Huffman table builder (orc_huffman_table, libavcodec's mjpegenc_huffman.c restated) on
 adversarial histograms, against properties that do not depend on tie order, computed with exact Python integers --
 among them the optimal cost of a 16-bit length-limited prefix code from a textbook package-merge."""
-import ctypes as C
-
 import numpy as np
 import pytest
 
@@ -13,15 +11,6 @@ from tests.support import histograms as H
 def tables():
     dc, ac = H.generate()
     return dc + ac
-
-
-def oracle_table(orc, hist):
-    bits = np.zeros(17, np.uint8)
-    vals = np.zeros(256, np.uint8)
-    nv = C.c_int(0)
-    h = np.ascontiguousarray(hist, np.uint32)
-    orc.oracle().orc_huffman_table(h.ctypes.data, bits.ctypes.data, vals.ctypes.data, C.byref(nv))
-    return bits, vals, nv.value
 
 
 def test_generator_covers_its_families(tables):
@@ -64,7 +53,7 @@ def test_reference_optimum_on_small_cases():
 def test_oracle_tables_are_optimal_length_limited_codes(orc, tables):
     deep = 0
     for i, (kind, hist) in enumerate(tables):
-        bits, vals, nv = oracle_table(orc, hist)
+        bits, vals, nv = H.oracle_table(orc, hist)
         bad = H.check_table(hist, bits, vals, nv)
         assert not bad, (i, kind, bad)
         deep += int(bits[16]) > 0
@@ -78,6 +67,6 @@ def test_length_limit_cuts_many_levels(orc):
         f.append(f[-1] + f[-2])
     hist = np.zeros(256, np.uint32)
     hist[:43] = f
-    bits, vals, nv = oracle_table(orc, hist)
+    bits, vals, nv = H.oracle_table(orc, hist)
     assert not H.check_table(hist, bits, vals, nv)
     assert int(bits[16]) >= 15 and sum(int(b) for b in bits[1:17]) == 43
