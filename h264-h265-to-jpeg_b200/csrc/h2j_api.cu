@@ -53,8 +53,12 @@ struct Slot {
     long long *h_sizes = nullptr;             // pinned (jpeg_bytes per frame)
     uint8_t *h_stage = nullptr;               // pinned staging for h2j_encode_frame / convert
     size_t h_stage_bytes = 0;
-    uint8_t *d_frames16 = nullptr;            // h2j_encode_frame16 (slot 0, allocated on its first call): the 16-bit planes ...
-    uint8_t *h_stage16 = nullptr;             // ... and their pinned staging
+    // the converting single-picture calls (h2j_encode_frame16, h2j_encode_frame_rgb; slot 0): the caller's picture as staged
+    // on the device, before the input stage converts it, and its pinned staging; allocated on first use, grown when a call
+    // needs more (reserve_convert)
+    uint8_t *d_convert = nullptr;
+    uint8_t *h_convert = nullptr;
+    size_t convert_bytes = 0;
     unsigned char *h_tail = nullptr;          // pinned: status .. jpeg_bytes of frame 0's FrameTab (h2j_encode_frame)
     size_t spec_bytes = 384 * 1024;           // JPEG bytes h2j_encode_frame copies back before it knows the size
     bool busy = false;
@@ -498,16 +502,17 @@ int check_slot(h2j_encoder *e, int slot)
     return H2J_OK;
 }
 
-// Upload one picture's three planes (rows[i] rows of row_bytes[i] bytes, strides[i] apart in host memory) to dev + off[i]
-// at pitch[i] on the slot's stream.  Pageable planes go through `stage` (pinned, laid out as on the device) in pieces,
-// every piece uploaded as soon as it is in place, so that the DMA of one piece runs under the memcpy of the next.
+// Upload one picture's planes (the first n_planes of three: rows[i] rows of row_bytes[i] bytes, strides[i] apart in host
+// memory) to dev + off[i] at pitch[i] on the slot's stream.  Pageable planes go through `stage` (pinned, laid out as on the
+// device) in pieces, every piece uploaded as soon as it is in place, so that the DMA of one piece runs under the memcpy of
+// the next.
 int upload_planes(h2j_encoder *e, Slot &sl, const uint8_t *const planes[3], const int strides[3], const int row_bytes[3], const int rows[3],
-                  const size_t off[3], const int pitch[3], uint8_t *dev, uint8_t *stage)
+                  const size_t off[3], const int pitch[3], uint8_t *dev, uint8_t *stage, int n_planes = 3)
 {
     constexpr int kMaxPieces = 96;
     CopyPiece pieces[kMaxPieces];
     int n_pieces = 0;
-    for (int p = 0; p < 3; p++) {
+    for (int p = 0; p < n_planes; p++) {
         const int ph = rows[p];
         // pieces of ~256 KiB, but never more than a third of the table per plane
         int rows_per_piece = std::max(1, (256 * 1024) / pitch[p]);
@@ -536,8 +541,10 @@ int upload_planes(h2j_encoder *e, Slot &sl, const uint8_t *const planes[3], cons
         }
         return at.type == cudaMemoryTypeHost;
     };
-    if (pinned(planes[0]) && pinned(planes[1]) && pinned(planes[2])) {
-        for (int p = 0; p < 3; p++)
+    bool all_pinned = true;
+    for (int p = 0; p < n_planes; p++) all_pinned = all_pinned && pinned(planes[p]);
+    if (all_pinned) {
+        for (int p = 0; p < n_planes; p++)
             CU(e, cudaMemcpy2DAsync(dev + off[p], pitch[p], planes[p], strides[p], row_bytes[p], rows[p], cudaMemcpyHostToDevice, sl.stream));
         n_pieces = 0;
     }
@@ -580,10 +587,10 @@ void free_slot(Slot &sl)
     if (sl.stream) cudaStreamSynchronize(sl.stream);
     cudaFree(sl.d_frames); cudaFree(sl.d_pitched); cudaFree(sl.d_images); cudaFree(sl.d_zero); cudaFree(sl.d_stage); cudaFree(sl.d_unit_info);
     cudaFree(sl.d_tabs); cudaFree(sl.d_scan); cudaFree(sl.d_out); cudaFree(sl.d_packed); cudaFree(sl.d_offsets); cudaFree(sl.d_status);
-    cudaFree(sl.d_frames16);
+    cudaFree(sl.d_convert);
     cudaFree(sl.d_desc);
     if (sl.h_desc) cudaFreeHost(sl.h_desc);
-    if (sl.h_stage16) cudaFreeHost(sl.h_stage16);
+    if (sl.h_convert) cudaFreeHost(sl.h_convert);
     if (sl.h_offsets) cudaFreeHost(sl.h_offsets);
     if (sl.h_status) cudaFreeHost(sl.h_status);
     if (sl.h_sizes) cudaFreeHost(sl.h_sizes);
@@ -663,13 +670,25 @@ struct Input {
     bool sp = false;    // semi-planar: the Cb/Cr pairs in one plane at u_off (= v_off)
     int bit_depth = 8;  // 9 .. 16: 16-bit words, converted to 8-bit planar frames
     int factor = 1;     // 2, 4, 8: box-filtered to 1/factor
+    int rgb = -1;       // an h2j_rgb_format: RGB pixels, converted to YCbCr planar frames
 };
+
+// the rgb_to_planar_kernel instantiation for an h2j_rgb_format and a chroma format
+template <int K>
+decltype(&rgb_to_planar_kernel<1, kFmt420>) rgb_kernel_fmt(int fmt)
+{
+    return fmt == kFmt422 ? rgb_to_planar_kernel<K, kFmt422> : fmt == kFmt444 ? rgb_to_planar_kernel<K, kFmt444> : rgb_to_planar_kernel<K, kFmt420>;
+}
+decltype(&rgb_to_planar_kernel<1, kFmt420>) rgb_kernel(int rgb, int fmt)
+{
+    return rgb == H2J_RGB_PLANAR ? rgb_kernel_fmt<1>(fmt) : rgb >= H2J_RGB_RGBX ? rgb_kernel_fmt<4>(fmt) : rgb_kernel_fmt<3>(fmt);
+}
 
 // The input stage of every submit, then the pipeline, for n frames described by m entry pairs (m = n, or 1: see Slot).  On
 // entry sl.h_desc[m + i] is the source of frame i where it lies, and sl.h_desc[i] the frame the pipeline encodes (at its
 // size: a downscaled frame's is smaller), read in place.  A frame is read
 // where it is unless it has to be copied:
-//   - 16-bit and downscaled frames are converted (depth_to_8_kernel, downscale_list_kernel);
+//   - 16-bit, downscaled and RGB frames are converted (depth_to_8_kernel, downscale_list_kernel, rgb_to_planar_kernel);
 //   - a semi-planar batch is read in place when every frame's rows start on 8-byte boundaries (K1 only looks at luma, K2's
 //     chroma roles fetch the pairs and keep their component in registers); otherwise, or with semiplanar_prepass, all of it
 //     is split into planes (nv12_to_i420_kernel);
@@ -682,7 +701,7 @@ int run_batch(h2j_encoder *e, Slot &sl, int n, int m, const Input &in, int tail)
 {
     FrameDesc *D = sl.h_desc, *S = sl.h_desc + m;
     const int fmt = e->s.chroma_format;
-    const bool convert = in.bit_depth > 8 || in.factor > 1;
+    const bool convert = in.bit_depth > 8 || in.factor > 1 || in.rgb >= 0;
     bool unaligned = false;
     for (int i = 0; i < m; i++) unaligned = unaligned || !S[i].L.aligned8;
     const bool split = in.sp && (unaligned || e->force_sp_prepass);
@@ -691,7 +710,9 @@ int run_batch(h2j_encoder *e, Slot &sl, int n, int m, const Input &in, int tail)
         cudaGetLastError();  // no room for the copies: the bytewise path still works
         sl.d_pitched = nullptr;
     }
-    int cols = 0, rows = 0;  // the largest copy: 16-byte columns of its widest row (semi-planar: of pairs), rows of all planes
+    // the largest copy: 16-byte columns of its widest row (semi-planar: of pairs), rows of all planes (RGB: 16-pixel columns,
+    // destination rows a warp makes)
+    int cols = 0, rows = 0;
     for (int i = 0; i < m; i++) {
         if (!convert && !split && (in.sp || S[i].L.aligned8 || !sl.d_pitched)) {
             S[i].base = nullptr;
@@ -703,6 +724,11 @@ int run_batch(h2j_encoder *e, Slot &sl, int n, int m, const Input &in, int tail)
         D[i].L.frame_stride = (long long)spacing;
         D[i].base = (convert || in.sp ? sl.d_frames : sl.d_pitched) + (size_t)i * spacing;
         const int w = D[i].L.w, h = D[i].L.h;
+        if (in.rgb >= 0) {
+            cols = std::max(cols, (w + 15) / 16);
+            rows = std::max(rows, fmt == kFmt420 ? (h + 1) / 2 : h);
+            continue;
+        }
         cols = std::max(cols, (std::max(w, (in.sp ? 2 : 1) * chroma_w(w, fmt)) + 15) / 16);
         rows = std::max(rows, h + (in.sp ? 1 : 2) * chroma_h(h, fmt));
     }
@@ -713,14 +739,17 @@ int run_batch(h2j_encoder *e, Slot &sl, int n, int m, const Input &in, int tail)
         CU(e, cudaMemcpyAsync(sl.d_desc, sl.h_desc, sizeof(FrameDesc) * (rows ? 2 * m : m), cudaMemcpyHostToDevice, sl.stream));
     if (rows) {
         static_assert(32 * kDownWarps == 128, "every copy kernel runs CTAs of 128 threads");
-        const int rows_per_cta = in.factor > 1 ? kDownWarps * 16 / in.factor : kPlaneRowsPerCta;
-        const dim3 grid(in.factor > 1 ? (cols + 31) / 32 : (cols + 127) / 128, (rows + rows_per_cta - 1) / rows_per_cta, n);
+        const bool warp_rows = in.factor > 1 || in.rgb >= 0;  // a warp per row, a lane per 16 bytes or pixels of it
+        const int rows_per_cta = in.rgb >= 0 ? kDownWarps * kRgbRowsPerWarp : in.factor > 1 ? kDownWarps * 16 / in.factor : kPlaneRowsPerCta;
+        const dim3 grid(warp_rows ? (cols + 31) / 32 : (cols + 127) / 128, (rows + rows_per_cta - 1) / rows_per_cta, n);
         decltype(&repitch_kernel) k = in.sp ? nv12_to_i420_kernel : repitch_kernel;
         if (in.factor == 2) k = in.sp ? downscale_list_kernel<2, true> : downscale_list_kernel<2, false>;
         else if (in.factor == 4) k = in.sp ? downscale_list_kernel<4, true> : downscale_list_kernel<4, false>;
         else if (in.factor == 8) k = in.sp ? downscale_list_kernel<8, true> : downscale_list_kernel<8, false>;
         const CopyTable t{sl.d_desc, m, D[0], S[0]};
         if (in.bit_depth > 8) (in.sp ? depth_to_8_kernel<true> : depth_to_8_kernel<false>)<<<grid, 128, 0, sl.stream>>>(t, in.bit_depth - 8);
+        else if (in.rgb >= 0)
+            rgb_kernel(in.rgb, fmt)<<<grid, 128, 0, sl.stream>>>(t, in.rgb == H2J_RGB_BGR24 || in.rgb == H2J_RGB_BGRX ? 0x3012u : 0x3210u);
         else k<<<grid, 128, 0, sl.stream>>>(t);
         e->launches++;
         CU(e, cudaGetLastError());
@@ -728,6 +757,63 @@ int run_batch(h2j_encoder *e, Slot &sl, int n, int m, const Input &in, int tail)
     int rc = launch_pipeline(e, sl, n, tail);
     if (rc) return rc;
     if (tail != TAIL_SINGLE) sl.busy = true;
+    return H2J_OK;
+}
+
+// slot 0's buffers of the converting single-picture calls hold at least `bytes` (grown if not): H2J_ERR_NOMEM, with none
+// held, when they cannot be had
+int reserve_convert(h2j_encoder *e, Slot &sl, size_t bytes)
+{
+    if (bytes <= sl.convert_bytes) return H2J_OK;
+    cudaFree(sl.d_convert);
+    if (sl.h_convert) cudaFreeHost(sl.h_convert);
+    sl.d_convert = nullptr;
+    sl.h_convert = nullptr;
+    sl.convert_bytes = 0;
+    if (cudaMalloc(&sl.d_convert, bytes) != cudaSuccess || cudaHostAlloc(&sl.h_convert, bytes, cudaHostAllocDefault) != cudaSuccess) {
+        cudaGetLastError();
+        cudaFree(sl.d_convert);
+        sl.d_convert = nullptr;
+        sl.h_convert = nullptr;
+        return fail(e, H2J_ERR_NOMEM, "no room for the %zu-byte staging of a picture to convert", bytes);
+    }
+    sl.convert_bytes = bytes;
+    return H2J_OK;
+}
+
+// bytes of a row of w pixels of an h2j_rgb_format (planar: of each plane); 0 for a bad format
+int rgb_row_bytes(int format, int w)
+{
+    switch (format) {
+    case H2J_RGB_RGB24: case H2J_RGB_BGR24: return 3 * w;
+    case H2J_RGB_RGBX: case H2J_RGB_BGRX: return 4 * w;
+    case H2J_RGB_PLANAR: return w;
+    default: return 0;
+    }
+}
+
+// Caller RGB frame i (h2j_submit_device_rgb) -> tab[i], the planar frame the pipeline encodes (range_mode 0: the YCbCr of
+// an RGB frame is full range by construction), and tab[n + i], the frame where it is (rows y_pitch apart, planar G and B
+// planes at u_off / v_off, extent: the bytes from its base that may be read)
+int rgb_frame_layout(h2j_encoder *e, int i, int n, int format, const h2j_frame_desc &F, FrameDesc *tab)
+{
+    if (!F.data) return fail(e, H2J_ERR_INVALID_ARG, "frame %d: null data", i);
+    FrameDesc &d = tab[i], &s = tab[n + i];
+    int rc = make_layout(e, nullptr, F.width, F.height, &d.L);
+    if (rc) return rc;
+    d.L.range_mode = 0;
+    const int row = rgb_row_bytes(format, F.width);
+    if (F.y_pitch < row) return fail(e, H2J_ERR_INVALID_ARG, "frame %d: pitch %d shorter than a row of %d bytes", i, F.y_pitch, row);
+    const size_t plane = (size_t)F.y_pitch * F.height;
+    const bool planar = format == H2J_RGB_PLANAR;
+    if (planar && (F.u_offset < plane || F.v_offset < plane))
+        return fail(e, H2J_ERR_INVALID_ARG, "frame %d: the G or B plane starts inside the R plane", i);
+    s = d;
+    s.L.y_pitch = s.L.c_pitch = F.y_pitch;
+    s.L.u_off = planar ? (long long)F.u_offset : 0;
+    s.L.v_off = planar ? (long long)F.v_offset : 0;
+    s.base = F.data;
+    s.extent = (long long)((planar ? std::max(F.u_offset, F.v_offset) : 0) + (size_t)F.y_pitch * (F.height - 1) + row);
     return H2J_OK;
 }
 
@@ -1063,6 +1149,25 @@ int h2j_submit_device_downscaled(h2j_encoder *e, int slot, int layout, const h2j
     return run_batch(e, sl, n, n, Input{sp, 8, factor}, TAIL_SIZES);
 }
 
+int h2j_submit_device_rgb(h2j_encoder *e, int slot, int format, const h2j_frame_desc *frames, int n)
+{
+    int rc = check_submit(e, slot, frames, n);
+    if (rc) return rc;
+    if (!rgb_row_bytes(format, 2)) return fail(e, H2J_ERR_INVALID_ARG, "bad RGB format %d", format);
+    Slot &sl = e->slots[slot];
+    std::vector<FrameDesc> tab(2 * (size_t)n);  // (every frame is checked before the slot's table is touched)
+    for (int i = 0; i < n; i++) {
+        rc = rgb_frame_layout(e, i, n, format, frames[i], tab.data());
+        if (rc) return rc;
+    }
+    memcpy(sl.h_desc, tab.data(), sizeof(FrameDesc) * 2 * n);
+    ON_DEVICE(e);
+    CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
+    Input in;
+    in.rgb = format;
+    return run_batch(e, sl, n, n, in, TAIL_SIZES);
+}
+
 int h2j_submit_host_list(h2j_encoder *e, int slot, const uint8_t *const *frames, const int *widths, const int *heights, int n)
 {
     int rc = check_submit(e, slot, widths && heights ? frames : nullptr, n);
@@ -1232,27 +1337,61 @@ int h2j_encode_frame16(h2j_encoder *e, const uint8_t *const planes[3], const int
     ON_DEVICE(e);
     // the 16-bit planes go to the device at 16-byte aligned row pitches, so that the conversion reads them with vector loads
     const int yp = (int)align_up((size_t)2 * width, 16), cp = (int)align_up((size_t)2 * fcw, 16);
-    if (!sl.d_frames16) {
+    {
         const int mcw = chroma_w(e->s.max_width, fmt), mch = chroma_h(e->s.max_height, fmt);
-        const size_t bytes = align_up((size_t)2 * e->s.max_width, 16) * e->s.max_height + 2 * align_up((size_t)2 * mcw, 16) * mch;
-        if (cudaMalloc(&sl.d_frames16, bytes) != cudaSuccess || cudaHostAlloc(&sl.h_stage16, bytes, cudaHostAllocDefault) != cudaSuccess) {
-            cudaGetLastError();
-            cudaFree(sl.d_frames16);
-            sl.d_frames16 = nullptr;
-            sl.h_stage16 = nullptr;
-            return fail(e, H2J_ERR_NOMEM, "no room for the 16-bit staging of a %dx%d picture", e->s.max_width, e->s.max_height);
-        }
+        const int rc = reserve_convert(e, sl, align_up((size_t)2 * e->s.max_width, 16) * e->s.max_height + 2 * align_up((size_t)2 * mcw, 16) * mch);
+        if (rc) return rc;
     }
     // a batch of one frame: the planes as staged on the device, converted by the input stage
-    const h2j_frame_desc F{sl.d_frames16, width, height, yp, cp, (size_t)yp * height, (size_t)yp * height + (size_t)cp * fch};
+    const h2j_frame_desc F{sl.d_convert, width, height, yp, cp, (size_t)yp * height, (size_t)yp * height + (size_t)cp * fch};
     int rc = describe_batch(e, sl, F, (size_t)yp * height + 2 * (size_t)cp * fch, false, 2);
     if (rc) return rc;
     CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
     const int row_bytes[3] = {2 * width, 2 * fcw, 2 * fcw}, rows[3] = {height, fch, fch}, pitch[3] = {yp, cp, cp};
     const size_t off[3] = {0, F.u_offset, F.v_offset};
-    rc = upload_planes(e, sl, planes, strides, row_bytes, rows, off, pitch, sl.d_frames16, sl.h_stage16);
+    rc = upload_planes(e, sl, planes, strides, row_bytes, rows, off, pitch, sl.d_convert, sl.h_convert);
     if (rc) return rc;
     rc = run_batch(e, sl, 1, 1, Input{false, bit_depth}, TAIL_SINGLE);
+    if (rc) return rc;
+    return finish_single(e, sl, out, out_capacity, out_size);
+}
+
+int h2j_encode_frame_rgb(h2j_encoder *e, int format, const uint8_t *const planes[3], const int strides[3], int width, int height,
+                         uint8_t *out, size_t out_capacity, size_t *out_size)
+{
+    if (!e) return H2J_ERR_INVALID_ARG;
+    const bool planar = format == H2J_RGB_PLANAR;
+    if (!planes || !strides || !planes[0] || (planar && (!planes[1] || !planes[2])) || !out || !out_size)
+        return fail(e, H2J_ERR_INVALID_ARG, "null plane/out pointer");
+    const int row = rgb_row_bytes(format, width);
+    if (!row) return fail(e, H2J_ERR_INVALID_ARG, "bad RGB format %d", format);
+    if (width < 2 || height < 2 || width > e->s.max_width || height > e->s.max_height)
+        return fail(e, H2J_ERR_UNSUPPORTED, "frame %dx%d outside 2x2 .. %dx%d", width, height, e->s.max_width, e->s.max_height);
+    Slot &sl = e->slots[0];
+    if (sl.busy) return fail(e, H2J_ERR_BUSY, "slot 0 has a batch in flight");
+    for (int p = 0; p < (planar ? 3 : 1); p++)
+        if (strides[p] < row) return fail(e, H2J_ERR_INVALID_ARG, "stride %d of plane %d smaller than a row of %d bytes", strides[p], p, row);
+    ON_DEVICE(e);
+    // the picture goes to the device at a 16-byte aligned row pitch, so that the conversion reads it with vector loads
+    const int pitch = (int)align_up((size_t)row, 16);
+    {
+        const size_t max_pitch = align_up((size_t)rgb_row_bytes(format, e->s.max_width), 16);
+        const int rc = reserve_convert(e, sl, max_pitch * e->s.max_height * (planar ? 3 : 1));
+        if (rc) return rc;
+    }
+    // a batch of one frame: the picture as staged on the device, converted by the input stage
+    const size_t plane = (size_t)pitch * height;
+    const h2j_frame_desc F{sl.d_convert, width, height, pitch, pitch, planar ? plane : 0, planar ? 2 * plane : 0};
+    int rc = rgb_frame_layout(e, 0, 1, format, F, sl.h_desc);
+    if (rc) return rc;
+    CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
+    const int row_bytes[3] = {row, row, row}, rows[3] = {height, height, height}, pitches[3] = {pitch, pitch, pitch};
+    const size_t off[3] = {0, plane, 2 * plane};
+    rc = upload_planes(e, sl, planes, strides, row_bytes, rows, off, pitches, sl.d_convert, sl.h_convert, planar ? 3 : 1);
+    if (rc) return rc;
+    Input in;
+    in.rgb = format;
+    rc = run_batch(e, sl, 1, 1, in, TAIL_SINGLE);
     if (rc) return rc;
     return finish_single(e, sl, out, out_capacity, out_size);
 }
@@ -1353,6 +1492,34 @@ int h2j_debug_coefficients(h2j_encoder *e, int slot, int frame, int16_t *out, si
         last_dc[comp] += rec[0];
         out[(size_t)b * 64] = (int16_t)last_dc[comp];
         for (int k = 1; k < 64; k++) out[(size_t)b * 64 + k] = rec[2 * (k & 31) + (k >> 5)];
+    }
+    return H2J_OK;
+}
+
+int h2j_debug_frame_planes(h2j_encoder *e, int slot, int frame, uint8_t *y, uint8_t *u, uint8_t *v)
+{
+    int rc = check_slot(e, slot);
+    if (rc) return rc;
+    Slot &sl = e->slots[slot];
+    if (!y || !u || !v || frame < 0 || frame >= sl.n) return fail(e, H2J_ERR_INVALID_ARG, "null plane or bad frame index %d", frame);
+    FrameDesc d = frame_desc(sl, frame);
+    if (sl.m == 1) d.base += (long long)frame * d.L.frame_stride;  // a batch of one layout at one stride
+    const FrameLayout &L = d.L;
+    const int cw = chroma_w(L.w, L.fmt), ch = chroma_h(L.h, L.fmt);
+    ON_DEVICE(e);
+    CU(e, cudaStreamSynchronize(sl.stream));
+    CU(e, cudaMemcpy2D(y, L.w, d.base, L.y_pitch, L.w, L.h, cudaMemcpyDeviceToHost));
+    if (!L.nv12) {
+        CU(e, cudaMemcpy2D(u, cw, d.base + L.u_off, L.c_pitch, cw, ch, cudaMemcpyDeviceToHost));
+        CU(e, cudaMemcpy2D(v, cw, d.base + L.v_off, L.c_pitch, cw, ch, cudaMemcpyDeviceToHost));
+        return H2J_OK;
+    }
+    // semi-planar, read in place: the rows of pairs, split here
+    std::vector<uint8_t> pairs((size_t)2 * cw * ch);
+    CU(e, cudaMemcpy2D(pairs.data(), 2 * cw, d.base + L.u_off, L.c_pitch, 2 * cw, ch, cudaMemcpyDeviceToHost));
+    for (size_t i = 0; i < (size_t)cw * ch; i++) {
+        u[i] = pairs[2 * i];
+        v[i] = pairs[2 * i + 1];
     }
     return H2J_OK;
 }

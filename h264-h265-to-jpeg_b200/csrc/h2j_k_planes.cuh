@@ -464,4 +464,119 @@ __global__ void __launch_bounds__(32 * kDownWarps, K == 2 ? 6 : 4) downscale_lis
     }
 }
 
+// ------------------------------------------------------------------------------------------------
+// RGB frames (h2j_submit_device_rgb, h2j_encode_frame_rgb) -> the planar frame C(frame) at the encoder's chroma format
+// (include/h2j_b200.h): per pixel JFIF / T.871 full-range YCbCr in libjpeg's 16-bit fixed point (jccolor.c), then Cb and Cr
+// box-averaged over 2x2 (4:2:0) or 2x1 (4:2:2) pixels, (S + c/2) / c over the c samples of a box inside the plane.
+// descs[f] is the destination (pitched_layout() in d_frames), descs[n + f] the caller's frame: rows S.y_pitch apart from its
+// base, the planar G and B planes at S.u_off / S.v_off.  K: bytes per pixel of a source row (3 or 4: packed; 1: three
+// planes).  order: the __byte_perm selector that puts a packed pixel's bytes in R, G, B order (0x3210: RGB, 0x3012: BGR).
+// grid (x, y, frames): a warp per destination row (4:2:0: per row pair, so that both luma rows and the chroma row they make
+// come from one pass over the source), kRgbRowsPerWarp of them one after the other, and a lane per 16 pixels of a row,
+// fetched with down_fetch (any alignment; nothing past a row's end is read); grid sized for the largest destination, CTAs
+// past their frame return.  Stores are aligned: rows of the destination are 16-byte aligned and hold 16 bytes from x0.
+// ------------------------------------------------------------------------------------------------
+constexpr int kRgbRowsPerWarp = 2;
+
+template <int K, int FMT>
+__global__ void __launch_bounds__(32 * kDownWarps) rgb_to_planar_kernel(const __grid_constant__ CopyTable t, unsigned order)
+{
+    static_assert(K == 1 || K == 3 || K == 4, "three planes, 3- or 4-byte pixels");
+    constexpr int kV = FMT == kFmt420 ? 2 : 1;             // luma rows per chroma row
+    constexpr int kBoxShift = FMT == kFmt420 ? 2 : 1;      // log2 of a full box (4:4:4: none)
+    const int f = blockIdx.z;
+    const FrameDesc &d = t.m > 1 ? t.descs[f] : t.d, &s = t.m > 1 ? t.descs[t.m + f] : t.s;
+    const FrameLayout &D = d.L, &S = s.L;
+    const int w = D.w, h = D.h;
+    const int x0 = (blockIdx.x * 32 + (threadIdx.x & 31)) * 16;  // the lane's first pixel
+    if (x0 >= w) return;
+    const bool inside = x0 + 16 <= w;
+    const int g0 = (blockIdx.y * kDownWarps + (threadIdx.x >> 5)) * kRgbRowsPerWarp;
+    uint8_t *const out = const_cast<uint8_t *>(d.base);
+    for (int g = g0; g < min(g0 + kRgbRowsPerWarp, (h + kV - 1) / kV); g++) {
+        const int rh = min(kV, h - kV * g);
+        unsigned cb[16], cr[16];  // 4:4:4: pixel i; otherwise the sum over box i (i < 8)
+#pragma unroll
+        for (int i = 0; i < 16; i++) cb[i] = cr[i] = 0;
+#pragma unroll
+        for (int j = 0; j < kV; j++) {
+            if (j >= rh) break;
+            const int row = kV * g + j;
+            const uint8_t *src = s.base + (long long)row * S.y_pitch;
+            unsigned wd[K == 1 ? 12 : 4 * K];  // K = 1: the R, G, B segments one after the other
+            if constexpr (K == 1) {
+                unsigned r[4], gr[4], b[4];
+                down_fetch<1>(src, x0, w, r);
+                down_fetch<1>(src + S.u_off, x0, w, gr);
+                down_fetch<1>(src + S.v_off, x0, w, b);
+#pragma unroll
+                for (int i = 0; i < 4; i++) { wd[i] = r[i]; wd[4 + i] = gr[i]; wd[8 + i] = b[i]; }
+            } else {
+                down_fetch<K>(src, K * x0, K * w, wd);
+            }
+            unsigned yw[4] = {0, 0, 0, 0};
+#pragma unroll
+            for (int i = 0; i < 16; i++) {
+                int R, G, B;
+                if constexpr (K == 1) {
+                    const int sh = 8 * (i & 3);
+                    R = (wd[i >> 2] >> sh) & 255;
+                    G = (wd[4 + (i >> 2)] >> sh) & 255;
+                    B = (wd[8 + (i >> 2)] >> sh) & 255;
+                } else {
+                    // the pixel's three bytes (K = 3: bytes o .. o + 2 of words b/4 and b/4 + 1), then in R G B order
+                    const int b = K * i, o = b & 3;
+                    unsigned px = K == 4 ? wd[i] : __byte_perm(wd[b >> 2], wd[min((b >> 2) + 1, 4 * K - 1)], o | (o + 1) << 4 | (o + 2) << 8);
+                    px = __byte_perm(px, 0, order);
+                    R = px & 255;
+                    G = (px >> 8) & 255;
+                    B = (px >> 16) & 255;
+                }
+                yw[i >> 2] |= (unsigned)((19595 * R + 38470 * G + 7471 * B + 32768) >> 16) << (8 * (i & 3));
+                // (128 << 16) + 32767 = 8421375: chroma rounds with ONE_HALF - 1; both always land in 0..255
+                const unsigned u = (unsigned)((-11059 * R - 21709 * G + 32768 * B + 8421375) >> 16);
+                const unsigned v = (unsigned)((32768 * R - 27439 * G - 5329 * B + 8421375) >> 16);
+                if constexpr (FMT == kFmt444) {
+                    cb[i] = u;
+                    cr[i] = v;
+                } else if (inside || x0 + i < w) {  // pixels past the row's end are no box's samples
+                    cb[i >> 1] += u;
+                    cr[i >> 1] += v;
+                }
+            }
+            *reinterpret_cast<uint4 *>(out + (long long)row * D.y_pitch + x0) = make_uint4(yw[0], yw[1], yw[2], yw[3]);
+        }
+        uint8_t *const ou = out + D.u_off + (long long)g * D.c_pitch, *const ov = out + D.v_off + (long long)g * D.c_pitch;
+        if constexpr (FMT == kFmt444) {
+            unsigned p[4] = {0, 0, 0, 0}, q[4] = {0, 0, 0, 0};
+#pragma unroll
+            for (int i = 0; i < 16; i++) {
+                p[i >> 2] |= cb[i] << (8 * (i & 3));
+                q[i >> 2] |= cr[i] << (8 * (i & 3));
+            }
+            *reinterpret_cast<uint4 *>(ou + x0) = make_uint4(p[0], p[1], p[2], p[3]);
+            *reinterpret_cast<uint4 *>(ov + x0) = make_uint4(q[0], q[1], q[2], q[3]);
+        } else {
+            const bool full = inside && rh == kV;
+            unsigned p[2] = {0, 0}, q[2] = {0, 0};
+#pragma unroll
+            for (int i = 0; i < 8; i++) {
+                unsigned a, b;
+                if (full) {
+                    a = (cb[i] + (1u << (kBoxShift - 1))) >> kBoxShift;
+                    b = (cr[i] + (1u << (kBoxShift - 1))) >> kBoxShift;
+                } else {
+                    const int c = min(2, w - x0 - 2 * i) * rh;  // samples of box i inside the plane
+                    a = c > 0 ? (cb[i] + (unsigned)(c >> 1)) / (unsigned)c : 0u;
+                    b = c > 0 ? (cr[i] + (unsigned)(c >> 1)) / (unsigned)c : 0u;
+                }
+                p[i >> 2] |= a << (8 * (i & 3));
+                q[i >> 2] |= b << (8 * (i & 3));
+            }
+            *reinterpret_cast<uint2 *>(ou + (x0 >> 1)) = make_uint2(p[0], p[1]);
+            *reinterpret_cast<uint2 *>(ov + (x0 >> 1)) = make_uint2(q[0], q[1]);
+        }
+    }
+}
+
 }  // namespace h2j

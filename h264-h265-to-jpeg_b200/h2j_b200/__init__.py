@@ -69,6 +69,13 @@ class Settings(C.Structure):
 LAYOUT_PLANAR = 0
 LAYOUT_SEMIPLANAR = 1
 
+# h2j_rgb_format: what submit_device_rgb / rgb2jpeg take
+RGB_RGB24 = 0   # R G B, 3 bytes per pixel (numpy / torch HWC)
+RGB_BGR24 = 1   # B G R (OpenCV)
+RGB_RGBX = 2    # R G B + one ignored byte (RGBA8)
+RGB_BGRX = 3    # B G R + one ignored byte (BGRA8)
+RGB_PLANAR = 4  # three planes R, G, B (torch CHW)
+
 
 class FrameDesc(C.Structure):
     """h2j_frame_desc: one device frame of a list submit (pitches and offsets in bytes)"""
@@ -108,7 +115,8 @@ EXPORTS = [
     "h2j_slot_kernel_ms", "h2j_set_profile", "h2j_slot_total_ms", "h2j_kernel_launches", "h2j_slot_set_stream",
     "h2j_slot_wait_event", "h2j_device_count", "h2j_debug_set_knob", "h2j_debug_read_device", "h2j_stream_copy",
     "h2j_submit_device_semiplanar16", "h2j_submit_device_pitched16", "h2j_encode_frame16", "h2j_submit_device_list",
-    "h2j_submit_host_list", "h2j_submit_device_downscaled",
+    "h2j_submit_host_list", "h2j_submit_device_downscaled", "h2j_submit_device_rgb", "h2j_encode_frame_rgb",
+    "h2j_debug_frame_planes",
 ]
 
 _lib = None
@@ -148,6 +156,9 @@ def load_library() -> C.CDLL:
     lib.h2j_submit_device_list.argtypes = [vp, ci, ci, C.POINTER(FrameDesc), ci]
     lib.h2j_submit_host_list.argtypes = [vp, ci, C.POINTER(vp), C.POINTER(ci), C.POINTER(ci), ci]
     lib.h2j_submit_device_downscaled.argtypes = [vp, ci, ci, C.POINTER(FrameDesc), ci, ci]
+    lib.h2j_submit_device_rgb.argtypes = [vp, ci, ci, C.POINTER(FrameDesc), ci]
+    lib.h2j_encode_frame_rgb.argtypes = [vp, ci, C.POINTER(vp), C.POINTER(ci), ci, ci, vp, sz, C.POINTER(sz)]
+    lib.h2j_debug_frame_planes.argtypes = [vp, ci, ci, vp, vp, vp]
     lib.h2j_collect.argtypes = [vp, ci, vp, sz, C.POINTER(sz), C.POINTER(ci)]
     lib.h2j_collect_device.argtypes = [vp, ci, C.POINTER(vp), C.POINTER(sz), C.POINTER(sz), C.POINTER(ci)]
     lib.h2j_wait.argtypes = [vp, ci]
@@ -355,6 +366,28 @@ class Encoder:
         self._check(self._lib.h2j_encode_frame16(self._h, planes, strides, bit_depth, w, h, out.ctypes.data, out.size, C.byref(n)))
         return out[: n.value].tobytes()
 
+    def rgb2jpeg(self, image, fmt: int) -> bytes:
+        """One RGB picture in host memory -> JPEG bytes (h2j_encode_frame_rgb).  Packed formats: a uint8 (H, W, 3) array
+        (RGB_RGB24, RGB_BGR24) or (H, W, 4) (RGB_RGBX, RGB_BGRX) whose pixels are contiguous, at any row stride.
+        RGB_PLANAR: a (3, H, W) uint8 array or three 2-D uint8 planes R, G, B, each with contiguous rows."""
+        if fmt == RGB_PLANAR:
+            planes = list(image)
+            if len(planes) != 3 or any(p.dtype != np.uint8 or p.ndim != 2 or p.strides[1] != 1 or p.shape != planes[0].shape for p in planes):
+                raise H2JError(ERR_INVALID_ARG, "planar RGB is three 2-D uint8 planes of one shape with contiguous rows")
+            h, w = planes[0].shape
+        else:
+            bpp = 4 if fmt in (RGB_RGBX, RGB_BGRX) else 3
+            if image.dtype != np.uint8 or image.ndim != 3 or image.shape[2] != bpp or image.strides[1:] != (bpp, 1):
+                raise H2JError(ERR_INVALID_ARG, f"packed RGB is a uint8 (H, W, {bpp}) array with contiguous pixels")
+            h, w = image.shape[:2]
+            planes = [image] * 3
+        ptrs = (C.c_void_p * 3)(*[p.ctypes.data for p in planes])
+        strides = (C.c_int * 3)(*[p.strides[0] for p in planes])
+        out = np.empty(self.out_capacity, np.uint8)
+        n = C.c_size_t(0)
+        self._check(self._lib.h2j_encode_frame_rgb(self._h, fmt, ptrs, strides, w, h, out.ctypes.data, out.size, C.byref(n)))
+        return out[: n.value].tobytes()
+
     def yuv2jpeg_into(self, y: np.ndarray, u: np.ndarray, v: np.ndarray, out: Optional[np.ndarray] = None) -> int:
         """Same call, JPEG bytes into a caller buffer (or a buffer kept by this object: ``self.last_out``); returns the
         size.  Nothing is allocated per call -- the form to time."""
@@ -425,6 +458,14 @@ class Encoder:
         (downscaled_size); only the downscaled frames must fit the encoder's maximum."""
         arr = (FrameDesc * max(1, len(descs)))(*descs)
         self._check(self._lib.h2j_submit_device_downscaled(self._h, slot, layout, arr, len(descs), factor))
+        self._n_in_slot[slot] = len(descs)
+
+    def submit_device_rgb(self, slot: int, fmt: int, descs: Sequence[FrameDesc]) -> None:
+        """RGB device frames (an RGB_* format for all), each at its own address and of its own size: packed formats use
+        data, width, height and y_pitch; RGB_PLANAR has G at data + u_offset and B at data + v_offset, rows y_pitch apart.
+        A (3, H, W) CUDA tensor t is FrameDesc(t.data_ptr(), W, H, t.stride(1), 0, t.stride(0), 2 * t.stride(0))."""
+        arr = (FrameDesc * max(1, len(descs)))(*descs)
+        self._check(self._lib.h2j_submit_device_rgb(self._h, slot, fmt, arr, len(descs)))
         self._n_in_slot[slot] = len(descs)
 
     def submit_host_list(self, slot: int, frames: Sequence[int], sizes: Sequence[Tuple[int, int]]) -> None:
@@ -522,6 +563,21 @@ class Encoder:
         out = np.empty((n_blocks, 64), np.int16)
         self._check(self._lib.h2j_debug_coefficients(self._h, slot, frame, out.ctypes.data, out.size))
         return out
+
+    def frame_planes(self, slot: int, frame: int, width: int, height: int) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """(y, u, v) of frame `frame` of the slot's last batch as the pipeline read it (h2j_debug_frame_planes); width x
+        height is that frame's size as encoded (a downscaled frame's: downscaled_size)."""
+        # the hook writes the frame's own size: buffers large enough for any frame of the MCU geometry the slot reports
+        info = self.frame_info(slot, frame)
+        mcu_px = 8 if self.chroma_format == CHROMA_444 else 16
+        if (info.mcu_w, info.mcu_h) != (-(-width // mcu_px), -(-height // 16)):
+            raise H2JError(ERR_INVALID_ARG, f"frame {frame} of slot {slot} is not {width}x{height}")
+        bw, bh = info.mcu_w * mcu_px, info.mcu_h * 16
+        bch, bcw = chroma_shape(bw, bh, self.chroma_format)
+        y, u, v = np.empty(bw * bh, np.uint8), np.empty(bch * bcw, np.uint8), np.empty(bch * bcw, np.uint8)
+        self._check(self._lib.h2j_debug_frame_planes(self._h, slot, frame, y.ctypes.data, u.ctypes.data, v.ctypes.data))
+        ch, cw = chroma_shape(width, height, self.chroma_format)
+        return y[: width * height].reshape(height, width), u[: cw * ch].reshape(ch, cw), v[: cw * ch].reshape(ch, cw)
 
     def kernel_ms(self, slot: int) -> List[Tuple[str, float]]:
         names = (C.c_char_p * 32)()

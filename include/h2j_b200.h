@@ -257,6 +257,54 @@ int h2j_submit_host_list(h2j_encoder *e, int slot, const uint8_t *const *frames,
  */
 int h2j_submit_device_downscaled(h2j_encoder *e, int slot, int layout, const h2j_frame_desc *frames, int n, int factor);
 
+/*
+ * RGB frames: torch tensors ((3, H, W) planar as torchvision.io.encode_jpeg takes them, or (H, W, 3)), model outputs and
+ * annotated frames, rendered RGBA8 surfaces, a hardware decoder's BGRA post-processing output, OpenCV / numpy images.
+ * Frame i's JPEG is byte-identical to the one h2j_submit_device writes, with the same fixed_qscale and chroma_format, for
+ * the planar frame C(frame i) built in two steps:
+ *   1. per pixel, JFIF / ITU-T T.871 full-range YCbCr in libjpeg's integer form (jccolor.c: 16 fraction bits,
+ *      FIX(x) = (int)(x * 65536 + 0.5), chroma rounded with ONE_HALF - 1):
+ *        Y  = ( 19595 R + 38470 G +  7471 B + 32768)              >> 16
+ *        Cb = (-11059 R - 21709 G + 32768 B + (128 << 16) + 32767) >> 16
+ *        Cr = ( 32768 R - 27439 G -  5329 B + (128 << 16) + 32767) >> 16
+ *      Every result lies in 0..255 (no clamp), and it is within 1 of the float T.871 formula rounded half up.  T.871 is the
+ *      only matrix: the JPEG carries component ids 1, 2, 3 and no JFIF or Adobe marker, which every decoder reads as T.871
+ *      YCbCr, so no other matrix would decode back to the caller's colours.
+ *   2. at 4:2:0 / 4:2:2, the 8-bit Cb and Cr planes are box-averaged over 2x2 / 2x1 pixels to the encoder's usual chroma
+ *      sizes (ceil(w/2) x ceil(h/2), ceil(w/2) x h; 4:4:4: w x h, no averaging): out = (S + c/2) / c in integers (rounded
+ *      half up), S the sum of the c samples of the box that lie inside the plane (fewer than the box's at the right and
+ *      bottom edges), as for D_k above.
+ * range_mode does not apply: the YCbCr of an RGB frame is full range by construction, and an encoder created with
+ * H2J_RANGE_LIMITED_TO_FULL writes the same RGB JPEGs as one created with H2J_RANGE_PASSTHROUGH.  Alpha / X bytes never
+ * reach the picture.
+ *
+ * h2j_submit_device_rgb: n device frames, each of its own size (at most max_width x max_height) at its own address, with
+ *   any alignment, described by h2j_frame_desc: packed formats use data, width, height and y_pitch (bytes between rows);
+ *   H2J_RGB_PLANAR has the R plane at data, G at data + u_offset and B at data + v_offset, every plane's rows y_pitch
+ *   apart.  Other fields are ignored.  One kernel converts the frames into the slot's own frame buffer, then the usual
+ *   pipeline runs (frames of one size run its batch form, others its list form).  Collect with h2j_collect /
+ *   h2j_collect_device; the device frames are read on the slot's stream, under the stream-ordering rule above.
+ * h2j_encode_frame_rgb: one picture from host memory, synchronously on slot 0, as h2j_encode_frame: packed formats take
+ *   planes[0] / strides[0] only, H2J_RGB_PLANAR the R, G and B planes with their own strides.  The picture is staged on
+ *   the device at a 16-byte aligned pitch in a buffer h2j_encode_frame16 shares, allocated on first use and grown when a
+ *   call needs more (H2J_ERR_NOMEM if that fails; the encoder stays usable), freed by h2j_destroy.
+ * H2J_ERR_INVALID_ARG: as h2j_submit_device_list, a bad format, a null data pointer, a pitch or stride shorter than a row
+ * (3w, 4w or w bytes), or a planar G or B plane that starts inside the R plane (offset < y_pitch * height).
+ * H2J_ERR_UNSUPPORTED: a size outside 2..65500 or above the encoder's maximum.  H2J_ERR_BUSY: the slot has a batch in
+ * flight.  Every frame is checked before anything is enqueued: a rejected call leaves the previous batch as it was.
+ */
+typedef enum h2j_rgb_format {
+    H2J_RGB_RGB24 = 0,   /* R G B, 3 bytes per pixel (numpy / torch HWC) */
+    H2J_RGB_BGR24 = 1,   /* B G R (OpenCV) */
+    H2J_RGB_RGBX = 2,    /* R G B + one ignored byte (RGBA8) */
+    H2J_RGB_BGRX = 3,    /* B G R + one ignored byte (BGRA8) */
+    H2J_RGB_PLANAR = 4   /* three planes R, G, B (torch CHW) */
+} h2j_rgb_format;
+
+int h2j_submit_device_rgb(h2j_encoder *e, int slot, int format, const h2j_frame_desc *frames, int n);
+int h2j_encode_frame_rgb(h2j_encoder *e, int format, const uint8_t *const planes[3], const int strides[3], int width,
+                         int height, uint8_t *out, size_t out_capacity, size_t *out_size);
+
 int h2j_collect(h2j_encoder *e, int slot, uint8_t *out, size_t out_capacity, size_t *offsets, int *status);
 int h2j_collect_device(h2j_encoder *e, int slot, const uint8_t **d_out, size_t *d_frame_capacity, size_t *sizes,
                        int *status);
@@ -304,6 +352,12 @@ int h2j_debug_frame_info(h2j_encoder *e, int slot, int frame, h2j_frame_info *in
 /* Quantised levels of one frame: mcu_w*mcu_h*6 blocks in MCU order (Y0 Y1 Y2 Y3 Cb Cr), 64 int16 each in
  * zigzag order (index 0 = quantised DC level, not the difference). */
 int h2j_debug_coefficients(h2j_encoder *e, int slot, int frame, int16_t *out, size_t out_elems);
+/* Frame `frame` of the slot's last batch as the pipeline read it (before range_mode's mapping), copied to tight host
+ * planes: Y width x height, U and V at the frame's chroma size (ceil-divided by the chroma format's subsampling).  A frame
+ * the input stage wrote (RGB, 16-bit, downscaled, split or repitched) is read from the slot's buffer; a frame read in place
+ * from the caller's memory, which must still hold it (semi-planar pairs are split on the host).  Same validity as above:
+ * JPEG byte equality can hide a one-off sample behind quantisation, these planes cannot. */
+int h2j_debug_frame_planes(h2j_encoder *e, int slot, int frame, uint8_t *y, uint8_t *u, uint8_t *v);
 
 /* Synchronous copy of `bytes` bytes of device memory on the encoder's device (e.g. a JPEG reported by h2j_collect_device)
  * to host memory: lets callers without a CUDA binding of their own look at device-resident results. */
