@@ -8,7 +8,9 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <map>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "h2j_kernels.cuh"
@@ -59,6 +61,12 @@ struct Slot {
     uint8_t *d_convert = nullptr;
     uint8_t *h_convert = nullptr;
     size_t convert_bytes = 0;
+    // h2j_submit_device_resized: the batch's coefficient arena (ResizeFrame per frame, then the axes' windows and
+    // coefficients) and its pinned mirror, allocated on first use and grown when a submit needs more; resize_used bytes of it
+    // are uploaded with one copy on the slot's stream (the busy-slot rule keeps the mirror as it is while that copy is pending)
+    uint8_t *d_resize = nullptr;
+    uint8_t *h_resize = nullptr;
+    size_t resize_bytes = 0, resize_used = 0;
     unsigned char *h_tail = nullptr;          // pinned: status .. jpeg_bytes of frame 0's FrameTab (h2j_encode_frame)
     size_t spec_bytes = 384 * 1024;           // JPEG bytes h2j_encode_frame copies back before it knows the size
     bool busy = false;
@@ -588,9 +596,11 @@ void free_slot(Slot &sl)
     cudaFree(sl.d_frames); cudaFree(sl.d_pitched); cudaFree(sl.d_images); cudaFree(sl.d_zero); cudaFree(sl.d_stage); cudaFree(sl.d_unit_info);
     cudaFree(sl.d_tabs); cudaFree(sl.d_scan); cudaFree(sl.d_out); cudaFree(sl.d_packed); cudaFree(sl.d_offsets); cudaFree(sl.d_status);
     cudaFree(sl.d_convert);
+    cudaFree(sl.d_resize);
     cudaFree(sl.d_desc);
     if (sl.h_desc) cudaFreeHost(sl.h_desc);
     if (sl.h_convert) cudaFreeHost(sl.h_convert);
+    if (sl.h_resize) cudaFreeHost(sl.h_resize);
     if (sl.h_offsets) cudaFreeHost(sl.h_offsets);
     if (sl.h_status) cudaFreeHost(sl.h_status);
     if (sl.h_sizes) cudaFreeHost(sl.h_sizes);
@@ -671,6 +681,7 @@ struct Input {
     int bit_depth = 8;  // 9 .. 16: 16-bit words, converted to 8-bit planar frames
     int factor = 1;     // 2, 4, 8: box-filtered to 1/factor
     int rgb = -1;       // an h2j_rgb_format: RGB pixels, converted to YCbCr planar frames
+    int filter = -1;    // an h2j_resize_filter: resized by the coefficient tables of the slot's arena (ResizeFrame)
 };
 
 // the rgb_to_planar_kernel instantiation for an h2j_rgb_format and a chroma format
@@ -701,7 +712,7 @@ int run_batch(h2j_encoder *e, Slot &sl, int n, int m, const Input &in, int tail)
 {
     FrameDesc *D = sl.h_desc, *S = sl.h_desc + m;
     const int fmt = e->s.chroma_format;
-    const bool convert = in.bit_depth > 8 || in.factor > 1 || in.rgb >= 0;
+    const bool convert = in.bit_depth > 8 || in.factor > 1 || in.rgb >= 0 || in.filter >= 0;
     bool unaligned = false;
     for (int i = 0; i < m; i++) unaligned = unaligned || !S[i].L.aligned8;
     const bool split = in.sp && (unaligned || e->force_sp_prepass);
@@ -724,6 +735,11 @@ int run_batch(h2j_encoder *e, Slot &sl, int n, int m, const Input &in, int tail)
         D[i].L.frame_stride = (long long)spacing;
         D[i].base = (convert || in.sp ? sl.d_frames : sl.d_pitched) + (size_t)i * spacing;
         const int w = D[i].L.w, h = D[i].L.h;
+        if (in.filter >= 0) {  // bands of output rows of every plane
+            cols = std::max(cols, (w + kResizeCols - 1) / kResizeCols);
+            rows = std::max(rows, (h + kResizeRows - 1) / kResizeRows + 2 * ((chroma_h(h, fmt) + kResizeRows - 1) / kResizeRows));
+            continue;
+        }
         if (in.rgb >= 0) {
             cols = std::max(cols, (w + 15) / 16);
             rows = std::max(rows, fmt == kFmt420 ? (h + 1) / 2 : h);
@@ -737,6 +753,7 @@ int run_batch(h2j_encoder *e, Slot &sl, int n, int m, const Input &in, int tail)
     long long stride;
     if (m > 1 && (rows || !batch_stride(sl, &stride)))  // (a table of one pair goes to the copy kernel by value)
         CU(e, cudaMemcpyAsync(sl.d_desc, sl.h_desc, sizeof(FrameDesc) * (rows ? 2 * m : m), cudaMemcpyHostToDevice, sl.stream));
+    if (in.filter >= 0) CU(e, cudaMemcpyAsync(sl.d_resize, sl.h_resize, sl.resize_used, cudaMemcpyHostToDevice, sl.stream));
     if (rows) {
         static_assert(32 * kDownWarps == 128, "every copy kernel runs CTAs of 128 threads");
         const bool warp_rows = in.factor > 1 || in.rgb >= 0;  // a warp per row, a lane per 16 bytes or pixels of it
@@ -748,6 +765,9 @@ int run_batch(h2j_encoder *e, Slot &sl, int n, int m, const Input &in, int tail)
         else if (in.factor == 8) k = in.sp ? downscale_list_kernel<8, true> : downscale_list_kernel<8, false>;
         const CopyTable t{sl.d_desc, m, D[0], S[0]};
         if (in.bit_depth > 8) (in.sp ? depth_to_8_kernel<true> : depth_to_8_kernel<false>)<<<grid, 128, 0, sl.stream>>>(t, in.bit_depth - 8);
+        else if (in.filter >= 0)
+            (in.sp ? resize_list_kernel<true> : resize_list_kernel<false>)<<<dim3(cols, rows, n), kResizeCols, 0, sl.stream>>>(
+                t, reinterpret_cast<const ResizeFrame *>(sl.d_resize));
         else if (in.rgb >= 0)
             rgb_kernel(in.rgb, fmt)<<<grid, 128, 0, sl.stream>>>(t, in.rgb == H2J_RGB_BGR24 || in.rgb == H2J_RGB_BGRX ? 0x3012u : 0x3210u);
         else k<<<grid, 128, 0, sl.stream>>>(t);
@@ -760,25 +780,30 @@ int run_batch(h2j_encoder *e, Slot &sl, int n, int m, const Input &in, int tail)
     return H2J_OK;
 }
 
-// slot 0's buffers of the converting single-picture calls hold at least `bytes` (grown if not): H2J_ERR_NOMEM, with none
-// held, when they cannot be had
+// A device buffer and its pinned mirror of a slot (the converting single-picture calls' staging, the resize arena) hold at
+// least `bytes` (grown if not): H2J_ERR_NOMEM, with none held, when they cannot be had.  The device buffer is asked for
+// first, so a request larger than the device pins no host memory.
+int reserve_mirrored(h2j_encoder *e, uint8_t *&d, uint8_t *&h, size_t &cap, size_t bytes, const char *what)
+{
+    if (bytes <= cap) return H2J_OK;
+    cudaFree(d);
+    if (h) cudaFreeHost(h);
+    d = nullptr;
+    h = nullptr;
+    cap = 0;
+    if (cudaMalloc(&d, bytes) != cudaSuccess || cudaHostAlloc(&h, bytes, cudaHostAllocDefault) != cudaSuccess) {
+        cudaGetLastError();
+        cudaFree(d);
+        d = nullptr;
+        h = nullptr;
+        return fail(e, H2J_ERR_NOMEM, "no room for the %zu-byte %s", bytes, what);
+    }
+    cap = bytes;
+    return H2J_OK;
+}
 int reserve_convert(h2j_encoder *e, Slot &sl, size_t bytes)
 {
-    if (bytes <= sl.convert_bytes) return H2J_OK;
-    cudaFree(sl.d_convert);
-    if (sl.h_convert) cudaFreeHost(sl.h_convert);
-    sl.d_convert = nullptr;
-    sl.h_convert = nullptr;
-    sl.convert_bytes = 0;
-    if (cudaMalloc(&sl.d_convert, bytes) != cudaSuccess || cudaHostAlloc(&sl.h_convert, bytes, cudaHostAllocDefault) != cudaSuccess) {
-        cudaGetLastError();
-        cudaFree(sl.d_convert);
-        sl.d_convert = nullptr;
-        sl.h_convert = nullptr;
-        return fail(e, H2J_ERR_NOMEM, "no room for the %zu-byte staging of a picture to convert", bytes);
-    }
-    sl.convert_bytes = bytes;
-    return H2J_OK;
+    return reserve_mirrored(e, sl.d_convert, sl.h_convert, sl.convert_bytes, bytes, "staging of a picture to convert");
 }
 
 // bytes of a row of w pixels of an h2j_rgb_format (planar: of each plane); 0 for a bad format
@@ -814,6 +839,104 @@ int rgb_frame_layout(h2j_encoder *e, int i, int n, int format, const h2j_frame_d
     s.L.v_off = planar ? (long long)F.v_offset : 0;
     s.base = F.data;
     s.extent = (long long)((planar ? std::max(F.u_offset, F.v_offset) : 0) + (size_t)F.y_pitch * (F.height - 1) + row);
+    return H2J_OK;
+}
+
+// ---- h2j_submit_device_resized: Pillow's coefficients (libImaging/Resample.c precompute_coeffs, normalize_coeffs_8bpc) ----
+// Built on the host in double, with Pillow's operations in Pillow's order.  This file's host code is compiled by g++ without
+// -march, which emits no FMA on x86-64: a contracted multiply-add (as nvcc makes of device code) would change the weights.
+double resize_filter(int filter, double x)
+{
+    if (filter == H2J_FILTER_BOX) return x > -0.5 && x <= 0.5 ? 1.0 : 0.0;
+    if (x < 0.0) x = -x;
+    if (filter == H2J_FILTER_BILINEAR) return x < 1.0 ? 1.0 - x : 0.0;
+    const double a = -0.5;
+    if (x < 1.0) return ((a + 2.0) * x - (a + 3.0)) * x * x + 1;
+    if (x < 2.0) return (((x - 5) * x + 8) * x - 4) * a;
+    return 0.0;
+}
+
+// One axis, in to out samples: win[o] = {first source sample, taps, first coefficient in coef} for every output o, and the
+// taps' coefficients in 22-bit fixed point.  in == out: the identity (Pillow skips the pass; one tap of 1 << 22 gives the
+// sample back).  win null: only counts.  Returns the number of coefficients.
+long long resize_axis(int filter, int in, int out, int4 *win, int *coef)
+{
+    const double scale = (double)in / out;
+    const double fs = scale < 1.0 ? 1.0 : scale;
+    const double support = (filter == H2J_FILTER_BOX ? 0.5 : filter == H2J_FILTER_BILINEAR ? 1.0 : 2.0) * fs;
+    std::vector<double> w;
+    long long k = 0;
+    for (int o = 0; o < out; o++) {
+        if (in == out) {
+            if (win) {
+                win[o] = make_int4(o, 1, o, 0);
+                coef[o] = 1 << kResizeBits;
+            }
+            k++;
+            continue;
+        }
+        const double center = (o + 0.5) * scale;
+        const double ss = 1.0 / fs;
+        int xmin = (int)(center - support + 0.5);
+        if (xmin < 0) xmin = 0;
+        int xmax = (int)(center + support + 0.5);
+        if (xmax > in) xmax = in;
+        const int n = xmax - xmin;
+        if (win) {
+            w.resize(n);
+            double ww = 0.0;
+            for (int x = 0; x < n; x++) {
+                w[x] = resize_filter(filter, (x + xmin - center + 0.5) * ss);
+                ww += w[x];
+            }
+            for (int x = 0; x < n; x++) {
+                if (ww != 0.0) w[x] /= ww;
+                coef[k + x] = w[x] < 0 ? (int)(-0.5 + w[x] * (1 << kResizeBits)) : (int)(0.5 + w[x] * (1 << kResizeBits));
+            }
+            win[o] = make_int4(xmin, n, (int)k, 0);
+        }
+        k += n;
+    }
+    return k;
+}
+
+// The arena of a resized batch: a ResizeFrame per frame, then per distinct (in, out) axis its windows, then its
+// coefficients.  axes[f * 4 + a] is frame f's axis a (luma x, luma y, chroma x, chroma y) as {in, out}.
+struct ResizeAxis {
+    int in, out;
+    size_t win_off, coef_off;  // bytes into the arena
+};
+int build_resize_arena(h2j_encoder *e, Slot &sl, int n, int filter, const std::vector<std::pair<int, int>> &axes)
+{
+    std::vector<ResizeAxis> uniq;
+    std::vector<int> which(axes.size());
+    std::map<std::pair<int, int>, int> seen;
+    size_t bytes = align_up(sizeof(ResizeFrame) * n, 16);
+    for (size_t a = 0; a < axes.size(); a++) {
+        auto it = seen.find(axes[a]);
+        if (it == seen.end()) {
+            it = seen.emplace(axes[a], (int)uniq.size()).first;
+            uniq.push_back(ResizeAxis{axes[a].first, axes[a].second, 0, 0});
+        }
+        which[a] = it->second;
+    }
+    for (ResizeAxis &x : uniq) {
+        x.win_off = bytes;
+        x.coef_off = bytes + sizeof(int4) * x.out;
+        bytes = align_up(x.coef_off + sizeof(int) * resize_axis(filter, x.in, x.out, nullptr, nullptr), 16);
+    }
+    int rc = reserve_mirrored(e, sl.d_resize, sl.h_resize, sl.resize_bytes, bytes, "coefficient tables of a resized batch");
+    if (rc) return rc;
+    sl.resize_used = bytes;
+    for (const ResizeAxis &x : uniq)
+        resize_axis(filter, x.in, x.out, reinterpret_cast<int4 *>(sl.h_resize + x.win_off), reinterpret_cast<int *>(sl.h_resize + x.coef_off));
+    ResizeFrame *rf = reinterpret_cast<ResizeFrame *>(sl.h_resize);
+    for (int f = 0; f < n; f++)
+        for (int a = 0; a < 4; a++) {
+            const ResizeAxis &x = uniq[which[(size_t)f * 4 + a]];
+            rf[f].win[a] = reinterpret_cast<const int4 *>(sl.d_resize + x.win_off);
+            rf[f].coef[a] = reinterpret_cast<const int *>(sl.d_resize + x.coef_off);
+        }
     return H2J_OK;
 }
 
@@ -1147,6 +1270,46 @@ int h2j_submit_device_downscaled(h2j_encoder *e, int slot, int layout, const h2j
     ON_DEVICE(e);
     CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
     return run_batch(e, sl, n, n, Input{sp, 8, factor}, TAIL_SIZES);
+}
+
+int h2j_submit_device_resized(h2j_encoder *e, int slot, int layout, const h2j_frame_desc *frames, int n, const int *out_widths,
+                              const int *out_heights, int filter)
+{
+    int rc = check_device_list(e, slot, layout, frames, n);
+    if (rc) return rc;
+    if (!out_widths || !out_heights) return fail(e, H2J_ERR_INVALID_ARG, "null out_widths / out_heights");
+    if (filter != H2J_FILTER_BOX && filter != H2J_FILTER_BILINEAR && filter != H2J_FILTER_BICUBIC)
+        return fail(e, H2J_ERR_INVALID_ARG, "bad resize filter %d", filter);
+    Slot &sl = e->slots[slot];
+    const bool sp = layout == H2J_LAYOUT_SEMIPLANAR;
+    const int fmt = e->s.chroma_format;
+    // tab[i]: the resized frame the pipeline encodes, tab[n + i]: the caller's frame.  Only the output size is held to the
+    // encoder's maximum.
+    std::vector<FrameDesc> tab(2 * (size_t)n);
+    std::vector<std::pair<int, int>> axes(4 * (size_t)n);
+    for (int i = 0; i < n; i++) {
+        const h2j_frame_desc &F = frames[i];
+        FrameDesc &src = tab[n + i];
+        rc = device_frame_layout(e, i, F, sp, 1, false, &src.L, &src.extent);
+        if (rc) return rc;
+        src.base = F.data;
+        const int w = out_widths[i], h = out_heights[i];
+        rc = make_layout(e, nullptr, w, h, &tab[i].L);
+        if (rc) return rc;
+        axes[4 * i] = {F.width, w};
+        axes[4 * i + 1] = {F.height, h};
+        axes[4 * i + 2] = {chroma_w(F.width, fmt), chroma_w(w, fmt)};
+        axes[4 * i + 3] = {chroma_h(F.height, fmt), chroma_h(h, fmt)};
+    }
+    ON_DEVICE(e);
+    rc = build_resize_arena(e, sl, n, filter, axes);
+    if (rc) return rc;
+    memcpy(sl.h_desc, tab.data(), sizeof(FrameDesc) * 2 * n);
+    CU(e, cudaEventRecord(sl.ev_begin, sl.stream));
+    Input in;
+    in.sp = sp;
+    in.filter = filter;
+    return run_batch(e, sl, n, n, in, TAIL_SIZES);
 }
 
 int h2j_submit_device_rgb(h2j_encoder *e, int slot, int format, const h2j_frame_desc *frames, int n)

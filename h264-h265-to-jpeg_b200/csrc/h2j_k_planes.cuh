@@ -579,4 +579,129 @@ __global__ void __launch_bounds__(32 * kDownWarps) rgb_to_planar_kernel(const __
     }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Resized frames (h2j_submit_device_resized): every plane of the caller's frame, at its decoder size, resized to the matching
+// plane of the W x H frame by Pillow's two-pass convolution (include/h2j_b200.h): a horizontal pass over every source row
+// the plane's output needs, clipped to 8 bits, then a vertical pass over those 8-bit rows, both in 22-bit fixed point with a
+// 32-bit sum.  The host builds the coefficients (an axis that keeps its size gets the identity: one tap of 1 << 22, which
+// gives back the sample, as Pillow's skipped pass does).  descs[f] is the destination (pitched_layout() in d_frames),
+// descs[n + f] the caller's frame (SP: the pair plane at u_off, component c of pair x at byte 2x + c).
+// grid (x, y, frames): a CTA owns kResizeCols output columns (a thread per column) by kResizeRows output rows of one plane
+// (y: the luma bands, then Cb's, then Cr's), grid sized for the largest frame, CTAs past their frame's planes return.  It
+// streams the source rows its band's vertical windows cover, in order, kResizeGroup at a time: the span of source samples the
+// tile's horizontal windows cover is staged in shared memory (16-byte loads where a chunk lies inside the span, bytes at the
+// cut ends: nothing outside a row's samples is read), each thread runs its column's horizontal window over it and keeps the
+// 8-bit results in its own column of s_h, then adds k_v * value over the part of every output row's vertical window that
+// lies in the group into that row's 32-bit sum (registers): only the taps, no test per (row, source row).  A span wider
+// than the staging buffer is staged one row at a time, in pieces.
+// ------------------------------------------------------------------------------------------------
+constexpr int kResizeCols = 128;
+constexpr int kResizeRows = 16;
+constexpr int kResizeGroup = 16;          // source rows staged at once, when their spans fit
+constexpr int kResizeStage = 16384;       // bytes of staged spans
+constexpr int kResizeBits = 22;           // Pillow's PRECISION_BITS
+
+// a frame's coefficient tables in the slot's arena: per output sample of an axis {first source sample, taps, first
+// coefficient}, and the axis's coefficients.  Axes: luma x, luma y, chroma x, chroma y.
+struct ResizeFrame {
+    const int4 *win[4];
+    const int *coef[4];
+};
+
+template <bool SP>
+__global__ void __launch_bounds__(kResizeCols, 4) resize_list_kernel(const __grid_constant__ CopyTable t, const ResizeFrame *__restrict__ frames)
+{
+    __shared__ __align__(16) uint8_t s_stage[kResizeStage];
+    __shared__ int4 s_win[kResizeRows];  // the band's vertical windows
+    __shared__ uint8_t s_h[kResizeGroup][kResizeCols];  // the group's horizontal results, a column per thread
+    const int f = blockIdx.z;
+    const FrameDesc &d = t.m > 1 ? t.descs[f] : t.d, &s = t.m > 1 ? t.descs[t.m + f] : t.s;
+    const FrameLayout &D = d.L, &S = s.L;
+    const int hs = fmt_hshift(S.fmt), vs = fmt_vshift(S.fmt);
+    const int dcw = (D.w + (1 << hs) - 1) >> hs, dch = (D.h + (1 << vs) - 1) >> vs;  // output chroma plane
+    const int luma_bands = (D.h + kResizeRows - 1) / kResizeRows, chroma_bands = (dch + kResizeRows - 1) / kResizeRows;
+    int band = blockIdx.y, plane = 0;
+    if (band >= luma_bands) {
+        band -= luma_bands;
+        plane = band >= chroma_bands ? 2 : 1;
+        if (plane == 2) band -= chroma_bands;
+        if (band >= chroma_bands) return;
+    }
+    const int ow = plane ? dcw : D.w, oh = plane ? dch : D.h;
+    const int c0 = blockIdx.x * kResizeCols, r0 = band * kResizeRows;
+    if (c0 >= ow) return;
+    const int nr = min(kResizeRows, oh - r0);
+    const bool pairs = SP && plane;
+    const int step = pairs ? 2 : 1, comp = pairs ? plane - 1 : 0;  // bytes per sample of a row; this component's byte
+    const uint8_t *src = s.base + (plane == 0 ? 0 : plane == 1 ? S.u_off : S.v_off) + comp;
+    const int spitch = plane ? S.c_pitch : S.y_pitch;
+    const ResizeFrame &rf = frames[f];
+    const int4 *xwin = rf.win[plane ? 2 : 0];
+    const int *xk = rf.coef[plane ? 2 : 0], *yk = rf.coef[plane ? 3 : 1];
+    if (threadIdx.x < kResizeRows) s_win[threadIdx.x] = threadIdx.x < nr ? rf.win[plane ? 3 : 1][r0 + threadIdx.x] : make_int4(0, 0, 0, 0);
+    const int o = c0 + threadIdx.x;
+    const bool active = o < ow;
+    const int4 w = active ? xwin[o] : make_int4(0, 0, 0, 0);
+    const int xa = xwin[c0].x;  // the tile's span of source samples: windows move right with the output sample
+    const int4 wl = xwin[min(c0 + kResizeCols, ow) - 1];
+    const int xb = wl.x + wl.y;
+    __syncthreads();
+    const int ja = s_win[0].x, jb = s_win[nr - 1].x + s_win[nr - 1].y;
+    // a piece of a row's span: at most the staging buffer (with the cut of its first chunk); as many rows of pieces as fit
+    const int piece = min(xb - xa, (kResizeStage - 16) / step - 1);
+    const int spitch_s = (piece * step + 31) & ~15;  // staged bytes per row: whole chunks from the 16-byte boundary below
+    const int group = piece < xb - xa ? 1 : min(kResizeGroup, kResizeStage / spitch_s);
+    const int chunks = spitch_s >> 4;
+    int acc[kResizeRows];
+#pragma unroll
+    for (int r = 0; r < kResizeRows; r++) acc[r] = 1 << (kResizeBits - 1);
+    int h = 1 << (kResizeBits - 1);  // a row staged in pieces (group 1): its horizontal sum so far
+    for (int j = ja; j < jb; j += group) {
+        const int g_n = min(group, jb - j);
+        for (int p0 = xa; p0 < xb; p0 += piece) {
+            const int p1 = min(xb, p0 + piece);
+            for (int c = threadIdx.x; c < g_n * chunks; c += kResizeCols) {
+                const int g = c / chunks, k = c - g * chunks;
+                const uint8_t *g0 = src + (long long)(j + g) * spitch + (long long)p0 * step, *g1 = g0 + (long long)(p1 - p0 - 1) * step + 1;
+                const uint8_t *q = reinterpret_cast<const uint8_t *>((uintptr_t)g0 & ~(uintptr_t)15) + 16 * k;
+                uint8_t *st = s_stage + g * spitch_s + 16 * k;
+                if (q >= g0 && q + 16 <= g1) *reinterpret_cast<uint4 *>(st) = ldg128(q);
+                else if (q < g1)
+                    for (int b = 0; b < 16; b++)
+                        if (q + b >= g0 && q + b < g1) st[b] = q[b];
+            }
+            __syncthreads();
+            for (int g = 0; g < g_n; g++) {
+                const int row = j + g;
+                int sum = p0 == xa ? 1 << (kResizeBits - 1) : h;
+                if (active) {
+                    const int cut = (int)((uintptr_t)(src + (long long)row * spitch + (long long)p0 * step) & 15u);
+                    const uint8_t *sp = s_stage + g * spitch_s + cut + (w.x - p0) * step;
+                    const int *kp = xk + w.z;
+                    const int t1 = min(w.y, p1 - w.x);
+                    for (int tt = max(0, p0 - w.x); tt < t1; tt++) sum += (int)sp[tt * step] * __ldg(kp + tt);
+                }
+                if (p1 < xb) h = sum;
+                else s_h[g][threadIdx.x] = (uint8_t)min(max(sum >> kResizeBits, 0), 255);
+            }
+            if (p1 == xb) {
+#pragma unroll
+                for (int r = 0; r < kResizeRows; r++) {
+                    const int4 yw = s_win[r];  // (rows past the band: an empty window)
+                    const int lo = max(yw.x, j), hi = min(yw.x + yw.y, j + g_n);
+                    const int *kp = yk + yw.z - yw.x;
+                    for (int row = lo; row < hi; row++) acc[r] += (int)s_h[row - j][threadIdx.x] * __ldg(kp + row);
+                }
+            }
+            __syncthreads();
+        }
+    }
+    if (!active) return;
+    uint8_t *out = const_cast<uint8_t *>(d.base) + (plane == 0 ? 0 : plane == 1 ? D.u_off : D.v_off) + o;
+    const int dpitch = plane ? D.c_pitch : D.y_pitch;
+#pragma unroll
+    for (int r = 0; r < kResizeRows; r++)
+        if (r < nr) out[(long long)(r0 + r) * dpitch] = (uint8_t)min(max(acc[r] >> kResizeBits, 0), 255);
+}
+
 }  // namespace h2j

@@ -76,6 +76,11 @@ RGB_RGBX = 2    # R G B + one ignored byte (RGBA8)
 RGB_BGRX = 3    # B G R + one ignored byte (BGRA8)
 RGB_PLANAR = 4  # three planes R, G, B (torch CHW)
 
+# h2j_resize_filter: what submit_device_resized takes (Pillow's Image.BOX, BILINEAR, BICUBIC)
+FILTER_BOX = 0
+FILTER_BILINEAR = 1
+FILTER_BICUBIC = 2
+
 
 class FrameDesc(C.Structure):
     """h2j_frame_desc: one device frame of a list submit (pitches and offsets in bytes)"""
@@ -116,7 +121,7 @@ EXPORTS = [
     "h2j_slot_wait_event", "h2j_device_count", "h2j_debug_set_knob", "h2j_debug_read_device", "h2j_stream_copy",
     "h2j_submit_device_semiplanar16", "h2j_submit_device_pitched16", "h2j_encode_frame16", "h2j_submit_device_list",
     "h2j_submit_host_list", "h2j_submit_device_downscaled", "h2j_submit_device_rgb", "h2j_encode_frame_rgb",
-    "h2j_debug_frame_planes",
+    "h2j_debug_frame_planes", "h2j_submit_device_resized",
 ]
 
 _lib = None
@@ -156,6 +161,7 @@ def load_library() -> C.CDLL:
     lib.h2j_submit_device_list.argtypes = [vp, ci, ci, C.POINTER(FrameDesc), ci]
     lib.h2j_submit_host_list.argtypes = [vp, ci, C.POINTER(vp), C.POINTER(ci), C.POINTER(ci), ci]
     lib.h2j_submit_device_downscaled.argtypes = [vp, ci, ci, C.POINTER(FrameDesc), ci, ci]
+    lib.h2j_submit_device_resized.argtypes = [vp, ci, ci, C.POINTER(FrameDesc), ci, C.POINTER(ci), C.POINTER(ci), ci]
     lib.h2j_submit_device_rgb.argtypes = [vp, ci, ci, C.POINTER(FrameDesc), ci]
     lib.h2j_encode_frame_rgb.argtypes = [vp, ci, C.POINTER(vp), C.POINTER(ci), ci, ci, vp, sz, C.POINTER(sz)]
     lib.h2j_debug_frame_planes.argtypes = [vp, ci, ci, vp, vp, vp]
@@ -459,6 +465,18 @@ class Encoder:
         arr = (FrameDesc * max(1, len(descs)))(*descs)
         self._check(self._lib.h2j_submit_device_downscaled(self._h, slot, layout, arr, len(descs), factor))
         self._n_in_slot[slot] = len(descs)
+
+    def submit_device_resized(self, slot: int, layout: int, descs: Sequence[FrameDesc], sizes: Sequence[Tuple[int, int]], filter: int) -> None:
+        """Device frames as for submit_device_list, frame i encoded resized to sizes[i] = (width, height) with a FILTER_* of
+        Pillow's (PIL.Image.resize on every plane); only the resized frames must fit the encoder's maximum."""
+        n = len(descs)
+        arr = (FrameDesc * max(1, n))(*descs)
+        ws = (C.c_int * max(1, len(sizes)))(*[w for w, _ in sizes])
+        hs = (C.c_int * max(1, len(sizes)))(*[h for _, h in sizes])
+        if len(sizes) != n:
+            raise H2JError(ERR_INVALID_ARG, f"{n} frames but {len(sizes)} sizes")
+        self._check(self._lib.h2j_submit_device_resized(self._h, slot, layout, arr, n, ws, hs, filter))
+        self._n_in_slot[slot] = n
 
     def submit_device_rgb(self, slot: int, fmt: int, descs: Sequence[FrameDesc]) -> None:
         """RGB device frames (an RGB_* format for all), each at its own address and of its own size: packed formats use

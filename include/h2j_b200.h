@@ -258,6 +258,39 @@ int h2j_submit_host_list(h2j_encoder *e, int slot, const uint8_t *const *frames,
 int h2j_submit_device_downscaled(h2j_encoder *e, int slot, int layout, const h2j_frame_desc *frames, int n, int factor);
 
 /*
+ * Resized device frames: thumbnails, previews and model inputs at any size (2/3, 1/6, a fixed 224x224, "longest side 512",
+ * an upscale to a fixed grid), with Pillow's BOX, BILINEAR or BICUBIC filter.  `layout` and `frames` are those of
+ * h2j_submit_device_list; frame i is encoded at out_widths[i] x out_heights[i] (W x H).  Frame i's JPEG is byte-identical to
+ * the one h2j_submit_device writes, with the same encoder settings, for the planar frame R(frame i):
+ *   every plane, at its decoder size (luma w x h, Cb and Cr at the encoder's chroma size of w x h; semi-planar Cb and Cr
+ *   separately), is resized as a Pillow "L" image to the matching plane of the W x H frame (luma W x H, chroma the
+ *   encoder's chroma size of W x H): PIL.Image.resize((pw_out, ph_out), filter) of Pillow's libImaging/Resample.c.  Per
+ *   axis, in to out samples: scale = in / out, fs = max(scale, 1), support = s_f * fs (s_f 0.5, 1, 2); output o has the
+ *   window xmin = max((int)(center - support + 0.5), 0) .. min((int)(center + support + 0.5), in), center = (o + 0.5) *
+ *   scale, weights f((x - center + 0.5) / fs) normalised by their sum, in double, and rounded to 22-bit fixed point
+ *   ((int)(w * 2^22 +- 0.5)).  The horizontal pass runs first, on every source row, and its result is clipped to 0..255;
+ *   the vertical pass runs on those 8-bit rows; each sums (2^21 + sum of sample * coefficient) in 32 bits and keeps
+ *   clamp(sum >> 22, 0, 255).  An axis whose size does not change has no pass, so W x H = w x h encodes the frame as
+ *   h2j_submit_device_list does.
+ * The resized samples are pinned bit for bit against Pillow itself (tests/test_resize_model.py); the JPEG is the existing
+ * encoder's.  BOX at an integer factor is NOT D_k above: Pillow rounds between its passes and its edge weights are not
+ * exact.  range_mode applies to the resized samples.  Sources may be 2..65500 on a side whatever max_width / max_height; only
+ * W x H must fit the encoder.  The coefficient tables are built on the host and kept in a per-slot buffer allocated on
+ * first use and grown when a submit needs more; one kernel writes the resized frames into the slot's own frame buffer,
+ * then the usual pipeline runs (frames of one size run its batch form).  Collect with h2j_collect / h2j_collect_device; the
+ * inspection calls answer for the resized frames; the device frames are read on the slot's stream, under the
+ * stream-ordering rule above.
+ * H2J_ERR_INVALID_ARG: as h2j_submit_device_list, null out_widths / out_heights, or a bad filter.  H2J_ERR_UNSUPPORTED: a
+ * source outside 2..65500, or an output size outside 2..65500 or above the encoder's maximum.  H2J_ERR_NOMEM: no room for
+ * the coefficient tables (the encoder stays usable).  H2J_ERR_BUSY: the slot has a batch in flight.  Every frame is checked
+ * before anything is enqueued: a rejected call leaves the previous batch as it was.
+ */
+typedef enum h2j_resize_filter { H2J_FILTER_BOX = 0, H2J_FILTER_BILINEAR = 1, H2J_FILTER_BICUBIC = 2 } h2j_resize_filter;
+
+int h2j_submit_device_resized(h2j_encoder *e, int slot, int layout, const h2j_frame_desc *frames, int n, const int *out_widths,
+                              const int *out_heights, int filter);
+
+/*
  * RGB frames: torch tensors ((3, H, W) planar as torchvision.io.encode_jpeg takes them, or (H, W, 3)), model outputs and
  * annotated frames, rendered RGBA8 surfaces, a hardware decoder's BGRA post-processing output, OpenCV / numpy images.
  * Frame i's JPEG is byte-identical to the one h2j_submit_device writes, with the same fixed_qscale and chroma_format, for
