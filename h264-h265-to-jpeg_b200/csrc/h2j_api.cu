@@ -106,6 +106,7 @@ struct h2j_encoder {
     int chunks_cap = 0;           // K5 chunks per frame
     int force_fdct_tiles = 0;     // h2j_debug_set_knob("fdct_tiles_per_cta"): exactly this many, whatever the batch size
     int force_sp_prepass = 0;     // h2j_debug_set_knob("semiplanar_prepass"): split semi-planar frames first even when aligned
+    int planar_copy = 1;          // h2j_debug_set_knob("planar_copy"): 0 = read unaligned planar frames in place, as without d_pitched
     size_t frame_bytes_cap = 0;
     uint8_t *d_qscale_lut = nullptr;
     char *d_comment = nullptr;
@@ -717,15 +718,16 @@ int run_batch(h2j_encoder *e, Slot &sl, int n, int m, const Input &in, int tail)
     for (int i = 0; i < m; i++) unaligned = unaligned || !S[i].L.aligned8;
     const bool split = in.sp && (unaligned || e->force_sp_prepass);
     const size_t pitched_cap = pitched_frame_bytes(e->s.max_width, e->s.max_height, fmt);
-    if (!convert && !in.sp && unaligned && !sl.d_pitched && cudaMalloc(&sl.d_pitched, pitched_cap * e->s.max_batch) != cudaSuccess) {
+    if (e->planar_copy && !convert && !in.sp && unaligned && !sl.d_pitched && cudaMalloc(&sl.d_pitched, pitched_cap * e->s.max_batch) != cudaSuccess) {
         cudaGetLastError();  // no room for the copies: the bytewise path still works
         sl.d_pitched = nullptr;
     }
+    uint8_t *const pitched = e->planar_copy ? sl.d_pitched : nullptr;
     // the largest copy: 16-byte columns of its widest row (semi-planar: of pairs), rows of all planes (RGB: 16-pixel columns,
     // destination rows a warp makes)
     int cols = 0, rows = 0;
     for (int i = 0; i < m; i++) {
-        if (!convert && !split && (in.sp || S[i].L.aligned8 || !sl.d_pitched)) {
+        if (!convert && !split && (in.sp || S[i].L.aligned8 || !pitched)) {
             S[i].base = nullptr;
             D[i].L.nv12 = in.sp ? 1 : 0;
             continue;
@@ -733,7 +735,7 @@ int run_batch(h2j_encoder *e, Slot &sl, int n, int m, const Input &in, int tail)
         const size_t spacing = convert || in.sp ? e->frame_bytes_cap : pitched_cap;
         D[i].L = pitched_layout(D[i].L);
         D[i].L.frame_stride = (long long)spacing;
-        D[i].base = (convert || in.sp ? sl.d_frames : sl.d_pitched) + (size_t)i * spacing;
+        D[i].base = (convert || in.sp ? sl.d_frames : pitched) + (size_t)i * spacing;
         const int w = D[i].L.w, h = D[i].L.h;
         if (in.filter >= 0) {  // bands of output rows of every plane
             cols = std::max(cols, (w + kResizeCols - 1) / kResizeCols);
@@ -1707,6 +1709,11 @@ int h2j_debug_set_knob(h2j_encoder *e, const char *name, int value)
     if (!strcmp(name, "semiplanar_prepass")) {
         if (value < 0 || value > 1) return fail(e, H2J_ERR_INVALID_ARG, "semiplanar_prepass %d is not 0 or 1", value);
         e->force_sp_prepass = value;
+        return H2J_OK;
+    }
+    if (!strcmp(name, "planar_copy")) {
+        if (value < 0 || value > 1) return fail(e, H2J_ERR_INVALID_ARG, "planar_copy %d is not 0 or 1", value);
+        e->planar_copy = value;
         return H2J_OK;
     }
     return fail(e, H2J_ERR_INVALID_ARG, "unknown knob %s", name);

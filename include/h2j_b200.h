@@ -399,7 +399,8 @@ int h2j_debug_read_device(h2j_encoder *e, const void *d_src, void *dst, size_t b
  * depend on a knob.  "fdct_tiles_per_cta": consecutive 16-MCU tiles one CTA of the FDCT kernel walks (0 = automatic:
  * 1 for small batches, up to 16 for large ones).  "semiplanar_prepass": 1 = h2j_submit_device_semiplanar /
  * h2j_submit_device_nv12 split the pairs into planes first even where the frames could be read in place (0 = by
- * alignment). */
+ * alignment).  "planar_copy": 0 = planar frames whose rows do not all start on 8-byte boundaries are read in place by the
+ * kernels' bytewise path, as when the slot has no room for their 16-byte-pitch copies (1 = copied first, the default). */
 int h2j_debug_set_knob(h2j_encoder *e, const char *name, int value);
 
 /* With settings.profile != 0: milliseconds each kernel of the slot's last batch took, measured with CUDA
